@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path
+  python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/*.npy
 
 One "step" is one pass of the audio-assembly hot path over one batch of
 synthetic utterances (default: BASELINE.json configs[2], 4096 sentences of ~200
@@ -58,7 +59,12 @@ def parse_args():
     ap.add_argument("--vocab", type=int, default=0,
                     help="draw the words from a Zipf vocabulary of this many types instead of the round-1 word list "
                          "(sensitivity of the word-region deduplication; the default line reports one such point itself)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/*.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def workload(args, rank: int):
@@ -200,6 +206,46 @@ def base_config(args) -> dict:
     """The `config` object: identical in both arms (ours and --impl reference)."""
     return {"workload": workload_name(args), "voice": VOICE,
             "l2": "inputs and outputs of a step (GBs) exceed the 126 MB L2; the 18 MB voice pool is L2-resident by design"}
+
+
+DUMP_PCM_BYTES = 48 << 20   # float32 PCM that --dump-outputs writes over all ranks; with the counts it stays under 64 MB
+
+
+def dump_outputs(out_dir: str, rp, counts: np.ndarray, rank: int, world: int) -> None:
+    """What the caller of the timed path (ctts_gpu_plan_run) receives from its last step, as .npy files:
+      counts.npy          samples of every utterance (float64)
+      pcm.npy             the PCM of a seeded sample of whole utterances, concatenated in batch order (float32)
+      pcm_utterances.npy  the utterances pcm.npy holds, ascending (float64)
+      pcm_strided.npy     every k-th sample of the batch's PCM (all utterances concatenated in batch order) from a
+                          seeded start, k as small as the budget allows (float32)
+    Each PCM file gets half of the budget.  The whole utterances are a seeded permutation's first ones whose counts
+    fit, so two correct builds run with the same arguments dump the same ones, whatever their output layout; with a
+    batch that fits, pcm.npy holds every utterance and pcm_strided.npy every sample.  Ranks > 1 add _rank<r> to the
+    names."""
+    budget = DUMP_PCM_BYTES // world // (2 * 4)                 # float32 samples of each of the two PCM files
+    off = rp.out_offsets().astype(np.int64)
+    cnt = counts.astype(np.int64)
+    order = np.random.default_rng(0).permutation(rp.n_utts)
+    pick = np.sort(order[np.cumsum(cnt[order]) <= budget])
+    starts = np.concatenate([[0], np.cumsum(cnt)])
+    stride = max(1, -(-int(starts[-1]) // budget))
+    first = int(np.random.default_rng(1).integers(stride))    # position of the first strided sample in the batch
+    picked = set(pick.tolist())
+    whole, strided = [np.zeros(0, np.int16)], [np.zeros(0, np.int16)]
+    for u in range(rp.n_utts):
+        lo = first + max(0, -(-(int(starts[u]) - first) // stride)) * stride - int(starts[u])
+        if u not in picked and lo >= cnt[u]:
+            continue
+        x = rp.read_pcm(int(off[u]), int(cnt[u]))
+        if u in picked:
+            whole.append(x)
+        strided.append(x[lo::stride].copy())                   # not a view: x is freed once used
+    sfx = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"counts{sfx}.npy"), counts.astype(np.float64))
+    np.save(os.path.join(out_dir, f"pcm{sfx}.npy"), np.concatenate(whole).astype(np.float32))
+    np.save(os.path.join(out_dir, f"pcm_utterances{sfx}.npy"), pick.astype(np.float64))
+    np.save(os.path.join(out_dir, f"pcm_strided{sfx}.npy"), np.concatenate(strided).astype(np.float32))
 
 
 def peak_hbm():
@@ -402,29 +448,31 @@ def main() -> int:
         torch.cuda.synchronize(local_rank)
 
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    for _ in range(args.warmup):
-        rp.run(d_out.data_ptr())
-    counts = rp.counts()
-    audio_s = float(counts.astype(np.int64).sum()) / SAMPLE_RATE
-    n_out = int(counts.astype(np.int64).sum())
-
-    sync_all()
-    if sampler:
-        sampler.wait_ready()
-        sampler.mark_begin()
-    evs = [torch.cuda.Event(enable_timing=True) for _ in range(args.steps + 1)]
-    with torch.cuda.stream(stream):
-        evs[0].record(stream)
-        for k in range(args.steps):
+    try:
+        for _ in range(args.warmup):
             rp.run(d_out.data_ptr())
-            evs[k + 1].record(stream)
-    sync_all()
-    if sampler:
-        sampler.mark_end()
-    clocks = sampler.stop() if sampler else None
+        sync_all()
+        if sampler:
+            sampler.wait_ready()
+            sampler.mark_begin()
+        evs = [torch.cuda.Event(enable_timing=True) for _ in range(args.steps + 1)]
+        with torch.cuda.stream(stream):
+            evs[0].record(stream)
+            for k in range(args.steps):
+                rp.run(d_out.data_ptr())
+                evs[k + 1].record(stream)
+        sync_all()
+        if sampler:
+            sampler.mark_end()
+    finally:   # a failed step must not leave nvidia-smi polling
+        clocks = sampler.stop() if sampler else None
     step_ms = [evs[k].elapsed_time(evs[k + 1]) for k in range(args.steps)]
     total_ms = evs[0].elapsed_time(evs[args.steps])
-    rp.counts()  # surfaces device error flags
+    counts = rp.counts()  # of the last timed step (there may be no warm-up); surfaces device error flags
+    audio_s = float(counts.astype(np.int64).sum()) / SAMPLE_RATE
+    n_out = int(counts.astype(np.int64).sum())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rp, counts, rank, world)
 
     # ---- the same resident plan with the word-region deduplication switched off (every region assembled): reported
     #      beside `value` so that the share of the speed-up that comes from repeated words in the batch is visible

@@ -20,8 +20,7 @@ def H():
 
 @pytest.fixture(scope="session")
 def golden(H):
-    import numpy as np
-    return np.load(os.path.join(H.GOLDEN, "ref_vectors.npz"), allow_pickle=False)
+    return H.golden_vectors()
 
 
 @pytest.fixture(scope="session")

@@ -1,5 +1,5 @@
-"""Generates tests/golden/ref_vectors.npz from the COMPILED, UNMODIFIED reference
-(oracle/_ref/libctts_ref.so, built from /root/reference/ctts.c by oracle/Makefile).
+"""Generates tests/golden/ref_vectors.npz.xz from the COMPILED, UNMODIFIED reference
+(oracle/_ref/libctts_ref.so, built from the reference's ctts.c by oracle/Makefile).
 
 Run where the reference tree exists:   python tests/golden/make_golden.py
 The fixture travels to the GPU box (the reference tree does not) and pins the
@@ -126,9 +126,8 @@ def main() -> None:
             assert rc == 0
             out[f"wsola_{sp}"] = np.ctypeslib.as_array(o, shape=(max(n.value, 1),))[:n.value].copy()
             L.ref_free(o)
-    path = os.path.join(HERE, "ref_vectors.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path), "bytes,", len(out), "arrays")
+    H.save_golden_vectors(out)
+    print("wrote", H.GOLDEN_VECTORS, os.path.getsize(H.GOLDEN_VECTORS), "bytes,", len(out), "arrays")
 
 
 if __name__ == "__main__":

@@ -281,6 +281,31 @@ def shipped_config():
     return front.load_config(SHIPPED_YAML)
 
 
+GOLDEN_VECTORS = os.path.join(GOLDEN, "ref_vectors.npz.xz")
+
+
+def save_golden_vectors(arrays: dict) -> None:
+    """Writes tests/golden/ref_vectors.npz.xz: an uncompressed .npz in one xz stream, every int16 array (all PCM)
+    stored as its first differences along the last axis.  Both make the file about half the size of
+    np.savez_compressed's."""
+    import io
+    import lzma
+    buf = io.BytesIO()
+    np.savez(buf, **{k: np.diff(v, prepend=np.int16(0)) if v.dtype == np.int16 else v for k, v in arrays.items()})
+    with open(GOLDEN_VECTORS, "wb") as f:
+        f.write(lzma.compress(buf.getvalue(), preset=9 | lzma.PRESET_EXTREME))
+
+
+def golden_vectors() -> dict:
+    """tests/golden/ref_vectors.npz.xz (make_golden.py), decoded: per-stage vectors and end-to-end PCM of the
+    compiled reference."""
+    import io
+    import lzma
+    with lzma.open(GOLDEN_VECTORS) as f:
+        z = np.load(io.BytesIO(f.read()), allow_pickle=False)
+        return {k: np.cumsum(v, axis=-1, dtype=np.int16) if v.dtype == np.int16 else v for k, v in z.items()}
+
+
 def golden_corpus() -> dict:
     """tests/golden/ref_corpus.json: SHA-1 / length of the compiled reference's PCM (make_golden_corpus.py)."""
     import json

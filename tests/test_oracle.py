@@ -10,6 +10,19 @@ def _i16(a):
     return np.ascontiguousarray(a, dtype=np.int16)
 
 
+def test_golden_vector_encoding_round_trips(H, tmp_path, monkeypatch):
+    """ref_vectors.npz.xz stores int16 arrays as first differences: they must decode exactly, whatever their shape."""
+    monkeypatch.setattr(H, "GOLDEN_VECTORS", str(tmp_path / "v.npz.xz"))
+    rng = np.random.default_rng(0)
+    arrays = {"pcm": rng.integers(-32768, 32768, 1000).astype(np.int16), "empty": np.zeros(0, np.int16),
+              "frames": rng.integers(-32768, 32768, (3, 50)).astype(np.int16), "f": rng.random(7).astype(np.float32)}
+    H.save_golden_vectors(arrays)
+    got = H.golden_vectors()
+    assert set(got) == set(arrays)
+    for k, v in arrays.items():
+        assert got[k].dtype == v.dtype and got[k].shape == v.shape and np.array_equal(got[k], v), k
+
+
 def test_tables_match_reference_bitwise(oracle_small, golden):
     luts, h256, h512 = oracle_small.tables()
     assert np.array_equal(luts.view(np.uint32), golden["luts"].view(np.uint32))
