@@ -156,8 +156,8 @@ __device__ void estimate_pitch_pair(const Smem& sm, const int16_t* a, const int1
     const int sig = pair ? (tid >> 6) & 1 : 0;
     const uint32_t lag0 = PITCH_LAG0 + PITCH_LPT * (uint32_t)(tid & (PITCH_TPS - 1));
     const bool lag_thread = lag0 <= hi;
-    // part boundaries are multiples of 4: every part keeps the float4 alignment
-    const uint32_t step = pair ? ((len >> 1) + 3u) & ~3u : (((len + 3u) >> 2) + 3u) & ~3u;
+    // part boundaries are multiples of 4: every part keeps the float4 alignment; the parts cover all len terms
+    const uint32_t step = pair ? (((len + 1u) >> 1) + 3u) & ~3u : (((len + 3u) >> 2) + 3u) & ~3u;
     if (!pair) cpart = reinterpret_cast<float4*>(Sb);   // signal b's prefix array is free: 3 x PITCH_TPS partials
     if (lag_thread) {
         const float* x = sig ? yb : ya;

@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import weakref
 
 import numpy as np
 
@@ -90,8 +91,13 @@ class ResidentPlan:
         self.n_utts = n_utts
 
     def close(self) -> None:
+        # a plan points into its context, so it is never destroyed after ctts_gpu_free.  GpuSynth.close destroys
+        # the plans it still knows first.  When the garbage collector frees a context and its plans together
+        # (a reference cycle) it clears the weak references before any finalizer runs, the context goes first
+        # and the plan's device memory is left allocated until the process ends: a leak, not a crash.
         if self._h:
-            lib().ctts_gpu_plan_destroy(self._h)
+            if self._ctx._h:
+                lib().ctts_gpu_plan_destroy(self._h)
             self._h = None
 
     def __del__(self):
@@ -160,9 +166,12 @@ class GpuSynth:
             raise GpuError(f"ctts_gpu_init failed: {rc}: {why.decode(errors='replace') if why else ''}")
         self._h = h
         self.device = device
+        self._plans = weakref.WeakSet()
 
     def close(self) -> None:
         if self._h:
+            for p in list(self._plans):
+                p.close()
             lib().ctts_gpu_free(self._h)
             self._h = None
 
@@ -275,7 +284,9 @@ class GpuSynth:
             out_offsets = np.ascontiguousarray(out_offsets, dtype=np.uint64)
             off_ptr = out_offsets.ctypes.data
         self._check(lib().ctts_gpu_plan_create(self._h, C.byref(cp), C.byref(params), off_ptr, C.byref(h)))
-        return ResidentPlan(self, h, plan.n_utts)
+        rp = ResidentPlan(self, h, plan.n_utts)
+        self._plans.add(rp)
+        return rp
 
 
 def multi_synth_batch(ctxs: list[GpuSynth], plan: BatchPlan, params: AssemblyParams, pcm_out: np.ndarray | None = None,

@@ -3,6 +3,8 @@ import ctypes as C
 import os
 import re
 
+import numpy as np
+
 import pytest
 
 
@@ -133,3 +135,39 @@ def test_c_command_line_has_no_cpu_fallback(H, small_db, tmp_path):
     (tmp_path / "voice.db").write_bytes(small_db)
     r = subprocess.run([exe, "synth", "voice.db", "olá mundo", "o.wav", "1.0"], cwd=tmp_path, capture_output=True, text=True)
     assert r.returncode == 1 and "no CPU fallback" in r.stderr and not (tmp_path / "o.wav").exists()
+
+
+def test_a_plan_is_never_destroyed_after_its_context(H, monkeypatch):
+    """ctts_gpu_plan_destroy reads the plan's context: closing the context first (explicitly, or the garbage
+    collector finalizing both in any order) must not lead to a destroy after ctts_gpu_free."""
+    gpu = H.importlib.import_module("2026-simple-c-tts_b200.gpu")
+    calls = []
+
+    class FakeLib:
+        def ctts_gpu_init(self, out, *_):
+            out._obj.value = 1
+            return 0
+
+        def ctts_gpu_plan_create(self, ctx, plan, prm, off, out):
+            out._obj.value = 100 + len(calls)
+            calls.append(("create", out._obj.value))
+            return 0
+
+        def ctts_gpu_plan_destroy(self, h):
+            calls.append(("destroy", h.value))
+
+        def ctts_gpu_free(self, h):
+            calls.append(("free", h.value))
+
+    monkeypatch.setattr(gpu, "_lib", FakeLib())
+    plan = H.front.BatchPlan(np.zeros(1, np.uint32), np.zeros(0, np.float32), np.zeros(0, H.front.OP_DTYPE))
+    g = gpu.GpuSynth(b"", 0)
+    a = g.create_plan(plan, H.front.AssemblyParams())
+    b = g.create_plan(plan, H.front.AssemblyParams())
+    b.close()
+    g.close()
+    a.close()
+    g.close()
+    assert [c[0] for c in calls].count("free") == 1
+    assert all(k != "destroy" for k, _ in calls[calls.index(("free", 1)):]), calls
+    assert sorted(h for k, h in calls if k == "destroy") == [100, 101]
