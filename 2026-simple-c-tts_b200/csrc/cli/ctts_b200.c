@@ -2,8 +2,11 @@
  * ctts_b200 -- the `ctts synth` command line (ctts.c:3970-4030) over the B200 back end, in the
  * reference's own language: plain C on top of the two C-ABI libraries, no Python, no CUDA headers.
  *
- *   ctts_b200 synth <database.db> "text" <output.wav> [speed]
- *   ctts_b200 synth-batch <database.db> <texts.tsv> <out_dir>     lines: speed<TAB>text
+ *   ctts_b200 synth <database.db> "text" <output.wav> [speed] [rate]
+ *   ctts_b200 synth-batch <database.db> <texts.tsv> <out_dir> [rate]     lines: speed<TAB>text
+ *
+ * rate: output sample rate in Hz (default 22050, the voice's own; ctts_gpu_set_output_rate lists the others),
+ * written into the WAV header.
  *
  * Like the reference it reads config.yaml and normalization.csv from the working directory
  * (ctts.c:3990, :3636), clamps the speed to [0.5, 2.0] (ctts.c:3976-3981) and takes default_speed
@@ -28,6 +31,7 @@ typedef struct {
     ctts_front_config cfg;
     ctts_front* front;
     ctts_gpu_ctx* gpu;
+    uint32_t rate;   /* output sample rate */
 } engine;
 
 static void engine_close(engine* e) {
@@ -38,7 +42,7 @@ static void engine_close(engine* e) {
 }
 
 /* ctts_init (ctts.c:1117) + ctts_load_config("config.yaml") + the rule table, for both halves */
-static int engine_open(engine* e, const char* db_path) {
+static int engine_open(engine* e, const char* db_path, uint32_t rate) {
     memset(e, 0, sizeof *e);
     FILE* f = fopen(db_path, "rb");
     if (!f) return -1;
@@ -63,14 +67,21 @@ static int engine_open(engine* e, const char* db_path) {
         engine_close(e);
         return rc;
     }
+    rc = ctts_gpu_set_output_rate(e->gpu, rate);
+    if (rc) {
+        fprintf(stderr, "output rate %u Hz: %s\n", rate, ctts_gpu_last_error(e->gpu));
+        engine_close(e);
+        return rc;
+    }
+    e->rate = rate;
     return 0;
 }
 
 /* ctts_write_wav, ctts.c:809: 44-byte RIFF/WAVE header (PCM, mono, 16 bit) + samples */
-static int write_wav(const char* path, const int16_t* samples, size_t count) {
+static int write_wav(const char* path, const int16_t* samples, size_t count, uint32_t rate) {
     FILE* f = fopen(path, "wb");
     if (!f) return -1;
-    const uint32_t data = (uint32_t)(count * sizeof(int16_t)), riff = 36 + data, fmt = 16, sr = SAMPLE_RATE, br = SAMPLE_RATE * 2;
+    const uint32_t data = (uint32_t)(count * sizeof(int16_t)), riff = 36 + data, fmt = 16, sr = rate, br = rate * 2;
     const uint16_t pcm = 1, ch = 1, align = 2, bits = 16;
     fwrite("RIFF", 1, 4, f); fwrite(&riff, 4, 1, f); fwrite("WAVE", 1, 4, f);
     fwrite("fmt ", 1, 4, f); fwrite(&fmt, 4, 1, f);
@@ -90,7 +101,7 @@ static int ctts_b200_synthesize_batch(engine* e, const char* const* texts, const
                                       int16_t** pcm, uint64_t** off, uint32_t** cnt, uint32_t* stats,
                                       ctts_gpu_chunk_fn on_chunk, void* user) {
     int rc = 0;
-    const uint64_t cap = ctts_b200_capacity_hint(e->front, texts, speeds, n);   /* replaces the SampleBuffer growth policy */
+    const uint64_t cap = ctts_b200_capacity_hint_rate(e->front, texts, speeds, n, e->rate);   /* replaces the SampleBuffer growth policy */
     *off = malloc(sizeof **off * ((size_t)n + 1));
     *cnt = calloc(n ? n : 1, sizeof **cnt);
     *pcm = ctts_gpu_host_alloc(sizeof(int16_t) * (cap ? cap : 8));
@@ -112,15 +123,23 @@ static int ctts_b200_synthesize_batch(engine* e, const char* const* texts, const
 
 static float clamp_speed(float s) { return s < 0.5f ? 0.5f : s > 2.0f ? 2.0f : s; }
 
+/* an output rate argument: digits only, else 0 (rejected by ctts_gpu_set_output_rate) */
+static uint32_t parse_rate(const char* a) {
+    char* end = NULL;
+    const unsigned long v = strtoul(a, &end, 10);
+    return (end && *end == 0 && end != a && v <= 0xffffffffu) ? (uint32_t)v : 0;
+}
+
 static int cmd_synth(int argc, char** argv) {
-    if (argc < 5) {
-        fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed]\n", argv[0]);
+    if (argc < 5 || argc > 7) {
+        fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed] [rate]\n", argv[0]);
         return 1;
     }
     float speed = 1.0f;
     if (argc > 5) speed = clamp_speed(strtof(argv[5], NULL));
+    const uint32_t rate = argc > 6 ? parse_rate(argv[6]) : SAMPLE_RATE;
     engine e;
-    if (engine_open(&e, argv[2])) {
+    if (engine_open(&e, argv[2], rate)) {
         fprintf(stderr, "Failed to load database: %s\n", argv[2]);
         return 1;
     }
@@ -131,9 +150,9 @@ static int cmd_synth(int argc, char** argv) {
     uint64_t* off;
     uint32_t *cnt, stats[2] = {0, 0};
     if (ctts_b200_synthesize_batch(&e, texts, &speed, 1, &pcm, &off, &cnt, stats, NULL, NULL)) { engine_close(&e); return 1; }
-    printf("Synthesized %u samples (%.2f seconds)\n", cnt[0], (float)cnt[0] / SAMPLE_RATE);
+    printf("Synthesized %u samples (%.2f seconds)\n", cnt[0], (float)cnt[0] / (float)e.rate);
     printf("Units found: %u, missing: %u\n", stats[0], stats[1]);
-    int rc = write_wav(argv[4], pcm + off[0], cnt[0]);
+    int rc = write_wav(argv[4], pcm + off[0], cnt[0], e.rate);
     if (rc) fprintf(stderr, "Failed to write WAV: %s\n", argv[4]);
     else printf("Written to %s\n", argv[4]);
     ctts_gpu_host_free(pcm);
@@ -147,6 +166,7 @@ static int cmd_synth(int argc, char** argv) {
  * working on later ones): state shared with the chunk callback */
 typedef struct {
     const char* dir;
+    uint32_t rate;
     uint32_t base;   /* first utterance of the group being synthesised */
     int16_t** pcm;
     uint64_t** off;
@@ -160,16 +180,17 @@ static void write_chunk(void* user, uint32_t u0, uint32_t u1) {
     for (uint32_t u = u0; u < u1 && !w->rc; u++) {
         char path[4096];
         snprintf(path, sizeof path, "%s/%06u.wav", w->dir, w->base + u);
-        w->rc = write_wav(path, *w->pcm + (*w->off)[u], (*w->cnt)[u]);
-        w->seconds += (double)(*w->cnt)[u] / SAMPLE_RATE;
+        w->rc = write_wav(path, *w->pcm + (*w->off)[u], (*w->cnt)[u], w->rate);
+        w->seconds += (double)(*w->cnt)[u] / w->rate;
     }
 }
 
 static int cmd_synth_batch(int argc, char** argv) {
-    if (argc != 5) {
-        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir>\n", argv[0]);
+    if (argc != 5 && argc != 6) {
+        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate]\n", argv[0]);
         return 1;
     }
+    const uint32_t rate = argc > 5 ? parse_rate(argv[5]) : SAMPLE_RATE;
     FILE* f = fopen(argv[3], "rb");
     if (!f) { fprintf(stderr, "cannot read %s\n", argv[3]); return 1; }
     char** texts = NULL;
@@ -197,7 +218,7 @@ static int cmd_synth_batch(int argc, char** argv) {
     free(line);
     fclose(f);
     engine e;
-    if (engine_open(&e, argv[2])) {
+    if (engine_open(&e, argv[2], rate)) {
         fprintf(stderr, "Failed to load database: %s\n", argv[2]);
         return 1;
     }
@@ -205,7 +226,7 @@ static int cmd_synth_batch(int argc, char** argv) {
     int16_t* pcm;
     uint64_t* off;
     uint32_t* cnt;
-    wav_sink sink = {argv[4], 0, &pcm, &off, &cnt, 0.0, 0};
+    wav_sink sink = {argv[4], e.rate, 0, &pcm, &off, &cnt, 0.0, 0};
     /* groups of 1024 utterances: the pinned buffer is sized from the texts alone (ctts_b200_capacity_hint) */
     int rc = 0;
     for (uint32_t g0 = 0; g0 < n && !rc; g0 += 1024) {
@@ -231,7 +252,7 @@ static int cmd_synth_batch(int argc, char** argv) {
 int main(int argc, char** argv) {
     if (argc >= 2 && strcmp(argv[1], "synth") == 0) return cmd_synth(argc, argv);
     if (argc >= 2 && strcmp(argv[1], "synth-batch") == 0) return cmd_synth_batch(argc, argv);
-    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed]\n       %s synth-batch <database.db> <texts.tsv> <out_dir>\n",
+    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed] [rate]\n       %s synth-batch <database.db> <texts.tsv> <out_dir> [rate]\n",
             argv[0], argv[0]);
     return 1;
 }

@@ -288,7 +288,21 @@ static void* planner(void* arg) {
 }
 
 uint64_t ctts_b200_capacity_hint(ctts_front* front, const char* const* texts, const float* speeds, uint32_t n) {
-    if (!front || (n && !texts)) return 0;
+    return ctts_b200_capacity_hint_rate(front, texts, speeds, n, CTTS_PLAN_SAMPLE_RATE);
+}
+
+static uint32_t gcd_u32(uint32_t a, uint32_t b) {
+    while (b) {
+        const uint32_t t = a % b;
+        a = b;
+        b = t;
+    }
+    return a;
+}
+
+uint64_t ctts_b200_capacity_hint_rate(ctts_front* front, const char* const* texts, const float* speeds, uint32_t n, uint32_t hz) {
+    if (!front || (n && !texts) || hz == 0) return 0;
+    const uint32_t g = gcd_u32(CTTS_PLAN_SAMPLE_RATE, hz), L = hz / g, M = CTTS_PLAN_SAMPLE_RATE / g;
     /* every character yields at most one unit or one pause; pauses are shorter than the longest unit for
      * any sane config, but take the larger of the two anyway */
     uint64_t per_char = ctts_front_max_unit_samples(front);
@@ -300,7 +314,8 @@ uint64_t ctts_b200_capacity_hint(ctts_front* front, const char* const* texts, co
             chars += (*c >= '0' && *c <= '9') ? 16 : 1;   /* a digit expands to words ("novecentos e ") */
         uint64_t s = chars * per_char;
         if (speeds && speeds[u] < 1.0f) s *= 2;   /* hop = 128 / speed <= 256 */
-        total += s + 1024;
+        s += 1024;
+        total += L == M ? s : (s * L + M - 1) / M + 8;   /* ceil(n L / M) at the output rate, rounded up to 8 */
     }
     return total;
 }

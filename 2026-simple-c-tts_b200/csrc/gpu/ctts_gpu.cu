@@ -21,9 +21,11 @@
 
 #include "assemble.cuh"
 #include "wsola.cuh"
+#include "resample.cuh"
 
 extern "C" void ctts_host_tables(float* fade_out, float* fade_in, float* sine, float* hann256,
                                  float* hann512);
+extern "C" void ctts_host_resample_taps(unsigned L, unsigned M, float* g);
 
 namespace {
 
@@ -109,6 +111,18 @@ struct ctts_gpu_ctx {
         std::vector<std::vector<std::pair<uint32_t, uint32_t>>> pitch_slots;   // per unit: (R, slot)
     };
     std::vector<NormPool*> norm_pools;
+    // output-rate conversion (DESIGN.md 3.4): one tap table per rate this context has seen; plans keep a
+    // pointer to the one they were created under, so tables live as long as the context
+    struct RsTable {
+        uint32_t hz = 0, L = 1, M = 1;
+        uint32_t kp = 0;            // taps per phase row (multiple of 4)
+        uint32_t c = 0;             // H * R: the filter's centre
+        uint32_t smem_floats = 0;   // bound on the input span of one resample_kernel tile
+        float* d_taps = nullptr;    // L rows of kp
+    };
+    std::vector<RsTable*> rs_tables;
+    RsTable* rs = nullptr;          // the output rate of the context; nullptr: the native 22 050 Hz
+    int rs_smem_attr = 48 * 1024;   // dynamic shared memory resample_kernel may use on this device
     uint64_t pool_samples = 0;
     uint32_t n_units = 0;
     uint32_t max_unit = 0;
@@ -123,8 +137,10 @@ struct ctts_gpu_ctx {
     static constexpr int kLanes = 4;
     struct Lane {
         Arena arena;                       // device workspace + pinned staging of the plan upload
-        int16_t* d_out = nullptr;          // the piece's output slots
+        int16_t* d_out = nullptr;          // the piece's output slots (native rate: where the kernels write)
         uint64_t d_out_cap = 0;
+        int16_t* d_rs = nullptr;           // output-rate slots (only when the context converts the rate)
+        uint64_t d_rs_cap = 0;
         int16_t* d_pack = nullptr;         // packed mode: the utterances' samples back to back
         uint64_t d_pack_cap = 0;
         unsigned long long* d_pack_off = nullptr;   // n + 1 (+ the n + 1 slot offsets behind them)
@@ -159,8 +175,16 @@ struct ctts_gpu_plan {
     ctts_gpu_ctx* ctx = nullptr;
     uint32_t n_utts = 0;
     ctts_assembly_params prm{};
-    std::vector<uint64_t> offsets;  // n_utts + 1
-    std::vector<uint64_t> bounds;
+    std::vector<uint64_t> offsets;  // n_utts + 1, output-rate slots (what callers see)
+    std::vector<uint64_t> bounds;   // output-rate bounds
+    ctts_gpu_ctx::RsTable* rs = nullptr;   // rate conversion the plan was created under (nullptr: native rate)
+    std::vector<uint64_t> n_offsets;       // native-rate slots, where the assembly and WSOLA kernels write (== offsets without rs)
+    std::vector<unsigned long long> rs_off_h;   // rs: native slot offsets [n + 1], then output-rate ones [n + 1]
+    unsigned long long* d_rs_off = nullptr;
+    uint32_t* d_rs_counts = nullptr;       // rs: output-rate counts
+    uint32_t* d_final_counts = nullptr;    // the counts callers see: d_rs_counts with rs, else d_counts
+    uint32_t rs_tiles = 0;                 // rs: grid.x of resample_kernel
+    int16_t* d_nat_owned = nullptr;        // resident plan with rs: its native slots
     Arena* arena = nullptr;         // device buffers live in a lane's arena (batch path); else cudaMalloc'ed
     uint32_t op0 = 0;               // first op of the plan's utterances in the caller's op array (ops are kept from there on)
     std::vector<void*> owned;       // else: cudaMalloc'ed buffers to free
@@ -246,6 +270,9 @@ uint64_t stretch_bound(uint64_t pre, uint32_t hop) {
     uint64_t frames = pre > 512 ? (pre - 512) / 128 + 1 : 1;
     return frames * hop + 512;
 }
+
+// samples at the output rate of n native samples: ceil(n * L / M)
+uint64_t rate_bound(const ctts_gpu_ctx::RsTable* rs, uint64_t n) { return rs ? (n * rs->L + rs->M - 1) / rs->M : n; }
 
 // Upper bound of the samples a UNIT op appends, given a lower bound L of the samples already in
 // the current region.  The crossfade consumes a = min(xf, count, n) samples of the tail
@@ -489,6 +516,10 @@ void ctts_gpu_free(ctts_gpu_ctx* ctx) {
     cudaFree(ctx->d_unit_off);
     cudaFree(ctx->d_unit_cnt);
     cudaFree(ctx->d_tables);
+    for (ctts_gpu_ctx::RsTable* t : ctx->rs_tables) {
+        cudaFree(t->d_taps);
+        delete t;
+    }
     for (ctts_gpu_ctx::NormPool* np : ctx->norm_pools) {
         cudaFree(np->d_pool);
         cudaFree(np->d_meta);
@@ -501,6 +532,7 @@ void ctts_gpu_free(ctts_gpu_ctx* ctx) {
         cudaFree(l.arena.d);
         if (l.arena.h) cudaFreeHost(l.arena.h);
         cudaFree(l.d_out);
+        cudaFree(l.d_rs);
         cudaFree(l.d_pack);
         cudaFree(l.d_pack_off);
         if (l.h_res) cudaFreeHost(l.h_res);
@@ -516,6 +548,62 @@ void ctts_gpu_free(ctts_gpu_ctx* ctx) {
 int ctts_gpu_set_stream(ctts_gpu_ctx* ctx, void* cuda_stream) {
     if (!ctx) return CTTS_GPU_ERR_INVALID_ARG;
     ctx->stream = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : ctx->own_stream;
+    return CTTS_GPU_OK;
+}
+
+int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz) {
+    if (!ctx) return CTTS_GPU_ERR_INVALID_ARG;
+    if (hz < 8000 || hz > 48000) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "output rate %u Hz outside [8000, 48000]", hz);
+    const uint32_t g = std::gcd<uint32_t>(CTTS_PLAN_SAMPLE_RATE, hz), L = hz / g, M = CTTS_PLAN_SAMPLE_RATE / g, R = std::max(L, M);
+    if (R > 1024) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "output rate %u Hz: the ratio %u/%u is not reduced enough (max(L, M) > 1024)", hz, L, M);
+    if (ctx->session) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "the output rate cannot change while a session is open");
+    if (hz == CTTS_PLAN_SAMPLE_RATE) {
+        ctx->rs = nullptr;
+        return CTTS_GPU_OK;
+    }
+    for (ctts_gpu_ctx::RsTable* t : ctx->rs_tables)
+        if (t->hz == hz) {
+            ctx->rs = t;
+            return CTTS_GPU_OK;
+        }
+    CU(ctx, cudaSetDevice(ctx->device));
+    const uint32_t N = 2u * 40u * R + 1u;
+    std::vector<float> taps(N);
+    ctts_host_resample_taps(L, M, taps.data());
+    // by phase, each row in the order the kernel walks it (resample.cuh), zero padded in front to a multiple of 4
+    const uint32_t kp = ((N + L - 1) / L + 3) & ~3u;
+    std::vector<float> rows((size_t)L * kp, 0.0f);
+    for (uint32_t phi = 0; phi < L; phi++)
+        for (uint32_t k = 0; k < kp; k++) {
+            const uint64_t i = (uint64_t)phi + (uint64_t)L * (kp - 1 - k);
+            if (i < N) rows[(size_t)phi * kp + k] = taps[i];
+        }
+    // input span of a tile of RS_THREADS work items: they cover at most d + 1 rows of L * RS_COPIES outputs
+    const uint64_t d = (uint64_t)(L - 1 + ctts::RS_THREADS - 1) / L;
+    const uint64_t out_span = d * L * ctts::RS_COPIES + (uint64_t)L * ctts::RS_COPIES;
+    const uint32_t smem_floats = (uint32_t)(((out_span * M) / L + 2 + kp + 3) & ~3ull);
+    const int smem_bytes = (int)(smem_floats * sizeof(float));
+    if (smem_bytes > ctx->smem_optin) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "output rate %u Hz: staging of %d bytes", hz, smem_bytes);
+    if (smem_bytes > ctx->rs_smem_attr) {
+        CU(ctx, cudaFuncSetAttribute(ctts::resample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+        ctx->rs_smem_attr = smem_bytes;
+    }
+    ctts_gpu_ctx::RsTable* t = new ctts_gpu_ctx::RsTable();
+    t->hz = hz;
+    t->L = L;
+    t->M = M;
+    t->kp = kp;
+    t->c = 40u * R;
+    t->smem_floats = smem_floats;
+    cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&t->d_taps), rows.size() * sizeof(float));
+    if (e == cudaSuccess) e = cudaMemcpy(t->d_taps, rows.data(), rows.size() * sizeof(float), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) {
+        cudaFree(t->d_taps);
+        delete t;
+        return fail(ctx, CTTS_GPU_ERR_CUDA, "output rate %u Hz: tap table: %s", hz, cudaGetErrorString(e));
+    }
+    ctx->rs_tables.push_back(t);
+    ctx->rs = t;
     return CTTS_GPU_OK;
 }
 
@@ -538,7 +626,7 @@ int ctts_gpu_plan_bounds(const ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, u
     uint32_t bad = 0;
     int rc = scan_plan(ctx, plan, ~0ull, &sc, &bad);
     if (rc) return rc;
-    std::copy(sc.bound.begin(), sc.bound.end(), out_bound);
+    for (uint32_t u = 0; u < plan->n_utts; u++) out_bound[u] = rate_bound(ctx->rs, sc.bound[u]);
     return CTTS_GPU_OK;
 }
 
@@ -565,6 +653,7 @@ void ctts_gpu_plan_destroy(ctts_gpu_plan* p) {
     }
     for (void* d : p->owned) cudaFree(d);
     cudaFree(p->d_out_owned);
+    cudaFree(p->d_nat_owned);
     delete p;
 }
 
@@ -734,7 +823,11 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     int rc = scan_plan(ctx, plan, scr_samples, &sc, &bad);
     if (rc) return fail(ctx, rc, "invalid plan (utterance %u)", bad);
     if (sc.bad_factor) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "WORD_END pitch factors must lie in [0, 2.05]");
-    const std::vector<uint64_t>&pre = sc.pre, &bound = sc.bound;
+    const std::vector<uint64_t>& pre = sc.pre;
+    ctts_gpu_ctx::RsTable* const rs = ctx->rs;
+    std::vector<uint64_t> bound(sc.bound);   // at the output rate
+    if (rs)
+        for (uint64_t& b : bound) b = rate_bound(rs, b);
 
     ctts_gpu_ctx::NormPool* np = nullptr;
     rc = norm_pool_for(ctx, params->target_rms, &np);
@@ -746,6 +839,7 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     p->n_utts = n;
     p->prm = *params;
     p->bounds = bound;
+    p->rs = rs;
     p->arena = arena;
     p->src = plan;
     p->op0 = n ? plan->utt_op_begin[0] : 0;
@@ -774,6 +868,30 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
             o += up8(bound[u]) + 8;
         }
         p->offsets[n] = o;
+    }
+    if (rs) {
+        // native slots packed by the native bounds; resample_kernel turns them into the slots above
+        p->n_offsets.resize((size_t)n + 1);
+        uint64_t o = 0, ob_max = 0;
+        for (uint32_t u = 0; u < n; u++) {
+            if (sc.bound[u] + 16 > 0xffffffffull) {
+                delete p;
+                return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "utterance %u too long (%llu samples)", u, (unsigned long long)sc.bound[u]);
+            }
+            p->n_offsets[u] = o;
+            o += up8(sc.bound[u]) + 8;
+            ob_max = std::max(ob_max, bound[u]);
+        }
+        p->n_offsets[n] = o;
+        p->rs_off_h.resize(2 * ((size_t)n + 1));
+        for (uint32_t u = 0; u <= n; u++) {
+            p->rs_off_h[u] = p->n_offsets[u];
+            p->rs_off_h[n + 1 + u] = p->offsets[u];
+        }
+        const uint64_t row = (uint64_t)rs->L * ctts::RS_COPIES;
+        p->rs_tiles = (uint32_t)std::max<uint64_t>(((ob_max + row - 1) / row * rs->L + ctts::RS_THREADS - 1) / ctts::RS_THREADS, 1);
+    } else {
+        p->n_offsets = p->offsets;
     }
 
     // ---- shared-memory geometry
@@ -838,8 +956,8 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
                 st.utt = u;
                 st.hop = hop;
                 st.pre_off = pre_total;
-                st.out_off = p->offsets[u];
-                st.out_cap = (uint32_t)(p->offsets[u + 1] - p->offsets[u]);
+                st.out_off = p->n_offsets[u];
+                st.out_cap = (uint32_t)(p->n_offsets[u + 1] - p->n_offsets[u]);
                 st.pos_off = (uint32_t)pos_total;
                 st.max_frames = (uint32_t)(pre[u] > 512 ? (pre[u] - 512) / 128 + 1 : 1);
                 if (st.max_frames > 1)
@@ -889,8 +1007,10 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         if (!stasks.empty())
             d_need += PlanAlloc::up256(stasks.size() * sizeof(ctts::StretchTask)) + 2 * PlanAlloc::up256(ola_task.size() * 4 + 4) +
                       PlanAlloc::up256(pre_total * 2 + 16) + PlanAlloc::up256(pos_total * 4 + 4) + PlanAlloc::up256(stasks.size() * 20) + 4096;
+        const size_t rs_bytes = rs ? PlanAlloc::up256(p->rs_off_h.size() * 8) : 0;
+        if (rs) d_need += rs_bytes + PlanAlloc::up256((size_t)n * 4);
         const size_t st_bytes = PlanAlloc::up256(stasks.size() * sizeof(ctts::StretchTask)) + 2 * PlanAlloc::up256(ola_task.size() * 4 + 4);
-        const size_t h_need = PlanAlloc::up256(ops_bytes) + PlanAlloc::up256(tasks_bytes) + st_bytes + 4096;
+        const size_t h_need = PlanAlloc::up256(ops_bytes) + PlanAlloc::up256(tasks_bytes) + st_bytes + rs_bytes + 4096;
         rc = ensure_arena(ctx, arena, d_need, h_need);
         if (rc) { delete p; return rc; }
         p->h_ops = reinterpret_cast<ctts_plan_op*>(arena->h);
@@ -913,6 +1033,12 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     p->d_counts = al.dev<uint32_t>(n);
     p->d_pre_counts = al.dev<uint32_t>(n);
     p->d_err = al.dev<uint32_t>(n);
+    p->d_final_counts = p->d_counts;
+    if (rs) {
+        p->d_rs_counts = al.dev<uint32_t>(n);
+        p->d_rs_off = al.dev<unsigned long long>(p->rs_off_h.size());
+        p->d_final_counts = p->d_rs_counts;
+    }
     if (sc.n_big_regions) {
         // rare (regions longer than ~51 k samples): always a separate allocation
         p->trim_words = (uint32_t)(2 * ((sc.big_region_max + 31) / 32) + 8);
@@ -956,6 +1082,16 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         CUP(cudaMemcpyAsync(p->d_ola_first, h_of, ola_first.size() * 4, cudaMemcpyHostToDevice, st));
         if (!arena) CUP(cudaStreamSynchronize(st));   // pageable vectors that are about to go out of scope
     }
+    if (rs) {
+        const void* h_ro = p->rs_off_h.data();   // (resident plans: lives as long as the plan)
+        if (arena) {
+            char* at = arena->h + PlanAlloc::up256(ops_bytes) + PlanAlloc::up256(tasks_bytes) +
+                       PlanAlloc::up256(stasks.size() * sizeof(ctts::StretchTask)) + 2 * PlanAlloc::up256(ola_task.size() * 4 + 4);
+            memcpy(at, p->rs_off_h.data(), p->rs_off_h.size() * 8);
+            h_ro = at;
+        }
+        CUP(cudaMemcpyAsync(p->d_rs_off, h_ro, p->rs_off_h.size() * 8, cudaMemcpyHostToDevice, st));
+    }
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ctts::assemble_kernel, ctts::ASM_THREADS, p->smem_bytes) != cudaSuccess || occ < 1)
         occ = 1;
@@ -964,6 +1100,7 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     p->info.kernel_launches = n_chunks;
     for (const PlanChunk& ch : p->chunks)   // scan, verify, repair (chain walk), overlap-add
         p->info.kernel_launches += ch.st_count ? 2 + (ch.verify_tiles && ctx->knobs.wsola_speculate ? 1 : 0) + (ch.ola_count ? 1 : 0) : 0;
+    if (rs) p->info.kernel_launches += (uint32_t)(((uint64_t)n + 65534) / 65535);   // resample_kernel
     p->info.n_stretch = p->n_stretch;
     p->info.bound_samples = std::accumulate(bound.begin(), bound.end(), (uint64_t)0);
     p->info.smem_bytes = p->smem_bytes;
@@ -1388,8 +1525,8 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
         const bool stretched = p->pre_off[u] != ~0ull;
         t.flags = (k + 1 == ht_begin[ui + 1] - ht_begin[ui] ? (uint32_t)ctts::TASK_LAST : 0u) | (stretched ? (uint32_t)ctts::TASK_TO_PRE : 0u);
         if (h.bound > wcap) { t.flags |= ctts::TASK_GLOBAL; p->n_global_tasks++; }
-        t.dst_cap = stretched ? (uint32_t)p->pre_cap[u] : (uint32_t)(p->offsets[u + 1] - p->offsets[u]);
-        t.dst_off = stretched ? p->pre_off[u] : p->offsets[u];
+        t.dst_cap = stretched ? (uint32_t)p->pre_cap[u] : (uint32_t)(p->n_offsets[u + 1] - p->n_offsets[u]);
+        t.dst_off = stretched ? p->pre_off[u] : p->n_offsets[u];
         t.big = 0xffffffffu;
         if (h.region_max > scr_samples) {
             if (p->n_big >= p->big_cap) build_rc = fail(ctx, CTTS_GPU_ERR_DEVICE, "internal: trim scratch slots");
@@ -1551,6 +1688,33 @@ int launch_stretch(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, int16_t* d_p
     return CTTS_GPU_OK;
 }
 
+// Enqueue the output-rate conversion of the whole plan (after the last chunk's kernels): native slots d_nat and
+// counts -> output-rate slots d_final and d_rs_counts.  Nothing at the native rate.
+int launch_resample(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const int16_t* d_nat, int16_t* d_final, cudaStream_t st) {
+    const ctts_gpu_ctx::RsTable* rs = p->rs;
+    if (!rs || !p->n_utts) return CTTS_GPU_OK;
+    const uint32_t n = p->n_utts;
+    for (uint32_t u0 = 0; u0 < n; u0 += 65535u) {   // grid.y limit
+        ctts::ResampleArgs r{};
+        r.in = d_nat;
+        r.in_off = p->d_rs_off + u0;
+        r.in_counts = p->d_counts + u0;
+        r.out = d_final;
+        r.out_off = p->d_rs_off + (n + 1) + u0;
+        r.out_counts = p->d_rs_counts + u0;
+        r.taps = reinterpret_cast<const float4*>(rs->d_taps);
+        r.L = rs->L;
+        r.M = rs->M;
+        r.kp = rs->kp;
+        r.c = rs->c;
+        r.smem_floats = rs->smem_floats;
+        const dim3 grid(p->rs_tiles, std::min<uint32_t>(n - u0, 65535u));
+        ctts::resample_kernel<<<grid, ctts::RS_THREADS, rs->smem_floats * sizeof(float), st>>>(r);
+        CU(ctx, cudaGetLastError());
+    }
+    return CTTS_GPU_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1593,11 +1757,18 @@ int ctts_gpu_plan_run(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out) {
     }
     p->d_out_last = d_pcm_out;
     if (p->n_utts == 0) return CTTS_GPU_OK;
+    int16_t* d_nat = d_pcm_out;   // where the assembly and WSOLA kernels write
+    if (p->rs) {
+        if (!p->d_nat_owned)
+            CU(ctx, cudaMalloc(reinterpret_cast<void**>(&p->d_nat_owned), std::max<uint64_t>(p->n_offsets[p->n_utts], 8) * sizeof(int16_t)));
+        d_nat = p->d_nat_owned;
+    }
     int rc = begin_run(ctx, p);
     for (uint32_t c = 0; !rc && c < p->chunks.size(); c++) {
-        rc = launch_chunk(ctx, p, c, d_pcm_out, ctx->stream);
-        if (!rc) rc = launch_stretch(ctx, p, c, d_pcm_out, ctx->stream);
+        rc = launch_chunk(ctx, p, c, d_nat, ctx->stream);
+        if (!rc) rc = launch_stretch(ctx, p, c, d_nat, ctx->stream);
     }
+    if (!rc) rc = launch_resample(ctx, p, d_nat, d_pcm_out, ctx->stream);
     return rc;
 }
 
@@ -1606,7 +1777,7 @@ int ctts_gpu_plan_read_counts(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t* out
     CU(ctx, cudaSetDevice(ctx->device));
     if (p->n_utts == 0) return CTTS_GPU_OK;
     std::vector<uint32_t> err(p->n_utts);
-    CU(ctx, cudaMemcpyAsync(out_counts, p->d_counts, (size_t)p->n_utts * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(out_counts, p->d_final_counts, (size_t)p->n_utts * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaMemcpyAsync(err.data(), p->d_err, (size_t)p->n_utts * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     for (uint32_t u = 0; u < p->n_utts; u++)
@@ -1761,7 +1932,7 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
             return bail(fail(ctx, CTTS_GPU_ERR_BOUNDS, "output slot of utterance %u is misaligned, outside the buffer or smaller than its bound %llu",
                              s->utts + u, (unsigned long long)p->bounds[u]));
     const uint64_t total = p->offsets[n];
-    auto grow = [&](int16_t** buf, uint64_t* cap_now) -> int {
+    auto grow = [&](int16_t** buf, uint64_t* cap_now, uint64_t total) -> int {
         if (total <= *cap_now) return 0;
         cudaFree(*buf);
         *buf = nullptr;
@@ -1774,8 +1945,10 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
         *cap_now = cap;
         return 0;
     };
-    if ((rc = grow(&l.d_out, &l.d_out_cap)) != 0) return bail(rc);
-    if (packed && (rc = grow(&l.d_pack, &l.d_pack_cap)) != 0) return bail(rc);
+    if ((rc = grow(&l.d_out, &l.d_out_cap, p->n_offsets[n])) != 0) return bail(rc);
+    if (p->rs && (rc = grow(&l.d_rs, &l.d_rs_cap, total)) != 0) return bail(rc);
+    if (packed && (rc = grow(&l.d_pack, &l.d_pack_cap, total)) != 0) return bail(rc);
+    int16_t* const d_final = p->rs ? l.d_rs : l.d_out;   // the slots callers see
     const size_t res_words = 2 * (size_t)n + 2 + 2 * ((size_t)n + 1);   // counts, flags, (aligned) slot offsets
     if (res_words > l.h_res_cap) {
         if (l.h_res) cudaFreeHost(l.h_res);
@@ -1801,7 +1974,7 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&l.counts_ready, cudaEventDisableTiming);
         if (e != cudaSuccess) return bail(fail(ctx, CTTS_GPU_ERR_CUDA, "event: %s", cudaGetErrorString(e)));
     }
-    p->d_out_last = l.d_out;
+    p->d_out_last = d_final;
     l.copy_pending = false;
     if (n) {
         rc = begin_run(ctx, p);
@@ -1809,6 +1982,7 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
         const auto tp2 = std::chrono::steady_clock::now();
         if (!rc) rc = launch_chunk(ctx, p, 0, l.d_out, ctx->stream);
         if (!rc) rc = launch_stretch(ctx, p, 0, l.d_out, ctx->stream);
+        if (!rc) rc = launch_resample(ctx, p, l.d_out, d_final, ctx->stream);
         if (rc) return bail(rc);
         if (ctx->knobs.trace) {
             auto msf = [](auto a, auto b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
@@ -1824,14 +1998,14 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
             unsigned long long* d_slot = l.d_pack_off + (n + 1);
             e = cudaMemcpyAsync(d_slot, h_slot, ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream);
             if (e == cudaSuccess) {
-                ctts::pack_scan_kernel<<<1, 1024, 0, ctx->stream>>>(p->d_counts, p->d_err, n, l.d_pack_off, l.h_res);
+                ctts::pack_scan_kernel<<<1, 1024, 0, ctx->stream>>>(p->d_final_counts, p->d_err, n, l.d_pack_off, l.h_res);
                 e = cudaGetLastError();
                 if (e == cudaSuccess) e = cudaEventRecord(l.counts_ready, ctx->stream);   // counts and flags are on the host
                 uint64_t max_slot = 0;
                 for (uint32_t u = 0; u < n; u++) max_slot = std::max<uint64_t>(max_slot, p->offsets[u + 1] - p->offsets[u]);
                 for (uint32_t u0 = 0; u0 < n && e == cudaSuccess; u0 += 65535u) {   // grid.y limit
                     const dim3 grid((unsigned)((max_slot + ctts::PACK_TILE - 1) / ctts::PACK_TILE), std::min<uint32_t>(n - u0, 65535u));
-                    ctts::pack_copy_kernel<<<grid, ctts::PACK_THREADS, 0, ctx->stream>>>(l.d_out, d_slot + u0, p->d_counts + u0, l.d_pack_off + u0, l.d_pack);
+                    ctts::pack_copy_kernel<<<grid, ctts::PACK_THREADS, 0, ctx->stream>>>(d_final, d_slot + u0, p->d_final_counts + u0, l.d_pack_off + u0, l.d_pack);
                     e = cudaGetLastError();
                 }
             }
@@ -1846,12 +2020,12 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
                    slot_cap[v] >= p->offsets[v + 1] - p->offsets[v])
                 v++;
             const uint64_t len = (p->offsets[v] - p->offsets[u]) + std::min<uint64_t>(p->offsets[v + 1] - p->offsets[v], slot_cap[v]);
-            if (len) e = cudaMemcpyAsync(s->pcm_out + slot_off[u], l.d_out + p->offsets[u], len * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
+            if (len) e = cudaMemcpyAsync(s->pcm_out + slot_off[u], d_final + p->offsets[u], len * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
             s->d2h_samples += len;
             u = v + 1;
         }
         if (e == cudaSuccess && !packed) {
-            e = cudaMemcpyAsync(l.h_res, p->d_counts, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->copy_stream);
+            e = cudaMemcpyAsync(l.h_res, p->d_final_counts, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->copy_stream);
             if (e == cudaSuccess) e = cudaMemcpyAsync(l.h_res + n, p->d_err, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->copy_stream);
             if (e == cudaSuccess) e = cudaEventRecord(l.copied, ctx->copy_stream);
         }
@@ -2043,6 +2217,9 @@ int ctts_gpu_multi_synth_batch(ctts_gpu_ctx* const* ctxs, uint32_t n_ctx, const 
     if (!ctxs || !n_ctx || !plan || !params || !pcm_out || !out_offsets || !out_counts) return CTTS_GPU_ERR_INVALID_ARG;
     for (uint32_t d = 0; d < n_ctx; d++)
         if (!ctxs[d]) return CTTS_GPU_ERR_INVALID_ARG;
+    for (uint32_t d = 1; d < n_ctx; d++)
+        if ((ctxs[d]->rs ? ctxs[d]->rs->hz : CTTS_PLAN_SAMPLE_RATE) != (ctxs[0]->rs ? ctxs[0]->rs->hz : CTTS_PLAN_SAMPLE_RATE))
+            return fail(ctxs[0], CTTS_GPU_ERR_INVALID_ARG, "context %u has another output rate than context 0", d);
     if (plan->n_utts && (!plan->utt_op_begin || !plan->speed)) return CTTS_GPU_ERR_INVALID_ARG;
     const uint32_t n = plan->n_utts;
     for (uint32_t u = 0; u < n; u++)

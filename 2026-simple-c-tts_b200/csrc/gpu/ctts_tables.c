@@ -10,6 +10,7 @@
  */
 #include <math.h>
 #include <stddef.h>
+#include <stdlib.h>
 
 #define CTTS_PI 3.14159265358979323846
 
@@ -23,4 +24,39 @@ void ctts_host_tables(float* fade_out, float* fade_in, float* sine, float* hann2
     for (int i = 0; i < 256; i++) hann256[i] = 0.5f * (1.0f - cosf(2.0f * CTTS_PI * i / 256));
     for (size_t i = 0; i < 512; i++)
         hann512[i] = 0.5f * (1.0f - cosf(2.0f * (float)CTTS_PI * (float)i / (float)512));
+}
+
+/* I0, the modified Bessel function of order 0, by its power series sum_k ((x/2)^k / k!)^2 */
+static double bessel_i0(double x) {
+    double term = 1.0, sum = 1.0;
+    const double q = 0.25 * x * x;
+    for (int k = 1; k < 500; k++) {
+        term *= q / ((double)k * (double)k);
+        sum += term;
+        if (term < 1e-17 * sum) break;
+    }
+    return sum;
+}
+
+/* The output-rate filter of DESIGN.md 3.4: g = L * firwin(N, 0.94 / R, window=('kaiser', beta)), N = 2*H*R + 1,
+ * H = 40, beta = 0.1102 * (70 - 8.7), computed in double and rounded to float once.  g receives N taps. */
+void ctts_host_resample_taps(unsigned L, unsigned M, float* g) {
+    const unsigned R = L > M ? L : M;
+    const unsigned N = 2u * 40u * R + 1u;
+    const double cutoff = 0.94 / (double)R, beta = 0.1102 * (70.0 - 8.7), half = 0.5 * (double)(N - 1);
+    const double i0b = bessel_i0(beta);
+    double* h = (double*)malloc(sizeof(double) * N);
+    double sum = 0.0;
+    if (!h) return;
+    for (unsigned i = 0; i < N; i++) {
+        const double m = (double)i - half;
+        const double a = CTTS_PI * cutoff * m;
+        const double sinc = m == 0.0 ? 1.0 : sin(a) / a;
+        const double r = m / half;
+        const double w = bessel_i0(beta * sqrt(r * r < 1.0 ? 1.0 - r * r : 0.0)) / i0b;
+        h[i] = cutoff * sinc * w;
+        sum += h[i];
+    }
+    for (unsigned i = 0; i < N; i++) g[i] = (float)((double)L * (h[i] / sum));
+    free(h);
 }

@@ -52,6 +52,7 @@ def lib(build: bool = True) -> C.CDLL:
         L.ctts_gpu_free.argtypes = [vp]
         L.ctts_gpu_free.restype = None
         L.ctts_gpu_set_stream.argtypes = [vp, vp]
+        L.ctts_gpu_set_output_rate.argtypes = [vp, C.c_uint32]
         L.ctts_gpu_last_error.argtypes = [vp]
         L.ctts_gpu_last_error.restype = C.c_char_p
         L.ctts_gpu_plan_bounds.argtypes = [vp, C.POINTER(CBatchPlan), vp]
@@ -188,6 +189,12 @@ class GpuSynth:
 
     def set_stream(self, cuda_stream_ptr: int | None) -> None:
         self._check(lib().ctts_gpu_set_stream(self._h, cuda_stream_ptr))
+
+    def set_output_rate(self, hz: int) -> None:
+        """ctts_gpu_set_output_rate: every later call of this context delivers PCM at `hz` (8000..48000, see
+        ctts_gpu.h for the accepted rates; 22050 is the voice's own), and every count, offset and bound is in
+        samples of that rate.  Plans created before keep their rate."""
+        self._check(lib().ctts_gpu_set_output_rate(self._h, int(hz)))
 
     def bounds(self, plan: BatchPlan) -> np.ndarray:
         b = np.zeros(max(plan.n_utts, 1), dtype=np.uint64)

@@ -39,6 +39,8 @@ def lib() -> C.CDLL:
                                             C.POINTER(C.c_uint64), C.POINTER(Options), C.POINTER(Timing)]
         L.ctts_b200_capacity_hint.argtypes = [vp, vp, vp, C.c_uint32]
         L.ctts_b200_capacity_hint.restype = C.c_uint64
+        L.ctts_b200_capacity_hint_rate.argtypes = [vp, vp, vp, C.c_uint32, C.c_uint32]
+        L.ctts_b200_capacity_hint_rate.restype = C.c_uint64
         L.ctts_b200_plan_cache_create.argtypes = [C.c_size_t]
         L.ctts_b200_plan_cache_create.restype = vp
         L.ctts_b200_plan_cache_destroy.argtypes = [vp]
@@ -89,8 +91,11 @@ class TextBatch:
         return None if self.speeds is None else self.speeds.ctypes.data
 
 
-def capacity_hint(front, batch: TextBatch) -> int:
-    return int(lib().ctts_b200_capacity_hint(front._h, batch.ptrs, batch.speeds_ptr, batch.n))
+def capacity_hint(front, batch: TextBatch, rate: int = 22050) -> int:
+    """Samples at output rate `rate` that are always enough for the batch (ctts_b200_capacity_hint_rate)."""
+    if rate == 22050:
+        return int(lib().ctts_b200_capacity_hint(front._h, batch.ptrs, batch.speeds_ptr, batch.n))
+    return int(lib().ctts_b200_capacity_hint_rate(front._h, batch.ptrs, batch.speeds_ptr, batch.n, rate))
 
 
 def synth_texts(front, gpu, batch: TextBatch, pcm_out: np.ndarray, piece_utts: int = 0, threads: int = 0,

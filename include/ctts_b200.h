@@ -49,7 +49,8 @@ typedef struct ctts_b200_timing {
     uint32_t reserved;
 } ctts_b200_timing;
 
-/* N texts -> PCM.  pcm_out (ctts_gpu_host_alloc) holds `capacity` samples; utterance u lands at
+/* N texts -> PCM at the output rate of `gpu` (ctts_gpu_set_output_rate; every count, offset and capacity is in
+ * samples of that rate).  pcm_out (ctts_gpu_host_alloc) holds `capacity` samples; utterance u lands at
  * pcm_out[out_offsets[u] .. out_offsets[u] + out_counts[u]) (out_offsets: n entries; the utterances are
  * packed back to back, each starting 16-byte aligned; *samples_used, may be NULL, = space taken).  speeds may be NULL
  * (all 1.0); stats may be NULL (2n: units found, missing per utterance, ctts.c:3861, :3866).
@@ -61,11 +62,13 @@ int ctts_b200_synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* cons
                           const ctts_b200_options* opt, ctts_b200_timing* timing);
 
 /* A capacity (samples) that is enough for the texts: characters x the longest unit x the slowest speed,
- * without planning anything. */
+ * without planning anything.  At another output rate: ctts_b200_capacity_hint_rate (ctts_b200_rate.h). */
 uint64_t ctts_b200_capacity_hint(ctts_front* front, const char* const* texts, const float* speeds, uint32_t n);
 
 #ifdef __cplusplus
 }
 #endif
+
+#include "ctts_b200_rate.h"
 
 #endif /* CTTS_B200_H */

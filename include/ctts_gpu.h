@@ -48,6 +48,19 @@ void ctts_gpu_free(ctts_gpu_ctx* ctx);
 /* Kernels and copies are issued on `cuda_stream` (a cudaStream_t); NULL
  * restores the context's own stream. */
 int ctts_gpu_set_stream(ctts_gpu_ctx* ctx, void* cuda_stream);
+/* Output sample rate of the context (DESIGN.md 3.4).  The back end assembles at the native 22 050 Hz
+ * (CTTS_PLAN_SAMPLE_RATE); any other rate converts every utterance on the device, after time stretching and
+ * before it is packed or copied: a Kaiser-windowed sinc of 2*40*max(L, M) + 1 taps at the reduced ratio L/M =
+ * hz/22050, utterance n samples long -> ceil(n*L/M) samples.  Accepted: integer hz in [8000, 48000] with
+ * max(L, M) <= 1024 (8000, 11025, 12000, 16000, 22050, 24000, 32000, 44100, 48000 among them).  Builds and uploads the
+ * tap table (once per rate and context).  CTTS_GPU_ERR_INVALID_ARG for any other rate and while a session is
+ * open; the context is then unchanged.  22050 (the default) enqueues no conversion at all.
+ *
+ * EVERY count, offset, capacity and bound of the context is in output-rate samples: ctts_gpu_plan_bounds, all
+ * ctts_gpu_synth_batch* calls, sessions, resident plans (out_samples, out_offsets, read_counts, read_pcm; a plan
+ * keeps the rate it was created under) and ctts_gpu_multi_synth_batch, which rejects contexts whose rates
+ * differ.  ctts_gpu_plan_read_pre stays at the native rate. */
+int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz);
 /* Text of the last error of a context; ctx == NULL: why the calling thread's last ctts_gpu_init failed. */
 const char* ctts_gpu_last_error(const ctts_gpu_ctx* ctx);
 
