@@ -27,6 +27,23 @@ extern "C" void ctts_host_tables(float* fade_out, float* fade_in, float* sine, f
                                  float* hann512);
 extern "C" void ctts_host_resample_taps(unsigned L, unsigned M, float* g);
 
+// Launch geometry of resample_kernel for the reduced ratio L/M (host only, no CUDA call; tests restate the kernel's
+// tile arithmetic against it): kp taps per phase row (a multiple of 4), the filter delay c, the staging bound
+// smem_floats of one tile, and the tiles (grid.x) that cover every output of an utterance of at most max_out
+// output samples.
+extern "C" void ctts_host_resample_geometry(uint32_t L, uint32_t M, uint64_t max_out, uint32_t* kp, uint32_t* c,
+                                            uint32_t* smem_floats, uint32_t* tiles) {
+    const uint32_t R = std::max(L, M), N = 2u * 40u * R + 1u;
+    *kp = ((N + L - 1) / L + 3) & ~3u;
+    *c = 40u * R;
+    // input span of a tile of RS_THREADS work items: they cover at most d + 1 rows of L * RS_COPIES outputs
+    const uint64_t d = (uint64_t)(L - 1 + ctts::RS_THREADS - 1) / L;
+    const uint64_t out_span = d * L * ctts::RS_COPIES + (uint64_t)L * ctts::RS_COPIES;
+    *smem_floats = (uint32_t)(((out_span * M) / L + 2 + *kp + 3) & ~3ull);
+    const uint64_t row = (uint64_t)L * ctts::RS_COPIES;
+    *tiles = (uint32_t)std::max<uint64_t>(((max_out + row - 1) / row * L + ctts::RS_THREADS - 1) / ctts::RS_THREADS, 1);
+}
+
 namespace {
 
 struct DbHeader {  // ctts.h:84-98
@@ -570,18 +587,15 @@ int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz) {
     const uint32_t N = 2u * 40u * R + 1u;
     std::vector<float> taps(N);
     ctts_host_resample_taps(L, M, taps.data());
+    uint32_t kp, c, smem_floats, tiles;
+    ctts_host_resample_geometry(L, M, 0, &kp, &c, &smem_floats, &tiles);
     // by phase, each row in the order the kernel walks it (resample.cuh), zero padded in front to a multiple of 4
-    const uint32_t kp = ((N + L - 1) / L + 3) & ~3u;
     std::vector<float> rows((size_t)L * kp, 0.0f);
     for (uint32_t phi = 0; phi < L; phi++)
         for (uint32_t k = 0; k < kp; k++) {
             const uint64_t i = (uint64_t)phi + (uint64_t)L * (kp - 1 - k);
             if (i < N) rows[(size_t)phi * kp + k] = taps[i];
         }
-    // input span of a tile of RS_THREADS work items: they cover at most d + 1 rows of L * RS_COPIES outputs
-    const uint64_t d = (uint64_t)(L - 1 + ctts::RS_THREADS - 1) / L;
-    const uint64_t out_span = d * L * ctts::RS_COPIES + (uint64_t)L * ctts::RS_COPIES;
-    const uint32_t smem_floats = (uint32_t)(((out_span * M) / L + 2 + kp + 3) & ~3ull);
     const int smem_bytes = (int)(smem_floats * sizeof(float));
     if (smem_bytes > ctx->smem_optin) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "output rate %u Hz: staging of %d bytes", hz, smem_bytes);
     if (smem_bytes > ctx->rs_smem_attr) {
@@ -593,7 +607,7 @@ int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz) {
     t->L = L;
     t->M = M;
     t->kp = kp;
-    t->c = 40u * R;
+    t->c = c;
     t->smem_floats = smem_floats;
     cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&t->d_taps), rows.size() * sizeof(float));
     if (e == cudaSuccess) e = cudaMemcpy(t->d_taps, rows.data(), rows.size() * sizeof(float), cudaMemcpyHostToDevice);
@@ -888,8 +902,8 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
             p->rs_off_h[u] = p->n_offsets[u];
             p->rs_off_h[n + 1 + u] = p->offsets[u];
         }
-        const uint64_t row = (uint64_t)rs->L * ctts::RS_COPIES;
-        p->rs_tiles = (uint32_t)std::max<uint64_t>(((ob_max + row - 1) / row * rs->L + ctts::RS_THREADS - 1) / ctts::RS_THREADS, 1);
+        uint32_t kp, c, smem_floats;
+        ctts_host_resample_geometry(rs->L, rs->M, ob_max, &kp, &c, &smem_floats, &p->rs_tiles);
     } else {
         p->n_offsets = p->offsets;
     }
@@ -1099,7 +1113,8 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
 
     p->info.kernel_launches = n_chunks;
     for (const PlanChunk& ch : p->chunks)   // scan, verify, repair (chain walk), overlap-add
-        p->info.kernel_launches += ch.st_count ? 2 + (ch.verify_tiles && ctx->knobs.wsola_speculate ? 1 : 0) + (ch.ola_count ? 1 : 0) : 0;
+        p->info.kernel_launches += ch.st_count ? 2 + (ch.verify_tiles && ctx->knobs.wsola_speculate ? (ch.st_count + 65534) / 65535 : 0) +
+                                                    (ch.ola_count ? 1 : 0) : 0;
     if (rs) p->info.kernel_launches += (uint32_t)(((uint64_t)n + 65534) / 65535);   // resample_kernel
     p->info.n_stretch = p->n_stretch;
     p->info.bound_samples = std::accumulate(bound.begin(), bound.end(), (uint64_t)0);
