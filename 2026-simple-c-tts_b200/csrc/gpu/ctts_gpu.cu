@@ -70,7 +70,7 @@ struct Knobs {
     int pitch_slots = 0;              // CTTS_GPU_PITCH_SLOTS: capacity of the unit-head pitch table (tests: a table that fills up)
     int ctas_per_sm = 3;              // CTTS_GPU_CTAS_PER_SM: occupancy the assembly window is sized for
     int window = 0;                   // CTTS_GPU_WINDOW: shared window in samples (tests: force the HBM-window path)
-    uint64_t chunk_samples = 192ull << 20;   // CTTS_GPU_CHUNK_SAMPLES: output samples per launch of ctts_gpu_synth_batch
+    uint64_t piece_samples = 192ull << 20;   // CTTS_GPU_CHUNK_SAMPLES: size of the pieces of the three batch calls (slot samples; packed: / 2800 ops)
     bool task_times = false;          // CTTS_GPU_TASK_TIMES=1: resident plans print the time their CTAs spent per task class
                                       // (only in a library built with -DCTTS_ASM_PROF=1)
     int region_dedup = 2;             // CTTS_GPU_REGION_DEDUP=0: assemble every word region of a batch, equal ones too;
@@ -88,7 +88,7 @@ struct Knobs {
         pitch_slots = (int)std::max(0ll, num("CTTS_GPU_PITCH_SLOTS", 0));
         ctas_per_sm = (int)std::max(1ll, std::min(8ll, num("CTTS_GPU_CTAS_PER_SM", 3)));
         window = (int)std::max(0ll, num("CTTS_GPU_WINDOW", 0));
-        chunk_samples = (uint64_t)std::max(1ll, num("CTTS_GPU_CHUNK_SAMPLES", 192ll << 20));
+        piece_samples = (uint64_t)std::max(1ll, num("CTTS_GPU_CHUNK_SAMPLES", 192ll << 20));
         region_dedup = (int)num("CTTS_GPU_REGION_DEDUP", 2);
         task_times = num("CTTS_GPU_TASK_TIMES", 0) != 0;
         wsola_speculate = num("CTTS_GPU_WSOLA_SPECULATE", 1) != 0;
@@ -178,16 +178,6 @@ struct ctts_gpu_ctx {
     char err[512] = {0};
 };
 
-// one kernel launch: a contiguous range of utterances (= a contiguous span of output slots)
-struct PlanChunk {
-    uint32_t utt_begin = 0, utt_end = 0;
-    uint32_t task_begin = 0, n_tasks = 0;
-    uint32_t grid = 0;
-    uint32_t st_begin = 0, st_count = 0;     // stretched utterances of the chunk (WSOLA tasks)
-    uint32_t ola_begin = 0, ola_count = 0;   // their overlap-add blocks
-    uint32_t verify_tiles = 0;               // tiles of the longest of them (grid.x of wsola_verify_kernel)
-};
-
 struct ctts_gpu_plan {
     ctts_gpu_ctx* ctx = nullptr;
     uint32_t n_utts = 0;
@@ -196,8 +186,7 @@ struct ctts_gpu_plan {
     std::vector<uint64_t> bounds;   // output-rate bounds
     ctts_gpu_ctx::RsTable* rs = nullptr;   // rate conversion the plan was created under (nullptr: native rate)
     std::vector<uint64_t> n_offsets;       // native-rate slots, where the assembly and WSOLA kernels write (== offsets without rs)
-    std::vector<unsigned long long> rs_off_h;   // rs: native slot offsets [n + 1], then output-rate ones [n + 1]
-    unsigned long long* d_rs_off = nullptr;
+    unsigned long long* d_rs_off = nullptr;   // rs: native slot offsets [n + 1], then output-rate ones [n + 1]
     uint32_t* d_rs_counts = nullptr;       // rs: output-rate counts
     uint32_t* d_final_counts = nullptr;    // the counts callers see: d_rs_counts with rs, else d_counts
     uint32_t rs_tiles = 0;                 // rs: grid.x of resample_kernel
@@ -209,14 +198,13 @@ struct ctts_gpu_plan {
     ctts_plan_op* d_ops = nullptr;
     ctts::RegionTask* d_tasks = nullptr;
     unsigned long long* d_chain = nullptr;
-    uint32_t* d_ticket = nullptr;   // one per chunk
+    uint32_t* d_ticket = nullptr;
     unsigned long long* d_prof = nullptr;   // CTTS_GPU_TASK_TIMES: per task class {ns, tasks}
     int16_t* d_region_store = nullptr;              // canonical word regions (see run_task in assemble.cuh)
     unsigned long long* d_region_state = nullptr;
-    size_t d_used = 0;              // arena mode: device bytes taken by prepare_plan (build_chunk continues from here)
-    std::vector<PlanChunk> chunks;
+    size_t d_used = 0;              // arena mode: device bytes taken by prepare_plan (build_tasks continues from here)
     uint32_t n_tasks = 0;
-    uint32_t n_global_tasks = 0;
+    uint32_t grid = 0;              // CTAs of assemble_kernel
     uint32_t epoch = 0;
     ctts::StretchTask* d_stasks = nullptr;
     uint32_t* d_counts = nullptr;
@@ -231,20 +219,18 @@ struct ctts_gpu_plan {
     uint32_t* d_ola_first = nullptr;
     uint32_t n_stretch = 0;
     uint32_t n_ola_blocks = 0;
+    uint32_t verify_tiles = 0;      // tiles of the longest stretched utterance (grid.x of wsola_verify_kernel)
     int16_t* d_out_owned = nullptr;
     int16_t* d_out_last = nullptr;
     std::vector<uint64_t> pre_off;   // per utterance (stretch only), else ~0
     std::vector<uint64_t> pre_cap;
     uint32_t wcap = 0, hcap = 0, smem_bytes = 0;
     ctts_gpu_run_info info{};
-    // builder state (chunks are compiled and uploaded one at a time, see build_chunk)
-    const ctts_batch_plan* src = nullptr;   // borrowed until the last chunk is built
-    ctts_plan_op* h_ops = nullptr;          // staging: pinned (context arena) or the vectors below
+    // builder state (prepare_plan -> build_tasks)
+    ctts_plan_op* h_ops = nullptr;          // staging: pinned (lane arena) or h_staging
     ctts::RegionTask* h_tasks = nullptr;
-    std::vector<ctts_plan_op> ops_vec;
-    std::vector<ctts::RegionTask> tasks_vec;
-    uint32_t built_chunks = 0, n_big = 0, big_cap = 0, occ = 1;
-    uint64_t gather = 0;
+    std::vector<char> h_staging;            // resident plans: pageable staging of the uploads, freed by build_tasks
+    uint32_t n_big = 0, big_cap = 0, occ = 1;
 };
 
 namespace {
@@ -675,24 +661,36 @@ void ctts_gpu_plan_destroy(ctts_gpu_plan* p) {
 
 namespace {
 
-// Device / pinned allocation for one plan: individual cudaMallocs (resident plans), or bump
-// allocation from the context's grow-only arenas (ctts_gpu_synth_batch: no malloc/free per call).
+// Workspace of one plan.  Device buffers: individual cudaMallocs (resident plans), or bump allocation from
+// a lane's grow-only arena (session pieces: no malloc/free per call).  Upload staging: bump allocation from
+// the arena's pinned block, or from the plan's pageable h_staging.  A measuring PlanAlloc allocates nothing
+// and returns nullptr: it only counts the bytes, so that one list of buffers both sizes and lays out the workspace.
 struct PlanAlloc {
-    ctts_gpu_ctx* ctx;
     ctts_gpu_plan* p;
-    size_t d_used = 0, h_used = 0;
-    cudaError_t err = cudaSuccess;
+    bool measure;
+    size_t d_used = 0, staged = 0;   // bytes
+    cudaError_t err = cudaSuccess;   // cudaErrorMemoryAllocation also when the list outgrows the arena
 
     static size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
 
-    // phase 1 (arena mode): reserve() everything, then commit() grows the arenas once
+    template <typename T>
+    T* host(size_t count) {
+        const size_t bytes = up256(std::max<size_t>(count, 1) * sizeof(T));
+        staged += bytes;
+        if (measure) return nullptr;
+        char* const base = p->arena ? p->arena->h : p->h_staging.data();
+        if (staged > (p->arena ? p->arena->h_cap : p->h_staging.size())) { err = cudaErrorMemoryAllocation; return nullptr; }
+        return reinterpret_cast<T*>(base + staged - bytes);
+    }
+
     template <typename T>
     T* dev(size_t count) {
         const size_t bytes = up256(std::max<size_t>(count, 1) * sizeof(T));
-        if (p->arena) {
-            T* r = reinterpret_cast<T*>(p->arena->d + d_used);
+        if (measure || p->arena) {
             d_used += bytes;
-            return r;
+            if (measure) return nullptr;
+            if (d_used > p->arena->d_cap) { err = cudaErrorMemoryAllocation; return nullptr; }
+            return reinterpret_cast<T*>(p->arena->d + d_used - bytes);
         }
         void* d = nullptr;
         cudaError_t e = cudaMalloc(&d, bytes);
@@ -815,9 +813,23 @@ int run_pitch_jobs(ctts_gpu_ctx* ctx, ctts_gpu_ctx::NormPool* np, const std::vec
     return CTTS_GPU_OK;
 }
 
+// Slots packed by their bounds, up8(bound) + 8 samples each: the n + 1 offsets.
+int pack_slots(ctts_gpu_ctx* ctx, const std::vector<uint64_t>& bound, std::vector<uint64_t>* off) {
+    off->resize(bound.size() + 1);
+    uint64_t o = 0;
+    for (uint32_t u = 0; u < bound.size(); u++) {
+        if (bound[u] + 16 > 0xffffffffull)
+            return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "utterance %u too long (%llu samples)", u, (unsigned long long)bound[u]);
+        (*off)[u] = o;
+        o += up8(bound[u]) + 8;
+    }
+    off->back() = o;
+    return CTTS_GPU_OK;
+}
+
 // The plan compiler, part 1: validation, bounds, output layout, workspace.  One launch of every kernel
 // per plan; a large batch is cut into pieces (plans) by the session code below.  `arena` != nullptr:
-// device / pinned workspace comes from that lane's grow-only arena.  build_chunk() is part 2.
+// device / pinned workspace comes from that lane's grow-only arena.  build_tasks() is part 2.
 int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_assembly_params* params,
                  const uint64_t* out_offsets, Arena* arena, ctts_gpu_plan** out) {
     if (!ctx || !plan || !params || !out) return CTTS_GPU_ERR_INVALID_ARG;
@@ -855,14 +867,12 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     p->bounds = bound;
     p->rs = rs;
     p->arena = arena;
-    p->src = plan;
     p->op0 = n ? plan->utt_op_begin[0] : 0;
     const uint32_t n_ops_local = n ? plan->utt_op_begin[n] - p->op0 : 0;   // (validated by the scan)
 
     // ---- output layout
-    p->offsets.resize((size_t)n + 1);
     if (out_offsets) {
-        for (uint32_t u = 0; u <= n; u++) p->offsets[u] = out_offsets[u];
+        p->offsets.assign(out_offsets, out_offsets + (size_t)n + 1);
         for (uint32_t u = 0; u < n; u++) {
             if ((out_offsets[u] & 7) || out_offsets[u + 1] < out_offsets[u] ||
                 out_offsets[u + 1] - out_offsets[u] < bound[u] || out_offsets[u + 1] - out_offsets[u] > 0xffffffffull) {
@@ -871,37 +881,17 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
                             (unsigned long long)bound[u]);
             }
         }
-    } else {
-        uint64_t o = 0;
-        for (uint32_t u = 0; u < n; u++) {
-            if (bound[u] + 16 > 0xffffffffull) {
-                delete p;
-                return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "utterance %u too long (%llu samples)", u, (unsigned long long)bound[u]);
-            }
-            p->offsets[u] = o;
-            o += up8(bound[u]) + 8;
-        }
-        p->offsets[n] = o;
+    } else if ((rc = pack_slots(ctx, bound, &p->offsets)) != 0) {
+        delete p;
+        return rc;
     }
     if (rs) {
         // native slots packed by the native bounds; resample_kernel turns them into the slots above
-        p->n_offsets.resize((size_t)n + 1);
-        uint64_t o = 0, ob_max = 0;
-        for (uint32_t u = 0; u < n; u++) {
-            if (sc.bound[u] + 16 > 0xffffffffull) {
-                delete p;
-                return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "utterance %u too long (%llu samples)", u, (unsigned long long)sc.bound[u]);
-            }
-            p->n_offsets[u] = o;
-            o += up8(sc.bound[u]) + 8;
-            ob_max = std::max(ob_max, bound[u]);
+        if ((rc = pack_slots(ctx, sc.bound, &p->n_offsets)) != 0) {
+            delete p;
+            return rc;
         }
-        p->n_offsets[n] = o;
-        p->rs_off_h.resize(2 * ((size_t)n + 1));
-        for (uint32_t u = 0; u <= n; u++) {
-            p->rs_off_h[u] = p->n_offsets[u];
-            p->rs_off_h[n + 1 + u] = p->offsets[u];
-        }
+        const uint64_t ob_max = n ? *std::max_element(bound.begin(), bound.end()) : 0;
         uint32_t kp, c, smem_floats;
         ctts_host_resample_geometry(rs->L, rs->M, ob_max, &kp, &c, &smem_floats, &p->rs_tiles);
     } else {
@@ -931,128 +921,116 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     p->hcap = hcap;
     p->smem_bytes = smem_for(wcap);
 
-    uint32_t n_stretched = 0;
+    // ---- slots of stretched utterances and WSOLA tasks, longest first
+    std::vector<uint32_t> order;
     if (sc.any_stretch)
         for (uint32_t u = 0; u < n; u++) {
             uint32_t hop = 0;
-            n_stretched += needs_stretch(plan->speed[u], &hop);
+            if (needs_stretch(plan->speed[u], &hop)) order.push_back(u);
         }
-    {
-        PlanChunk ch;
-        ch.utt_end = n;
-        p->chunks.push_back(ch);
-    }
-
-    // ---- slots of stretched utterances and WSOLA tasks, chunk by chunk, longest first inside a chunk
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return pre[a] > pre[b]; });
     std::vector<ctts::StretchTask> stasks;
     std::vector<uint32_t> ola_task, ola_first;
     p->pre_off.assign(n, ~0ull);
     p->pre_cap.assign(n, 0);
     uint64_t pre_total = 0, pos_total = 0;
-    if (n_stretched) {
-        std::vector<uint32_t> order;
-        for (PlanChunk& ch : p->chunks) {
-            ch.st_begin = (uint32_t)stasks.size();
-            ch.ola_begin = (uint32_t)ola_task.size();
-            order.resize(ch.utt_end - ch.utt_begin);
-            std::iota(order.begin(), order.end(), ch.utt_begin);
-            std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return pre[a] > pre[b]; });
-            for (const uint32_t u : order) {
-                uint32_t hop = 0;
-                if (!needs_stretch(plan->speed[u], &hop)) continue;
-                if (pre[u] + 16 > 0xffffffffull) {
-                    delete p;
-                    return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "utterance %u too long", u);
-                }
-                p->pre_off[u] = pre_total;
-                p->pre_cap[u] = (uint32_t)(up8(pre[u]) + 8);
-                ctts::StretchTask st;
-                st.utt = u;
-                st.hop = hop;
-                st.pre_off = pre_total;
-                st.out_off = p->n_offsets[u];
-                st.out_cap = (uint32_t)(p->n_offsets[u + 1] - p->n_offsets[u]);
-                st.pos_off = (uint32_t)pos_total;
-                st.max_frames = (uint32_t)(pre[u] > 512 ? (pre[u] - 512) / 128 + 1 : 1);
-                if (st.max_frames > 1)
-                    ch.verify_tiles = std::max(ch.verify_tiles, (st.max_frames - 1 + ctts::WV_FRAMES - 1) / ctts::WV_FRAMES);
-                const uint64_t used_max = (uint64_t)st.max_frames * hop + 512;
-                const uint32_t per_block = ctts::ola_block_span(hop);
-                for (uint64_t f = 0; f < used_max; f += per_block) {
-                    ola_task.push_back((uint32_t)stasks.size());
-                    ola_first.push_back((uint32_t)f);
-                }
-                stasks.push_back(st);
-                pre_total += p->pre_cap[u];
-                pos_total += st.max_frames;
-                if (pos_total > 0xffffffffull) {
-                    delete p;
-                    return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "too many WSOLA frames in one batch");
-                }
-            }
-            ch.st_count = (uint32_t)stasks.size() - ch.st_begin;
-            ch.ola_count = (uint32_t)ola_task.size() - ch.ola_begin;
+    for (const uint32_t u : order) {
+        uint32_t hop = 0;
+        needs_stretch(plan->speed[u], &hop);
+        if (pre[u] + 16 > 0xffffffffull) {
+            delete p;
+            return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "utterance %u too long", u);
+        }
+        p->pre_off[u] = pre_total;
+        p->pre_cap[u] = (uint32_t)(up8(pre[u]) + 8);
+        ctts::StretchTask st;
+        st.utt = u;
+        st.hop = hop;
+        st.pre_off = pre_total;
+        st.out_off = p->n_offsets[u];
+        st.out_cap = (uint32_t)(p->n_offsets[u + 1] - p->n_offsets[u]);
+        st.pos_off = (uint32_t)pos_total;
+        st.max_frames = (uint32_t)(pre[u] > 512 ? (pre[u] - 512) / 128 + 1 : 1);
+        if (st.max_frames > 1)
+            p->verify_tiles = std::max(p->verify_tiles, (st.max_frames - 1 + ctts::WV_FRAMES - 1) / ctts::WV_FRAMES);
+        const uint64_t used_max = (uint64_t)st.max_frames * hop + 512;
+        const uint32_t per_block = ctts::ola_block_span(hop);
+        for (uint64_t f = 0; f < used_max; f += per_block) {
+            ola_task.push_back((uint32_t)stasks.size());
+            ola_first.push_back((uint32_t)f);
+        }
+        stasks.push_back(st);
+        pre_total += p->pre_cap[u];
+        pos_total += st.max_frames;
+        if (pos_total > 0xffffffffull) {
+            delete p;
+            return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "too many WSOLA frames in one batch");
         }
     }
     p->n_stretch = (uint32_t)stasks.size();
     p->n_ola_blocks = (uint32_t)ola_task.size();
-    const uint32_t n_chunks = (uint32_t)p->chunks.size();
     if (sc.n_regions + 1 > 0x7fffffffull) {
         delete p;
         return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "too many region tasks");
     }
 
-    // ---- workspace.  The private op copy and the tasks are built directly in (pinned) staging.
-    const size_t ops_bytes = std::max<size_t>(n_ops_local, 1) * sizeof(ctts_plan_op);
+    // ---- workspace: one list of device buffers and upload staging, run once to measure it (the arena, or the
+    // pageable staging, is sized from that) and once to lay it out.  The private op copy and the tasks are built
+    // directly in the staging.
     // merging only lowers the count of region tasks; canonical word regions (each stands for >= 2 tasks) add at most half
     const size_t tasks_cap = (size_t)sc.n_regions + (size_t)sc.n_regions / 2 + 2;
-    uint64_t pre_sum = 0;
-    for (uint32_t u = 0; u < n; u++) pre_sum += pre[u];
-    // region store: the canonical regions' slots and the shared whole tasks' (each <= half of all region samples,
-    // a slot per two tasks at most) + their tables
-    const size_t region_bytes = PlanAlloc::up256((pre_sum + 16 * (sc.n_regions + 2)) * sizeof(int16_t)) +
-                                2 * PlanAlloc::up256((sc.n_regions + 2) * 8);
-    const size_t tasks_bytes = tasks_cap * sizeof(ctts::RegionTask);
+    ctts::StretchTask* h_st = nullptr;
+    uint32_t *h_ot = nullptr, *h_of = nullptr;
+    unsigned long long* h_ro = nullptr;
+    auto layout = [&](PlanAlloc& al) {
+        p->d_ops = al.dev<ctts_plan_op>(n_ops_local);
+        p->d_tasks = al.dev<ctts::RegionTask>(tasks_cap);
+        p->d_chain = al.dev<unsigned long long>(tasks_cap);
+        p->d_ticket = al.dev<uint32_t>(1);
+        if (ctx->knobs.task_times && !arena) p->d_prof = al.dev<unsigned long long>(16);
+        p->d_counts = al.dev<uint32_t>(n);
+        p->d_pre_counts = al.dev<uint32_t>(n);
+        p->d_err = al.dev<uint32_t>(n);
+        p->d_final_counts = p->d_counts;
+        if (rs) {
+            p->d_rs_counts = al.dev<uint32_t>(n);
+            p->d_rs_off = al.dev<unsigned long long>(2 * ((size_t)n + 1));
+            p->d_final_counts = p->d_rs_counts;
+        }
+        if (p->n_stretch) {
+            p->d_stasks = al.dev<ctts::StretchTask>(stasks.size());
+            p->d_ola_task = al.dev<uint32_t>(ola_task.size());
+            p->d_ola_first = al.dev<uint32_t>(ola_first.size());
+            p->d_pre = al.dev<int16_t>(pre_total);
+            p->d_frame_pos = al.dev<uint32_t>(pos_total);
+            p->d_n_frames = al.dev<uint32_t>(5 * (size_t)p->n_stretch);   // frames, exact evaluations, first bad frame, first silent frame, tier-2 candidates
+        }
+        p->h_ops = al.host<ctts_plan_op>(n_ops_local);
+        p->h_tasks = al.host<ctts::RegionTask>(tasks_cap);
+        if (p->n_stretch) {
+            h_st = al.host<ctts::StretchTask>(stasks.size());
+            h_ot = al.host<uint32_t>(ola_task.size());
+            h_of = al.host<uint32_t>(ola_first.size());
+        }
+        if (rs) h_ro = al.host<unsigned long long>(2 * ((size_t)n + 1));
+    };
+    PlanAlloc al{p, true};
+    layout(al);
     if (arena) {
-        // device side: ops, tasks, chain, tickets, counts, pre_counts, err (+ the stretch buffers)
-        size_t d_need = PlanAlloc::up256(ops_bytes) + PlanAlloc::up256(tasks_bytes) + PlanAlloc::up256(tasks_cap * 8) +
-                        PlanAlloc::up256((size_t)n_chunks * 4) + 3 * PlanAlloc::up256(std::max<size_t>(n, 1) * 4) + 65536 +
-                        (ctx->knobs.region_dedup ? region_bytes + 4096 : 0);
-        if (!stasks.empty())
-            d_need += PlanAlloc::up256(stasks.size() * sizeof(ctts::StretchTask)) + 2 * PlanAlloc::up256(ola_task.size() * 4 + 4) +
-                      PlanAlloc::up256(pre_total * 2 + 16) + PlanAlloc::up256(pos_total * 4 + 4) + PlanAlloc::up256(stasks.size() * 20) + 4096;
-        const size_t rs_bytes = rs ? PlanAlloc::up256(p->rs_off_h.size() * 8) : 0;
-        if (rs) d_need += rs_bytes + PlanAlloc::up256((size_t)n * 4);
-        const size_t st_bytes = PlanAlloc::up256(stasks.size() * sizeof(ctts::StretchTask)) + 2 * PlanAlloc::up256(ola_task.size() * 4 + 4);
-        const size_t h_need = PlanAlloc::up256(ops_bytes) + PlanAlloc::up256(tasks_bytes) + st_bytes + rs_bytes + 4096;
-        rc = ensure_arena(ctx, arena, d_need, h_need);
+        // + the region store, carved by build_tasks once the regions are known; reserved here at its upper bound:
+        // the canonical regions' slots and the shared whole tasks' (each <= half of all region samples, a slot per
+        // two tasks at most) + their tables
+        const uint64_t pre_sum = std::accumulate(pre.begin(), pre.end(), (uint64_t)0);
+        const size_t region_bytes = !ctx->knobs.region_dedup ? 0 :
+            PlanAlloc::up256((pre_sum + 16 * (sc.n_regions + 2)) * sizeof(int16_t)) + 2 * PlanAlloc::up256((sc.n_regions + 2) * 8);
+        rc = ensure_arena(ctx, arena, al.d_used + region_bytes, al.staged);
         if (rc) { delete p; return rc; }
-        p->h_ops = reinterpret_cast<ctts_plan_op*>(arena->h);
-        p->h_tasks = reinterpret_cast<ctts::RegionTask*>(arena->h + PlanAlloc::up256(ops_bytes));
     } else {
-        p->ops_vec.resize(std::max<size_t>(n_ops_local, 1));
-        p->tasks_vec.resize(tasks_cap);
-        p->h_ops = p->ops_vec.data();
-        p->h_tasks = p->tasks_vec.data();
+        p->h_staging.resize(al.staged);
     }
-    PlanAlloc al{ctx, p};
-    p->d_ops = al.dev<ctts_plan_op>(n_ops_local);
-    p->d_tasks = al.dev<ctts::RegionTask>(tasks_cap);
-    p->d_chain = al.dev<unsigned long long>(tasks_cap);
-    p->d_ticket = al.dev<uint32_t>(n_chunks);
-    if (ctx->knobs.task_times && !arena) {
-        p->d_prof = al.dev<unsigned long long>(16);
-        if (p->d_prof) cudaMemset(p->d_prof, 0, 16 * 8);
-    }
-    p->d_counts = al.dev<uint32_t>(n);
-    p->d_pre_counts = al.dev<uint32_t>(n);
-    p->d_err = al.dev<uint32_t>(n);
-    p->d_final_counts = p->d_counts;
-    if (rs) {
-        p->d_rs_counts = al.dev<uint32_t>(n);
-        p->d_rs_off = al.dev<unsigned long long>(p->rs_off_h.size());
-        p->d_final_counts = p->d_rs_counts;
-    }
+    al = PlanAlloc{p, false};
+    layout(al);
+    if (p->d_prof) cudaMemset(p->d_prof, 0, 16 * 8);
     if (sc.n_big_regions) {
         // rare (regions longer than ~51 k samples): always a separate allocation
         p->trim_words = (uint32_t)(2 * ((sc.big_region_max + 31) / 32) + 8);
@@ -1061,60 +1039,39 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         if (cudaMalloc(&d, (size_t)p->big_cap * p->trim_words * 4) != cudaSuccess) al.err = cudaErrorMemoryAllocation;
         else { p->owned.push_back(d); p->d_trim = static_cast<uint32_t*>(d); }
     }
-    if (p->n_stretch) {
-        p->d_stasks = al.dev<ctts::StretchTask>(stasks.size());
-        p->d_ola_task = al.dev<uint32_t>(ola_task.size());
-        p->d_ola_first = al.dev<uint32_t>(ola_first.size());
-        p->d_pre = al.dev<int16_t>(pre_total);
-        p->d_frame_pos = al.dev<uint32_t>(pos_total);
-        p->d_n_frames = al.dev<uint32_t>(5 * (size_t)p->n_stretch);   // frames, exact evaluations, first bad frame, first silent frame, tier-2 candidates
-    }
     if (al.err != cudaSuccess) {
         ctts_gpu_plan_destroy(p);
         return fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "plan workspace: %s", cudaGetErrorString(al.err));
     }
     p->d_used = al.d_used;
+    // arena: through the lane's pinned staging, truly asynchronous, no stream drain per piece (the staging is
+    // reused only after the lane's piece has completed)
     cudaStream_t st = ctx->stream;
     CUP(cudaMemsetAsync(p->d_chain, 0, tasks_cap * 8, st));
     if (p->n_stretch) {
-        const void *h_st = stasks.data(), *h_ot = ola_task.data(), *h_of = ola_first.data();
-        if (arena) {
-            // through the lane's pinned staging: truly asynchronous, no stream drain per piece (the staging is
-            // reused only after the lane's piece has completed)
-            char* at = arena->h + PlanAlloc::up256(ops_bytes) + PlanAlloc::up256(tasks_bytes);
-            memcpy(at, stasks.data(), stasks.size() * sizeof(ctts::StretchTask));
-            h_st = at;
-            at += PlanAlloc::up256(stasks.size() * sizeof(ctts::StretchTask));
-            memcpy(at, ola_task.data(), ola_task.size() * 4);
-            h_ot = at;
-            at += PlanAlloc::up256(ola_task.size() * 4 + 4);
-            memcpy(at, ola_first.data(), ola_first.size() * 4);
-            h_of = at;
-        }
+        memcpy(h_st, stasks.data(), stasks.size() * sizeof(ctts::StretchTask));
+        memcpy(h_ot, ola_task.data(), ola_task.size() * 4);
+        memcpy(h_of, ola_first.data(), ola_first.size() * 4);
         CUP(cudaMemcpyAsync(p->d_stasks, h_st, stasks.size() * sizeof(ctts::StretchTask), cudaMemcpyHostToDevice, st));
         CUP(cudaMemcpyAsync(p->d_ola_task, h_ot, ola_task.size() * 4, cudaMemcpyHostToDevice, st));
         CUP(cudaMemcpyAsync(p->d_ola_first, h_of, ola_first.size() * 4, cudaMemcpyHostToDevice, st));
-        if (!arena) CUP(cudaStreamSynchronize(st));   // pageable vectors that are about to go out of scope
     }
     if (rs) {
-        const void* h_ro = p->rs_off_h.data();   // (resident plans: lives as long as the plan)
-        if (arena) {
-            char* at = arena->h + PlanAlloc::up256(ops_bytes) + PlanAlloc::up256(tasks_bytes) +
-                       PlanAlloc::up256(stasks.size() * sizeof(ctts::StretchTask)) + 2 * PlanAlloc::up256(ola_task.size() * 4 + 4);
-            memcpy(at, p->rs_off_h.data(), p->rs_off_h.size() * 8);
-            h_ro = at;
+        for (uint32_t u = 0; u <= n; u++) {
+            h_ro[u] = p->n_offsets[u];
+            h_ro[n + 1 + u] = p->offsets[u];
         }
-        CUP(cudaMemcpyAsync(p->d_rs_off, h_ro, p->rs_off_h.size() * 8, cudaMemcpyHostToDevice, st));
+        CUP(cudaMemcpyAsync(p->d_rs_off, h_ro, 2 * ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, st));
     }
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ctts::assemble_kernel, ctts::ASM_THREADS, p->smem_bytes) != cudaSuccess || occ < 1)
         occ = 1;
     p->occ = (uint32_t)occ;
 
-    p->info.kernel_launches = n_chunks;
-    for (const PlanChunk& ch : p->chunks)   // scan, verify, repair (chain walk), overlap-add
-        p->info.kernel_launches += ch.st_count ? 2 + (ch.verify_tiles && ctx->knobs.wsola_speculate ? (ch.st_count + 65534) / 65535 : 0) +
-                                                    (ch.ola_count ? 1 : 0) : 0;
+    p->info.kernel_launches = 1;   // assemble_kernel, counted also when a plan without tasks skips it
+    if (p->n_stretch)   // scan, verify, repair (chain walk), overlap-add
+        p->info.kernel_launches += 2 + (p->verify_tiles && ctx->knobs.wsola_speculate ? (p->n_stretch + 65534) / 65535 : 0) +
+                                   (p->n_ola_blocks ? 1 : 0);
     if (rs) p->info.kernel_launches += (uint32_t)(((uint64_t)n + 65534) / 65535);   // resample_kernel
     p->info.n_stretch = p->n_stretch;
     p->info.bound_samples = std::accumulate(bound.begin(), bound.end(), (uint64_t)0);
@@ -1128,20 +1085,17 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
 }
 
 // The plan compiler, part 2: private op copy (with provably dead fade-outs turned into
-// no-ops), regions -> tasks, ticket order, upload -- for chunk c.  Chunks are built in order.
-int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st) {
-    if (c != p->built_chunks || c >= p->chunks.size() || !p->src) return CTTS_GPU_ERR_INVALID_ARG;
-    const ctts_batch_plan* plan = p->src;
-    PlanChunk& ch = p->chunks[c];
-    const uint32_t u0 = ch.utt_begin, u1 = ch.utt_end;
+// no-ops), regions -> tasks, ticket order, upload.  `plan` is the one prepare_plan() was given.
+int build_tasks(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const ctts_batch_plan* plan, cudaStream_t st) {
+    const uint32_t n = p->n_utts;
     const uint32_t* ub = plan->utt_op_begin;
     const std::vector<uint32_t>& ucnt = ctx->unit_cnt;
     const uint32_t wcap = p->wcap;
     const uint64_t scr_samples = (uint64_t)(ctts::SCR_WORDS - 4) / 2 * 32;
     ctts_plan_op* h_ops = p->h_ops;
     const uint32_t op0 = p->op0;   // h_ops / d_ops hold the caller's ops from op0 on
-    const uint32_t op_lo = u1 > u0 ? ub[u0] : op0, op_hi = u1 > u0 ? ub[u1] : op0;
-    if (op_hi > op_lo) memcpy(h_ops + (op_lo - op0), plan->ops + op_lo, (size_t)(op_hi - op_lo) * sizeof(ctts_plan_op));
+    const uint32_t n_ops = n ? ub[n] - op0 : 0;
+    if (n_ops) memcpy(h_ops, plan->ops + op0, (size_t)n_ops * sizeof(ctts_plan_op));
 
     // A fade-out that provably acts on zeros (or on an empty buffer) becomes a no-op, so that a
     // pause-only region never has to reach back into its predecessor's samples.  Trailing zeros:
@@ -1156,10 +1110,10 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
     std::vector<HostTask> ht;
     std::vector<uint3> pitch_jobs;
     std::vector<uint32_t> pitch_job_units;   // unit of every new table entry (to take them back if the fill fails)
-    std::vector<uint32_t> ht_begin(u1 - u0 + 1, 0);   // CSR: tasks of utterance u0 + i
+    std::vector<uint32_t> ht_begin(n + 1, 0);   // CSR: tasks of utterance u
     uint32_t max_rows = 0;
-    for (uint32_t u = u0; u < u1; u++) {
-        ht_begin[u - u0] = (uint32_t)ht.size();
+    for (uint32_t u = 0; u < n; u++) {
+        ht_begin[u] = (uint32_t)ht.size();
         uint64_t tz = 0, count_ub = 0, rb = 0, L = 0;
         uint64_t count_lb = 0, word_lb = 0, region_lb = 0;   // lower bounds: of the count, at the last MARK, at the start of the open region
         uint32_t r_units = 0, r_begin = ub[u];
@@ -1167,7 +1121,7 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
         auto close_region = [&](uint32_t r_end) {
             if (r_end == r_begin) return;
             const bool tiny = r_units == 0 || rb <= 2048;
-            if (ht.size() > ht_begin[u - u0] && tiny && ht.back().bound + rb <= wcap) {
+            if (ht.size() > ht_begin[u] && tiny && ht.back().bound + rb <= wcap) {
                 ht.back().op_end = r_end;
                 ht.back().bound += rb;
                 ht.back().region_max = (uint32_t)std::max<uint64_t>(ht.back().region_max, rb);
@@ -1203,7 +1157,7 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
                     memcpy(&op.f2, &slot1, 4);
                     count_ub += cn;
                     count_lb += (op.flags & CTTS_UNIT_AFTER_BOUNDARY) ? cn : cn - std::min(op.b, cn);
-                    p->gather += cn;
+                    p->info.gather_samples += cn;
                     rb += unit_append_bound(op, cn, L);
                     r_units++;
                     if (cn) { tz = 0; audio = true; }
@@ -1231,9 +1185,9 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
             }
         }
         close_region(ub[u + 1]);
-        max_rows = std::max<uint32_t>(max_rows, (uint32_t)ht.size() - ht_begin[u - u0]);
+        max_rows = std::max<uint32_t>(max_rows, (uint32_t)ht.size() - ht_begin[u]);
     }
-    ht_begin[u1 - u0] = (uint32_t)ht.size();
+    ht_begin[n] = (uint32_t)ht.size();
     {
         const int rcj = run_pitch_jobs(ctx, p->np, pitch_jobs);
         if (rcj) {
@@ -1348,7 +1302,7 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
         }
         if (ctx->knobs.trace) {
             uint64_t single = 0, single_bound = 0, first = 0, first_bound = 0;
-            for (uint32_t ui = 0; ui < u1 - u0; ui++)
+            for (uint32_t ui = 0; ui < n; ui++)
                 for (uint32_t ti = ht_begin[ui]; ti < ht_begin[ui + 1]; ti++) {
                     if (dd[ti].group == ctts::NO_REGION) continue;
                     if (groups[dd[ti].group].count < 2) { single++; single_bound += ht[ti].bound; }
@@ -1394,7 +1348,7 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
                 if (memcmp(&h_ops[dd[ta].w_op + i - op0], &h_ops[dd[tb].w_op + i - op0], 12) != 0) return false;
             return true;
         };
-        for (uint32_t ui = 0; ui < u1 - u0; ui++) {
+        for (uint32_t ui = 0; ui < n; ui++) {
             for (uint32_t ti = ht_begin[ui]; ti < ht_begin[ui + 1]; ti++) {
                 const Dedup& d = dd[ti];
                 if (d.group == ctts::NO_REGION || groups[d.group].canon == ctts::NO_REGION) continue;
@@ -1442,16 +1396,16 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
     // copy waits for memory), those whose source is in the same row close it (and so run well after it)
     std::vector<uint32_t> order;              // ht indices in ticket order
     std::vector<uint32_t> ht_ui(ht.size());
-    for (uint32_t ui = 0; ui < u1 - u0; ui++)
+    for (uint32_t ui = 0; ui < n; ui++)
         for (uint32_t ti = ht_begin[ui]; ti < ht_begin[ui + 1]; ti++) ht_ui[ti] = ui;
     order.reserve(ht.size());
     std::vector<uint8_t> is_reuse(ht.size(), 0);
     uint32_t n_sources = 0;
     {
-        std::vector<uint32_t> row(u1 - u0), tail, kept, early;
+        std::vector<uint32_t> row(n), tail, kept, early;
         for (uint32_t k = 0; k < max_rows; k++) {
             uint32_t m = 0;
-            for (uint32_t i = 0; i < u1 - u0; i++)
+            for (uint32_t i = 0; i < n; i++)
                 if (k < ht_begin[i + 1] - ht_begin[i]) row[m++] = i;
             std::sort(row.begin(), row.begin() + m, [&](uint32_t a, uint32_t b) {
                 const uint64_t ba = ht[ht_begin[a] + k].bound, bb = ht[ht_begin[b] + k].bound;
@@ -1495,18 +1449,17 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
     for (uint32_t c = 0; c < n_store; c++) region_off[c + 1] += region_off[c];
     if (region_off.back() >> 3 > 0xffffffffull) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "region store larger than 2^35 samples");
     if (n_store) {
-        PlanAlloc al{ctx, p};
+        PlanAlloc al{p, false};
         al.d_used = p->d_used;
         p->d_region_store = al.dev<int16_t>(region_off.back());
         p->d_region_state = al.dev<unsigned long long>(n_store);
         p->d_used = al.d_used;
-        if (al.err != cudaSuccess || (p->arena && p->d_used > p->arena->d_cap))
+        if (al.err != cudaSuccess)
             return fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "region store");
         CU(ctx, cudaMemsetAsync(p->d_region_state, 0, (size_t)n_store * 8, st));
     }
 
-    ch.task_begin = p->n_tasks;
-    uint32_t nt = p->n_tasks;
+    uint32_t nt = 0;
     for (uint32_t c = 0; c < canon_groups.size(); c++) {
         const uint32_t ti = groups[canon_groups[c]].first_task;
         const HostTask& h = ht[ti];
@@ -1524,22 +1477,22 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
         t.w_op = dd[ti].w_op - op0;
         p->h_tasks[nt++] = t;
     }
-    p->info.n_canon_tasks += (uint32_t)canon_groups.size();
-    std::vector<int32_t> last_index(u1 - u0, -1);
+    p->info.n_canon_tasks = n_canon;
+    std::vector<int32_t> last_index(n, -1);
     int build_rc = CTTS_GPU_OK;
     auto make_task = [&](uint32_t hti) {
-        const uint32_t ui = ht_ui[hti], u = u0 + ui;
-        const uint32_t k = hti - ht_begin[ui];
+        const uint32_t u = ht_ui[hti];
+        const uint32_t k = hti - ht_begin[u];
         const HostTask& h = ht[hti];
         ctts::RegionTask t{};
         t.utt = u;
         t.op_begin = h.op_begin - op0;
         t.op_end = h.op_end - op0;
         t.bound = (uint32_t)std::min<uint64_t>(h.bound, 0xffffffffull);
-        t.pred = last_index[ui];
+        t.pred = last_index[u];
         const bool stretched = p->pre_off[u] != ~0ull;
-        t.flags = (k + 1 == ht_begin[ui + 1] - ht_begin[ui] ? (uint32_t)ctts::TASK_LAST : 0u) | (stretched ? (uint32_t)ctts::TASK_TO_PRE : 0u);
-        if (h.bound > wcap) { t.flags |= ctts::TASK_GLOBAL; p->n_global_tasks++; }
+        t.flags = (k + 1 == ht_begin[u + 1] - ht_begin[u] ? (uint32_t)ctts::TASK_LAST : 0u) | (stretched ? (uint32_t)ctts::TASK_TO_PRE : 0u);
+        if (h.bound > wcap) { t.flags |= ctts::TASK_GLOBAL; p->info.n_global_tasks++; }
         t.dst_cap = stretched ? (uint32_t)p->pre_cap[u] : (uint32_t)(p->n_offsets[u + 1] - p->n_offsets[u]);
         t.dst_off = stretched ? p->pre_off[u] : p->n_offsets[u];
         t.big = 0xffffffffu;
@@ -1575,42 +1528,28 @@ int build_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, cudaStream_t st
     };
     for (size_t oi = 0; oi < order.size(); oi++) {
         p->h_tasks[nt] = make_task(order[oi]);
-        last_index[ht_ui[order[oi]]] = (int32_t)(nt - ch.task_begin);   // index inside this chunk's launch
+        last_index[ht_ui[order[oi]]] = (int32_t)nt;
         nt++;
     }
     if (build_rc) return build_rc;
-    ch.n_tasks = nt - ch.task_begin;
     p->n_tasks = nt;
-    ch.grid = (uint32_t)std::min<uint64_t>((uint64_t)p->occ * (uint64_t)ctx->sm_count, std::max<uint32_t>(ch.n_tasks, 1));
-
-    if (op_hi > op_lo)
-        CU(ctx, cudaMemcpyAsync(p->d_ops + (op_lo - op0), h_ops + (op_lo - op0), (size_t)(op_hi - op_lo) * sizeof(ctts_plan_op),
-                                cudaMemcpyHostToDevice, st));
-    if (ch.n_tasks)
-        CU(ctx, cudaMemcpyAsync(p->d_tasks + ch.task_begin, p->h_tasks + ch.task_begin, (size_t)ch.n_tasks * sizeof(ctts::RegionTask),
-                                cudaMemcpyHostToDevice, st));
-    p->built_chunks++;
-    p->info.n_tasks = p->n_tasks;
-    p->info.n_global_tasks = p->n_global_tasks;
-    p->info.gather_samples = p->gather;
-    p->info.grid = std::max(p->info.grid, ch.grid);
-    if (p->built_chunks == p->chunks.size()) {
-        p->src = nullptr;
-        if (!p->arena) {
-            // pageable staging must outlive the async copies
-            CU(ctx, cudaStreamSynchronize(st));
-            std::vector<ctts_plan_op>().swap(p->ops_vec);
-            std::vector<ctts::RegionTask>().swap(p->tasks_vec);
-        }
+    p->grid = (uint32_t)std::min<uint64_t>((uint64_t)p->occ * (uint64_t)ctx->sm_count, std::max<uint32_t>(nt, 1));
+    p->info.n_tasks = nt;
+    p->info.grid = p->grid;
+    if (n_ops) CU(ctx, cudaMemcpyAsync(p->d_ops, h_ops, (size_t)n_ops * sizeof(ctts_plan_op), cudaMemcpyHostToDevice, st));
+    if (nt) CU(ctx, cudaMemcpyAsync(p->d_tasks, p->h_tasks, (size_t)nt * sizeof(ctts::RegionTask), cudaMemcpyHostToDevice, st));
+    if (!p->arena) {
+        // pageable staging must outlive the async copies
+        CU(ctx, cudaStreamSynchronize(st));
+        std::vector<char>().swap(p->h_staging);
     }
     return CTTS_GPU_OK;
 }
 #undef CUP
 
-// Enqueue one chunk's assembly kernel on the context stream.
-int launch_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, int16_t* d_pcm_out, cudaStream_t st) {
-    const PlanChunk& ch = p->chunks[c];
-    if (ch.n_tasks == 0) return CTTS_GPU_OK;
+// Enqueue the plan's assembly kernel.
+int launch_assemble(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out, cudaStream_t st) {
+    if (p->n_tasks == 0) return CTTS_GPU_OK;
     ctts::AsmArgs a{};
     a.pool = p->np->d_pool;
     a.unit_meta = p->np->d_meta;
@@ -1625,8 +1564,8 @@ int launch_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, int16_t* d_pcm
     a.tab.hann512 = ctx->d_tables + 3328;
     a.tab.xfade4 = reinterpret_cast<const float4*>(ctx->d_tables + 3840);
     a.ops = p->d_ops;
-    a.tasks = p->d_tasks + ch.task_begin;
-    a.n_tasks = ch.n_tasks;
+    a.tasks = p->d_tasks;
+    a.n_tasks = p->n_tasks;
     a.dst_final = d_pcm_out;
     a.dst_pre = p->d_pre;
     a.out_counts = p->d_counts;
@@ -1636,14 +1575,14 @@ int launch_chunk(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, int16_t* d_pcm
     a.trim_scratch_words = p->trim_words;
     a.region_store = p->d_region_store;
     a.region_state = p->d_region_state;
-    a.chain = p->d_chain + ch.task_begin;
-    a.ticket = p->d_ticket + c;
+    a.chain = p->d_chain;
+    a.ticket = p->d_ticket;
     a.prof = p->d_prof;
     a.epoch = p->epoch;
     a.prm = p->prm;
     a.wcap = p->wcap;
     a.hcap = p->hcap;
-    ctts::assemble_kernel<<<ch.grid, ctts::ASM_THREADS, p->smem_bytes, st>>>(a);
+    ctts::assemble_kernel<<<p->grid, ctts::ASM_THREADS, p->smem_bytes, st>>>(a);
     CU(ctx, cudaGetLastError());
     return CTTS_GPU_OK;
 }
@@ -1653,20 +1592,19 @@ int begin_run(ctts_gpu_ctx* ctx, ctts_gpu_plan* p) {
     CU(ctx, cudaMemsetAsync(p->d_counts, 0, (size_t)p->n_utts * 4, st));
     CU(ctx, cudaMemsetAsync(p->d_pre_counts, 0, (size_t)p->n_utts * 4, st));
     CU(ctx, cudaMemsetAsync(p->d_err, 0, (size_t)p->n_utts * 4, st));
-    CU(ctx, cudaMemsetAsync(p->d_ticket, 0, p->chunks.size() * 4, st));
+    CU(ctx, cudaMemsetAsync(p->d_ticket, 0, 4, st));
     p->epoch++;
     if (p->epoch == 0) p->epoch = 1;   // (2^32 runs later) the chain words of the last lap are long gone
     return CTTS_GPU_OK;
 }
 
-// Enqueue the WSOLA kernels of one chunk's stretched utterances (after its assembly kernel).
-int launch_stretch(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, int16_t* d_pcm_out, cudaStream_t st) {
-    const PlanChunk& ch = p->chunks[c];
-    if (!ch.st_count) return CTTS_GPU_OK;
+// Enqueue the WSOLA kernels of the plan's stretched utterances (after its assembly kernel).
+int launch_stretch(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out, cudaStream_t st) {
+    const uint32_t ns = p->n_stretch;
+    if (!ns) return CTTS_GPU_OK;
     ctts::WsolaArgs w{};
     w.tasks = p->d_stasks;
-    w.n_tasks = p->n_stretch;
-    w.task_first = ch.st_begin;
+    w.n_tasks = ns;
     w.pre = p->d_pre;
     w.pre_counts = p->d_pre_counts;
     w.out = d_pcm_out;
@@ -1676,34 +1614,34 @@ int launch_stretch(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t c, int16_t* d_p
     w.first_bad = p->d_n_frames + 2 * (size_t)p->n_stretch;
     w.first_silent = p->d_n_frames + 3 * (size_t)p->n_stretch;
     w.tier2 = p->d_n_frames + 4 * (size_t)p->n_stretch;
-    w.task_count = ch.st_count;
+    w.task_count = ns;
     w.speculate = ctx->knobs.wsola_speculate ? 1u : 0u;
     w.force_bad = ctx->knobs.wsola_force_bad;
     w.hann512 = ctx->d_tables + 3328;
-    w.ola_block_task = p->d_ola_task + ch.ola_begin;
-    w.ola_block_first = p->d_ola_first + ch.ola_begin;
+    w.ola_block_task = p->d_ola_task;
+    w.ola_block_first = p->d_ola_first;
     // speculate (scan) -> verify every frame in parallel -> walk the chain only where that failed -> overlap-add
-    ctts::wsola_scan_kernel<<<(ch.st_count + 7) / 8, 256, 0, st>>>(w);
+    ctts::wsola_scan_kernel<<<(ns + 7) / 8, 256, 0, st>>>(w);
     CU(ctx, cudaGetLastError());
-    if (w.speculate && ch.verify_tiles) {
-        for (uint32_t t0 = 0; t0 < ch.st_count; t0 += 65535u) {   // grid.y limit
+    if (w.speculate && p->verify_tiles) {
+        for (uint32_t t0 = 0; t0 < ns; t0 += 65535u) {   // grid.y limit
             ctts::WsolaArgs wv = w;
-            wv.task_first = ch.st_begin + t0;
-            const dim3 grid(ch.verify_tiles, std::min<uint32_t>(ch.st_count - t0, 65535u));
+            wv.task_first = t0;
+            const dim3 grid(p->verify_tiles, std::min<uint32_t>(ns - t0, 65535u));
             ctts::wsola_verify_kernel<<<grid, ctts::WV_THREADS, sizeof(ctts::WvSmem), st>>>(wv);
             CU(ctx, cudaGetLastError());
         }
     }
-    ctts::wsola_search_kernel<<<ch.st_count, ctts::WS_THREADS, 0, st>>>(w);
+    ctts::wsola_search_kernel<<<ns, ctts::WS_THREADS, 0, st>>>(w);
     CU(ctx, cudaGetLastError());
-    if (ch.ola_count) {
-        ctts::wsola_ola_kernel<<<ch.ola_count, ctts::OLA_THREADS, 0, st>>>(w);
+    if (p->n_ola_blocks) {
+        ctts::wsola_ola_kernel<<<p->n_ola_blocks, ctts::OLA_THREADS, 0, st>>>(w);
         CU(ctx, cudaGetLastError());
     }
     return CTTS_GPU_OK;
 }
 
-// Enqueue the output-rate conversion of the whole plan (after the last chunk's kernels): native slots d_nat and
+// Enqueue the output-rate conversion of the plan (after its WSOLA kernels): native slots d_nat and
 // counts -> output-rate slots d_final and d_rs_counts.  Nothing at the native rate.
 int launch_resample(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const int16_t* d_nat, int16_t* d_final, cudaStream_t st) {
     const ctts_gpu_ctx::RsTable* rs = p->rs;
@@ -1738,7 +1676,7 @@ int ctts_gpu_plan_create(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const c
                          const uint64_t* out_offsets, ctts_gpu_plan** out) {
     ctts_gpu_plan* p = nullptr;
     int rc = prepare_plan(ctx, plan, params, out_offsets, nullptr, &p);
-    for (uint32_t c = 0; !rc && c < p->chunks.size(); c++) rc = build_chunk(ctx, p, c, ctx->stream);
+    if (!rc) rc = build_tasks(ctx, p, plan, ctx->stream);
     if (rc) {
         ctts_gpu_plan_destroy(p);
         return rc;
@@ -1779,10 +1717,8 @@ int ctts_gpu_plan_run(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out) {
         d_nat = p->d_nat_owned;
     }
     int rc = begin_run(ctx, p);
-    for (uint32_t c = 0; !rc && c < p->chunks.size(); c++) {
-        rc = launch_chunk(ctx, p, c, d_nat, ctx->stream);
-        if (!rc) rc = launch_stretch(ctx, p, c, d_nat, ctx->stream);
-    }
+    if (!rc) rc = launch_assemble(ctx, p, d_nat, ctx->stream);
+    if (!rc) rc = launch_stretch(ctx, p, d_nat, ctx->stream);
     if (!rc) rc = launch_resample(ctx, p, d_nat, d_pcm_out, ctx->stream);
     return rc;
 }
@@ -1993,10 +1929,10 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
     l.copy_pending = false;
     if (n) {
         rc = begin_run(ctx, p);
-        if (!rc) rc = build_chunk(ctx, p, 0, ctx->stream);
+        if (!rc) rc = build_tasks(ctx, p, piece, ctx->stream);
         const auto tp2 = std::chrono::steady_clock::now();
-        if (!rc) rc = launch_chunk(ctx, p, 0, l.d_out, ctx->stream);
-        if (!rc) rc = launch_stretch(ctx, p, 0, l.d_out, ctx->stream);
+        if (!rc) rc = launch_assemble(ctx, p, l.d_out, ctx->stream);
+        if (!rc) rc = launch_stretch(ctx, p, l.d_out, ctx->stream);
         if (!rc) rc = launch_resample(ctx, p, l.d_out, d_final, ctx->stream);
         if (rc) return bail(rc);
         if (ctx->knobs.trace) {
@@ -2100,6 +2036,29 @@ int enqueue_packed_copy(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l) {
     return CTTS_GPU_OK;
 }
 
+// Caller-defined slots: utterance u goes to pcm_out[off[u] ..), cap[u] samples of room.  The batch is cut into
+// pieces of about piece_samples samples of slot space: the device->host copy of one overlaps the kernels of the
+// next and the host-side compilation of the one after.
+int submit_slot_pieces(ctts_gpu_session* s, const ctts_batch_plan* plan, const uint64_t* off, const uint64_t* cap,
+                       uint32_t* out_counts) {
+    const uint32_t n = plan->n_utts;
+    int rc = CTTS_GPU_OK;
+    uint64_t acc = 0;
+    for (uint32_t u0 = 0, u = 0; u < n && !rc; u++) {
+        acc += cap[u];
+        if (acc >= s->ctx->knobs.piece_samples || u + 1 == n) {
+            ctts_batch_plan piece = *plan;
+            piece.n_utts = u + 1 - u0;
+            piece.utt_op_begin = plan->utt_op_begin + u0;
+            piece.speed = plan->speed + u0;
+            rc = submit_piece(s, &piece, off + u0, cap + u0, nullptr, out_counts + u0);
+            u0 = u + 1;
+            acc = 0;
+        }
+    }
+    return rc;
+}
+
 }  // namespace
 
 extern "C" {
@@ -2164,24 +2123,9 @@ int ctts_gpu_synth_batch_stream(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, 
     ctts_gpu_session* s = nullptr;
     int rc = ctts_gpu_session_begin(ctx, params, pcm_out, n ? out_offsets[n] : 0, on_chunk, user, &s);
     if (rc) return rc;
-    // pieces of about chunk_samples samples of slot space: the device->host copy of one overlaps the kernels of
-    // the next and the host-side compilation of the one after
     std::vector<uint64_t> cap(std::max<uint32_t>(n, 1));
     for (uint32_t u = 0; u < n; u++) cap[u] = out_offsets[u + 1] - out_offsets[u];
-    const uint64_t chunk = ctx->knobs.chunk_samples;
-    uint64_t acc = 0;
-    for (uint32_t u0 = 0, u = 0; u < n && !rc; u++) {
-        acc += cap[u];
-        if (acc >= chunk || u + 1 == n) {
-            ctts_batch_plan piece = *plan;
-            piece.n_utts = u + 1 - u0;
-            piece.utt_op_begin = plan->utt_op_begin + u0;
-            piece.speed = plan->speed + u0;
-            rc = submit_piece(s, &piece, out_offsets + u0, cap.data() + u0, nullptr, out_counts + u0);
-            u0 = u + 1;
-            acc = 0;
-        }
-    }
+    rc = submit_slot_pieces(s, plan, out_offsets, cap.data(), out_counts);
     const int rc_end = ctts_gpu_session_end(s, nullptr);
     return rc ? rc : rc_end;
 }
@@ -2201,10 +2145,10 @@ int ctts_gpu_synth_batch_packed(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, 
     ctts_gpu_session* s = nullptr;
     int rc = ctts_gpu_session_begin(ctx, params, pcm_out, capacity, nullptr, nullptr, &s);
     if (rc) return rc;
-    // pieces of about chunk_samples / 2400 utterances ... by ops: an op appends at most a few thousand samples, so
+    // pieces of about piece_samples / 2400 utterances ... by ops: an op appends at most a few thousand samples, so
     // cut by op count (no bounds are known before a piece is compiled): ~70 k ops ~ 192 sentences of 200 characters (measured: text -> PCM of a mixed-speed batch 105 ms with pieces of
     // 128, 97 with 192, 99 with 256; at speed 1.0 no difference)
-    const uint64_t ops_per_piece = std::max<uint64_t>(ctx->knobs.chunk_samples / 2800, 64);
+    const uint64_t ops_per_piece = std::max<uint64_t>(ctx->knobs.piece_samples / 2800, 64);
     for (uint32_t u0 = 0, u = 0; u < n && !rc; u++) {
         if (plan->utt_op_begin[u + 1] - plan->utt_op_begin[u0] >= ops_per_piece || u + 1 == n) {
             ctts_batch_plan piece = *plan;
@@ -2295,20 +2239,7 @@ int ctts_gpu_multi_synth_batch(ctts_gpu_ctx* const* ctxs, uint32_t n_ctx, const 
         ctts_gpu_session* s = nullptr;
         int rc = ctts_gpu_session_begin(ctx, params, pcm_out, out_offsets[n], nullptr, nullptr, &s);
         if (rc) { rcs[d] = rc; return; }
-        const uint64_t chunk = ctx->knobs.chunk_samples;
-        uint64_t acc = 0;
-        for (uint32_t i0 = 0, i = 0; i < m && !rc; i++) {
-            acc += cap[i];
-            if (acc >= chunk || i + 1 == m) {
-                ctts_batch_plan piece = sub;
-                piece.n_utts = i + 1 - i0;
-                piece.utt_op_begin = begin.data() + i0;
-                piece.speed = speed.data() + i0;
-                rc = submit_piece(s, &piece, off.data() + i0, cap.data() + i0, nullptr, counts.data() + i0);
-                i0 = i + 1;
-                acc = 0;
-            }
-        }
+        rc = submit_slot_pieces(s, &sub, off.data(), cap.data(), counts.data());
         const int rc_end = ctts_gpu_session_end(s, nullptr);
         rcs[d] = rc ? rc : rc_end;
         for (uint32_t i = 0; i < m; i++) out_counts[mine[i]] = counts[i];
