@@ -107,6 +107,9 @@ __device__ __forceinline__ void run_task(const Smem& sm, const AsmArgs& A, uint3
     // Second level: tasks that are equal as a whole (same canonical region, same WORD_END bit for bit, nothing but
     // fade-outs / pauses / marks behind it).  The first of them in ticket order (TASK_SOURCE) stores what it flushes in
     // the region store too, the others (TASK_REUSE) copy that and run nothing.
+    // Regions longer than the window (TASK_GLOBAL) take part as well: a canonical one is assembled in its region-store
+    // slot, an occurrence copies the store straight into its utterance slot and resumes there, a source copies what it
+    // appended to its slot into the store.
     // the task's ops, asynchronously (an op fetched from HBM per step would stall the whole CTA)
     {
         const uint32_t n_pref = min(task.op_end - task.op_begin, TASK_OPS_SMEM);
@@ -119,6 +122,11 @@ __device__ __forceinline__ void run_task(const Smem& sm, const AsmArgs& A, uint3
         s.dst = A.region_store + task.dst_off;
         s.have_base = true;
         s.base = CANON_BASE;
+        if (task.flags & TASK_GLOBAL) {   // in place in the region store: nothing reaches back (the plan compiler proves it)
+            s.in_smem = false;
+            s.w = s.dst;
+            s.cap = task.dst_cap;
+        }
     } else if (task.region != NO_REGION) {
         // One round trip for everything this task waits for: lane 0 the predecessor's chain word, lane 1 the
         // canonical region's state, lane 2 the shared whole task's (their producers hold smaller tickets: running or
@@ -145,32 +153,42 @@ __device__ __forceinline__ void run_task(const Smem& sm, const AsmArgs& A, uint3
         }
         if (s.base >= task.thresh) {
             const uint32_t len_whole = sm.bcast[4], len_region = sm.bcast[2];
+            const uint32_t cap = (task.flags & TASK_GLOBAL) ? NO_REGION : s.cap;   // TASK_GLOBAL: the slot's, checked below
             uint32_t len = NO_REGION;
             unsigned long long at = 0;
-            if (len_whole != NO_REGION && len_whole <= s.cap) {
+            if (len_whole != NO_REGION && len_whole <= cap) {
                 len = len_whole;
                 at = 8ull * task.whole_at;
                 k_first = task.op_end;
-            } else if (len_region != NO_REGION && len_region <= s.cap) {
+            } else if (len_region != NO_REGION && len_region <= cap) {
                 len = len_region;
                 at = 8ull * task.region_at;
                 k_first = task.w_op;
                 resumed = true;
             }
-            if (len != NO_REGION) {   // region store -> window (written by another CTA during this launch: L2, not the read-only path)
-                const int4* src = reinterpret_cast<const int4*>(A.region_store + at);
-                int4* dstw = reinterpret_cast<int4*>(sm.win);
-                for (uint32_t v = tid; v < (len + 7) >> 3; v += ASM_THREADS) cp_async16(dstw + v, src + v);
+            if (len != NO_REGION) {
                 s.cnt = len;
+                if (!(task.flags & TASK_GLOBAL)) {   // region store -> window (written by another CTA during this launch: L2, not the read-only path)
+                    const int4* src = reinterpret_cast<const int4*>(A.region_store + at);
+                    int4* dstw = reinterpret_cast<int4*>(sm.win);
+                    for (uint32_t v = tid; v < (len + 7) >> 3; v += ASM_THREADS) cp_async16(dstw + v, src + v);
+                }
             }
         }
     }
-    if (task.flags & TASK_GLOBAL) {
+    if ((task.flags & TASK_GLOBAL) && !canon) {
         // the region does not fit the shared window: assemble it in place in the HBM slot
         need_base(s, sm, A);
         s.in_smem = false;
         s.w = s.dst + s.base;
         s.cap = s.dst_cap > s.base ? s.dst_cap - s.base : 0u;
+        if (s.cnt > s.cap) {   // the stored samples do not fit the slot: assemble them, and fail, as without the store
+            s.cnt = 0;
+            k_first = task.op_begin;
+            resumed = false;
+        } else if (k_first != task.op_begin) {
+            copy_from_store(s.w, A.region_store + 8ull * (resumed ? task.region_at : task.whole_at), s.cnt);
+        }
         __threadfence();
     }
     cp_async_wait_all();
@@ -227,10 +245,11 @@ __device__ __forceinline__ void run_task(const Smem& sm, const AsmArgs& A, uint3
     }
 
     if (canon) {
-        // ---- the canonical region goes to the region store; a region that left the window (cannot happen for
-        //      regions the plan compiler accepts) or failed is marked unusable: its occurrences assemble themselves
-        const bool ok = !s.err && s.in_smem && s.cnt <= task.dst_cap;
-        if (ok) {
+        // ---- the canonical region goes to the region store (TASK_GLOBAL: it is there already); a region that left
+        //      the window (cannot happen for regions the plan compiler accepts) or failed is marked unusable: its
+        //      occurrences assemble themselves
+        const bool ok = !s.err && s.in_smem == !(task.flags & TASK_GLOBAL) && s.cnt <= task.dst_cap;
+        if (ok && s.in_smem) {
             const int4* srcw = reinterpret_cast<const int4*>(sm.win);
             int4* d = reinterpret_cast<int4*>(s.dst);
             for (uint32_t v = tid; v < (s.cnt + 7) >> 3; v += ASM_THREADS) d[v] = srcw[v];
@@ -242,8 +261,13 @@ __device__ __forceinline__ void run_task(const Smem& sm, const AsmArgs& A, uint3
     }
     if (task.flags & TASK_SOURCE) {
         // ---- what this task appends goes to the region store as well, unless it depends on more than the task's ops
-        const bool ok = resumed && sm.bcast[3] == 0u && !s.err && s.in_smem && s.cnt <= task.bound;
-        if (ok) {
+        //      (TASK_GLOBAL: from the utterance slot, where it was appended)
+        const bool global = (task.flags & TASK_GLOBAL) != 0;
+        const bool ok = resumed && sm.bcast[3] == 0u && !s.err && s.in_smem == !global && s.cnt <= task.bound;
+        if (ok && global) {
+            __syncthreads();   // every thread's last samples are in the slot
+            copy_to_store(A.region_store + 8ull * task.whole_at, s.dst + s.base, s.cnt);
+        } else if (ok) {
             const int4* srcw = reinterpret_cast<const int4*>(sm.win);
             int4* d = reinterpret_cast<int4*>(A.region_store + 8ull * task.whole_at);
             for (uint32_t v = tid; v < (s.cnt + 7) >> 3; v += ASM_THREADS) d[v] = srcw[v];

@@ -1018,8 +1018,11 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     layout(al);
     if (arena) {
         // + the region store, carved by build_tasks once the regions are known; reserved here at its upper bound:
-        // the canonical regions' slots and the shared whole tasks' (each <= half of all region samples, a slot per
-        // two tasks at most) + their tables
+        // the canonical regions' slots and the shared whole tasks' + their tables.  A slot takes up8(bound) + 8
+        // samples and every slot can be charged to a task of its own: a canonical region (a group of >= 2 tasks) to
+        // the task whose bound sizes it, a shared whole task (>= 2 tasks with equal ops, so equal bounds) to one of
+        // its tasks that is not that first task of the group.  So the slots hold at most the sum of the bounds +
+        // 16 samples per task, whatever the window (build_tasks still checks that the store fits the arena).
         const uint64_t pre_sum = std::accumulate(pre.begin(), pre.end(), (uint64_t)0);
         const size_t region_bytes = !ctx->knobs.region_dedup ? 0 :
             PlanAlloc::up256((pre_sum + 16 * (sc.n_regions + 2)) * sizeof(int16_t)) + 2 * PlanAlloc::up256((sc.n_regions + 2) * 8);
@@ -1200,7 +1203,8 @@ int build_tasks(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const ctts_batch_plan* plan
 
     // ---- word-region deduplication (run_task in assemble.cuh).  A task is ELIGIBLE when the window it holds on
     // reaching the contour of its first WORD_END is a function of the ops before it alone:
-    //   * no MARK before that WORD_END (the region starts with the task), the task fits the shared window;
+    //   * no MARK before that WORD_END (the region starts with the task), its silence mask fits the shared scratch
+    //     (a task longer than the window takes part as well: it is assembled / resumed in place, TASK_GLOBAL);
     //   * every join finds its crossfade / energy window min(xf, n) and its pitch-analysis window min(2 xf, n/2)
     //     inside the region (nothing reaches back into an earlier region), every live fade-out too;
     //   * the remaining count clamps (count >= 200, count / 2 >= analysis window, ctts.c:1983-1987) do not bind,
@@ -1224,10 +1228,10 @@ int build_tasks(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const ctts_batch_plan* plan
                 if (memcmp(&h_ops[a0 + i - op0], &h_ops[b0 + i - op0], 12) != 0) return false;
             return ((h_ops[a1 - op0].flags ^ h_ops[b1 - op0].flags) & CTTS_WE_TRIM) == 0;
         };
-        uint64_t why[4] = {0, 0, 0, 0}, why_bound[4] = {0, 0, 0, 0};   // trace: too big, reaches back / no WORD_END, (unused), eligible
+        uint64_t why[4] = {0, 0, 0, 0}, why_bound[4] = {0, 0, 0, 0};   // trace: mask beyond the scratch, reaches back / no WORD_END, (unused), eligible
         for (size_t ti = 0; ti < ht.size(); ti++) {
             const HostTask& h = ht[ti];
-            if (h.bound > wcap || h.region_max > scr_samples) { why[0]++; why_bound[0] += h.bound; continue; }
+            if (h.region_max > scr_samples) { why[0]++; why_bound[0] += h.bound; continue; }
             uint64_t cnt = 0, T = 0, hash = 1469598103934665603ull;
             bool ok = true, found = false;
             uint32_t k = h.op_begin;
@@ -1308,14 +1312,15 @@ int build_tasks(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const ctts_batch_plan* plan
                     if (groups[dd[ti].group].count < 2) { single++; single_bound += ht[ti].bound; }
                     else if (ti == ht_begin[ui] && dd[ti].thresh) { first++; first_bound += ht[ti].bound; }
                 }
-            fprintf(stderr, "ctts_gpu: region dedup, %zu tasks: too big %llu (%llu samples), not a function of their ops %llu (%llu), "
+            fprintf(stderr, "ctts_gpu: region dedup, %zu tasks: mask beyond the scratch %llu (%llu samples), not a function of their ops %llu (%llu), "
                             "eligible %llu (%llu) of which unique %llu (%llu), first of an utterance with clamps %llu (%llu)\n",
                     ht.size(), (unsigned long long)why[0], (unsigned long long)why_bound[0], (unsigned long long)why[1],
                     (unsigned long long)why_bound[1], (unsigned long long)why[3], (unsigned long long)why_bound[3],
                     (unsigned long long)single, (unsigned long long)single_bound, (unsigned long long)first, (unsigned long long)first_bound);
         }
     }
-    // canonical tasks: first in ticket order (an occurrence waits for a SMALLER ticket only), longest first
+    // canonical tasks: first in ticket order (an occurrence waits for a SMALLER ticket only), longest first (those
+    // longer than the window, the slowest, start first: their occurrences wait the least)
     std::vector<uint32_t> canon_groups;
     for (uint32_t gi = 0; gi < groups.size(); gi++)
         if (groups[gi].count >= 2) canon_groups.push_back(gi);
@@ -1468,7 +1473,7 @@ int build_tasks(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const ctts_batch_plan* plan
         t.op_end = dd[ti].w_op + 1 - op0;
         t.bound = (uint32_t)h.bound;
         t.pred = -1;
-        t.flags = ctts::TASK_CANON;
+        t.flags = ctts::TASK_CANON | (h.bound > wcap ? (uint32_t)ctts::TASK_GLOBAL : 0u);   // assembled in its slot
         t.dst_cap = (uint32_t)(region_off[c + 1] - region_off[c]);
         t.dst_off = region_off[c];
         t.big = 0xffffffffu;
