@@ -2,11 +2,12 @@
  * ctts_b200 -- the `ctts synth` command line (ctts.c:3970-4030) over the B200 back end, in the
  * reference's own language: plain C on top of the two C-ABI libraries, no Python, no CUDA headers.
  *
- *   ctts_b200 synth <database.db> "text" <output.wav> [speed] [rate]
- *   ctts_b200 synth-batch <database.db> <texts.tsv> <out_dir> [rate]     lines: speed<TAB>text
+ *   ctts_b200 synth <database.db> "text" <output.wav|output.flac> [speed] [rate]
+ *   ctts_b200 synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac]     lines: speed<TAB>text
  *
  * rate: output sample rate in Hz (default 22050, the voice's own; ctts_gpu_set_output_rate lists the others),
- * written into the WAV header.
+ * written into the WAV header.  An output name ending in ".flac", or synth-batch's "flac", writes lossless FLAC files
+ * encoded on the device (ctts_b200_synth_texts_flac) instead of 16-bit WAV.
  *
  * Like the reference it reads config.yaml and normalization.csv from the working directory
  * (ctts.c:3990, :3636), clamps the speed to [0.5, 2.0] (ctts.c:3976-3981) and takes default_speed
@@ -92,33 +93,60 @@ static int write_wav(const char* path, const int16_t* samples, size_t count, uin
     return fclose(f) == 0 ? 0 : -1;
 }
 
-/* N texts -> N PCM spans of one pinned buffer through ctts_b200_synth_texts (the front end's planner threads
- * feed the device piece by piece): *pcm (release with ctts_gpu_host_free), off[u] and cnt[u] (malloc'ed, n
- * entries each); stats may be NULL (2n: found, missing).  on_chunk (may be NULL) is called as soon as a range of
- * utterances is in host memory; it finds the three arrays through *pcm, *off, *cnt, which are set before the
- * device starts. */
-static int ctts_b200_synthesize_batch(engine* e, const char* const* texts, const float* speeds, uint32_t n,
-                                      int16_t** pcm, uint64_t** off, uint32_t** cnt, uint32_t* stats,
-                                      ctts_gpu_chunk_fn on_chunk, void* user) {
+/* N texts -> N PCM spans (or, with flac, N .flac files) of one pinned buffer through ctts_b200_synth_texts(_flac)
+ * (the front end's planner threads feed the device piece by piece): r->out (release with ctts_gpu_host_free),
+ * r->off[u], r->bytes[u] (FLAC: file sizes) and r->cnt[u] (malloc'ed, n entries each); stats may be NULL (2n: found,
+ * missing).  on_chunk (may be NULL) is called as soon as a range of utterances is in host memory; it finds the
+ * arrays through r, which is filled before the device starts. */
+typedef struct {
+    void* out;   /* int16_t PCM, or the FLAC files */
+    uint64_t* off;
+    uint32_t* bytes;
+    uint32_t* cnt;
+} batch_result;
+
+static void result_free(batch_result* r) {
+    ctts_gpu_host_free(r->out);
+    free(r->off);
+    free(r->bytes);
+    free(r->cnt);
+    memset(r, 0, sizeof *r);
+}
+
+static int ctts_b200_synthesize_batch(engine* e, const char* const* texts, const float* speeds, uint32_t n, int flac,
+                                      batch_result* r, uint32_t* stats, ctts_gpu_chunk_fn on_chunk, void* user) {
     int rc = 0;
-    const uint64_t cap = ctts_b200_capacity_hint_rate(e->front, texts, speeds, n, e->rate);   /* replaces the SampleBuffer growth policy */
-    *off = malloc(sizeof **off * ((size_t)n + 1));
-    *cnt = calloc(n ? n : 1, sizeof **cnt);
-    *pcm = ctts_gpu_host_alloc(sizeof(int16_t) * (cap ? cap : 8));
-    if (!*off || !*cnt || !*pcm) rc = CTTS_GPU_ERR_OUT_OF_MEMORY;
+    /* replaces the SampleBuffer growth policy */
+    const uint64_t cap = flac ? ctts_b200_capacity_hint_flac(e->front, texts, speeds, n, e->rate)
+                              : ctts_b200_capacity_hint_rate(e->front, texts, speeds, n, e->rate);
+    r->off = malloc(sizeof *r->off * ((size_t)n + 1));
+    r->bytes = calloc(n ? n : 1, sizeof *r->bytes);
+    r->cnt = calloc(n ? n : 1, sizeof *r->cnt);
+    r->out = ctts_gpu_host_alloc((flac ? 1 : sizeof(int16_t)) * (cap ? cap : 16));
+    if (!r->off || !r->bytes || !r->cnt || !r->out) rc = CTTS_GPU_ERR_OUT_OF_MEMORY;
     ctts_b200_options opt;
     memset(&opt, 0, sizeof opt);
     opt.on_piece = on_chunk;
     opt.user = user;
-    if (!rc) rc = ctts_b200_synth_texts(e->front, e->gpu, texts, speeds, n, *pcm, cap, *off, *cnt, stats, NULL, &opt, NULL);
+    if (!rc && flac) rc = ctts_b200_synth_texts_flac(e->front, e->gpu, texts, speeds, n, r->out, cap, r->off, r->bytes, r->cnt, stats, NULL, &opt, NULL);
+    else if (!rc) rc = ctts_b200_synth_texts(e->front, e->gpu, texts, speeds, n, r->out, cap, r->off, r->cnt, stats, NULL, &opt, NULL);
     if (rc) {
         fprintf(stderr, "synthesis failed: %d %s\n", rc, ctts_gpu_last_error(e->gpu));
-        ctts_gpu_host_free(*pcm);
-        free(*off);
-        free(*cnt);
-        *pcm = NULL; *off = NULL; *cnt = NULL;
+        result_free(r);
     }
     return rc;
+}
+
+static int write_flac(const char* path, const uint8_t* data, size_t bytes) {
+    FILE* f = fopen(path, "wb");
+    if (!f) return -1;
+    const int ok = fwrite(data, 1, bytes, f) == bytes;
+    return fclose(f) == 0 && ok ? 0 : -1;
+}
+
+static int ends_with(const char* s, const char* tail) {
+    const size_t a = strlen(s), b = strlen(tail);
+    return a >= b && strcmp(s + a - b, tail) == 0;
 }
 
 static float clamp_speed(float s) { return s < 0.5f ? 0.5f : s > 2.0f ? 2.0f : s; }
@@ -146,18 +174,17 @@ static int cmd_synth(int argc, char** argv) {
     if (argc <= 5 && e.cfg.default_speed != 1.0f) speed = e.cfg.default_speed;
     printf("Loaded database with %u units\n", ctts_front_unit_count(e.front));
     const char* texts[1] = {argv[3]};
-    int16_t* pcm;
-    uint64_t* off;
-    uint32_t *cnt, stats[2] = {0, 0};
-    if (ctts_b200_synthesize_batch(&e, texts, &speed, 1, &pcm, &off, &cnt, stats, NULL, NULL)) { engine_close(&e); return 1; }
-    printf("Synthesized %u samples (%.2f seconds)\n", cnt[0], (float)cnt[0] / (float)e.rate);
+    const int flac = ends_with(argv[4], ".flac");
+    batch_result r;
+    uint32_t stats[2] = {0, 0};
+    if (ctts_b200_synthesize_batch(&e, texts, &speed, 1, flac, &r, stats, NULL, NULL)) { engine_close(&e); return 1; }
+    printf("Synthesized %u samples (%.2f seconds)\n", r.cnt[0], (float)r.cnt[0] / (float)e.rate);
     printf("Units found: %u, missing: %u\n", stats[0], stats[1]);
-    int rc = write_wav(argv[4], pcm + off[0], cnt[0], e.rate);
-    if (rc) fprintf(stderr, "Failed to write WAV: %s\n", argv[4]);
+    int rc = flac ? write_flac(argv[4], (const uint8_t*)r.out + r.off[0], r.bytes[0])
+                  : write_wav(argv[4], (const int16_t*)r.out + r.off[0], r.cnt[0], e.rate);
+    if (rc) fprintf(stderr, "Failed to write %s: %s\n", flac ? "FLAC" : "WAV", argv[4]);
     else printf("Written to %s\n", argv[4]);
-    ctts_gpu_host_free(pcm);
-    free(off);
-    free(cnt);
+    result_free(&r);
     engine_close(&e);
     return rc ? 1 : 0;
 }
@@ -168,9 +195,8 @@ typedef struct {
     const char* dir;
     uint32_t rate;
     uint32_t base;   /* first utterance of the group being synthesised */
-    int16_t** pcm;
-    uint64_t** off;
-    uint32_t** cnt;
+    int flac;
+    const batch_result* r;
     double seconds;
     int rc;
 } wav_sink;
@@ -179,18 +205,20 @@ static void write_chunk(void* user, uint32_t u0, uint32_t u1) {
     wav_sink* w = user;
     for (uint32_t u = u0; u < u1 && !w->rc; u++) {
         char path[4096];
-        snprintf(path, sizeof path, "%s/%06u.wav", w->dir, w->base + u);
-        w->rc = write_wav(path, *w->pcm + (*w->off)[u], (*w->cnt)[u], w->rate);
-        w->seconds += (double)(*w->cnt)[u] / w->rate;
+        snprintf(path, sizeof path, "%s/%06u.%s", w->dir, w->base + u, w->flac ? "flac" : "wav");
+        w->rc = w->flac ? write_flac(path, (const uint8_t*)w->r->out + w->r->off[u], w->r->bytes[u])
+                        : write_wav(path, (const int16_t*)w->r->out + w->r->off[u], w->r->cnt[u], w->rate);
+        w->seconds += (double)w->r->cnt[u] / w->rate;
     }
 }
 
 static int cmd_synth_batch(int argc, char** argv) {
-    if (argc != 5 && argc != 6) {
-        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate]\n", argv[0]);
+    if (argc < 5 || argc > 7 || (argc == 7 && strcmp(argv[6], "flac") != 0)) {
+        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac]\n", argv[0]);
         return 1;
     }
     const uint32_t rate = argc > 5 ? parse_rate(argv[5]) : SAMPLE_RATE;
+    const int flac = argc == 7;
     FILE* f = fopen(argv[3], "rb");
     if (!f) { fprintf(stderr, "cannot read %s\n", argv[3]); return 1; }
     char** texts = NULL;
@@ -223,24 +251,20 @@ static int cmd_synth_batch(int argc, char** argv) {
         return 1;
     }
     if (mkdir(argv[4], 0777) != 0 && errno != EEXIST) { fprintf(stderr, "cannot create %s\n", argv[4]); engine_close(&e); return 1; }
-    int16_t* pcm;
-    uint64_t* off;
-    uint32_t* cnt;
-    wav_sink sink = {argv[4], e.rate, 0, &pcm, &off, &cnt, 0.0, 0};
+    batch_result r;
+    wav_sink sink = {argv[4], e.rate, 0, flac, &r, 0.0, 0};
     /* groups of 1024 utterances: the pinned buffer is sized from the texts alone (ctts_b200_capacity_hint) */
     int rc = 0;
     for (uint32_t g0 = 0; g0 < n && !rc; g0 += 1024) {
         const uint32_t gn = n - g0 < 1024 ? n - g0 : 1024;
         sink.base = g0;
-        rc = ctts_b200_synthesize_batch(&e, (const char* const*)texts + g0, speeds + g0, gn, &pcm, &off, &cnt, NULL, write_chunk, &sink);
+        rc = ctts_b200_synthesize_batch(&e, (const char* const*)texts + g0, speeds + g0, gn, flac, &r, NULL, write_chunk, &sink);
         if (!rc) {
             rc = sink.rc;
-            ctts_gpu_host_free(pcm);
-            free(off);
-            free(cnt);
+            result_free(&r);
         }
     }
-    if (rc) fprintf(stderr, "Failed to write WAV files into %s\n", argv[4]);
+    if (rc) fprintf(stderr, "Failed to write %s files into %s\n", flac ? "FLAC" : "WAV", argv[4]);
     else printf("Synthesized %u utterances (%.1f seconds of audio) into %s\n", n, sink.seconds, argv[4]);
     for (uint32_t u = 0; u < n; u++) free(texts[u]);
     free(texts);
@@ -252,7 +276,7 @@ static int cmd_synth_batch(int argc, char** argv) {
 int main(int argc, char** argv) {
     if (argc >= 2 && strcmp(argv[1], "synth") == 0) return cmd_synth(argc, argv);
     if (argc >= 2 && strcmp(argv[1], "synth-batch") == 0) return cmd_synth_batch(argc, argv);
-    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed] [rate]\n       %s synth-batch <database.db> <texts.tsv> <out_dir> [rate]\n",
+    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav|output.flac> [speed] [rate]\n       %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac]\n",
             argv[0], argv[0]);
     return 1;
 }

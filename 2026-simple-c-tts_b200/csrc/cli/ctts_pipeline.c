@@ -300,7 +300,9 @@ static uint32_t gcd_u32(uint32_t a, uint32_t b) {
     return a;
 }
 
-uint64_t ctts_b200_capacity_hint_rate(ctts_front* front, const char* const* texts, const float* speeds, uint32_t n, uint32_t hz) {
+/* the capacity hint of every utterance at output rate hz, in samples (flac == 0) or in bytes of its FLAC file
+ * (ctts_gpu_flac_bound, rounded up to 16) */
+static uint64_t capacity_hint(ctts_front* front, const char* const* texts, const float* speeds, uint32_t n, uint32_t hz, int flac) {
     if (!front || (n && !texts) || hz == 0) return 0;
     const uint32_t g = gcd_u32(CTTS_PLAN_SAMPLE_RATE, hz), L = hz / g, M = CTTS_PLAN_SAMPLE_RATE / g;
     /* every character yields at most one unit or one pause; pauses are shorter than the longest unit for
@@ -315,16 +317,26 @@ uint64_t ctts_b200_capacity_hint_rate(ctts_front* front, const char* const* text
         uint64_t s = chars * per_char;
         if (speeds && speeds[u] < 1.0f) s *= 2;   /* hop = 128 / speed <= 256 */
         s += 1024;
-        total += L == M ? s : (s * L + M - 1) / M + 8;   /* ceil(n L / M) at the output rate, rounded up to 8 */
+        s = L == M ? s : (s * L + M - 1) / M + 8;   /* ceil(n L / M) at the output rate, rounded up to 8 */
+        total += flac ? (ctts_gpu_flac_bound(s) + 15) & ~15ull : s;
     }
     return total;
 }
 
-int ctts_b200_synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* const* texts, const float* speeds,
-                          uint32_t n, int16_t* pcm_out, uint64_t capacity, uint64_t* out_offsets,
-                          uint32_t* out_counts, uint32_t* stats, uint64_t* samples_used,
-                          const ctts_b200_options* opt, ctts_b200_timing* timing) {
-    if (!front || !gpu || (n && (!texts || !out_offsets || !out_counts))) return CTTS_GPU_ERR_INVALID_ARG;
+uint64_t ctts_b200_capacity_hint_rate(ctts_front* front, const char* const* texts, const float* speeds, uint32_t n, uint32_t hz) {
+    return capacity_hint(front, texts, speeds, n, hz, 0);
+}
+
+uint64_t ctts_b200_capacity_hint_flac(ctts_front* front, const char* const* texts, const float* speeds, uint32_t n, uint32_t hz) {
+    return capacity_hint(front, texts, speeds, n, hz, 1);
+}
+
+/* ctts_b200_synth_texts and ctts_b200_synth_texts_flac: the same pipeline over a PCM or a FLAC session */
+static int synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* const* texts, const float* speeds, uint32_t n,
+                       int flac, int16_t* pcm_out, uint8_t* flac_out, uint64_t capacity, uint64_t* out_offsets, uint32_t* out_bytes,
+                       uint32_t* out_counts, uint32_t* stats, uint64_t* used, const ctts_b200_options* opt,
+                       ctts_b200_timing* timing) {
+    if (!front || !gpu || (n && (!texts || !out_offsets || !out_counts || (flac && !out_bytes)))) return CTTS_GPU_ERR_INVALID_ARG;
     pipeline P;
     memset(&P, 0, sizeof P);
     P.front = front;
@@ -350,7 +362,8 @@ int ctts_b200_synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* cons
     ctts_assembly_params prm;
     ctts_front_params(front, &prm);
     ctts_gpu_session* ses = NULL;
-    int rc = ctts_gpu_session_begin(gpu, &prm, pcm_out, capacity, opt ? opt->on_piece : NULL, opt ? opt->user : NULL, &ses);
+    int rc = flac ? ctts_gpu_session_begin_flac(gpu, &prm, flac_out, capacity, opt ? opt->on_piece : NULL, opt ? opt->user : NULL, &ses)
+                      : ctts_gpu_session_begin(gpu, &prm, pcm_out, capacity, opt ? opt->on_piece : NULL, opt ? opt->user : NULL, &ses);
     if (rc) {
         free(P.piece_begin);
         return rc;
@@ -437,7 +450,8 @@ int ctts_b200_synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* cons
             joined.ops = j_ops;
             piece = &joined;
         }
-        rc = ctts_gpu_session_submit(ses, piece, out_offsets + u0, out_counts + u0);
+        rc = flac ? ctts_gpu_session_submit_flac(ses, piece, out_offsets + u0, out_bytes + u0, out_counts + u0)
+                      : ctts_gpu_session_submit(ses, piece, out_offsets + u0, out_counts + u0);
         for (uint32_t k = i; k < j; k++) {
             ctts_front_plan_free(&P.slots[k].plan);   /* the session keeps nothing of the plan */
             P.slots[k].state = 2;
@@ -460,7 +474,7 @@ int ctts_b200_synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* cons
     for (uint32_t t = 0; t < started; t++) pthread_join(tids[t], NULL);
     for (uint32_t i = 0; i < P.n_pieces; i++)
         if (P.slots[i].state == 1) ctts_front_plan_free(&P.slots[i].plan);
-    const int rc_end = ctts_gpu_session_end(ses, samples_used);
+    const int rc_end = ctts_gpu_session_end(ses, used);
     if (!rc) rc = rc_end;
     if (timing) {
         timing->first_plan_s = P.first_plan_s;
@@ -477,4 +491,20 @@ int ctts_b200_synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* cons
     free(tids);
     free(P.piece_begin);
     return rc;
+}
+
+int ctts_b200_synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* const* texts, const float* speeds,
+                          uint32_t n, int16_t* pcm_out, uint64_t capacity, uint64_t* out_offsets,
+                          uint32_t* out_counts, uint32_t* stats, uint64_t* samples_used,
+                          const ctts_b200_options* opt, ctts_b200_timing* timing) {
+    return synth_texts(front, gpu, texts, speeds, n, 0, pcm_out, NULL, capacity, out_offsets, NULL, out_counts, stats,
+                       samples_used, opt, timing);
+}
+
+int ctts_b200_synth_texts_flac(ctts_front* front, ctts_gpu_ctx* gpu, const char* const* texts, const float* speeds,
+                               uint32_t n, uint8_t* out, uint64_t capacity_bytes, uint64_t* out_offsets,
+                               uint32_t* out_bytes, uint32_t* out_counts, uint32_t* stats, uint64_t* bytes_used,
+                               const ctts_b200_options* opt, ctts_b200_timing* timing) {
+    return synth_texts(front, gpu, texts, speeds, n, 1, NULL, out, capacity_bytes, out_offsets, out_bytes,
+                       out_counts, stats, bytes_used, opt, timing);
 }

@@ -22,6 +22,7 @@
 #include "assemble.cuh"
 #include "wsola.cuh"
 #include "resample.cuh"
+#include "flac.cuh"
 
 extern "C" void ctts_host_tables(float* fade_out, float* fade_in, float* sine, float* hann256,
                                  float* hann512);
@@ -162,12 +163,20 @@ struct ctts_gpu_ctx {
         uint64_t d_pack_cap = 0;
         unsigned long long* d_pack_off = nullptr;   // n + 1 (+ the n + 1 slot offsets behind them)
         size_t d_pack_off_cap = 0;
-        uint32_t* h_res = nullptr;         // pinned: counts [n], then device error flags [n], then (8-byte aligned) slot offsets [n + 1]
+        uint8_t* d_flac = nullptr;         // FLAC sessions: the utterances' files back to back (DESIGN.md 3.5)
+        uint64_t d_flac_cap = 0;           // bytes
+        ctts::FlacFrame* d_frames = nullptr;   // FLAC sessions: one descriptor per frame a slot can hold
+        uint64_t d_frames_cap = 0;         // bytes
+        uint32_t* d_flac_info = nullptr;   // FLAC sessions: per utterance file bytes, min and max frame bytes
+        uint64_t d_flac_info_cap = 0;      // bytes
+        uint32_t* h_res = nullptr;         // pinned: counts [n], then device error flags [n], (FLAC: file bytes [n],) then
+                                           // (8-byte aligned) slot offsets [n + 1] (FLAC: and frame bases [n + 1])
         size_t h_res_cap = 0;              // in 4-byte words
         cudaEvent_t kernels_done = nullptr, counts_ready = nullptr, copied = nullptr;
         ctts_gpu_plan* plan = nullptr;     // piece in flight
         uint32_t* user_counts = nullptr;   // where its counts go
         uint64_t* user_offsets = nullptr;  // packed mode: where its offsets go
+        uint32_t* user_bytes = nullptr;    // FLAC sessions: where its file sizes go
         bool copy_pending = false;         // packed mode: the PCM copy is enqueued once the counts are on the host
         uint32_t utt_base = 0, n = 0;      // its utterances in the session's numbering
         bool busy = false;
@@ -538,6 +547,9 @@ void ctts_gpu_free(ctts_gpu_ctx* ctx) {
         cudaFree(l.d_rs);
         cudaFree(l.d_pack);
         cudaFree(l.d_pack_off);
+        cudaFree(l.d_flac);
+        cudaFree(l.d_frames);
+        cudaFree(l.d_flac_info);
         if (l.h_res) cudaFreeHost(l.h_res);
         if (l.kernels_done) cudaEventDestroy(l.kernels_done);
         if (l.counts_ready) cudaEventDestroy(l.counts_ready);
@@ -1791,6 +1803,8 @@ struct ctts_gpu_session {
     ctts_gpu_ctx* ctx = nullptr;
     ctts_assembly_params prm{};
     int16_t* pcm_out = nullptr;
+    uint8_t* flac_out = nullptr;  // FLAC session: the files go here, and capacity and cursor count bytes
+    bool flac = false;
     uint64_t capacity = 0;        // samples
     uint64_t cursor = 0;          // next free sample (library-chosen layout)
     uint32_t submitted = 0, harvested = 0;   // pieces
@@ -1799,7 +1813,7 @@ struct ctts_gpu_session {
     ctts_gpu_chunk_fn on_piece = nullptr;
     void* user = nullptr;
     int error = 0;
-    uint64_t d2h_samples = 0;     // samples copied to the host
+    uint64_t d2h_samples = 0;     // samples (FLAC: bytes) copied to the host
     std::chrono::steady_clock::time_point t0;
 };
 
@@ -1843,6 +1857,7 @@ int harvest_one(ctts_gpu_session* s) {
         const uint32_t* h_cnt = l.h_res;
         const uint32_t* h_err = l.h_res + l.n;
         if (l.user_counts) memcpy(l.user_counts, h_cnt, (size_t)l.n * 4);
+        if (l.user_bytes) memcpy(l.user_bytes, l.h_res + 2 * (size_t)l.n, (size_t)l.n * 4);
         for (uint32_t u = 0; u < l.n && !rc; u++)
             if (h_err[u]) rc = fail(ctx, CTTS_GPU_ERR_DEVICE, "utterance %u: device error %u", l.utt_base + u, h_err[u]);
     }
@@ -1864,8 +1879,9 @@ int harvest_one(ctts_gpu_session* s) {
 // One piece: compile, launch, copy.  Utterance i of the piece is delivered to pcm_out[slot_off[i] ..),
 // slot_cap[i] samples of room (>= its bound); slot_off == nullptr: the library appends packed slots at the
 // session's cursor and reports them through offsets_out.  Asynchronous: returns once everything is enqueued.
+// A FLAC session (packed only) encodes every utterance into a file instead and reports the sizes through out_bytes.
 int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64_t* slot_off, const uint64_t* slot_cap,
-                 uint64_t* offsets_out, uint32_t* out_counts) {
+                 uint64_t* offsets_out, uint32_t* out_counts, uint32_t* out_bytes = nullptr) {
     ctts_gpu_ctx* ctx = s->ctx;
     const uint32_t n = piece->n_utts;
     ctts_gpu_ctx::Lane& l = ctx->lane[s->submitted % ctts_gpu_ctx::kLanes];
@@ -1903,9 +1919,35 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
     };
     if ((rc = grow(&l.d_out, &l.d_out_cap, p->n_offsets[n])) != 0) return bail(rc);
     if (p->rs && (rc = grow(&l.d_rs, &l.d_rs_cap, total)) != 0) return bail(rc);
-    if (packed && (rc = grow(&l.d_pack, &l.d_pack_cap, total)) != 0) return bail(rc);
+    const bool flac = s->flac;
+    if (packed && !flac && (rc = grow(&l.d_pack, &l.d_pack_cap, total)) != 0) return bail(rc);
+    // FLAC: the files and the frame descriptors are sized by the slots (>= the bounds): ctts_gpu_flac_bound each
+    uint64_t flac_bytes = 0, n_frames = 0, max_frames = 1;
+    for (uint32_t u = 0; u < n && flac; u++) {
+        const uint64_t frames = (p->offsets[u + 1] - p->offsets[u] + ctts::FLAC_BLOCK - 1) / ctts::FLAC_BLOCK;
+        flac_bytes += (ctts_gpu_flac_bound(p->offsets[u + 1] - p->offsets[u]) + 15) & ~15ull;
+        n_frames += frames;
+        max_frames = std::max(max_frames, frames);
+    }
+    auto grow_raw = [&](void** buf, uint64_t* cap_now, uint64_t bytes, const char* what) -> int {
+        if (bytes <= *cap_now) return 0;
+        cudaFree(*buf);
+        *buf = nullptr;
+        *cap_now = 0;
+        const uint64_t cap = std::max<uint64_t>(bytes + bytes / 8, 64);
+        if (cudaMalloc(buf, cap) != cudaSuccess) return fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "%s of %llu bytes", what, (unsigned long long)cap);
+        *cap_now = cap;
+        return 0;
+    };
+    if (flac) {
+        if ((rc = grow_raw(reinterpret_cast<void**>(&l.d_flac), &l.d_flac_cap, flac_bytes, "FLAC output")) != 0) return bail(rc);
+        if ((rc = grow_raw(reinterpret_cast<void**>(&l.d_frames), &l.d_frames_cap, n_frames * sizeof(ctts::FlacFrame), "FLAC frames")) != 0) return bail(rc);
+        if ((rc = grow_raw(reinterpret_cast<void**>(&l.d_flac_info), &l.d_flac_info_cap, 3 * (uint64_t)n * 4, "FLAC sizes")) != 0) return bail(rc);
+    }
     int16_t* const d_final = p->rs ? l.d_rs : l.d_out;   // the slots callers see
-    const size_t res_words = 2 * (size_t)n + 2 + 2 * ((size_t)n + 1);   // counts, flags, (aligned) slot offsets
+    // h_res: counts, flags (, FLAC: file bytes), then 8-byte aligned: slot offsets (, FLAC: frame bases)
+    const size_t res_head = ((flac ? 3 : 2) * (size_t)n + 1) & ~(size_t)1;
+    const size_t res_words = res_head + 2 + (flac ? 4 : 2) * ((size_t)n + 1);
     if (res_words > l.h_res_cap) {
         if (l.h_res) cudaFreeHost(l.h_res);
         l.h_res = nullptr;
@@ -1915,11 +1957,12 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
             return bail(fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "pinned counts"));
         l.h_res_cap = cap;
     }
-    if (packed && 2 * ((size_t)n + 1) > l.d_pack_off_cap) {
+    const size_t off_words = (flac ? 3 : 2) * ((size_t)n + 1);   // packed offsets, slot offsets (, FLAC: frame bases)
+    if (packed && off_words > l.d_pack_off_cap) {
         cudaFree(l.d_pack_off);
         l.d_pack_off = nullptr;
         l.d_pack_off_cap = 0;
-        const size_t cap = 2 * ((size_t)n + 1) + 4096;
+        const size_t cap = off_words + 4096;
         if (cudaMalloc(reinterpret_cast<void**>(&l.d_pack_off), cap * 8) != cudaSuccess)
             return bail(fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "pack offsets"));
         l.d_pack_off_cap = cap;
@@ -1949,11 +1992,32 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
         if (packed) {
             // device prefix sum of the counts -> packed positions -> gather; the scan kernel also stores counts
             // and flags into page-locked host memory, and the PCM copy is enqueued once they are here
-            unsigned long long* h_slot = reinterpret_cast<unsigned long long*>(l.h_res + ((2 * (size_t)n + 1) & ~(size_t)1));
+            unsigned long long* h_slot = reinterpret_cast<unsigned long long*>(l.h_res + res_head);
             for (uint32_t u = 0; u <= n; u++) h_slot[u] = p->offsets[u];
+            for (uint32_t u = 0, fb = 0; u <= n && flac; u++) {   // first frame descriptor of every utterance
+                h_slot[n + 1 + u] = fb;
+                if (u < n) fb += (uint32_t)((p->offsets[u + 1] - p->offsets[u] + ctts::FLAC_BLOCK - 1) / ctts::FLAC_BLOCK);
+            }
             unsigned long long* d_slot = l.d_pack_off + (n + 1);
-            e = cudaMemcpyAsync(d_slot, h_slot, ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream);
-            if (e == cudaSuccess) {
+            e = cudaMemcpyAsync(d_slot, h_slot, (flac ? 2 : 1) * ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream);
+            if (e == cudaSuccess && flac) {
+                // analyse every frame -> sizes and packed byte offsets (counts, flags and sizes into h_res) -> emit
+                const ctts::FlacArgs fa{d_final, d_slot, p->d_final_counts, d_slot + (n + 1), l.d_frames, l.d_pack_off,
+                                        l.d_flac_info, l.d_flac, p->rs ? p->rs->hz : (uint32_t)CTTS_PLAN_SAMPLE_RATE};
+                for (uint32_t u0 = 0; u0 < n && e == cudaSuccess; u0 += 65535u) {   // grid.y limit
+                    ctts::flac_analyze_kernel<<<dim3((unsigned)max_frames, std::min<uint32_t>(n - u0, 65535u)), ctts::FLAC_THREADS, 0, ctx->stream>>>(fa, u0);
+                    e = cudaGetLastError();
+                }
+                if (e == cudaSuccess) {
+                    ctts::flac_scan_kernel<<<1, 1024, 0, ctx->stream>>>(fa, p->d_err, n, l.h_res);
+                    e = cudaGetLastError();
+                }
+                if (e == cudaSuccess) e = cudaEventRecord(l.counts_ready, ctx->stream);   // counts, flags and sizes are on the host
+                for (uint32_t u0 = 0; u0 < n && e == cudaSuccess; u0 += 65535u) {
+                    ctts::flac_emit_kernel<<<dim3((unsigned)max_frames, std::min<uint32_t>(n - u0, 65535u)), ctts::FLAC_THREADS, 0, ctx->stream>>>(fa, u0);
+                    e = cudaGetLastError();
+                }
+            } else if (e == cudaSuccess) {
                 ctts::pack_scan_kernel<<<1, 1024, 0, ctx->stream>>>(p->d_final_counts, p->d_err, n, l.d_pack_off, l.h_res);
                 e = cudaGetLastError();
                 if (e == cudaSuccess) e = cudaEventRecord(l.counts_ready, ctx->stream);   // counts and flags are on the host
@@ -1994,6 +2058,7 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
     l.plan = p;
     l.user_counts = out_counts;
     l.user_offsets = offsets_out;
+    l.user_bytes = out_bytes;
     l.utt_base = s->utts;
     l.n = n;
     l.busy = true;
@@ -2019,18 +2084,21 @@ int enqueue_packed_copy(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l) {
         return s->error;
     }
     const uint32_t* h_cnt = l.h_res;
+    const uint32_t* h_bytes = l.h_res + 2 * (size_t)l.n;   // FLAC: file sizes
     uint64_t o = s->cursor;
     for (uint32_t u = 0; u < l.n; u++) {
         if (l.user_offsets) l.user_offsets[u] = o;
-        o += up8(h_cnt[u]);
+        o += s->flac ? (h_bytes[u] + 15ull) & ~15ull : up8(h_cnt[u]);
     }
     const uint64_t len = o - s->cursor;
     if (o > s->capacity) {
         if (!s->error)
-            s->error = fail(ctx, CTTS_GPU_ERR_BOUNDS, "output buffer too small: %llu samples needed up to utterance %u", (unsigned long long)o, l.utt_base + l.n);
+            s->error = fail(ctx, CTTS_GPU_ERR_BOUNDS, "output buffer too small: %llu %s needed up to utterance %u", (unsigned long long)o,
+                            s->flac ? "bytes" : "samples", l.utt_base + l.n);
         return s->error;
     }
-    if (len) e = cudaMemcpyAsync(s->pcm_out + s->cursor, l.d_pack, len * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
+    if (len && s->flac) e = cudaMemcpyAsync(s->flac_out + s->cursor, l.d_flac, len, cudaMemcpyDeviceToHost, ctx->copy_stream);
+    else if (len) e = cudaMemcpyAsync(s->pcm_out + s->cursor, l.d_pack, len * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
     if (e == cudaSuccess) e = cudaEventRecord(l.copied, ctx->copy_stream);
     if (e != cudaSuccess) {
         if (!s->error) s->error = fail(ctx, CTTS_GPU_ERR_CUDA, "D2H: %s", cudaGetErrorString(e));
@@ -2090,10 +2158,36 @@ int ctts_gpu_session_begin(ctts_gpu_ctx* ctx, const ctts_assembly_params* params
 
 int ctts_gpu_session_submit(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets, uint32_t* out_counts) {
     if (!s || !piece || !out_counts || (piece->n_utts && !out_offsets)) return CTTS_GPU_ERR_INVALID_ARG;
+    if (s->flac) return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, "a FLAC session takes ctts_gpu_session_submit_flac");
     if (s->error) return s->error;
     ctts_gpu_ctx* ctx = s->ctx;
     CU(ctx, cudaSetDevice(ctx->device));
     return submit_piece(s, piece, nullptr, nullptr, out_offsets, out_counts);
+}
+
+uint64_t ctts_gpu_flac_bound(uint64_t samples) {
+    return ctts::FLAC_HEADER_BYTES + (samples + ctts::FLAC_BLOCK - 1) / ctts::FLAC_BLOCK * ctts::FLAC_FRAME_MAX;
+}
+
+int ctts_gpu_session_begin_flac(ctts_gpu_ctx* ctx, const ctts_assembly_params* params, uint8_t* out, uint64_t capacity_bytes,
+                                ctts_gpu_chunk_fn on_piece, void* user, ctts_gpu_session** s) {
+    if (capacity_bytes && !out) return CTTS_GPU_ERR_INVALID_ARG;
+    const int rc = ctts_gpu_session_begin(ctx, params, nullptr, 0, on_piece, user, s);
+    if (rc) return rc;
+    (*s)->flac = true;
+    (*s)->flac_out = out;
+    (*s)->capacity = capacity_bytes;
+    return CTTS_GPU_OK;
+}
+
+int ctts_gpu_session_submit_flac(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets, uint32_t* out_bytes,
+                                 uint32_t* out_counts) {
+    if (!s || !piece || (piece->n_utts && (!out_offsets || !out_bytes || !out_counts))) return CTTS_GPU_ERR_INVALID_ARG;
+    if (!s->flac) return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, "a PCM session takes ctts_gpu_session_submit");
+    if (s->error) return s->error;
+    ctts_gpu_ctx* ctx = s->ctx;
+    CU(ctx, cudaSetDevice(ctx->device));
+    return submit_piece(s, piece, nullptr, nullptr, out_offsets, out_counts, out_bytes);
 }
 
 int ctts_gpu_session_end(ctts_gpu_session* s, uint64_t* samples_used) {
@@ -2104,7 +2198,7 @@ int ctts_gpu_session_end(ctts_gpu_session* s, uint64_t* samples_used) {
     if (samples_used) *samples_used = s->cursor;
     if (ctx->knobs.trace)
         fprintf(stderr, "ctts_gpu session: %u utterances in %u pieces, %.1f MB to the host, %.1f ms\n", s->utts, s->submitted,
-                2e-6 * (double)s->d2h_samples, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - s->t0).count());
+                (s->flac ? 1e-6 : 2e-6) * (double)s->d2h_samples, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - s->t0).count());
     const int rc = s->error;
     ctx->session = nullptr;
     delete s;

@@ -72,6 +72,10 @@ def lib(build: bool = True) -> C.CDLL:
         L.ctts_gpu_session_begin.argtypes = [vp, C.POINTER(AssemblyParams), vp, C.c_uint64, vp, vp, C.POINTER(vp)]
         L.ctts_gpu_session_submit.argtypes = [vp, C.POINTER(CBatchPlan), vp, vp]
         L.ctts_gpu_session_end.argtypes = [vp, u64p]
+        L.ctts_gpu_session_begin_flac.argtypes = [vp, C.POINTER(AssemblyParams), vp, C.c_uint64, vp, vp, C.POINTER(vp)]
+        L.ctts_gpu_session_submit_flac.argtypes = [vp, C.POINTER(CBatchPlan), vp, vp, vp]
+        L.ctts_gpu_flac_bound.argtypes = [C.c_uint64]
+        L.ctts_gpu_flac_bound.restype = C.c_uint64
         L.ctts_gpu_synth_batch_packed.argtypes = [vp, C.POINTER(CBatchPlan), C.POINTER(AssemblyParams), vp, C.c_uint64, vp, vp, u64p]
         L.ctts_gpu_multi_synth_batch.argtypes = [C.POINTER(vp), C.c_uint32, C.POINTER(CBatchPlan), C.POINTER(AssemblyParams),
                                                  vp, vp, vp, vp]
@@ -278,6 +282,34 @@ class GpuSynth:
         rc_end = L.ctts_gpu_session_end(h, C.byref(used))
         self._check(rc or rc_end)
         return off[:n], cnt[:n]
+
+    def synth_pieces_flac(self, pieces: list[BatchPlan], params: AssemblyParams, out: np.ndarray):
+        """A FLAC session fed with the given plans, one piece each (ctts_gpu_session_begin_flac / _submit_flac): every
+        utterance becomes one .flac file in the uint8 buffer `out`.  Returns (byte offsets, file bytes, sample counts,
+        bytes used) over all utterances of all pieces, in order."""
+        assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
+        L = lib()
+        h = C.c_void_p()
+        self._check(L.ctts_gpu_session_begin_flac(self._h, C.byref(params), out.ctypes.data, out.size, None, None, C.byref(h)))
+        n = sum(p.n_utts for p in pieces)
+        off = np.zeros(max(n, 1), dtype=np.uint64)
+        nbytes = np.zeros(max(n, 1), dtype=np.uint32)
+        cnt = np.zeros(max(n, 1), dtype=np.uint32)
+        at, rc = 0, 0
+        for p in pieces:
+            cp = p.as_c()
+            rc = L.ctts_gpu_session_submit_flac(h, C.byref(cp), off[at:].ctypes.data, nbytes[at:].ctypes.data, cnt[at:].ctypes.data)
+            if rc:
+                break
+            at += p.n_utts
+        used = C.c_uint64()
+        rc_end = L.ctts_gpu_session_end(h, C.byref(used))
+        self._check(rc or rc_end)
+        return off[:n], nbytes[:n], cnt[:n], int(used.value)
+
+    def flac_bound(self, plan: BatchPlan) -> int:
+        """Bytes that are always enough for a FLAC session over the plan: ctts_gpu_flac_bound of every bound, rounded up to 16."""
+        return sum((int(lib().ctts_gpu_flac_bound(int(b))) + 15) // 16 * 16 for b in self.bounds(plan))
 
     def synth_list(self, plan: BatchPlan, params: AssemblyParams) -> list[np.ndarray]:
         pcm, off, cnt = self.synth_batch(plan, params)

@@ -41,6 +41,10 @@ def lib() -> C.CDLL:
         L.ctts_b200_capacity_hint.restype = C.c_uint64
         L.ctts_b200_capacity_hint_rate.argtypes = [vp, vp, vp, C.c_uint32, C.c_uint32]
         L.ctts_b200_capacity_hint_rate.restype = C.c_uint64
+        L.ctts_b200_synth_texts_flac.argtypes = [vp, vp, vp, vp, C.c_uint32, vp, C.c_uint64, vp, vp, vp, vp,
+                                                 C.POINTER(C.c_uint64), C.POINTER(Options), C.POINTER(Timing)]
+        L.ctts_b200_capacity_hint_flac.argtypes = [vp, vp, vp, C.c_uint32, C.c_uint32]
+        L.ctts_b200_capacity_hint_flac.restype = C.c_uint64
         L.ctts_b200_plan_cache_create.argtypes = [C.c_size_t]
         L.ctts_b200_plan_cache_create.restype = vp
         L.ctts_b200_plan_cache_destroy.argtypes = [vp]
@@ -117,3 +121,29 @@ def synth_texts(front, gpu, batch: TextBatch, pcm_out: np.ndarray, piece_utts: i
         raise _gpu.GpuError(f"ctts_b200_synth_texts: {rc}: {msg.decode(errors='replace') if msg else ''}")
     res = (off[:n], cnt[:n], int(used.value), tm)
     return res + (stats[:2 * n].reshape(n, 2),) if want_stats else res
+
+
+def capacity_hint_flac(front, batch: TextBatch, rate: int = 22050) -> int:
+    """Bytes that are always enough for synth_texts_flac at output rate `rate` (ctts_b200_capacity_hint_flac)."""
+    return int(lib().ctts_b200_capacity_hint_flac(front._h, batch.ptrs, batch.speeds_ptr, batch.n, rate))
+
+
+def synth_texts_flac(front, gpu, batch: TextBatch, out: np.ndarray, piece_utts: int = 0, threads: int = 0,
+                     cache: PlanCache | None = None):
+    """ctts_b200_synth_texts_flac: one .flac file per utterance in the uint8 buffer `out`.
+    Returns (byte offsets[n], file bytes[n], sample counts[n], bytes_used, Timing)."""
+    assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
+    n = batch.n
+    off = np.zeros(max(n, 1), dtype=np.uint64)
+    nbytes = np.zeros(max(n, 1), dtype=np.uint32)
+    cnt = np.zeros(max(n, 1), dtype=np.uint32)
+    used = C.c_uint64()
+    opt = Options(piece_utts, threads, None, None, cache._h if cache is not None else None)
+    tm = Timing()
+    rc = lib().ctts_b200_synth_texts_flac(front._h, gpu._h, batch.ptrs, batch.speeds_ptr, n, out.ctypes.data, out.size,
+                                          off.ctypes.data, nbytes.ctypes.data, cnt.ctypes.data, None, C.byref(used),
+                                          C.byref(opt), C.byref(tm))
+    if rc != 0:
+        msg = _gpu.lib().ctts_gpu_last_error(gpu._h)
+        raise _gpu.GpuError(f"ctts_b200_synth_texts_flac: {rc}: {msg.decode(errors='replace') if msg else ''}")
+    return off[:n], nbytes[:n], cnt[:n], int(used.value), tm

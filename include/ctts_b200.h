@@ -70,5 +70,6 @@ uint64_t ctts_b200_capacity_hint(ctts_front* front, const char* const* texts, co
 #endif
 
 #include "ctts_b200_rate.h"
+#include "ctts_b200_flac.h"
 
 #endif /* CTTS_B200_H */

@@ -130,6 +130,26 @@ int ctts_gpu_session_submit(ctts_gpu_session* s, const ctts_batch_plan* piece, u
                             uint32_t* out_counts);
 int ctts_gpu_session_end(ctts_gpu_session* s, uint64_t* samples_used);
 
+/* ---- FLAC sessions: the same session, every utterance delivered as one .flac file (DESIGN.md 3.5) ----------------
+ * Lossless: a file decodes to exactly the PCM a PCM session delivers for the same piece.  Each file is complete and
+ * self-contained (RFC 9639): "fLaC", one STREAMINFO block (the context's output rate, mono, 16 bit, the utterance's
+ * sample count, MD5 all zero), frames of 4096 samples (the last one holds the remainder) with CONSTANT, FIXED
+ * (orders 0-4, Rice-coded residuals) or VERBATIM subframes.  The encoder is deterministic.
+ * begin_flac   as ctts_gpu_session_begin; out (page-locked for full copy speed) holds capacity_bytes bytes.
+ * submit_flac  as ctts_gpu_session_submit; the files are packed back to back in out, each starting at a multiple of
+ *              16 bytes (the padding is zero).  out_offsets[i] (bytes), out_bytes[i] (file size) and out_counts[i]
+ *              (samples) are written when the piece has arrived.  A buffer that turns out too small ends the session
+ *              with CTTS_GPU_ERR_BOUNDS; ctts_gpu_flac_bound of every bound (rounded up to 16) is always enough.
+ * ctts_gpu_session_end closes it; *samples_used is then the number of BYTES taken in out.  ctts_gpu_session_submit on
+ * a FLAC session, or ctts_gpu_session_submit_flac on a PCM session, is CTTS_GPU_ERR_INVALID_ARG. */
+int ctts_gpu_session_begin_flac(ctts_gpu_ctx* ctx, const ctts_assembly_params* params, uint8_t* out,
+                                uint64_t capacity_bytes, ctts_gpu_chunk_fn on_piece, void* user, ctts_gpu_session** s);
+int ctts_gpu_session_submit_flac(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets,
+                                 uint32_t* out_bytes, uint32_t* out_counts);
+/* Largest .flac file of an utterance of `samples` samples: 42 + ceil(samples / 4096) * (16 + 1 + 8192 + 2) bytes
+ * (a VERBATIM subframe caps every frame). */
+uint64_t ctts_gpu_flac_bound(uint64_t samples);
+
 /* ---- one batch on several GPUs of one box ---------------------------------------------------------
  * ctxs[d] is a context on device d (each holds its own replica of the voice: ctts_gpu_init per device).
  * The batch is partitioned by utterance (greedy longest-processing-time on the slot sizes, WSOLA
