@@ -2,12 +2,13 @@
  * ctts_b200 -- the `ctts synth` command line (ctts.c:3970-4030) over the B200 back end, in the
  * reference's own language: plain C on top of the two C-ABI libraries, no Python, no CUDA headers.
  *
- *   ctts_b200 synth <database.db> "text" <output.wav|output.flac> [speed] [rate]
- *   ctts_b200 synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac]     lines: speed<TAB>text
+ *   ctts_b200 synth <database.db> "text" <output.wav|output.flac> [speed] [rate] [lufs=<target>]
+ *   ctts_b200 synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target>]     lines: speed<TAB>text
  *
  * rate: output sample rate in Hz (default 22050, the voice's own; ctts_gpu_set_output_rate lists the others),
  * written into the WAV header.  An output name ending in ".flac", or synth-batch's "flac", writes lossless FLAC files
- * encoded on the device (ctts_b200_synth_texts_flac) instead of 16-bit WAV.
+ * encoded on the device (ctts_b200_synth_texts_flac) instead of 16-bit WAV.  lufs=<target> normalizes every utterance
+ * to <target> LUFS (ITU-R BS.1770-4, in [-60, -5]) with its sample peak held to -1 dBFS (ctts_gpu_set_loudness).
  *
  * Like the reference it reads config.yaml and normalization.csv from the working directory
  * (ctts.c:3990, :3636), clamps the speed to [0.5, 2.0] (ctts.c:3976-3981) and takes default_speed
@@ -43,7 +44,7 @@ static void engine_close(engine* e) {
 }
 
 /* ctts_init (ctts.c:1117) + ctts_load_config("config.yaml") + the rule table, for both halves */
-static int engine_open(engine* e, const char* db_path, uint32_t rate) {
+static int engine_open(engine* e, const char* db_path, uint32_t rate, float lufs) {
     memset(e, 0, sizeof *e);
     FILE* f = fopen(db_path, "rb");
     if (!f) return -1;
@@ -74,8 +75,25 @@ static int engine_open(engine* e, const char* db_path, uint32_t rate) {
         engine_close(e);
         return rc;
     }
+    if (lufs != 0.0f && (rc = ctts_gpu_set_loudness(e->gpu, lufs, -1.0f)) != 0) {
+        fprintf(stderr, "loudness target %g LUFS: %s\n", (double)lufs, ctts_gpu_last_error(e->gpu));
+        engine_close(e);
+        return rc;
+    }
     e->rate = rate;
     return 0;
+}
+
+/* An optional last argument lufs=<target> (after the output argument): taken off the argument list.  *lufs = 0 without one; -1 when it is not a
+ * number (any other value is checked by ctts_gpu_set_loudness). */
+static int take_lufs(int* argc, char** argv, float* lufs) {
+    *lufs = 0.0f;
+    if (*argc < 6 || strncmp(argv[*argc - 1], "lufs=", 5) != 0) return 0;   /* behind the required arguments only */
+    const char* v = argv[*argc - 1] + 5;
+    char* end = NULL;
+    *lufs = strtof(v, &end);
+    (*argc)--;
+    return (*v && end && *end == '\0') ? 0 : -1;
 }
 
 /* ctts_write_wav, ctts.c:809: 44-byte RIFF/WAVE header (PCM, mono, 16 bit) + samples */
@@ -159,15 +177,16 @@ static uint32_t parse_rate(const char* a) {
 }
 
 static int cmd_synth(int argc, char** argv) {
-    if (argc < 5 || argc > 7) {
-        fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed] [rate]\n", argv[0]);
+    float lufs;
+    if (take_lufs(&argc, argv, &lufs) || argc < 5 || argc > 7) {
+        fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed] [rate] [lufs=<target>]\n", argv[0]);
         return 1;
     }
     float speed = 1.0f;
     if (argc > 5) speed = clamp_speed(strtof(argv[5], NULL));
     const uint32_t rate = argc > 6 ? parse_rate(argv[6]) : SAMPLE_RATE;
     engine e;
-    if (engine_open(&e, argv[2], rate)) {
+    if (engine_open(&e, argv[2], rate, lufs)) {
         fprintf(stderr, "Failed to load database: %s\n", argv[2]);
         return 1;
     }
@@ -213,8 +232,9 @@ static void write_chunk(void* user, uint32_t u0, uint32_t u1) {
 }
 
 static int cmd_synth_batch(int argc, char** argv) {
-    if (argc < 5 || argc > 7 || (argc == 7 && strcmp(argv[6], "flac") != 0)) {
-        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac]\n", argv[0]);
+    float lufs;
+    if (take_lufs(&argc, argv, &lufs) || argc < 5 || argc > 7 || (argc == 7 && strcmp(argv[6], "flac") != 0)) {
+        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target>]\n", argv[0]);
         return 1;
     }
     const uint32_t rate = argc > 5 ? parse_rate(argv[5]) : SAMPLE_RATE;
@@ -246,7 +266,7 @@ static int cmd_synth_batch(int argc, char** argv) {
     free(line);
     fclose(f);
     engine e;
-    if (engine_open(&e, argv[2], rate)) {
+    if (engine_open(&e, argv[2], rate, lufs)) {
         fprintf(stderr, "Failed to load database: %s\n", argv[2]);
         return 1;
     }
@@ -276,7 +296,7 @@ static int cmd_synth_batch(int argc, char** argv) {
 int main(int argc, char** argv) {
     if (argc >= 2 && strcmp(argv[1], "synth") == 0) return cmd_synth(argc, argv);
     if (argc >= 2 && strcmp(argv[1], "synth-batch") == 0) return cmd_synth_batch(argc, argv);
-    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav|output.flac> [speed] [rate]\n       %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac]\n",
+    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav|output.flac> [speed] [rate] [lufs=<target>]\n       %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target>]\n",
             argv[0], argv[0]);
     return 1;
 }

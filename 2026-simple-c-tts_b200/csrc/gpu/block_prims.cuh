@@ -3,7 +3,8 @@
 // The assembly path needs exact integer reductions (sums of squares and DC sums
 // are order-free because they are integers: SURVEY.md 7.3) and max/min scans for
 // the silence-run analysis; float sums are NEVER reduced in parallel anywhere in
-// this back end because the reference's float accumulations are sequential.
+// this back end because the reference's float accumulations are sequential.  (The loudness measurement of
+// loudness.cuh is the one exception: it is not part of the reference, and its contract carries a tolerance.)
 #pragma once
 #include <cstdint>
 

@@ -23,10 +23,14 @@
 #include "wsola.cuh"
 #include "resample.cuh"
 #include "flac.cuh"
+#include "loudness.cuh"
 
 extern "C" void ctts_host_tables(float* fade_out, float* fade_in, float* sine, float* hann256,
                                  float* hann512);
 extern "C" void ctts_host_resample_taps(unsigned L, unsigned M, float* g);
+extern "C" void ctts_host_loudness_filter(unsigned fs, double* shelf, double* hp);
+extern "C" void ctts_host_loudness_gains(unsigned* table);
+extern "C" unsigned ctts_host_loudness_ceiling(float ceiling_dbfs);
 
 // Launch geometry of resample_kernel for the reduced ratio L/M (host only, no CUDA call; tests restate the kernel's
 // tile arithmetic against it): kp taps per phase row (a multiple of 4), the filter delay c, the staging bound
@@ -141,6 +145,17 @@ struct ctts_gpu_ctx {
     std::vector<RsTable*> rs_tables;
     RsTable* rs = nullptr;          // the output rate of the context; nullptr: the native 22 050 Hz
     int rs_smem_attr = 48 * 1024;   // dynamic shared memory resample_kernel may use on this device
+    // loudness normalization (DESIGN.md 3.6): one setting per (output rate, target, ceiling) this context has seen;
+    // plans keep a pointer to the one they were created under
+    struct LdTable {
+        uint32_t hz = 0;
+        float target = 0, ceiling = 0;
+        uint32_t ceiling_q = 0;     // A
+        ctts::LdFilter f{};         // the K-weighting at hz and its transitions (kernel parameters)
+    };
+    std::vector<LdTable*> ld_tables;
+    LdTable* ld = nullptr;          // nullptr: the stage is off
+    uint32_t* d_ld_gains = nullptr; // the gain table, uploaded by the first ctts_gpu_set_loudness that turns the stage on
     uint64_t pool_samples = 0;
     uint32_t n_units = 0;
     uint32_t max_unit = 0;
@@ -200,6 +215,14 @@ struct ctts_gpu_plan {
     uint32_t* d_final_counts = nullptr;    // the counts callers see: d_rs_counts with rs, else d_counts
     uint32_t rs_tiles = 0;                 // rs: grid.x of resample_kernel
     int16_t* d_nat_owned = nullptr;        // resident plan with rs: its native slots
+    const ctts_gpu_ctx::LdTable* ld = nullptr;   // loudness setting the plan was created under (nullptr: off)
+    unsigned long long* d_ld_off = nullptr;      // ld: output-rate slot offsets [n + 1], then first chunks [n + 1]
+    double* d_ld_state = nullptr;                // ld: 4 per chunk
+    double* d_ld_energy = nullptr;               // ld: per chunk
+    uint32_t* d_ld_peak = nullptr;               // ld: per chunk
+    double* d_ld_lufs = nullptr;                 // ld: per utterance
+    uint32_t* d_ld_gain = nullptr;               // ld: per utterance
+    uint32_t ld_tiles = 0, ld_apply_tiles = 0;   // ld: grid.x of the chunk passes and of ld_apply_kernel
     Arena* arena = nullptr;         // device buffers live in a lane's arena (batch path); else cudaMalloc'ed
     uint32_t op0 = 0;               // first op of the plan's utterances in the caller's op array (ops are kept from there on)
     std::vector<void*> owned;       // else: cudaMalloc'ed buffers to free
@@ -532,6 +555,8 @@ void ctts_gpu_free(ctts_gpu_ctx* ctx) {
         cudaFree(t->d_taps);
         delete t;
     }
+    for (ctts_gpu_ctx::LdTable* t : ctx->ld_tables) delete t;
+    cudaFree(ctx->d_ld_gains);
     for (ctts_gpu_ctx::NormPool* np : ctx->norm_pools) {
         cudaFree(np->d_pool);
         cudaFree(np->d_meta);
@@ -566,6 +591,61 @@ int ctts_gpu_set_stream(ctts_gpu_ctx* ctx, void* cuda_stream) {
     return CTTS_GPU_OK;
 }
 
+}  // extern "C"
+
+namespace {
+
+// The loudness setting (target, ceiling) at the context's current output rate: found among the context's tables or
+// built.  The transitions A^len of the scan come from running the cascade itself on the unit states.
+void ld_select(ctts_gpu_ctx* ctx, float target, float ceiling) {
+    const uint32_t hz = ctx->rs ? ctx->rs->hz : (uint32_t)CTTS_PLAN_SAMPLE_RATE;
+    for (ctts_gpu_ctx::LdTable* t : ctx->ld_tables)
+        if (t->hz == hz && t->target == target && t->ceiling == ceiling) {
+            ctx->ld = t;
+            return;
+        }
+    ctts_gpu_ctx::LdTable* t = new ctts_gpu_ctx::LdTable();
+    t->hz = hz;
+    t->target = target;
+    t->ceiling = ceiling;
+    t->ceiling_q = ctts_host_loudness_ceiling(ceiling);
+    double shelf[5], hp[2];
+    ctts_host_loudness_filter(hz, shelf, hp);
+    ctts::LdFilter& f = t->f;
+    f.b0 = shelf[0] / 32768.0;
+    f.b1 = shelf[1] / 32768.0;
+    f.b2 = shelf[2] / 32768.0;
+    f.a1 = shelf[3];
+    f.a2 = shelf[4];
+    f.h1 = hp[0];
+    f.h2 = hp[1];
+    f.fs = hz;
+    f.lo = hz / 10;
+    for (int r = 0; r < 2; r++)
+        for (int i = 0; i < 4; i++) {
+            double v[4] = {0.0, 0.0, 0.0, 0.0};
+            v[i] = 1.0;
+            ctts::LdState s{v[0], v[1], v[2], v[3]};
+            for (uint32_t j = 0; j < f.lo + (uint32_t)r; j++) ctts::ld_step(f, s, 0.0);
+            f.pw[r][0 * 4 + i] = s.s1;
+            f.pw[r][1 * 4 + i] = s.s2;
+            f.pw[r][2 * 4 + i] = s.t1;
+            f.pw[r][3 * 4 + i] = s.t2;
+        }
+    ctx->ld_tables.push_back(t);
+    ctx->ld = t;
+}
+
+// after a change of the output rate: the loudness setting moves to the new rate
+int ld_follow_rate(ctts_gpu_ctx* ctx) {
+    if (ctx->ld) ld_select(ctx, ctx->ld->target, ctx->ld->ceiling);
+    return CTTS_GPU_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
 int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz) {
     if (!ctx) return CTTS_GPU_ERR_INVALID_ARG;
     if (hz < 8000 || hz > 48000) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "output rate %u Hz outside [8000, 48000]", hz);
@@ -574,12 +654,12 @@ int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz) {
     if (ctx->session) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "the output rate cannot change while a session is open");
     if (hz == CTTS_PLAN_SAMPLE_RATE) {
         ctx->rs = nullptr;
-        return CTTS_GPU_OK;
+        return ld_follow_rate(ctx);
     }
     for (ctts_gpu_ctx::RsTable* t : ctx->rs_tables)
         if (t->hz == hz) {
             ctx->rs = t;
-            return CTTS_GPU_OK;
+            return ld_follow_rate(ctx);
         }
     CU(ctx, cudaSetDevice(ctx->device));
     const uint32_t N = 2u * 40u * R + 1u;
@@ -616,6 +696,33 @@ int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz) {
     }
     ctx->rs_tables.push_back(t);
     ctx->rs = t;
+    return ld_follow_rate(ctx);
+}
+
+int ctts_gpu_set_loudness(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_dbfs) {
+    if (!ctx) return CTTS_GPU_ERR_INVALID_ARG;
+    if (!std::isfinite(target_lufs) || (target_lufs != 0.0f && (target_lufs < -60.0f || target_lufs > -5.0f)))
+        return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "loudness target %g LUFS: neither 0 nor in [-60, -5]", (double)target_lufs);
+    if (!std::isfinite(ceiling_dbfs) || ceiling_dbfs < -20.0f || ceiling_dbfs > 0.0f)
+        return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "peak ceiling %g dBFS outside [-20, 0]", (double)ceiling_dbfs);
+    if (ctx->session) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "the loudness setting cannot change while a session is open");
+    if (target_lufs == 0.0f) {
+        ctx->ld = nullptr;
+        return CTTS_GPU_OK;
+    }
+    if (!ctx->d_ld_gains) {
+        std::vector<uint32_t> gains(2 * ctts::LD_K_MAX + 1);
+        ctts_host_loudness_gains(gains.data());
+        CU(ctx, cudaSetDevice(ctx->device));
+        cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&ctx->d_ld_gains), gains.size() * 4);
+        if (e == cudaSuccess) e = cudaMemcpy(ctx->d_ld_gains, gains.data(), gains.size() * 4, cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) {
+            cudaFree(ctx->d_ld_gains);
+            ctx->d_ld_gains = nullptr;
+            return fail(ctx, CTTS_GPU_ERR_CUDA, "loudness gain table: %s", cudaGetErrorString(e));
+        }
+    }
+    ld_select(ctx, target_lufs, ceiling_dbfs);
     return CTTS_GPU_OK;
 }
 
@@ -909,6 +1016,22 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     } else {
         p->n_offsets = p->offsets;
     }
+    // loudness: one chunk per 100 ms sub-block that can start before the bound
+    const ctts_gpu_ctx::LdTable* const ld = ctx->ld;
+    p->ld = ld;
+    std::vector<uint64_t> ld_chunk0;
+    if (ld) {
+        ld_chunk0.resize((size_t)n + 1, 0);
+        uint64_t max_chunks = 0, max_bound = 0;
+        for (uint32_t u = 0; u < n; u++) {
+            const uint64_t k = (bound[u] * 10 + ld->hz - 1) / ld->hz;
+            ld_chunk0[u + 1] = ld_chunk0[u] + k;
+            max_chunks = std::max(max_chunks, k);
+            max_bound = std::max(max_bound, bound[u]);
+        }
+        p->ld_tiles = (uint32_t)std::max<uint64_t>((max_chunks + ctts::LD_THREADS - 1) / ctts::LD_THREADS, 1);
+        p->ld_apply_tiles = (uint32_t)std::max<uint64_t>((max_bound + ctts::LD_APPLY_TILE - 1) / ctts::LD_APPLY_TILE, 1);
+    }
 
     // ---- shared-memory geometry
     const uint32_t max_unit = ctx->max_unit, xf_max = sc.xf_max;
@@ -994,6 +1117,7 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     ctts::StretchTask* h_st = nullptr;
     uint32_t *h_ot = nullptr, *h_of = nullptr;
     unsigned long long* h_ro = nullptr;
+    unsigned long long* h_lo = nullptr;
     auto layout = [&](PlanAlloc& al) {
         p->d_ops = al.dev<ctts_plan_op>(n_ops_local);
         p->d_tasks = al.dev<ctts::RegionTask>(tasks_cap);
@@ -1008,6 +1132,15 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
             p->d_rs_counts = al.dev<uint32_t>(n);
             p->d_rs_off = al.dev<unsigned long long>(2 * ((size_t)n + 1));
             p->d_final_counts = p->d_rs_counts;
+        }
+        if (ld) {
+            const uint64_t chunks = ld_chunk0[n];
+            p->d_ld_off = al.dev<unsigned long long>(2 * ((size_t)n + 1));
+            p->d_ld_state = al.dev<double>(4 * chunks);
+            p->d_ld_energy = al.dev<double>(chunks);
+            p->d_ld_peak = al.dev<uint32_t>(chunks);
+            p->d_ld_lufs = al.dev<double>(n);
+            p->d_ld_gain = al.dev<uint32_t>(n);
         }
         if (p->n_stretch) {
             p->d_stasks = al.dev<ctts::StretchTask>(stasks.size());
@@ -1025,6 +1158,7 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
             h_of = al.host<uint32_t>(ola_first.size());
         }
         if (rs) h_ro = al.host<unsigned long long>(2 * ((size_t)n + 1));
+        if (ld) h_lo = al.host<unsigned long long>(2 * ((size_t)n + 1));
     };
     PlanAlloc al{p, true};
     layout(al);
@@ -1078,6 +1212,13 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         }
         CUP(cudaMemcpyAsync(p->d_rs_off, h_ro, 2 * ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, st));
     }
+    if (ld) {
+        for (uint32_t u = 0; u <= n; u++) {
+            h_lo[u] = p->offsets[u];
+            h_lo[n + 1 + u] = ld_chunk0[u];
+        }
+        CUP(cudaMemcpyAsync(p->d_ld_off, h_lo, 2 * ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, st));
+    }
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ctts::assemble_kernel, ctts::ASM_THREADS, p->smem_bytes) != cudaSuccess || occ < 1)
         occ = 1;
@@ -1088,6 +1229,8 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         p->info.kernel_launches += 2 + (p->verify_tiles && ctx->knobs.wsola_speculate ? (p->n_stretch + 65534) / 65535 : 0) +
                                    (p->n_ola_blocks ? 1 : 0);
     if (rs) p->info.kernel_launches += (uint32_t)(((uint64_t)n + 65534) / 65535);   // resample_kernel
+    if (ld && n)   // the two chunk passes and ld_apply_kernel per grid.y slice, ld_scan_kernel, ld_gain_kernel
+        p->info.kernel_launches += 3 * (uint32_t)(((uint64_t)n + 65534) / 65535) + 2;
     p->info.n_stretch = p->n_stretch;
     p->info.bound_samples = std::accumulate(bound.begin(), bound.end(), (uint64_t)0);
     p->info.smem_bytes = p->smem_bytes;
@@ -1685,6 +1828,46 @@ int launch_resample(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const int16_t* d_nat, i
     return CTTS_GPU_OK;
 }
 
+// Enqueue the loudness normalization of the plan (after its output-rate conversion), in place on the output-rate
+// slots d_final.  Nothing when the stage is off.
+int launch_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_final, cudaStream_t st) {
+    const ctts_gpu_ctx::LdTable* ld = p->ld;
+    if (!ld || !p->n_utts) return CTTS_GPU_OK;
+    const uint32_t n = p->n_utts;
+    ctts::LdArgs a{};
+    a.pcm = d_final;
+    a.off = p->d_ld_off;
+    a.counts = p->d_final_counts;
+    a.state = p->d_ld_state;
+    a.energy = p->d_ld_energy;
+    a.peak = p->d_ld_peak;
+    a.lufs = p->d_ld_lufs;
+    a.gain = p->d_ld_gain;
+    a.table = ctx->d_ld_gains;
+    a.gate_abs = pow(10.0, (-70.0 + 0.691) / 10.0);
+    a.n = n;
+    a.ceiling = ld->ceiling_q;
+    a.target = ld->target;
+    a.f = ld->f;
+    auto sliced = [&](auto kernel, uint32_t tiles, int threads) -> int {
+        for (uint32_t u0 = 0; u0 < n; u0 += 65535u) {   // grid.y limit
+            a.u0 = u0;
+            kernel<<<dim3(tiles, std::min<uint32_t>(n - u0, 65535u)), threads, 0, st>>>(a);
+            CU(ctx, cudaGetLastError());
+        }
+        a.u0 = 0;
+        return CTTS_GPU_OK;
+    };
+    int rc = sliced(ctts::ld_chunk_kernel<false>, p->ld_tiles, ctts::LD_THREADS);
+    if (rc) return rc;
+    ctts::ld_scan_kernel<<<(n + ctts::LD_SCAN_THREADS - 1) / ctts::LD_SCAN_THREADS, ctts::LD_SCAN_THREADS, 0, st>>>(a);
+    CU(ctx, cudaGetLastError());
+    if ((rc = sliced(ctts::ld_chunk_kernel<true>, p->ld_tiles, ctts::LD_THREADS)) != 0) return rc;
+    ctts::ld_gain_kernel<<<n, ctts::LD_GAIN_THREADS, 0, st>>>(a);
+    CU(ctx, cudaGetLastError());
+    return sliced(ctts::ld_apply_kernel, p->ld_apply_tiles, ctts::LD_APPLY_THREADS);
+}
+
 }  // namespace
 
 extern "C" {
@@ -1737,6 +1920,7 @@ int ctts_gpu_plan_run(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out) {
     if (!rc) rc = launch_assemble(ctx, p, d_nat, ctx->stream);
     if (!rc) rc = launch_stretch(ctx, p, d_nat, ctx->stream);
     if (!rc) rc = launch_resample(ctx, p, d_nat, d_pcm_out, ctx->stream);
+    if (!rc) rc = launch_loudness(ctx, p, d_pcm_out, ctx->stream);
     return rc;
 }
 
@@ -1757,6 +1941,17 @@ int ctts_gpu_plan_read_pcm(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* dst, ui
     if (!ctx || !p || !dst || !p->d_out_last || first + n > p->offsets[p->n_utts]) return CTTS_GPU_ERR_INVALID_ARG;
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, cudaMemcpyAsync(dst, p->d_out_last + first, n * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return CTTS_GPU_OK;
+}
+
+int ctts_gpu_plan_read_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, double* lufs, uint32_t* gain) {
+    if (!ctx || !p || p->ctx != ctx || !lufs || !gain) return CTTS_GPU_ERR_INVALID_ARG;
+    if (!p->ld) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "the plan was created with loudness normalization off");
+    if (p->n_utts == 0) return CTTS_GPU_OK;
+    CU(ctx, cudaSetDevice(ctx->device));
+    CU(ctx, cudaMemcpyAsync(lufs, p->d_ld_lufs, (size_t)p->n_utts * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(gain, p->d_ld_gain, (size_t)p->n_utts * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return CTTS_GPU_OK;
 }
@@ -1982,6 +2177,7 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
         if (!rc) rc = launch_assemble(ctx, p, l.d_out, ctx->stream);
         if (!rc) rc = launch_stretch(ctx, p, l.d_out, ctx->stream);
         if (!rc) rc = launch_resample(ctx, p, l.d_out, d_final, ctx->stream);
+        if (!rc) rc = launch_loudness(ctx, p, d_final, ctx->stream);
         if (rc) return bail(rc);
         if (ctx->knobs.trace) {
             auto msf = [](auto a, auto b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
@@ -2278,6 +2474,11 @@ int ctts_gpu_multi_synth_batch(ctts_gpu_ctx* const* ctxs, uint32_t n_ctx, const 
     for (uint32_t d = 1; d < n_ctx; d++)
         if ((ctxs[d]->rs ? ctxs[d]->rs->hz : CTTS_PLAN_SAMPLE_RATE) != (ctxs[0]->rs ? ctxs[0]->rs->hz : CTTS_PLAN_SAMPLE_RATE))
             return fail(ctxs[0], CTTS_GPU_ERR_INVALID_ARG, "context %u has another output rate than context 0", d);
+    for (uint32_t d = 1; d < n_ctx; d++) {
+        const ctts_gpu_ctx::LdTable *a = ctxs[d]->ld, *b = ctxs[0]->ld;
+        if ((a == nullptr) != (b == nullptr) || (a && (a->target != b->target || a->ceiling != b->ceiling)))
+            return fail(ctxs[0], CTTS_GPU_ERR_INVALID_ARG, "context %u has another loudness setting than context 0", d);
+    }
     if (plan->n_utts && (!plan->utt_op_begin || !plan->speed)) return CTTS_GPU_ERR_INVALID_ARG;
     const uint32_t n = plan->n_utts;
     for (uint32_t u = 0; u < n; u++)

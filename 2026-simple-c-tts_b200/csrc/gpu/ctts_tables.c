@@ -60,3 +60,32 @@ void ctts_host_resample_taps(unsigned L, unsigned M, float* g) {
     for (unsigned i = 0; i < N; i++) g[i] = (float)((double)L * (h[i] / sum));
     free(h);
 }
+
+/* K-weighting of ITU-R BS.1770-4 at fs Hz (DESIGN.md 3.6), in libebur128's parameterisation.  shelf receives the
+ * pre-filter (high shelf) b0, b1, b2, a1, a2; hp receives a1, a2 of the RLB high-pass, whose numerator is 1, -2, 1.
+ * At 48 kHz these are the two tables of BS.1770-4. */
+void ctts_host_loudness_filter(unsigned fs, double* shelf, double* hp) {
+    double f0 = 1681.974450955533, Q = 0.7071752369554196, K = tan(CTTS_PI * f0 / (double)fs);
+    const double G = 3.999843853973347, Vh = pow(10.0, G / 20.0), Vb = pow(Vh, 0.4996667741545416);
+    const double a0 = 1.0 + K / Q + K * K;
+    shelf[0] = (Vh + Vb * K / Q + K * K) / a0;
+    shelf[1] = 2.0 * (K * K - Vh) / a0;
+    shelf[2] = (Vh - Vb * K / Q + K * K) / a0;
+    shelf[3] = 2.0 * (K * K - 1.0) / a0;
+    shelf[4] = (1.0 - K / Q + K * K) / a0;
+    f0 = 38.13547087602444;
+    Q = 0.5003270373238773;
+    K = tan(CTTS_PI * f0 / (double)fs);
+    hp[0] = 2.0 * (K * K - 1.0) / (1.0 + K / Q + K * K);
+    hp[1] = (1.0 - K / Q + K * K) / (1.0 + K / Q + K * K);
+}
+
+/* The loudness gains in Q16, steps of 0.01 dB: table[k + 8000] = floor(65536 * 10^(k / 2000)), k = -8000 .. 8000. */
+void ctts_host_loudness_gains(unsigned* table) {
+    for (int k = -8000; k <= 8000; k++) table[k + 8000] = (unsigned)floor(65536.0 * pow(10.0, (double)k / 2000.0));
+}
+
+/* The sample-peak ceiling of C dBFS as an int16 magnitude: floor(32767 * 10^(C / 20)). */
+unsigned ctts_host_loudness_ceiling(float ceiling_dbfs) {
+    return (unsigned)floor(32767.0 * pow(10.0, (double)ceiling_dbfs / 20.0));
+}

@@ -53,6 +53,8 @@ def lib(build: bool = True) -> C.CDLL:
         L.ctts_gpu_free.restype = None
         L.ctts_gpu_set_stream.argtypes = [vp, vp]
         L.ctts_gpu_set_output_rate.argtypes = [vp, C.c_uint32]
+        L.ctts_gpu_set_loudness.argtypes = [vp, C.c_float, C.c_float]
+        L.ctts_gpu_plan_read_loudness.argtypes = [vp, vp, vp, vp]
         L.ctts_gpu_last_error.argtypes = [vp]
         L.ctts_gpu_last_error.restype = C.c_char_p
         L.ctts_gpu_plan_bounds.argtypes = [vp, C.POINTER(CBatchPlan), vp]
@@ -139,6 +141,14 @@ class ResidentPlan:
         self._ctx._check(lib().ctts_gpu_plan_read_pcm(self._ctx._h, self._h, out.ctypes.data, first, n))
         return out[:n]
 
+    def loudness(self) -> tuple[np.ndarray, np.ndarray]:
+        """After a run of a plan created with loudness normalization on (ctts_gpu_plan_read_loudness): every
+        utterance's integrated loudness in LUFS (-inf when undefined) and the Q16 gain applied to it."""
+        lufs = np.zeros(max(self.n_utts, 1), dtype=np.float64)
+        gain = np.zeros(max(self.n_utts, 1), dtype=np.uint32)
+        self._ctx._check(lib().ctts_gpu_plan_read_loudness(self._ctx._h, self._h, lufs.ctypes.data, gain.ctypes.data))
+        return lufs[:self.n_utts], gain[:self.n_utts]
+
     def read_pre(self, u: int, cap: int) -> np.ndarray:
         out = np.zeros(max(cap, 1), dtype=np.int16)
         n = C.c_uint64()
@@ -199,6 +209,12 @@ class GpuSynth:
         ctts_gpu.h for the accepted rates; 22050 is the voice's own), and every count, offset and bound is in
         samples of that rate.  Plans created before keep their rate."""
         self._check(lib().ctts_gpu_set_output_rate(self._h, int(hz)))
+
+    def set_loudness(self, target_lufs: float, ceiling_dbfs: float = -1.0) -> None:
+        """ctts_gpu_set_loudness: every later call of this context normalizes each utterance to target_lufs LUFS
+        (ITU-R BS.1770-4, in [-60, -5]) without letting its sample peak pass ceiling_dbfs dBFS (in [-20, 0]).
+        target_lufs == 0 turns it off.  Plans created before keep their setting."""
+        self._check(lib().ctts_gpu_set_loudness(self._h, float(target_lufs), float(ceiling_dbfs)))
 
     def bounds(self, plan: BatchPlan) -> np.ndarray:
         b = np.zeros(max(plan.n_utts, 1), dtype=np.uint64)

@@ -61,6 +61,25 @@ int ctts_gpu_set_stream(ctts_gpu_ctx* ctx, void* cuda_stream);
  * keeps the rate it was created under) and ctts_gpu_multi_synth_batch, which rejects contexts whose rates
  * differ.  ctts_gpu_plan_read_pre stays at the native rate. */
 int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz);
+/* Loudness normalization of the context (DESIGN.md 3.6), off by default.  Every utterance's integrated loudness L is
+ * measured after ITU-R BS.1770-4 on its output-rate samples x (K-weighting in double, 400 ms blocks, absolute gate
+ * -70 LUFS, relative gate -10 LU; L is undefined for utterances shorter than 400 ms or with no block above the gates),
+ * and one gain per utterance is applied on the device, after the rate conversion and before the output is packed,
+ * encoded or copied:
+ *   k = clamp(floor(100 * (T - L) + 0.5), -8000, 8000), G = min(floor(65536 * 10^(k / 2000)), floor(A * 65536 / P))
+ *   with A = floor(32767 * 10^(C / 20)) and P = max |x|; G = 65536 when L is undefined;  y = (x * G + 32768) >> 16.
+ * So an utterance reaches T LUFS to 0.005 LU unless its SAMPLE peak would pass C dBFS (there is no true-peak,
+ * oversampled, limiting and no compression); G = 65536 leaves it exactly as it was; counts do not change.
+ * Accepted: target_lufs a finite T in [-60, -5] with ceiling_dbfs a finite C in [-20, 0]; target_lufs == 0 turns the
+ * stage off (then nothing is enqueued: bytes and kernel launches are those of a context that never set it).
+ * Builds the K-weighting of the context's output rate (and keeps it consistent when the rate changes) and, once per
+ * context, uploads the gain table.  CTTS_GPU_ERR_INVALID_ARG for anything else and while a session is open; the context
+ * is then unchanged.
+ *
+ * It applies to every path: resident plans (a plan keeps the setting it was created under), all ctts_gpu_synth_batch*
+ * calls, PCM and FLAC sessions, ctts_b200_synth_texts(_flac) and ctts_gpu_multi_synth_batch, which rejects contexts
+ * whose settings differ. */
+int ctts_gpu_set_loudness(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_dbfs);
 /* Text of the last error of a context; ctx == NULL: why the calling thread's last ctts_gpu_init failed. */
 const char* ctts_gpu_last_error(const ctts_gpu_ctx* ctx);
 
@@ -182,6 +201,9 @@ int ctts_gpu_plan_read_counts(ctts_gpu_ctx* ctx, ctts_gpu_plan* plan, uint32_t* 
 /* Device -> host copy of the plan-owned PCM buffer range [first, first+n). */
 int ctts_gpu_plan_read_pcm(ctts_gpu_ctx* ctx, ctts_gpu_plan* plan, int16_t* dst, uint64_t first,
                            uint64_t n);
+/* After a run of a plan created with loudness normalization on: L (LUFS, -INFINITY when undefined) and G (Q16) of
+ * every utterance, n_utts entries each.  CTTS_GPU_ERR_INVALID_ARG for a plan created with the stage off. */
+int ctts_gpu_plan_read_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* plan, double* lufs, uint32_t* gain);
 /* Debug / tests: pre-stretch buffer of utterance u (only for speed != 1.0f utterances). */
 int ctts_gpu_plan_read_pre(ctts_gpu_ctx* ctx, ctts_gpu_plan* plan, uint32_t u, int16_t* dst,
                            uint64_t cap, uint64_t* n);
