@@ -14,6 +14,10 @@ config / assembly-parameter changes it needs:
                        47 .. 64 cuttable runs in a region (inside and beyond the trim's candidate
                        pre-pass), a negative silence threshold
 
+family_signals builds a voice that delivers chosen int16 signals unchanged, one per utterance, so the stages
+behind the assembly (output rate, loudness, FLAC) can be fed any samples through the real device path:
+loudness_signals, long_signal, flac_signals and piece_signals are the ones their GPU tests use.
+
 Every family goes through the front end.  Units are named by syllables (consonant + vowel, or one
 vowel), so a word is parsed in exactly one way and the crossfade of a join is set by the class of the
 next unit's first letter (the previous unit always ends in a vowel): plosive, fricative, other
@@ -555,6 +559,172 @@ def family_trim(seed: int = 16, negative: bool = False, min_silence_ms: float | 
                   info={"limit": limit, "min_sil": min_sil, "S": S, "P": P, "many": many})
 
 
+# ---------------------------------------------------------------------------------- chosen samples
+
+def family_signals(name: str, signals: list) -> Family:
+    """One single-unit utterance per signal, delivered unchanged: no pause, fades, trim, crossfade, intonation
+    contour (max_pitch_change 0 leaves every sample alone), RMS gain, DC removal or fade-in, and speed 1.0.  The
+    native output of utterance u is signals[u] itself (witnessed in test_edge_voices.py), so any int16 signal
+    reaches the output-rate, loudness and FLAC stages through the real device path.  A signal object that appears
+    more than once becomes one unit shared by its utterances."""
+    cfg = H.shipped_config()
+    cfg.word_pause_ms = 0.0
+    cfg.fade_in_ms = 0.0
+    cfg.fade_out_ms = 0.0
+    cfg.crossfade_ms = 0.0
+    cfg.remove_word_silence = 0
+    cfg.max_pitch_change = 0.0
+    names = Names()
+    classes = iter(["other"] * 75 + ["plosive"] * 90 + ["fricative"] * 75)
+    units, unit_of, words = [], {}, []
+    for x in signals:
+        if id(x) not in unit_of:
+            unit_of[id(x)] = names.take(next(classes))
+            units.append((unit_of[id(x)], np.ascontiguousarray(x, dtype=np.int16)))
+        words.append([[unit_of[id(x)]]])
+    return Family(name, units, words, [1.0] * len(words), cfg,
+                  params={"fade_in_samples": 0, "target_rms": 0.0, "remove_dc_offset": 0}, info={"signals": signals})
+
+
+def tone(n: int, f: float, amp: float, phase: float = 0.3) -> np.ndarray:
+    return i16(amp * np.sin(2 * np.pi * f * np.arange(n) / SR + phase))
+
+
+# ---------------------------------------------------------------------------------- L: loudness signals
+
+LD_SETTINGS = ((-16.0, -1.0), (-23.0, -3.0))     # (T, C), as test_gpu_loudness.SETTINGS
+LD_SUBS = (31, 32, 33, 128, 129, 259, 260, 261)   # warp staging of 32 chunks, chunk grid.x >= 2, nb past 256
+
+
+def ld_counts(hz: int) -> list:
+    """Output lengths at hz, s(k) = floor(k hz / 10): empty, one sample, one sample short of a block, one block, a
+    block and a partial sub-block, and s(k), s(k) + 1 for the sub-block counts of LD_SUBS."""
+    s = [k * hz // 10 for k in range(max(LD_SUBS) + 1)]
+    return sorted({0, 1, s[4] - 1, s[4], s[4] + 1} | {s[k] + d for k in LD_SUBS for d in (0, 1)})
+
+
+def native_lengths(hz: int, t: int) -> list:
+    """Native lengths whose output at hz has t samples; where upsampling skips t, the nearest on either side."""
+    import resample_oracle as R
+    L, M = R.ratio(hz)
+    least = lambda c: 0 if c <= 0 else (c - 1) * M // L + 1     # the least native length with >= c outputs
+    return sorted({least(t), least(t + 1) - 1} - {-1})
+
+
+def unity_amplitude(hz: int, T: float, C: float, n: int, f: float = 997.0) -> float:
+    """The amplitude of a tone of n native samples whose output at hz measures within 0.3 hundredths of a dB of T,
+    so the oracle's k is 0 and G is unity: L is log-linear in the amplitude, so a few corrections converge."""
+    import loudness_oracle as O
+    import resample_oracle as R
+    a = 3000.0
+    for _ in range(30):
+        y = R.resample(tone(n, f, a), hz)
+        L = O.lufs(y, hz)
+        if abs(100.0 * (float(np.float32(T)) - L)) < 0.3 and O.normalize(y, hz, T, C)[2] == O.UNITY:
+            return a
+        a *= 10.0 ** ((T - L) / 20.0)
+    raise AssertionError(f"no unity tone at {hz} Hz for T = {T}")
+
+
+def loudness_signals(hz: int, seed: int = 31) -> list:
+    """(case, native signal) pairs for one launch at output rate hz: every length of ld_counts, and signals that drive
+    each gate and gain decision (witnessed on the resampled signal in test_loudness.py)."""
+    rng = np.random.default_rng(seed + hz)
+    out = []
+    for t in ld_counts(hz):
+        for n in native_lengths(hz, t):
+            out.append((f"len{t}", harmonic(rng, n)))
+    two = 2 * SR
+    loud = harmonic(rng, two, peak=16000.0)
+    out.append(("two_levels", np.concatenate([loud, i16(loud.astype(np.float64) / 100.0)])))     # 40 dB apart
+    env = np.geomspace(2.0, 80.0, 4 * SR)      # a 997 Hz tone from about -91 to -59 LUFS
+    out.append(("straddles_abs_gate", i16(env * np.sin(2 * np.pi * 997.0 * np.arange(4 * SR) / SR))))
+    out.append(("faint", tone(5 * SR // 2, 997.0, 2.0)))
+    burst = np.zeros(3 * SR + 4 * SR // 10, np.int16)
+    burst[-4 * SR // 10:] = tone(4 * SR // 10, 440.0, 20000.0)
+    out.append(("last_block_burst", burst))
+    lone = np.zeros(2 * SR, np.int16)
+    lone[SR] = -32768
+    out.append(("lone_min", lone))
+    sq = harmonic(rng, 2 * SR, peak=300.0)
+    sq[SR:SR + 40] = np.where(np.arange(40) < 20, 32767, -32767)   # one period of a full-scale square
+    sq[SR] = -32768
+    out.append(("square_burst", sq))
+    out.append(("loud", tone(2 * SR, 997.0, 32000.0)))
+    for T, C in LD_SETTINGS:
+        n = 5 * SR // 2
+        out.append((f"unity{int(T)}", tone(n, 997.0, unity_amplitude(hz, T, C, n))))
+    return out
+
+
+# ---------------------------------------------------------------------------------- one long utterance
+
+LONG_FRAMES = 2049      # FLAC frame numbers 0 .. 2048: coded in one, two and three bytes
+
+
+def long_signal(seed: int = 33) -> np.ndarray:
+    """6.3 minutes at 22 050 Hz (2 049 FLAC frames and a partial one): speech-like levels that change every
+    second, with silent seconds between, so both loudness gates act over thousands of 100 ms chunks."""
+    rng = np.random.default_rng(seed)
+    n = LONG_FRAMES * 4096 + 1234
+    x = harmonic(rng, n, f0=130.0, peak=8000.0).astype(np.float64)
+    sec = np.arange(n) // SR
+    level = 10.0 ** (rng.uniform(-45.0, 0.0, sec[-1] + 1) / 20.0)
+    level[rng.random(len(level)) < 0.15] = 0.0
+    return i16(x * level[sec])
+
+
+# ---------------------------------------------------------------------------------- Q: FLAC signals
+
+FLAC_LAST = (1, 2, 3, 4, 5, 8, 15, 16, 17, 31, 32, 256, 257, 2048, 4095)
+
+
+def _fixed_order(x: np.ndarray) -> int:
+    """The encoder's order rule (DESIGN.md 3.5): least sum of |residual| over samples 4 .. n - 1, ties to the lower."""
+    r = x.astype(np.int64)
+    sums = []
+    for o in range(5):
+        sums.append(int(np.abs(r[4 - o:]).sum()))
+        r = np.diff(r)
+    return int(np.argmin(sums))
+
+
+def order_tones(n: int = 4096, amp: float = 3000.0, seed: int = 35) -> list:
+    """Noisy tones of one frame each whose fixed order is 0, 1, 2, 3 and 4 in turn.  (An integer polynomial of
+    degree d >= 2 cannot fill 4 096 samples in int16, and a rounded one leaves rounding noise that favours low
+    orders.  A tone's order-d residual scales with (2 sin(pi f / fs))^d and white noise's with sqrt(C(2d, d)), so
+    the frequency and the noise level set which order is least.)"""
+    nz = np.random.default_rng(seed).normal(0.0, 1.0, n)
+    out = {}
+    for sigma in (0.0, 100.0):
+        for f in np.geomspace(6000.0, 5.0, 200):
+            x = i16(amp * np.sin(2 * np.pi * f * np.arange(n) / SR + 0.3) + sigma * nz)
+            out.setdefault(_fixed_order(x), x)
+    return [out[d] for d in range(5)]
+
+
+def flac_signals(seed: int = 34) -> list:
+    """(case, native signal) pairs that drive each decision of the FLAC encoder (witnessed by the decoder's frame
+    report in test_flac.py)."""
+    rng = np.random.default_rng(seed)
+    noise = lambda n: rng.integers(-32768, 32768, n).astype(np.int16)
+    out = [("constant_then_fixed", np.concatenate([np.full(2 * 4096, -1234, np.int16), harmonic(rng, 2 * 4096)]))]
+    out.append(("noise", noise(5 * 4096)))
+    half = np.zeros(3 * 4096, np.int16)
+    for f in range(3):
+        half[f * 4096:f * 4096 + 2048] = noise(2048)
+    out.append(("half_noise", half))
+    out.append(("alternating", np.where(np.arange(2 * 4096 + 100) % 2, -32768, 32767).astype(np.int16)))
+    out += [(f"order{d}", x) for d, x in enumerate(order_tones())]
+    out.append(("ramp", (np.arange(12000) * 5 - 30000).astype(np.int16)))
+    for r in FLAC_LAST:
+        # a smooth tone (order 4) whose last sample jumps: the partition that holds it wants a large Rice parameter
+        x = tone(2 * 4096 + r, 527.0, 30000.0)
+        x[-1] = i16(x[-1] - 20000.0 * np.sign(float(x[-1]) or 1.0))
+        out.append((f"last{r}", x))
+    return out
+
+
 FAMILIES = {
     "short_units": family_short_units,
     "pitch": family_pitch,
@@ -573,4 +743,39 @@ _built: dict = {}
 def family(name: str) -> Family:
     if name not in _built:
         _built[name] = FAMILIES[name]()
+    return _built[name]
+
+
+# ---------------------------------------------------------------------------------- the signal families
+
+LD_RATES = (22050, 11025, 8015, 46035, 8001, 47971)   # 22 050 is the control: every sub-block fs / 10 long
+PIECE_SIZES = (2000, 70000)   # a FLAC piece past one 1 024-utterance scan pass, and one past grid.y = 65 535
+
+
+def piece_signals(seed: int = 36) -> list:
+    """A handful of short signals (0 .. 3 frames) for the piece-size tests; utterance u uses signal u % 7 (7 divides
+    neither 1 024 nor 65 535, so neighbours across each limit differ)."""
+    rng = np.random.default_rng(seed)
+    return [np.zeros(0, np.int16), harmonic(rng, 1), harmonic(rng, 1000), np.full(3000, 77, np.int16),
+            harmonic(rng, 4096), rng.integers(-32768, 32768, 5000).astype(np.int16), harmonic(rng, 9000)]
+
+
+def _signal_family(name: str) -> Family:
+    if name == "flac":
+        return family_signals(name, [x for _, x in flac_signals()])
+    if name == "long":
+        return family_signals(name, [long_signal()])
+    if name == "pieces":
+        sig = piece_signals()
+        return family_signals(name, [sig[u % len(sig)] for u in range(sum(PIECE_SIZES))])
+    hz = int(name.split("_")[1])
+    return family_signals(name, [x for _, x in loudness_signals(hz)])
+
+
+SIGNAL_FAMILIES = ["flac", "long", "pieces"] + [f"loudness_{hz}" for hz in LD_RATES]
+
+
+def signal_family(name: str) -> Family:
+    if name not in _built:
+        _built[name] = _signal_family(name)
     return _built[name]

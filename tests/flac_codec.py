@@ -16,6 +16,9 @@ BLOCK = 4096
 FRAME_MAX = 16 + 1 + 2 * BLOCK + 2
 INFO_FIELDS = ("min_blocksize", "max_blocksize", "min_framesize", "max_framesize", "sample_rate", "channels",
                "bits_per_sample", "total_samples", "md5_zero")
+# per frame, what the decoder parsed (ctts_flac_decode_report); kind 0 CONSTANT, 1 VERBATIM, 2 FIXED, 3 LPC
+REPORT_FIELDS = ("number", "blocksize", "header_bytes", "kind", "order", "po", "kmin", "kmax")
+CONSTANT, VERBATIM, FIXED = 0, 1, 2
 
 
 class DecodeError(ValueError):
@@ -50,6 +53,9 @@ def _lib(name: str) -> C.CDLL:
         else:
             L.ctts_flac_decode.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p]
             L.ctts_flac_decode.restype = C.c_int64
+            L.ctts_flac_decode_report.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p,
+                                                  C.c_uint64, C.POINTER(C.c_uint64)]
+            L.ctts_flac_decode_report.restype = C.c_int64
         _libs[name] = L
     return _libs[name]
 
@@ -69,16 +75,25 @@ def encode(x, hz: int) -> bytes:
     return buf[:got].tobytes()
 
 
-def decode(data: bytes, cap: int | None = None) -> tuple[np.ndarray, dict]:
-    """The independent decoder: .flac bytes -> (int16 PCM, STREAMINFO fields); DecodeError for a malformed stream."""
+def decode(data: bytes, cap: int | None = None, report: bool = False):
+    """The independent decoder: .flac bytes -> (int16 PCM, STREAMINFO fields); DecodeError for a malformed stream.
+    With report, also a record array of the frames as parsed (REPORT_FIELDS), the decoder's witness of what the
+    encoder chose."""
     src = np.frombuffer(data, np.uint8)
     if cap is None:   # STREAMINFO's total, when the header is there to read
         cap = int.from_bytes(data[21:26], "big") & ((1 << 36) - 1) if len(data) >= 26 else 0
         cap = max(cap, 1 << 16)
     out = np.zeros(max(cap, 1), np.int16)
     info = np.zeros(len(INFO_FIELDS), np.uint64)
-    got = _lib("decode").ctts_flac_decode(src.ctypes.data if len(src) else None, len(src), out.ctypes.data, cap,
-                                          info.ctypes.data)
+    rep_cap = len(data) // 6 + 1 if report else 0   # a frame takes at least 6 bytes
+    rep = np.zeros((max(rep_cap, 1), len(REPORT_FIELDS)), np.uint32)
+    frames = C.c_uint64()
+    got = _lib("decode").ctts_flac_decode_report(src.ctypes.data if len(src) else None, len(src), out.ctypes.data, cap,
+                                                 info.ctypes.data, rep.ctypes.data if report else None, rep_cap,
+                                                 C.byref(frames))
     if got < 0:
         raise DecodeError(f"flac_decode: error {got}")
-    return out[:got].copy(), dict(zip(INFO_FIELDS, (int(v) for v in info)))
+    res = out[:got].copy(), dict(zip(INFO_FIELDS, (int(v) for v in info)))
+    if not report:
+        return res
+    return res + (np.rec.fromarrays(list(rep[:frames.value].astype(np.int64).T), names=REPORT_FIELDS),)

@@ -9,10 +9,22 @@
  *   int64_t ctts_flac_decode(const uint8_t* in, uint64_t len, int16_t* out, uint64_t cap, uint64_t* info)
  *     -> samples decoded (< 0: an error code below).  info (may be NULL) receives 9 values: min and max blocksize,
  *        min and max frame size, sample rate, channels, bits per sample, total samples, 1 if the MD5 is all zero.
+ *
+ *   int64_t ctts_flac_decode_report(..., uint32_t* rep, uint64_t rep_cap, uint64_t* frames)
+ *     -> the same, and for every frame (at most rep_cap) what was parsed, REPORT_FIELDS values: the coded frame
+ *        number, the blocksize, the header length in bytes (CRC-8 included), the subframe kind (0 CONSTANT,
+ *        1 VERBATIM, 2 FIXED, 3 LPC), the predictor order, the partition order, the least and the largest Rice
+ *        parameter (15: the escape code; 0 for CONSTANT and VERBATIM).  *frames receives the frames decoded.
  */
 #include <stdint.h>
 #include <stdlib.h>
 #include <string.h>
+
+enum { REPORT_FIELDS = 8, K_NONE = 255 };
+
+typedef struct {   /* what one frame's subframe and residual said */
+    uint32_t kind, order, po, kmin, kmax;
+} parsed;
 
 enum {
     E_MARKER = -1, E_METADATA = -2, E_SYNC = -3, E_RESERVED = -4, E_CRC8 = -5, E_CRC16 = -6, E_SUBFRAME = -7,
@@ -68,17 +80,20 @@ static uint16_t crc16_of(const uint8_t* p, uint64_t n) {
     return c;
 }
 
-static int residual(br* b, uint32_t bs, uint32_t order, int64_t* r) {
+static int residual(br* b, uint32_t bs, uint32_t order, int64_t* r, parsed* rp) {
     const uint32_t method = (uint32_t)rd(b, 2);
     if (method > 1) return E_RESIDUAL;
     const uint32_t pbits = method ? 5 : 4, esc = method ? 31 : 15;
     const uint32_t po = (uint32_t)rd(b, 4);
     const uint32_t P = 1u << po;
     if (bs % P || (bs >> po) < order) return E_RESIDUAL;
+    rp->po = po;
     uint32_t i = order;
     for (uint32_t j = 0; j < P && !b->err; j++) {
         const uint32_t end = (j + 1) * (bs >> po);
         const uint32_t k = (uint32_t)rd(b, pbits);
+        if (k < rp->kmin) rp->kmin = k;
+        if (k > rp->kmax) rp->kmax = k;
         if (k == esc) {
             const uint32_t w = (uint32_t)rd(b, 5);
             for (; i < end && !b->err; i++) r[i] = rd_signed(b, w);
@@ -93,9 +108,10 @@ static int residual(br* b, uint32_t bs, uint32_t order, int64_t* r) {
     return b->err;
 }
 
-static int subframe(br* b, uint32_t bs, uint32_t bps, int64_t* s, int64_t* r) {
+static int subframe(br* b, uint32_t bs, uint32_t bps, int64_t* s, int64_t* r, parsed* rp) {
     if (rd(b, 1) != 0) return E_RESERVED;
     const uint32_t type = (uint32_t)rd(b, 6);
+    *rp = (parsed){type >= 32 ? 3 : type >= 8 ? 2 : type, type >= 32 ? type - 31 : type >= 8 ? type - 8 : 0, 0, K_NONE, 0};
     uint32_t wasted = 0;
     if (rd(b, 1)) wasted = (uint32_t)rd_unary(b) + 1;
     if (wasted >= bps) return E_SUBFRAME;
@@ -110,7 +126,7 @@ static int subframe(br* b, uint32_t bs, uint32_t bps, int64_t* s, int64_t* r) {
         const uint32_t order = type - 8;
         if (order > bs) return E_SUBFRAME;
         for (uint32_t i = 0; i < order; i++) s[i] = rd_signed(b, w);
-        int rc = residual(b, bs, order, r);
+        int rc = residual(b, bs, order, r, rp);
         if (rc) return rc;
         for (uint32_t i = order; i < bs; i++) {
             int64_t p = 0;
@@ -127,7 +143,7 @@ static int subframe(br* b, uint32_t bs, uint32_t bps, int64_t* s, int64_t* r) {
         if (shift < 0) return E_SUBFRAME;
         int64_t c[32];
         for (uint32_t j = 0; j < order; j++) c[j] = rd_signed(b, prec);
-        int rc = residual(b, bs, order, r);
+        int rc = residual(b, bs, order, r, rp);
         if (rc) return rc;
         for (uint32_t i = order; i < bs; i++) {
             int64_t p = 0;
@@ -141,7 +157,8 @@ static int subframe(br* b, uint32_t bs, uint32_t bps, int64_t* s, int64_t* r) {
     return b->err;
 }
 
-static int64_t decode(const uint8_t* in, uint64_t len, int16_t* out, uint64_t cap, uint64_t* info, int64_t* s, int64_t* r) {
+static int64_t decode(const uint8_t* in, uint64_t len, int16_t* out, uint64_t cap, uint64_t* info, int64_t* s, int64_t* r,
+                      uint32_t* rep, uint64_t rep_cap, uint64_t* frames) {
     br b = {in, len, 0, 0};
     if (len < 4 || memcmp(in, "fLaC", 4) != 0) return E_MARKER;
     b.pos = 32;
@@ -229,8 +246,15 @@ static int64_t decode(const uint8_t* in, uint64_t len, int16_t* out, uint64_t ca
         if (fbps != bps) return E_STREAMINFO;
         if (variable ? num != done : num != frame_no) return E_FRAMENUM;
         if (bs > max_bs) return E_STREAMINFO;
-        int e = subframe(&b, bs, bps, s, r);
+        const uint64_t hdr = (b.pos >> 3) - start;
+        parsed p;
+        int e = subframe(&b, bs, bps, s, r, &p);
         if (e) return e;
+        if (rep && frame_no < rep_cap) {
+            const uint32_t v[REPORT_FIELDS] = {(uint32_t)num, bs, (uint32_t)hdr, p.kind, p.order, p.po,
+                                               p.kmin == K_NONE ? 0 : p.kmin, p.kmax};
+            memcpy(rep + REPORT_FIELDS * frame_no, v, sizeof v);
+        }
         b.pos = (b.pos + 7) & ~7ull;
         const uint64_t crc16 = rd(&b, 16);
         if (b.err) return b.err;
@@ -246,14 +270,20 @@ static int64_t decode(const uint8_t* in, uint64_t len, int16_t* out, uint64_t ca
         frame_no++;
     }
     if (total && done != total) return E_STREAMINFO;
+    if (frames) *frames = frame_no;
     return (int64_t)done;
 }
 
-int64_t ctts_flac_decode(const uint8_t* in, uint64_t len, int16_t* out, uint64_t cap, uint64_t* info) {
+int64_t ctts_flac_decode_report(const uint8_t* in, uint64_t len, int16_t* out, uint64_t cap, uint64_t* info, uint32_t* rep,
+                                uint64_t rep_cap, uint64_t* frames) {
     int64_t* s = malloc(65536 * sizeof *s);   /* the largest blocksize */
     int64_t* r = malloc(65536 * sizeof *r);
-    const int64_t rc = s && r ? decode(in, len, out, cap, info, s, r) : E_CAPACITY;
+    const int64_t rc = s && r ? decode(in, len, out, cap, info, s, r, rep, rep_cap, frames) : E_CAPACITY;
     free(s);
     free(r);
     return rc;
+}
+
+int64_t ctts_flac_decode(const uint8_t* in, uint64_t len, int16_t* out, uint64_t cap, uint64_t* info) {
+    return ctts_flac_decode_report(in, len, out, cap, info, NULL, 0, NULL);
 }

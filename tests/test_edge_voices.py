@@ -257,3 +257,19 @@ def test_trim_runs_at_min_silence_on_every_residue(name):
         assert {47, 48, 49, 64} <= prepass, sorted(prepass)
     else:
         assert longest > 200000, longest      # beyond the shared-memory trim mask
+
+
+@pytest.mark.parametrize("name", E.SIGNAL_FAMILIES)
+def test_signal_families_deliver_their_samples(name):
+    """The pass-through the loudness and FLAC signal tests rely on: the oracle's native output of every utterance is
+    its signal bit for bit, the longest unit (6.3 minutes) included."""
+    fam = E.signal_family(name)
+    plan, prm, orc = fam.plan(), fam.prm(), fam.oracle()
+    sig = fam.info["signals"]
+    first = {}
+    for u, ws in enumerate(fam.words):
+        first.setdefault(ws[0][0], u)
+    assert len(first) == len(fam.units)   # utterances of one signal share its unit: one of them stands for all
+    for u in first.values():
+        got = orc.synth(prm, plan.utt_ops(u), 1.0)[0]
+        assert np.array_equal(got, sig[u]), f"{name}: utterance {u} ({len(sig[u])} samples) is not its signal"

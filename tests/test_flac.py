@@ -181,3 +181,109 @@ def test_library_bound_covers_every_case(H):
         assert len(F.encode(x, 22050)) <= b, name
     noise = CASES["white_noise"][:5 * 4096]   # whole frames: VERBATIM everywhere
     assert int(L.ctts_gpu_flac_bound(len(noise))) <= 1.01 * len(F.encode(noise, 22050))
+
+
+# ---------------------------------------------------------------------------------- frame numbers (RFC 9639 9.1.5)
+
+def _coded_number(v):
+    """RFC 9639's coding of a frame number: 7 bits in one byte below 2^7; else a first byte of (extra + 1) one-bits,
+    a zero and the top bits, then `extra` bytes 10xxxxxx of six bits each, with extra the least of 1 .. 6 for which
+    the value fits 6 + 5 extra bits (11 bits in two bytes, 16 in three, 21 in four)."""
+    if v < 0x80:
+        return bytes([v])
+    extra = next(e for e in range(1, 7) if v < 1 << (5 * e + 6))
+    first = (0xFF00 >> (extra + 1)) & 0xFF | v >> (6 * extra)
+    return bytes([first] + [0x80 | (v >> (6 * i)) & 0x3F for i in range(extra - 1, -1, -1)])
+
+
+def test_frame_number_coding_known_answers():
+    """A constant signal of 2 049 whole frames and one sample: every frame is CONSTANT (6-byte subframe and CRC), so
+    frame f starts at 42 + sum of the earlier frames' 4 + len(code) + 1 + 3 + 2 bytes.  The header bytes of frames
+    127, 128, 2047 and 2048 are the RFC's codes, and the decoder reads every number back."""
+    assert [_coded_number(v).hex() for v in (127, 128, 2047, 2048, 65535, 65536)] == \
+        ["7f", "c280", "dfbf", "e0a080", "efbfbf", "f0908080"]
+    n = 2049 * 4096 + 1
+    x = np.full(n, 321, np.int16)
+    data = F.encode(x, 22050)
+    at, starts = 42, []
+    for f in range(2050):
+        starts.append(at)
+        at += 4 + len(_coded_number(f)) + (1 if f == 2049 else 0) + 1 + 3 + 2   # frame 2049: 1 sample, 8-bit blocksize
+    assert at == len(data)
+    for f, code in ((127, "7f"), (128, "c280"), (2047, "dfbf"), (2048, "e0a080")):
+        assert data[starts[f]:starts[f] + 2] == b"\xff\xf8"
+        assert data[starts[f] + 4:starts[f] + 4 + len(code) // 2].hex() == code, f
+    got, info, rep = F.decode(data, report=True)
+    assert np.array_equal(got, x) and info["total_samples"] == n
+    assert rep.number.tolist() == list(range(2050))
+    assert rep.header_bytes.tolist() == [4 + len(_coded_number(f)) + (f == 2049) + 1 for f in range(2050)]
+    assert (rep.kind == F.CONSTANT).all() and rep.blocksize[-1] == 1
+
+
+# ---------------------------------------------------------------------------------- the device tests' signals
+
+def _rice_bits(z):
+    """The least bits of one partition of zigzag residuals: 4-bit parameter, then k + 1 + (u >> k) per residual."""
+    return 4 + min(len(z) * (k + 1) + int((z >> k).sum()) for k in range(15))
+
+
+def _fixed_bits(x, order, po):
+    """Partition bits of a FIXED subframe of x with the given order and partition order."""
+    r = x.astype(np.int64)
+    for _ in range(order):
+        r = np.diff(r)
+    z = np.where(r >= 0, 2 * r, -2 * r - 1)     # residuals of samples order .. n - 1
+    m = len(x) >> po
+    return sum(_rice_bits(z[max(j * m - order, 0):(j + 1) * m - order]) for j in range(1 << po))
+
+
+def _residual_sums(x):
+    r, out = x.astype(np.int64), []
+    for o in range(5):
+        out.append(int(np.abs(r[4 - o:]).sum()))
+        r = np.diff(r)
+    return out
+
+
+def test_device_signals_reach_their_decisions():
+    """CPU witness of test_gpu_flac_signals.py: the oracle's file of each constructed signal, as the decoder parsed
+    it, makes the decision the signal is built for."""
+    import edge_voices as E
+    reports = {}
+    for case, x in E.flac_signals():
+        data = F.encode(x, 22050)
+        got, _, rep = F.decode(data, report=True)
+        assert np.array_equal(got, x)
+        assert rep.blocksize.tolist() == [4096] * (len(x) // 4096) + ([len(x) % 4096] if len(x) % 4096 else [])
+        reports[case] = (x, data, rep)
+    assert reports["constant_then_fixed"][2].kind.tolist() == [F.CONSTANT] * 2 + [F.FIXED] * 2
+    x, data, rep = reports["noise"]
+    assert (rep.kind == F.VERBATIM).all() and 0.99 * F.bound(len(x)) <= len(data) <= F.bound(len(x))
+    rep = reports["half_noise"][2]
+    assert (rep.kind == F.FIXED).all() and (rep.kmin == 0).all() and (rep.kmax == 14).all()
+    x, _, rep = reports["alternating"]
+    r = x.astype(np.int64)
+    for _ in range(4):
+        r = np.diff(r)
+    assert np.abs(r).max() == 16 * 32767 + 8 and (rep.kind == F.VERBATIM).all()   # order-4 zigzag near 2^20
+    assert [reports[f"order{d}"][2].order.tolist() for d in range(5)] == [[d] for d in range(5)]
+    assert all((reports[f"order{d}"][2].kind == F.FIXED).all() for d in range(5))
+    x, _, rep = reports["ramp"]
+    assert (rep.kind == F.FIXED).all() and (rep.order == 2).all()
+    for f in range(len(rep)):
+        s = _residual_sums(x[4096 * f:4096 * (f + 1)])
+        assert s[1] > 0 and s[2] == s[3] == s[4] == 0      # orders 2, 3 and 4 tie: the lowest wins
+    binding = []
+    for r in E.FLAC_LAST:
+        x, _, rep = reports[f"last{r}"]
+        assert rep.blocksize[-1] == r and (rep.order[:-1] == 4).all()
+        last = rep[-1]
+        tail = x[-r:]
+        assert last.kind == (F.CONSTANT if r == 1 else F.VERBATIM if r <= 8 else F.FIXED)   # few samples: raw is cheaper
+        if last.kind == F.FIXED:
+            assert last.order == 4 and (r >> last.po) > 4 and r % (1 << last.po) == 0
+            # the partition order the rule (n >> po) > order rules out, with m = order samples per partition
+            po_out = next((p for p in range(9) if r % (1 << p) == 0 and r >> p == 4), None)
+            if po_out is not None and _fixed_bits(tail, 4, po_out) < _fixed_bits(tail, 4, int(last.po)):
+                binding.append(r)
+    assert 16 in binding, binding     # the rule, not the bit count, decides the last frame's partition order

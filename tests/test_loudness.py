@@ -27,21 +27,31 @@ def _product(fs):
     return shelf, hp
 
 
-def _scipy_lufs(x, fs):
-    """BS.1770-4 restated with scipy.signal.lfilter, independently of the oracle."""
+GATE_ABS = 10 ** ((-70 + 0.691) / 10)
+
+
+def _scipy_blocks(x, fs):
+    """BS.1770-4's 400 ms block energies z_j, restated with scipy.signal.lfilter independently of the oracle (empty
+    when there is no complete block)."""
     sb, sa, hb, ha = O.filter_coeffs(fs)
     y = S.lfilter(hb, ha, S.lfilter(sb, sa, np.asarray(x, np.float64) / 32768.0))
     starts = [k * fs // 10 for k in range(len(y) * 10 // fs + 2)]
     subs = [k for k in range(len(starts) - 1) if starts[k + 1] <= len(y)]
-    if len(subs) < 4:
-        return -np.inf
-    y2 = y * y
-    z = np.array([y2[starts[j]:starts[j + 4]].mean() for j in range(len(subs) - 3)])
-    z1 = z[z > 10 ** ((-70 + 0.691) / 10)]
+    c = np.concatenate([[0.0], np.cumsum(y * y)])
+    return np.array([(c[starts[j + 4]] - c[starts[j]]) / (starts[j + 4] - starts[j]) for j in range(len(subs) - 3)])
+
+
+def _gated_lufs(z):
+    z1 = z[z > GATE_ABS]
     if not len(z1):
         return -np.inf
     z2 = z1[z1 > z1.mean() / 10]
     return -0.691 + 10 * np.log10(z2.mean())
+
+
+def _scipy_lufs(x, fs):
+    """BS.1770-4 restated with scipy.signal.lfilter, independently of the oracle."""
+    return _gated_lufs(_scipy_blocks(x, fs))
 
 
 def _sine(fs, seconds, amp, f=997.0):
@@ -157,3 +167,83 @@ def test_target_reached_within_a_step():
     for target in (-16.0, -23.0, -30.0):
         y, L, G = O.normalize(x, fs, target, 0.0)
         assert abs(O.lufs(y, fs) - target) < 0.05
+
+
+# ---------------------------------------------------------------------------------- the device tests' signals
+
+def _resampled_cases(hz):
+    import edge_voices as E
+    import resample_oracle as R
+    return [(case, R.resample(x, hz)) for case, x in E.loudness_signals(hz)]
+
+
+@pytest.mark.parametrize("hz", (22050, 11025, 8015, 46035, 8001, 47971))
+def test_device_signals_reach_their_paths(hz):
+    """CPU witness of test_gpu_loudness_signals.py: at output rate hz, each constructed signal drives the gate or gain
+    decision it is built for, by the scipy restatement of the blocks; the lengths reach every sub-block count they
+    aim at; the oracle agrees with the restatement; and no utterance sits on a rounding tie of k, so the device
+    tests compare every gain."""
+    import edge_voices as E
+    cases = _resampled_cases(hz)
+    seen = set()
+    counts = sorted({len(y) for case, y in cases if case.startswith("len")})
+    for t in E.ld_counts(hz):   # every target count, or both neighbours where the conversion skips it
+        assert t in counts or (any(c < t for c in counts) and any(c > t for c in counts)), t
+    full = lambda n: (n * 10 + 10 + hz - 1) // hz - 1     # complete sub-blocks (ld_gain_kernel)
+    chunks = lambda n: (n * 10 + hz - 1) // hz
+    nbs = {max(full(len(y)) - 3, 0) for case, y in cases if case.startswith("len")}
+    assert {0, 1, 256, 257, 258} <= nbs and max(chunks(c) for c in counts) > 256
+    assert any(chunks(c) == 129 for c in counts) and any(full(c) < chunks(c) for c in counts)
+    for case, y in cases:
+        z = _scipy_blocks(y, hz)
+        L = O.lufs(y, hz)
+        assert (L == -np.inf and _gated_lufs(z) == -np.inf) or abs(L - _gated_lufs(z)) <= 1e-9, (case, L)
+        peak = int(np.abs(y.astype(np.int32)).max()) if len(y) else 0
+        for T, C in E.LD_SETTINGS:
+            assert not O.near_tie(L, T), (case, T, L)
+            _, L2, G = O.normalize(y, hz, T, C)
+            assert L2 == L
+            k = int(np.clip(np.floor(100 * (float(np.float32(T)) - L) + 0.5), -O.K_MAX, O.K_MAX)) if np.isfinite(L) else 0
+            table = int(O.table()[k + O.K_MAX])
+            lim = O.ceiling(C) * 65536 // peak if peak else None
+            if case == "two_levels":
+                z1 = z[z > GATE_ABS]
+                assert (z1 <= z1.mean() / 10).sum() >= 1    # blocks past the absolute gate, dropped by the relative one
+                seen.add(case)
+            elif case == "straddles_abs_gate":
+                assert (z <= GATE_ABS).sum() >= 1 and (z > GATE_ABS).sum() >= 1
+                seen.add(case)
+            elif case == "faint":
+                assert len(z) >= 4 and (z <= GATE_ABS).all() and G == O.UNITY    # long enough, too quiet
+                seen.add(case)
+            elif case == "last_block_burst":
+                assert np.argmax(z) == len(z) - 1 and _gated_lufs(z[:-1]) < _gated_lufs(z) - 0.5
+                seen.add(case)
+            elif case in ("lone_min", "square_burst"):
+                assert np.isfinite(L) and lim < table and G == lim    # the peak limits the gain
+                assert peak == 32768 or (case == "lone_min" and hz != 22050)   # (resampling spreads the lone sample)
+                seen.add(case)
+            elif case == "loud":
+                assert k < 0 and G == table < O.UNITY
+                seen.add(case)
+            elif case == f"unity{int(T)}":
+                assert np.isfinite(L) and G == O.UNITY and (lim is None or lim > O.UNITY)
+                seen.add(case)
+            elif case.startswith("unity"):
+                assert G != O.UNITY     # scaled under the other setting
+    assert len(seen) == 9, seen
+
+
+def test_long_utterance_spans_thousands_of_chunks():
+    import edge_voices as E
+    import resample_oracle as R
+    x = E.long_signal()
+    for hz in (22050, 11025):
+        y = x if hz == 22050 else R.resample(x, hz)
+        z = _scipy_blocks(y, hz)
+        assert len(y) * 10 // hz >= 3000 and len(y) >= 5 * 60 * hz
+        z1 = z[z > GATE_ABS]
+        assert (z <= GATE_ABS).sum() > 100 and (z1 <= z1.mean() / 10).sum() > 100   # both gates drop many blocks
+        assert abs(O.lufs(y, hz) - _gated_lufs(z)) <= 1e-9
+        for T, _ in E.LD_SETTINGS:
+            assert not O.near_tie(O.lufs(y, hz), T)
