@@ -2,13 +2,15 @@
  * ctts_b200 -- the `ctts synth` command line (ctts.c:3970-4030) over the B200 back end, in the
  * reference's own language: plain C on top of the two C-ABI libraries, no Python, no CUDA headers.
  *
- *   ctts_b200 synth <database.db> "text" <output.wav|output.flac> [speed] [rate] [lufs=<target>]
- *   ctts_b200 synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target>]     lines: speed<TAB>text
+ *   ctts_b200 synth <database.db> "text" <output.wav|output.flac> [speed] [rate] [lufs=<target> [dbtp=<ceiling>]]
+ *   ctts_b200 synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target> [dbtp=<ceiling>]]
+ *                                                                                          lines: speed<TAB>text
  *
  * rate: output sample rate in Hz (default 22050, the voice's own; ctts_gpu_set_output_rate lists the others),
  * written into the WAV header.  An output name ending in ".flac", or synth-batch's "flac", writes lossless FLAC files
  * encoded on the device (ctts_b200_synth_texts_flac) instead of 16-bit WAV.  lufs=<target> normalizes every utterance
- * to <target> LUFS (ITU-R BS.1770-4, in [-60, -5]) with its sample peak held to -1 dBFS (ctts_gpu_set_loudness).
+ * to <target> LUFS (ITU-R BS.1770-4, in [-60, -5]) with its sample peak held to -1 dBFS (ctts_gpu_set_loudness);
+ * dbtp=<ceiling> next to it holds the true peak to <ceiling> dBTP instead (in [-20, 0], ctts_gpu_set_loudness_true_peak).
  *
  * Like the reference it reads config.yaml and normalization.csv from the working directory
  * (ctts.c:3990, :3636), clamps the speed to [0.5, 2.0] (ctts.c:3976-3981) and takes default_speed
@@ -27,6 +29,12 @@
 
 #define SAMPLE_RATE CTTS_PLAN_SAMPLE_RATE
 
+/* the loudness options: lufs = 0 without lufs=; true_peak when dbtp= was given */
+typedef struct {
+    float lufs, dbtp;
+    int true_peak;
+} loudness_arg;
+
 typedef struct {
     void* db;
     size_t db_size;
@@ -44,7 +52,7 @@ static void engine_close(engine* e) {
 }
 
 /* ctts_init (ctts.c:1117) + ctts_load_config("config.yaml") + the rule table, for both halves */
-static int engine_open(engine* e, const char* db_path, uint32_t rate, float lufs) {
+static int engine_open(engine* e, const char* db_path, uint32_t rate, const loudness_arg* ld) {
     memset(e, 0, sizeof *e);
     FILE* f = fopen(db_path, "rb");
     if (!f) return -1;
@@ -75,8 +83,9 @@ static int engine_open(engine* e, const char* db_path, uint32_t rate, float lufs
         engine_close(e);
         return rc;
     }
-    if (lufs != 0.0f && (rc = ctts_gpu_set_loudness(e->gpu, lufs, -1.0f)) != 0) {
-        fprintf(stderr, "loudness target %g LUFS: %s\n", (double)lufs, ctts_gpu_last_error(e->gpu));
+    if (ld->lufs != 0.0f && (rc = ld->true_peak ? ctts_gpu_set_loudness_true_peak(e->gpu, ld->lufs, ld->dbtp)
+                                                : ctts_gpu_set_loudness(e->gpu, ld->lufs, -1.0f)) != 0) {
+        fprintf(stderr, "loudness target %g LUFS: %s\n", (double)ld->lufs, ctts_gpu_last_error(e->gpu));
         engine_close(e);
         return rc;
     }
@@ -84,16 +93,30 @@ static int engine_open(engine* e, const char* db_path, uint32_t rate, float lufs
     return 0;
 }
 
-/* An optional last argument lufs=<target> (after the output argument): taken off the argument list.  *lufs = 0 without one; -1 when it is not a
- * number (any other value is checked by ctts_gpu_set_loudness). */
-static int take_lufs(int* argc, char** argv, float* lufs) {
-    *lufs = 0.0f;
-    if (*argc < 6 || strncmp(argv[*argc - 1], "lufs=", 5) != 0) return 0;   /* behind the required arguments only */
-    const char* v = argv[*argc - 1] + 5;
-    char* end = NULL;
-    *lufs = strtof(v, &end);
-    (*argc)--;
-    return (*v && end && *end == '\0') ? 0 : -1;
+/* Optional last arguments lufs=<target> and dbtp=<ceiling>, in either order (after the output argument): taken off the
+ * argument list.  ld->lufs = 0 without lufs=; -1 when a value is not a number, an option repeats or dbtp= comes
+ * without lufs= (any other value is checked by ctts_gpu_set_loudness(_true_peak)). */
+static int take_lufs(int* argc, char** argv, loudness_arg* ld) {
+    memset(ld, 0, sizeof *ld);
+    int have_lufs = 0;
+    while (*argc >= 6) {   /* behind the required arguments only */
+        const char* a = argv[*argc - 1];
+        const int is_lufs = strncmp(a, "lufs=", 5) == 0, is_dbtp = strncmp(a, "dbtp=", 5) == 0;
+        if (!is_lufs && !is_dbtp) break;
+        if (is_lufs ? have_lufs : ld->true_peak) return -1;
+        char* end = NULL;
+        const float v = strtof(a + 5, &end);
+        if (!a[5] || !end || *end != '\0') return -1;
+        if (is_lufs) {
+            ld->lufs = v;
+            have_lufs = 1;
+        } else {
+            ld->dbtp = v;
+            ld->true_peak = 1;
+        }
+        (*argc)--;
+    }
+    return ld->true_peak && !have_lufs ? -1 : 0;
 }
 
 /* ctts_write_wav, ctts.c:809: 44-byte RIFF/WAVE header (PCM, mono, 16 bit) + samples */
@@ -177,16 +200,16 @@ static uint32_t parse_rate(const char* a) {
 }
 
 static int cmd_synth(int argc, char** argv) {
-    float lufs;
-    if (take_lufs(&argc, argv, &lufs) || argc < 5 || argc > 7) {
-        fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed] [rate] [lufs=<target>]\n", argv[0]);
+    loudness_arg ld;
+    if (take_lufs(&argc, argv, &ld) || argc < 5 || argc > 7) {
+        fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed] [rate] [lufs=<target> [dbtp=<ceiling>]]\n", argv[0]);
         return 1;
     }
     float speed = 1.0f;
     if (argc > 5) speed = clamp_speed(strtof(argv[5], NULL));
     const uint32_t rate = argc > 6 ? parse_rate(argv[6]) : SAMPLE_RATE;
     engine e;
-    if (engine_open(&e, argv[2], rate, lufs)) {
+    if (engine_open(&e, argv[2], rate, &ld)) {
         fprintf(stderr, "Failed to load database: %s\n", argv[2]);
         return 1;
     }
@@ -232,9 +255,9 @@ static void write_chunk(void* user, uint32_t u0, uint32_t u1) {
 }
 
 static int cmd_synth_batch(int argc, char** argv) {
-    float lufs;
-    if (take_lufs(&argc, argv, &lufs) || argc < 5 || argc > 7 || (argc == 7 && strcmp(argv[6], "flac") != 0)) {
-        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target>]\n", argv[0]);
+    loudness_arg ld;
+    if (take_lufs(&argc, argv, &ld) || argc < 5 || argc > 7 || (argc == 7 && strcmp(argv[6], "flac") != 0)) {
+        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target> [dbtp=<ceiling>]]\n", argv[0]);
         return 1;
     }
     const uint32_t rate = argc > 5 ? parse_rate(argv[5]) : SAMPLE_RATE;
@@ -266,7 +289,7 @@ static int cmd_synth_batch(int argc, char** argv) {
     free(line);
     fclose(f);
     engine e;
-    if (engine_open(&e, argv[2], rate, lufs)) {
+    if (engine_open(&e, argv[2], rate, &ld)) {
         fprintf(stderr, "Failed to load database: %s\n", argv[2]);
         return 1;
     }
@@ -296,7 +319,7 @@ static int cmd_synth_batch(int argc, char** argv) {
 int main(int argc, char** argv) {
     if (argc >= 2 && strcmp(argv[1], "synth") == 0) return cmd_synth(argc, argv);
     if (argc >= 2 && strcmp(argv[1], "synth-batch") == 0) return cmd_synth_batch(argc, argv);
-    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav|output.flac> [speed] [rate] [lufs=<target>]\n       %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target>]\n",
+    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav|output.flac> [speed] [rate] [lufs=<target> [dbtp=<ceiling>]]\n       %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target> [dbtp=<ceiling>]]\n",
             argv[0], argv[0]);
     return 1;
 }

@@ -31,6 +31,7 @@ extern "C" void ctts_host_resample_taps(unsigned L, unsigned M, float* g);
 extern "C" void ctts_host_loudness_filter(unsigned fs, double* shelf, double* hp);
 extern "C" void ctts_host_loudness_gains(unsigned* table);
 extern "C" unsigned ctts_host_loudness_ceiling(float ceiling_dbfs);
+extern "C" void ctts_host_true_peak_taps(float* h);
 
 // Launch geometry of resample_kernel for the reduced ratio L/M (host only, no CUDA call; tests restate the kernel's
 // tile arithmetic against it): kp taps per phase row (a multiple of 4), the filter delay c, the staging bound
@@ -150,8 +151,10 @@ struct ctts_gpu_ctx {
     struct LdTable {
         uint32_t hz = 0;
         float target = 0, ceiling = 0;
+        bool true_peak = false;     // the ceiling holds the true (4x oversampled) peak, not the sample peak
         uint32_t ceiling_q = 0;     // A
         ctts::LdFilter f{};         // the K-weighting at hz and its transitions (kernel parameters)
+        float tp_h[3][12] = {};     // true_peak: the interpolator's phases 1 .. 3 as LdArgs::tp_h lays them out
     };
     std::vector<LdTable*> ld_tables;
     LdTable* ld = nullptr;          // nullptr: the stage is off
@@ -216,13 +219,16 @@ struct ctts_gpu_plan {
     uint32_t rs_tiles = 0;                 // rs: grid.x of resample_kernel
     int16_t* d_nat_owned = nullptr;        // resident plan with rs: its native slots
     const ctts_gpu_ctx::LdTable* ld = nullptr;   // loudness setting the plan was created under (nullptr: off)
-    unsigned long long* d_ld_off = nullptr;      // ld: output-rate slot offsets [n + 1], then first chunks [n + 1]
+    unsigned long long* d_ld_off = nullptr;      // ld: output-rate slot offsets [n + 1], then first chunks [n + 1] (+ first tiles [n + 1] for a true peak)
     double* d_ld_state = nullptr;                // ld: 4 per chunk
     double* d_ld_energy = nullptr;               // ld: per chunk
     uint32_t* d_ld_peak = nullptr;               // ld: per chunk
     double* d_ld_lufs = nullptr;                 // ld: per utterance
     uint32_t* d_ld_gain = nullptr;               // ld: per utterance
     uint32_t ld_tiles = 0, ld_apply_tiles = 0;   // ld: grid.x of the chunk passes and of ld_apply_kernel
+    float* d_ld_tp_tile = nullptr;               // ld->true_peak: per (utterance, tile) of ld_true_peak_kernel
+    float* d_ld_tp = nullptr;                    // ld->true_peak: P per utterance
+    uint32_t ld_tp_tiles = 0;                    // ld->true_peak: grid.x of ld_true_peak_kernel
     Arena* arena = nullptr;         // device buffers live in a lane's arena (batch path); else cudaMalloc'ed
     uint32_t op0 = 0;               // first op of the plan's utterances in the caller's op array (ops are kept from there on)
     std::vector<void*> owned;       // else: cudaMalloc'ed buffers to free
@@ -597,10 +603,10 @@ namespace {
 
 // The loudness setting (target, ceiling) at the context's current output rate: found among the context's tables or
 // built.  The transitions A^len of the scan come from running the cascade itself on the unit states.
-void ld_select(ctts_gpu_ctx* ctx, float target, float ceiling) {
+void ld_select(ctts_gpu_ctx* ctx, float target, float ceiling, bool true_peak) {
     const uint32_t hz = ctx->rs ? ctx->rs->hz : (uint32_t)CTTS_PLAN_SAMPLE_RATE;
     for (ctts_gpu_ctx::LdTable* t : ctx->ld_tables)
-        if (t->hz == hz && t->target == target && t->ceiling == ceiling) {
+        if (t->hz == hz && t->target == target && t->ceiling == ceiling && t->true_peak == true_peak) {
             ctx->ld = t;
             return;
         }
@@ -608,7 +614,14 @@ void ld_select(ctts_gpu_ctx* ctx, float target, float ceiling) {
     t->hz = hz;
     t->target = target;
     t->ceiling = ceiling;
+    t->true_peak = true_peak;
     t->ceiling_q = ctts_host_loudness_ceiling(ceiling);
+    if (true_peak) {
+        float h[49];
+        ctts_host_true_peak_taps(h);
+        for (int r = 1; r <= 3; r++)
+            for (int i = 0; i < 12; i++) t->tp_h[r - 1][i] = h[44 - 4 * i + r];
+    }
     double shelf[5], hp[2];
     ctts_host_loudness_filter(hz, shelf, hp);
     ctts::LdFilter& f = t->f;
@@ -638,7 +651,7 @@ void ld_select(ctts_gpu_ctx* ctx, float target, float ceiling) {
 
 // after a change of the output rate: the loudness setting moves to the new rate
 int ld_follow_rate(ctts_gpu_ctx* ctx) {
-    if (ctx->ld) ld_select(ctx, ctx->ld->target, ctx->ld->ceiling);
+    if (ctx->ld) ld_select(ctx, ctx->ld->target, ctx->ld->ceiling, ctx->ld->true_peak);
     return CTTS_GPU_OK;
 }
 
@@ -699,12 +712,13 @@ int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz) {
     return ld_follow_rate(ctx);
 }
 
-int ctts_gpu_set_loudness(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_dbfs) {
+// ctts_gpu_set_loudness and ctts_gpu_set_loudness_true_peak: the same rules, the ceiling kind apart
+static int ld_set(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_db, bool true_peak) {
     if (!ctx) return CTTS_GPU_ERR_INVALID_ARG;
     if (!std::isfinite(target_lufs) || (target_lufs != 0.0f && (target_lufs < -60.0f || target_lufs > -5.0f)))
         return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "loudness target %g LUFS: neither 0 nor in [-60, -5]", (double)target_lufs);
-    if (!std::isfinite(ceiling_dbfs) || ceiling_dbfs < -20.0f || ceiling_dbfs > 0.0f)
-        return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "peak ceiling %g dBFS outside [-20, 0]", (double)ceiling_dbfs);
+    if (!std::isfinite(ceiling_db) || ceiling_db < -20.0f || ceiling_db > 0.0f)
+        return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "peak ceiling %g %s outside [-20, 0]", (double)ceiling_db, true_peak ? "dBTP" : "dBFS");
     if (ctx->session) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "the loudness setting cannot change while a session is open");
     if (target_lufs == 0.0f) {
         ctx->ld = nullptr;
@@ -722,8 +736,16 @@ int ctts_gpu_set_loudness(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_db
             return fail(ctx, CTTS_GPU_ERR_CUDA, "loudness gain table: %s", cudaGetErrorString(e));
         }
     }
-    ld_select(ctx, target_lufs, ceiling_dbfs);
+    ld_select(ctx, target_lufs, ceiling_db, true_peak);
     return CTTS_GPU_OK;
+}
+
+int ctts_gpu_set_loudness(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_dbfs) {
+    return ld_set(ctx, target_lufs, ceiling_dbfs, false);
+}
+
+int ctts_gpu_set_loudness_true_peak(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_dbtp) {
+    return ld_set(ctx, target_lufs, ceiling_dbtp, true);
 }
 
 const char* ctts_gpu_last_error(const ctts_gpu_ctx* ctx) { return ctx ? ctx->err : g_init_err; }
@@ -1019,7 +1041,9 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     // loudness: one chunk per 100 ms sub-block that can start before the bound
     const ctts_gpu_ctx::LdTable* const ld = ctx->ld;
     p->ld = ld;
-    std::vector<uint64_t> ld_chunk0;
+    // (true peak: and one ld_true_peak_kernel tile per LD_TP_TILE positions -6 .. bound + 5)
+    std::vector<uint64_t> ld_chunk0, ld_tile0;
+    const bool tp = ld && ld->true_peak;
     if (ld) {
         ld_chunk0.resize((size_t)n + 1, 0);
         uint64_t max_chunks = 0, max_bound = 0;
@@ -1031,6 +1055,11 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         }
         p->ld_tiles = (uint32_t)std::max<uint64_t>((max_chunks + ctts::LD_THREADS - 1) / ctts::LD_THREADS, 1);
         p->ld_apply_tiles = (uint32_t)std::max<uint64_t>((max_bound + ctts::LD_APPLY_TILE - 1) / ctts::LD_APPLY_TILE, 1);
+        if (tp) {
+            ld_tile0.resize((size_t)n + 1, 0);
+            for (uint32_t u = 0; u < n; u++) ld_tile0[u + 1] = ld_tile0[u] + ctts::ld_tp_tiles(bound[u]);
+            p->ld_tp_tiles = (uint32_t)ctts::ld_tp_tiles(max_bound);
+        }
     }
 
     // ---- shared-memory geometry
@@ -1135,12 +1164,16 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         }
         if (ld) {
             const uint64_t chunks = ld_chunk0[n];
-            p->d_ld_off = al.dev<unsigned long long>(2 * ((size_t)n + 1));
+            p->d_ld_off = al.dev<unsigned long long>((tp ? 3 : 2) * ((size_t)n + 1));
             p->d_ld_state = al.dev<double>(4 * chunks);
             p->d_ld_energy = al.dev<double>(chunks);
             p->d_ld_peak = al.dev<uint32_t>(chunks);
             p->d_ld_lufs = al.dev<double>(n);
             p->d_ld_gain = al.dev<uint32_t>(n);
+            if (tp) {
+                p->d_ld_tp_tile = al.dev<float>(ld_tile0[n]);
+                p->d_ld_tp = al.dev<float>(n);
+            }
         }
         if (p->n_stretch) {
             p->d_stasks = al.dev<ctts::StretchTask>(stasks.size());
@@ -1158,7 +1191,7 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
             h_of = al.host<uint32_t>(ola_first.size());
         }
         if (rs) h_ro = al.host<unsigned long long>(2 * ((size_t)n + 1));
-        if (ld) h_lo = al.host<unsigned long long>(2 * ((size_t)n + 1));
+        if (ld) h_lo = al.host<unsigned long long>((tp ? 3 : 2) * ((size_t)n + 1));
     };
     PlanAlloc al{p, true};
     layout(al);
@@ -1216,8 +1249,9 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         for (uint32_t u = 0; u <= n; u++) {
             h_lo[u] = p->offsets[u];
             h_lo[n + 1 + u] = ld_chunk0[u];
+            if (tp) h_lo[2 * ((size_t)n + 1) + u] = ld_tile0[u];
         }
-        CUP(cudaMemcpyAsync(p->d_ld_off, h_lo, 2 * ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, st));
+        CUP(cudaMemcpyAsync(p->d_ld_off, h_lo, (tp ? 3 : 2) * ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, st));
     }
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ctts::assemble_kernel, ctts::ASM_THREADS, p->smem_bytes) != cudaSuccess || occ < 1)
@@ -1230,7 +1264,7 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
                                    (p->n_ola_blocks ? 1 : 0);
     if (rs) p->info.kernel_launches += (uint32_t)(((uint64_t)n + 65534) / 65535);   // resample_kernel
     if (ld && n)   // the two chunk passes and ld_apply_kernel per grid.y slice, ld_scan_kernel, ld_gain_kernel
-        p->info.kernel_launches += 3 * (uint32_t)(((uint64_t)n + 65534) / 65535) + 2;
+        p->info.kernel_launches += (tp ? 4 : 3) * (uint32_t)(((uint64_t)n + 65534) / 65535) + 2;   // + ld_true_peak_kernel
     p->info.n_stretch = p->n_stretch;
     p->info.bound_samples = std::accumulate(bound.begin(), bound.end(), (uint64_t)0);
     p->info.smem_bytes = p->smem_bytes;
@@ -1849,6 +1883,11 @@ int launch_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_final, cudaS
     a.ceiling = ld->ceiling_q;
     a.target = ld->target;
     a.f = ld->f;
+    if (ld->true_peak) {
+        a.tp_tile = p->d_ld_tp_tile;
+        a.tp_peak = p->d_ld_tp;
+        memcpy(a.tp_h, ld->tp_h, sizeof a.tp_h);
+    }
     auto sliced = [&](auto kernel, uint32_t tiles, int threads) -> int {
         for (uint32_t u0 = 0; u0 < n; u0 += 65535u) {   // grid.y limit
             a.u0 = u0;
@@ -1863,7 +1902,12 @@ int launch_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_final, cudaS
     ctts::ld_scan_kernel<<<(n + ctts::LD_SCAN_THREADS - 1) / ctts::LD_SCAN_THREADS, ctts::LD_SCAN_THREADS, 0, st>>>(a);
     CU(ctx, cudaGetLastError());
     if ((rc = sliced(ctts::ld_chunk_kernel<true>, p->ld_tiles, ctts::LD_THREADS)) != 0) return rc;
-    ctts::ld_gain_kernel<<<n, ctts::LD_GAIN_THREADS, 0, st>>>(a);
+    if (ld->true_peak) {
+        if ((rc = sliced(ctts::ld_true_peak_kernel, p->ld_tp_tiles, ctts::LD_TP_THREADS)) != 0) return rc;
+        ctts::ld_gain_kernel<true><<<n, ctts::LD_GAIN_THREADS, 0, st>>>(a);
+    } else {
+        ctts::ld_gain_kernel<false><<<n, ctts::LD_GAIN_THREADS, 0, st>>>(a);
+    }
     CU(ctx, cudaGetLastError());
     return sliced(ctts::ld_apply_kernel, p->ld_apply_tiles, ctts::LD_APPLY_THREADS);
 }
@@ -1952,6 +1996,16 @@ int ctts_gpu_plan_read_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, double* luf
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, cudaMemcpyAsync(lufs, p->d_ld_lufs, (size_t)p->n_utts * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaMemcpyAsync(gain, p->d_ld_gain, (size_t)p->n_utts * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return CTTS_GPU_OK;
+}
+
+int ctts_gpu_plan_read_true_peak(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, float* peak) {
+    if (!ctx || !p || p->ctx != ctx || !peak) return CTTS_GPU_ERR_INVALID_ARG;
+    if (!p->ld || !p->ld->true_peak) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "the plan was not created with a true-peak ceiling");
+    if (p->n_utts == 0) return CTTS_GPU_OK;
+    CU(ctx, cudaSetDevice(ctx->device));
+    CU(ctx, cudaMemcpyAsync(peak, p->d_ld_tp, (size_t)p->n_utts * 4, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return CTTS_GPU_OK;
 }
@@ -2476,7 +2530,7 @@ int ctts_gpu_multi_synth_batch(ctts_gpu_ctx* const* ctxs, uint32_t n_ctx, const 
             return fail(ctxs[0], CTTS_GPU_ERR_INVALID_ARG, "context %u has another output rate than context 0", d);
     for (uint32_t d = 1; d < n_ctx; d++) {
         const ctts_gpu_ctx::LdTable *a = ctxs[d]->ld, *b = ctxs[0]->ld;
-        if ((a == nullptr) != (b == nullptr) || (a && (a->target != b->target || a->ceiling != b->ceiling)))
+        if ((a == nullptr) != (b == nullptr) || (a && (a->target != b->target || a->ceiling != b->ceiling || a->true_peak != b->true_peak)))
             return fail(ctxs[0], CTTS_GPU_ERR_INVALID_ARG, "context %u has another loudness setting than context 0", d);
     }
     if (plan->n_utts && (!plan->utt_op_begin || !plan->speed)) return CTTS_GPU_ERR_INVALID_ARG;

@@ -89,3 +89,15 @@ void ctts_host_loudness_gains(unsigned* table) {
 unsigned ctts_host_loudness_ceiling(float ceiling_dbfs) {
     return (unsigned)floor(32767.0 * pow(10.0, (double)ceiling_dbfs / 20.0));
 }
+
+/* The true-peak interpolator (DESIGN.md 3.6): 4x oversampling, 49 taps, the windowed sinc libebur128 uses below
+ * 96 kHz.  h[j] = sinc((j - 24) / 4) * 0.5 * (1 - cos(2 pi j / 48)), j = 0 .. 48, in double; |h[j]| <= 1e-9 becomes
+ * exactly 0 (the non-centre taps of phase 0, so phase j mod 4 = 0 is the identity); each tap is rounded to float once. */
+void ctts_host_true_peak_taps(float* h) {
+    for (int j = 0; j <= 48; j++) {
+        const double t = (double)(j - 24) / 4.0;
+        const double s = j == 24 ? 1.0 : sin(CTTS_PI * t) / (CTTS_PI * t);
+        const double v = s * 0.5 * (1.0 - cos(2.0 * CTTS_PI * (double)j / 48.0));
+        h[j] = fabs(v) <= 1e-9 ? 0.0f : (float)v;
+    }
+}

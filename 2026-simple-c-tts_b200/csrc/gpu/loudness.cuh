@@ -1,6 +1,7 @@
 // loudness.cuh -- loudness normalization of every utterance (DESIGN.md 3.6): integrated loudness after
 // ITU-R BS.1770-4 (K-weighting, 400 ms blocks, absolute and relative gates), one Q16 gain per utterance that reaches
-// the target without the sample peak exceeding the ceiling, applied in place on the output-rate slots.
+// the target without the sample peak (or, under a true-peak setting, the 4x oversampled peak of BS.1770-4 Annex 2)
+// exceeding the ceiling, applied in place on the output-rate slots.
 //
 // The K-weighting is an IIR cascade in double, sequential by nature.  It is cut into chunks, one per 100 ms
 // sub-block k = [floor(k*fs/10), floor((k+1)*fs/10)) (the last one clipped at the count):
@@ -8,6 +9,7 @@
 //   ld_scan_kernel          per utterance, the true start state of every chunk: s_{k+1} = A^len_k s_k + e_k, with the
 //                           zero-input transitions A^lo, A^(lo+1) of the two sub-block lengths tabulated on the host
 //   ld_chunk_kernel<true>   every chunk again from its true state: sum of y^2
+//   ld_true_peak_kernel     true-peak plans only: max |v| of the 4x oversampled signal per tile of 2048 positions
 //   ld_gain_kernel          per utterance: block energies, both gates, L, the gain
 //   ld_apply_kernel         y = (x * G + 32768) >> 16 in place, skipped where G is unity
 // The filter state of a chunk is not its exact sequential value (the scan reassociates the recurrence), so L agrees
@@ -26,6 +28,11 @@ constexpr int LD_SCAN_BATCH = 8;       // chunk end states loaded ahead of the s
 constexpr int LD_GAIN_THREADS = 256;   // one CTA per utterance
 constexpr int LD_APPLY_THREADS = 256;
 constexpr uint32_t LD_APPLY_TILE = 8u * LD_APPLY_THREADS * 4u;
+constexpr int LD_TP_THREADS = 256;
+constexpr int LD_TP_PER = 8;           // consecutive positions per thread, from one register window
+constexpr uint32_t LD_TP_TILE = LD_TP_THREADS * LD_TP_PER;
+constexpr int LD_TP_HALO = 6;          // samples staged on each side of a tile
+constexpr uint32_t LD_TP_STAGE = LD_TP_TILE + 2 * LD_TP_HALO;
 constexpr int LD_K_MAX = 8000;         // gain table: k = -LD_K_MAX .. LD_K_MAX hundredths of a dB
 constexpr uint32_t LD_UNITY = 65536;   // G = 1 in Q16: y == x
 
@@ -58,6 +65,7 @@ __host__ __device__ __forceinline__ double ld_step(const LdFilter& f, LdState& s
 struct LdArgs {
     int16_t* pcm;                     // output-rate slots, scaled in place by ld_apply_kernel
     const unsigned long long* off;    // slot offsets [n + 1], then the first chunk of every utterance [n + 1]
+                                      // (true peak: then its first ld_true_peak_kernel tile [n + 1])
     const uint32_t* counts;           // output-rate counts
     double* state;                    // 4 per chunk: zero-state end state, overwritten by the scan with the start state
     double* energy;                   // per chunk: sum of y^2
@@ -71,6 +79,10 @@ struct LdArgs {
     uint32_t ceiling;                 // A = floor(32767 * 10^(C / 20))
     float target;                     // T, LUFS
     LdFilter f;
+    // true-peak plans only (the fields above keep their offsets, so the sample-peak kernels are unchanged)
+    float* tp_tile;                   // per (utterance, tile): max |v| over the tile's positions
+    float* tp_peak;                   // per utterance: P
+    float tp_h[3][12];                // phases r = 1 .. 3: tp_h[r - 1][i] = h[44 - 4i + r], the tap of x[q - 5 + i]
 };
 
 __device__ __forceinline__ unsigned long long ld_sub_start(unsigned long long k, uint32_t fs) { return k * fs / 10u; }
@@ -178,7 +190,60 @@ __global__ void __launch_bounds__(LD_SCAN_THREADS) ld_scan_kernel(LdArgs a) {
     }
 }
 
-// One CTA per utterance: the gated mean of the 400 ms block energies, L, and G = min(table[k], A * 65536 / P).
+// Tiles of the true-peak pass of an utterance of cnt samples: positions q = -6 .. cnt + 5 in tiles of LD_TP_TILE.
+__host__ __device__ __forceinline__ unsigned long long ld_tp_tiles(unsigned long long cnt) {
+    return (cnt + 2 * LD_TP_HALO + LD_TP_TILE - 1) / LD_TP_TILE;
+}
+
+// Utterance u0 + blockIdx.y, positions q = blockIdx.x * LD_TP_TILE - 6 + [0, LD_TP_TILE): for every q the phases
+// v[4q + r] = sum over j = q - 5 .. q + 6 (ascending) of x[j] * h[4(q - j) + r + 24], r = 1 .. 3, one fmaf per term
+// from 0.0f, and v[4q] = x[q]; the tile's max |v| goes to tp_tile at the utterance's first tile (off[2(n + 1) + u])
+// plus blockIdx.x.  Samples outside [0, cnt) read as zeros, so positions past cnt + 5 add nothing.  The staged
+// samples are stored at l + l / 8: thread t reads its 19-sample window l = 8t + 1 .. 8t + 19 at stride 9 words,
+// conflict-free.  Every |v| is a non-negative float, whose bits order like its value: the maximum is exact.
+__global__ void __launch_bounds__(LD_TP_THREADS) ld_true_peak_kernel(LdArgs a) {
+    __shared__ float stage[LD_TP_STAGE + LD_TP_STAGE / 8 + 1];
+    __shared__ unsigned red[LD_TP_THREADS / 32];
+    const uint32_t u = a.u0 + blockIdx.y;
+    const long long cnt = a.counts[u];
+    const long long t0 = (long long)blockIdx.x * LD_TP_TILE;
+    if ((unsigned long long)t0 >= (unsigned long long)cnt + 2 * LD_TP_HALO) return;   // the whole CTA
+    const int16_t* x = a.pcm + a.off[u];
+    const long long j0 = t0 - 2 * LD_TP_HALO;   // sample of stage position 0 (positions start at t0 - 6)
+    for (uint32_t l = threadIdx.x; l < LD_TP_STAGE; l += LD_TP_THREADS) {
+        const long long j = j0 + l;
+        stage[l + l / 8] = (j >= 0 && j < cnt) ? (float)x[j] : 0.0f;
+    }
+    __syncthreads();
+    const uint32_t b = LD_TP_PER * threadIdx.x + 1;
+    float w[LD_TP_PER + 11];
+#pragma unroll
+    for (int k = 0; k < LD_TP_PER + 11; k++) w[k] = stage[b + k + (b + k) / 8];
+    float m = 0.0f;
+#pragma unroll
+    for (int p = 0; p < LD_TP_PER; p++) {
+        m = fmaxf(m, fabsf(w[p + 5]));   // phase 0: x[q]
+#pragma unroll
+        for (int r = 0; r < 3; r++) {
+            float v = 0.0f;
+#pragma unroll
+            for (int i = 0; i < 12; i++) v = __fmaf_rn(w[p + i], a.tp_h[r][i], v);
+            m = fmaxf(m, fabsf(v));
+        }
+    }
+    const unsigned wm = __reduce_max_sync(0xffffffffu, __float_as_uint(m));
+    if ((threadIdx.x & 31u) == 0) red[threadIdx.x >> 5] = wm;
+    __syncthreads();
+    if (threadIdx.x) return;
+    unsigned bits = red[0];
+#pragma unroll
+    for (int k = 1; k < LD_TP_THREADS / 32; k++) bits = max(bits, red[k]);
+    a.tp_tile[a.off[2 * (a.n + 1) + u] + blockIdx.x] = __uint_as_float(bits);
+}
+
+// One CTA per utterance: the gated mean of the 400 ms block energies, L, and G = min(table[k], A * 65536 / P) with
+// the sample peak P; TRUE_PEAK: G = min(table[k], floor((A - 1) * 65536 / P)) with the true peak P, which is stored.
+template <bool TRUE_PEAK>
 __global__ void __launch_bounds__(LD_GAIN_THREADS) ld_gain_kernel(LdArgs a) {
     __shared__ double red_d[LD_GAIN_THREADS / 32];
     __shared__ unsigned red_u[LD_GAIN_THREADS / 32];
@@ -191,7 +256,12 @@ __global__ void __launch_bounds__(LD_GAIN_THREADS) ld_gain_kernel(LdArgs a) {
     const unsigned long long full = min(((unsigned long long)cnt * 10u + 10u + fs - 1u) / fs - 1u, nch);
     const unsigned long long nb = full >= 4 ? full - 3 : 0;
     unsigned pk = 0;
-    for (unsigned long long k = threadIdx.x; k < nch; k += LD_GAIN_THREADS) pk = max(pk, a.peak[c0 + k]);
+    if (TRUE_PEAK) {
+        const unsigned long long t0 = a.off[2 * (a.n + 1) + u], nt = ld_tp_tiles(cnt);
+        for (unsigned long long t = threadIdx.x; t < nt; t += LD_GAIN_THREADS) pk = max(pk, __float_as_uint(a.tp_tile[t0 + t]));
+    } else {
+        for (unsigned long long k = threadIdx.x; k < nch; k += LD_GAIN_THREADS) pk = max(pk, a.peak[c0 + k]);
+    }
     pk = block_allreduce<LD_GAIN_THREADS>(pk, LdMaxU{}, red_u);
     const double* E = a.energy + c0;
     auto z_of = [&](unsigned long long j) {
@@ -223,14 +293,21 @@ __global__ void __launch_bounds__(LD_GAIN_THREADS) ld_gain_kernel(LdArgs a) {
         L = -0.691 + 10.0 * log10(sum2 / (double)m2);
         const double k = fmin(fmax(floor(100.0 * ((double)a.target - L) + 0.5), (double)-LD_K_MAX), (double)LD_K_MAX);
         G = a.table[(int)k + LD_K_MAX];
-        if (pk) G = (uint32_t)min((unsigned long long)G, (unsigned long long)a.ceiling * LD_UNITY / pk);
+        if (TRUE_PEAK) {
+            // exact operands: (A - 1) * 65536 < 2^31 and a float P; the quotient is rounded once, then floored
+            if (pk) G = (uint32_t)fmin((double)G, floor((double)(a.ceiling - 1u) * (double)LD_UNITY / (double)__uint_as_float(pk)));
+        } else {
+            if (pk) G = (uint32_t)min((unsigned long long)G, (unsigned long long)a.ceiling * LD_UNITY / pk);
+        }
     }
     a.lufs[u] = L;
     a.gain[u] = G;
+    if (TRUE_PEAK) a.tp_peak[u] = __uint_as_float(pk);
 }
 
 // Utterance u0 + blockIdx.y, tile blockIdx.x of LD_APPLY_TILE samples, 16-byte vectors (slots start 16-byte aligned).
-// Samples past the count are left as they are.  |y| <= A follows from G <= A * 65536 / P: no saturation.
+// Samples past the count are left as they are.  |y| <= A follows from G <= A * 65536 / P (sample peak) and from the
+// true-peak guarantee of DESIGN.md 5: no saturation.
 __global__ void __launch_bounds__(LD_APPLY_THREADS) ld_apply_kernel(LdArgs a) {
     const uint32_t u = a.u0 + blockIdx.y;
     const uint32_t G = a.gain[u];

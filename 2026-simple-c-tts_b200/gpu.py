@@ -55,6 +55,8 @@ def lib(build: bool = True) -> C.CDLL:
         L.ctts_gpu_set_output_rate.argtypes = [vp, C.c_uint32]
         L.ctts_gpu_set_loudness.argtypes = [vp, C.c_float, C.c_float]
         L.ctts_gpu_plan_read_loudness.argtypes = [vp, vp, vp, vp]
+        L.ctts_gpu_set_loudness_true_peak.argtypes = [vp, C.c_float, C.c_float]
+        L.ctts_gpu_plan_read_true_peak.argtypes = [vp, vp, vp]
         L.ctts_gpu_last_error.argtypes = [vp]
         L.ctts_gpu_last_error.restype = C.c_char_p
         L.ctts_gpu_plan_bounds.argtypes = [vp, C.POINTER(CBatchPlan), vp]
@@ -149,6 +151,13 @@ class ResidentPlan:
         self._ctx._check(lib().ctts_gpu_plan_read_loudness(self._ctx._h, self._h, lufs.ctypes.data, gain.ctypes.data))
         return lufs[:self.n_utts], gain[:self.n_utts]
 
+    def true_peak(self) -> np.ndarray:
+        """After a run of a plan created under a true-peak ceiling (ctts_gpu_plan_read_true_peak): every utterance's
+        true peak P (4x oversampled, int16 units, float32) before the gain."""
+        peak = np.zeros(max(self.n_utts, 1), dtype=np.float32)
+        self._ctx._check(lib().ctts_gpu_plan_read_true_peak(self._ctx._h, self._h, peak.ctypes.data))
+        return peak[:self.n_utts]
+
     def read_pre(self, u: int, cap: int) -> np.ndarray:
         out = np.zeros(max(cap, 1), dtype=np.int16)
         n = C.c_uint64()
@@ -210,11 +219,13 @@ class GpuSynth:
         samples of that rate.  Plans created before keep their rate."""
         self._check(lib().ctts_gpu_set_output_rate(self._h, int(hz)))
 
-    def set_loudness(self, target_lufs: float, ceiling_dbfs: float = -1.0) -> None:
+    def set_loudness(self, target_lufs: float, ceiling_dbfs: float = -1.0, true_peak: bool = False) -> None:
         """ctts_gpu_set_loudness: every later call of this context normalizes each utterance to target_lufs LUFS
         (ITU-R BS.1770-4, in [-60, -5]) without letting its sample peak pass ceiling_dbfs dBFS (in [-20, 0]).
+        true_peak=True (ctts_gpu_set_loudness_true_peak): the ceiling is in dBTP and holds the 4x oversampled peak.
         target_lufs == 0 turns it off.  Plans created before keep their setting."""
-        self._check(lib().ctts_gpu_set_loudness(self._h, float(target_lufs), float(ceiling_dbfs)))
+        f = lib().ctts_gpu_set_loudness_true_peak if true_peak else lib().ctts_gpu_set_loudness
+        self._check(f(self._h, float(target_lufs), float(ceiling_dbfs)))
 
     def bounds(self, plan: BatchPlan) -> np.ndarray:
         b = np.zeros(max(plan.n_utts, 1), dtype=np.uint64)

@@ -68,8 +68,8 @@ int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz);
  * encoded or copied:
  *   k = clamp(floor(100 * (T - L) + 0.5), -8000, 8000), G = min(floor(65536 * 10^(k / 2000)), floor(A * 65536 / P))
  *   with A = floor(32767 * 10^(C / 20)) and P = max |x|; G = 65536 when L is undefined;  y = (x * G + 32768) >> 16.
- * So an utterance reaches T LUFS to 0.005 LU unless its SAMPLE peak would pass C dBFS (there is no true-peak,
- * oversampled, limiting and no compression); G = 65536 leaves it exactly as it was; counts do not change.
+ * So an utterance reaches T LUFS to 0.005 LU unless its SAMPLE peak would pass C dBFS (no compression; for a
+ * true-peak ceiling see ctts_gpu_set_loudness_true_peak); G = 65536 leaves it exactly as it was; counts do not change.
  * Accepted: target_lufs a finite T in [-60, -5] with ceiling_dbfs a finite C in [-20, 0]; target_lufs == 0 turns the
  * stage off (then nothing is enqueued: bytes and kernel launches are those of a context that never set it).
  * Builds the K-weighting of the context's output rate (and keeps it consistent when the rate changes) and, once per
@@ -80,6 +80,18 @@ int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz);
  * calls, PCM and FLAC sessions, ctts_b200_synth_texts(_flac) and ctts_gpu_multi_synth_batch, which rejects contexts
  * whose settings differ. */
 int ctts_gpu_set_loudness(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_dbfs);
+/* The same loudness normalization with a TRUE-PEAK ceiling of C dBTP (ITU-R BS.1770-4 Annex 2, DESIGN.md 3.6), for
+ * delivery specifications such as EBU R128 (-1 dBTP).  The peak is that of the signal interpolated 4x with the 49-tap
+ * windowed sinc h[j] = sinc((j - 24) / 4) * 0.5 * (1 - cos(2 pi j / 48)), j = 0 .. 48 (|h[j]| <= 1e-9 set to 0, taps
+ * rounded to float once), the utterance taken as zero outside its n samples:
+ *   v[m] = sum over j of x[j] * h[m - 4j + 24] for m = -24 .. 4(n - 1) + 24 (ascending j, one fmaf per term from 0.0f),
+ *   P = max |v[m]| (>= max |x|, since v[4j] = x[j]),  G = min(floor(65536 * 10^(k / 2000)), floor((A - 1) * 65536 / P))
+ *   (the division in double), everything else as ctts_gpu_set_loudness.
+ * Guarantee: the interpolated peak of the delivered y (same taps, exact arithmetic) is <= A, so |y| <= A.
+ * The same acceptance rules; it replaces the context's loudness setting, whichever kind that was, and
+ * ctts_gpu_set_loudness replaces it back.  Plans keep the kind, it follows the output rate, and
+ * ctts_gpu_multi_synth_batch rejects contexts whose kinds differ.  A plan adds ceil(n / 65535) kernel launches. */
+int ctts_gpu_set_loudness_true_peak(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_dbtp);
 /* Text of the last error of a context; ctx == NULL: why the calling thread's last ctts_gpu_init failed. */
 const char* ctts_gpu_last_error(const ctts_gpu_ctx* ctx);
 
@@ -204,6 +216,9 @@ int ctts_gpu_plan_read_pcm(ctts_gpu_ctx* ctx, ctts_gpu_plan* plan, int16_t* dst,
 /* After a run of a plan created with loudness normalization on: L (LUFS, -INFINITY when undefined) and G (Q16) of
  * every utterance, n_utts entries each.  CTTS_GPU_ERR_INVALID_ARG for a plan created with the stage off. */
 int ctts_gpu_plan_read_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* plan, double* lufs, uint32_t* gain);
+/* After a run of a plan created under a true-peak setting (ctts_gpu_set_loudness_true_peak): every utterance's true
+ * peak P before the gain (int16 units), n_utts entries.  CTTS_GPU_ERR_INVALID_ARG for any other plan. */
+int ctts_gpu_plan_read_true_peak(ctts_gpu_ctx* ctx, ctts_gpu_plan* plan, float* peak);
 /* Debug / tests: pre-stretch buffer of utterance u (only for speed != 1.0f utterances). */
 int ctts_gpu_plan_read_pre(ctts_gpu_ctx* ctx, ctts_gpu_plan* plan, uint32_t u, int16_t* dst,
                            uint64_t cap, uint64_t* n);

@@ -1,11 +1,11 @@
 """Loudness normalization on the bench workload (DESIGN.md 3.6): one JSON line.
 
   resident   the resident-plan step of the bench workload (4096 utterances, ~200 characters, speed 1.0) at 22050 and
-             16000 Hz with the stage off and at -16 LUFS (-1 dBFS ceiling), off and on alternated round by round in
-             one process (CUDA events), medians of the rounds
+             16000 Hz with the stage off, at -16 LUFS with a -1 dBFS sample-peak ceiling and at -16 LUFS with a
+             -1 dBTP true-peak ceiling, the three alternated round by round in one process (CUDA events), medians
   kernels    the loudness kernels' own time per step, from torch.profiler (CUDA activity) in a run of its own
   e2e        text -> pinned host PCM (ctts_b200_synth_texts) and text -> pinned host FLAC (ctts_b200_synth_texts_flac),
-             off and on alternated round by round
+             the three settings alternated round by round
 
 The device name and power limit are read in the same run.  Usage:
   python tools/bench_loudness.py [--utts 4096] [--rounds 3] [--steps 5] [--out FILE]
@@ -28,8 +28,9 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
         sys.path.insert(0, p)
 
 RATES = (22050, 16000)
-TARGETS = (0.0, -16.0)   # 0: off
-KERNELS = ("ld_chunk_kernel", "ld_scan_kernel", "ld_gain_kernel", "ld_apply_kernel")
+TARGETS = (0.0, -16.0, "tp")   # 0: off; "tp": -16 LUFS with a -1 dBTP true-peak ceiling
+LABEL = {0.0: "off", -16.0: "minus16", "tp": "minus16_tp"}
+KERNELS = ("ld_chunk_kernel", "ld_scan_kernel", "ld_true_peak_kernel", "ld_gain_kernel", "ld_apply_kernel")
 
 
 def power_limit_w(index: int) -> float | None:
@@ -72,7 +73,7 @@ def main() -> int:
 
     def configure(hz, target):
         g.set_output_rate(hz)
-        g.set_loudness(target, -1.0)
+        g.set_loudness(-16.0 if target == "tp" else target, -1.0, true_peak=target == "tp")
 
     plans, outs, launches = {}, {}, {}
     for hz in RATES:
@@ -89,6 +90,13 @@ def main() -> int:
         lufs, gain = plans[hz, -16.0].loudness()
         gains[hz] = {"defined": int(np.isfinite(lufs).sum()), "unity": int((gain == 65536).sum()),
                      "lufs_median": round(float(np.median(lufs[np.isfinite(lufs)])), 2)}
+        _, gain_tp = plans[hz, "tp"].loudness()
+        peak = plans[hz, "tp"].true_peak()
+        gains[hz]["true_peak_limited"] = int((gain_tp < gain).sum())
+        # the stage-off output of the same batch: the sample peaks
+        pk = np.array([np.abs(u.astype(np.int32)).max() if len(u) else 0 for u in plans[hz, 0.0].utterances()], np.float64)
+        ok = pk > 0
+        gains[hz]["true_peak_over_sample_peak_db_max"] = round(float(np.max(20 * np.log10(peak[ok] / pk[ok]))), 3)
 
     step_ms = {(hz, t): [] for hz in RATES for t in TARGETS}
     with torch.cuda.stream(stream):
@@ -107,16 +115,17 @@ def main() -> int:
     kernel_ms = {}
     from torch.profiler import ProfilerActivity, profile
     for hz in RATES:
-        with profile(activities=[ProfilerActivity.CUDA]) as prof:
-            for _ in range(args.steps):
-                plans[hz, -16.0].run(outs[hz, -16.0].data_ptr())
-            torch.cuda.synchronize(dev)
-        tot = {k: 0.0 for k in KERNELS}
-        for e in prof.events():
-            for k in KERNELS:
-                if k in e.name:
-                    tot[k] += e.device_time_total if hasattr(e, "device_time_total") else e.cuda_time_total
-        kernel_ms[hz] = {k: round(v / 1e3 / args.steps, 3) for k, v in tot.items()}
+        for t in (-16.0, "tp"):
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                for _ in range(args.steps):
+                    plans[hz, t].run(outs[hz, t].data_ptr())
+                torch.cuda.synchronize(dev)
+            tot = {k: 0.0 for k in KERNELS}
+            for e in prof.events():
+                for k in KERNELS:
+                    if k in e.name:
+                        tot[k] += e.device_time_total if hasattr(e, "device_time_total") else e.cuda_time_total
+            kernel_ms[f"{hz}_{LABEL[t]}"] = {k: round(v / 1e3 / args.steps, 3) for k, v in tot.items()}
 
     tb = pipe.TextBatch(texts)
     e2e = {}
@@ -139,8 +148,8 @@ def main() -> int:
                 s = time.perf_counter()
                 _, _, _, used["flac", t], _ = pipe.synth_texts_flac(fr, g, tb, flac)
                 res["flac", t].append(1e3 * (time.perf_counter() - s))
-        e2e[hz] = {f"{k}_{'off' if t == 0 else 'minus16'}_ms": _med(v) for (k, t), v in res.items()}
-        e2e[hz]["bytes"] = {f"{k}_{'off' if t == 0 else 'minus16'}": int(v) * (2 if k == "pcm" else 1) for (k, t), v in used.items()}
+        e2e[hz] = {f"{k}_{LABEL[t]}_ms": _med(v) for (k, t), v in res.items()}
+        e2e[hz]["bytes"] = {f"{k}_{LABEL[t]}": int(v) * (2 if k == "pcm" else 1) for (k, t), v in used.items()}
 
     line = {
         "tool": "tools/bench_loudness.py",
@@ -149,9 +158,10 @@ def main() -> int:
         "utterances": args.utts,
         "workload": "corpus.batch(n, seed=1234, target_chars=200), speed 1.0 (bench.py's default workload)",
         "setting_on": {"target_lufs": -16.0, "ceiling_dbfs": -1.0},
-        "resident_step_ms": {f"{hz}_{'off' if t == 0 else 'minus16'}": _med(v) for (hz, t), v in step_ms.items()},
-        "kernel_launches": {f"{hz}_{'off' if t == 0 else 'minus16'}": v for (hz, t), v in launches.items()},
-        "loudness_kernels_ms_per_step": {str(hz): v for hz, v in kernel_ms.items()},
+        "setting_tp": {"target_lufs": -16.0, "ceiling_dbtp": -1.0},
+        "resident_step_ms": {f"{hz}_{LABEL[t]}": _med(v) for (hz, t), v in step_ms.items()},
+        "kernel_launches": {f"{hz}_{LABEL[t]}": v for (hz, t), v in launches.items()},
+        "loudness_kernels_ms_per_step": kernel_ms,
         "utterances_at_minus16": {str(hz): v for hz, v in gains.items()},
         "e2e": {str(hz): v for hz, v in e2e.items()},
         "rounds": args.rounds, "steps": args.steps,
