@@ -101,7 +101,7 @@ def build_cli(force: bool = False) -> str:
     """The plain-C drop-in command line (csrc/cli/ctts_b200.c) linked against the three libraries."""
     src = os.path.join(CSRC, "cli", "ctts_b200.c")
     build_pipeline(force)
-    deps = [src, FRONT_SO, GPU_SO, PIPE_SO] + _headers()
+    deps = [src, os.path.join(CSRC, "cli", "g711_wav.h"), FRONT_SO, GPU_SO, PIPE_SO] + _headers()
     if not force and _newer(CLI_BIN, deps):
         return CLI_BIN
     cc = shutil.which("gcc") or "cc"

@@ -3,14 +3,18 @@
  * reference's own language: plain C on top of the two C-ABI libraries, no Python, no CUDA headers.
  *
  *   ctts_b200 synth <database.db> "text" <output.wav|output.flac> [speed] [rate] [lufs=<target> [dbtp=<ceiling>]]
+ *                   [g711=ulaw|alaw]
  *   ctts_b200 synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target> [dbtp=<ceiling>]]
- *                                                                                          lines: speed<TAB>text
+ *                         [g711=ulaw|alaw]                                                 lines: speed<TAB>text
  *
  * rate: output sample rate in Hz (default 22050, the voice's own; ctts_gpu_set_output_rate lists the others),
  * written into the WAV header.  An output name ending in ".flac", or synth-batch's "flac", writes lossless FLAC files
  * encoded on the device (ctts_b200_synth_texts_flac) instead of 16-bit WAV.  lufs=<target> normalizes every utterance
  * to <target> LUFS (ITU-R BS.1770-4, in [-60, -5]) with its sample peak held to -1 dBFS (ctts_gpu_set_loudness);
  * dbtp=<ceiling> next to it holds the true peak to <ceiling> dBTP instead (in [-20, 0], ctts_gpu_set_loudness_true_peak).
+ * g711=ulaw or g711=alaw writes 8-bit G.711 .wav files (format tag 7 or 6, with a fact chunk) encoded on the device
+ * (ctts_b200_synth_texts_g711), for telephony: with rate 8000 they are what IVR systems play.  It does not combine with
+ * FLAC output.  The trailing options may come in any order.
  *
  * Like the reference it reads config.yaml and normalization.csv from the working directory
  * (ctts.c:3990, :3636), clamps the speed to [0.5, 2.0] (ctts.c:3976-3981) and takes default_speed
@@ -26,6 +30,7 @@
 #include <sys/stat.h>
 
 #include "ctts_b200.h"
+#include "g711_wav.h"
 
 #define SAMPLE_RATE CTTS_PLAN_SAMPLE_RATE
 
@@ -93,14 +98,23 @@ static int engine_open(engine* e, const char* db_path, uint32_t rate, const loud
     return 0;
 }
 
-/* Optional last arguments lufs=<target> and dbtp=<ceiling>, in either order (after the output argument): taken off the
- * argument list.  ld->lufs = 0 without lufs=; -1 when a value is not a number, an option repeats or dbtp= comes
- * without lufs= (any other value is checked by ctts_gpu_set_loudness(_true_peak)). */
-static int take_lufs(int* argc, char** argv, loudness_arg* ld) {
+/* Optional last arguments lufs=<target>, dbtp=<ceiling> and g711=ulaw|alaw, in any order (after the output argument):
+ * taken off the argument list.  ld->lufs = 0 without lufs=; *law = 0 without g711=, else CTTS_GPU_G711_ULAW or
+ * CTTS_GPU_G711_ALAW.  -1 when a value is not a number or not a law, an option repeats or dbtp= comes without lufs=
+ * (any other value is checked by ctts_gpu_set_loudness(_true_peak)). */
+static int take_options(int* argc, char** argv, loudness_arg* ld, int* law) {
     memset(ld, 0, sizeof *ld);
+    *law = 0;
     int have_lufs = 0;
     while (*argc >= 6) {   /* behind the required arguments only */
         const char* a = argv[*argc - 1];
+        if (strncmp(a, "g711=", 5) == 0) {
+            if (*law) return -1;
+            *law = strcmp(a + 5, "ulaw") == 0 ? CTTS_GPU_G711_ULAW : strcmp(a + 5, "alaw") == 0 ? CTTS_GPU_G711_ALAW : -1;
+            if (*law < 0) return -1;
+            (*argc)--;
+            continue;
+        }
         const int is_lufs = strncmp(a, "lufs=", 5) == 0, is_dbtp = strncmp(a, "dbtp=", 5) == 0;
         if (!is_lufs && !is_dbtp) break;
         if (is_lufs ? have_lufs : ld->true_peak) return -1;
@@ -134,13 +148,25 @@ static int write_wav(const char* path, const int16_t* samples, size_t count, uin
     return fclose(f) == 0 ? 0 : -1;
 }
 
-/* N texts -> N PCM spans (or, with flac, N .flac files) of one pinned buffer through ctts_b200_synth_texts(_flac)
- * (the front end's planner threads feed the device piece by piece): r->out (release with ctts_gpu_host_free),
- * r->off[u], r->bytes[u] (FLAC: file sizes) and r->cnt[u] (malloc'ed, n entries each); stats may be NULL (2n: found,
- * missing).  on_chunk (may be NULL) is called as soon as a range of utterances is in host memory; it finds the
- * arrays through r, which is filled before the device starts. */
+/* G.711 .wav (g711_wav.h): the header, the count code bytes and a pad byte when the count is odd */
+static int write_g711_wav(const char* path, const uint8_t* codes, size_t count, uint32_t rate, int law) {
+    FILE* f = fopen(path, "wb");
+    if (!f) return -1;
+    uint8_t h[G711_WAV_HEADER_BYTES];
+    g711_wav_header(h, law, rate, (uint32_t)count);
+    const uint8_t pad = 0;
+    int ok = fwrite(h, 1, sizeof h, f) == sizeof h && fwrite(codes, 1, count, f) == count;
+    if (count & 1) ok = ok && fwrite(&pad, 1, 1, f) == 1;
+    return fclose(f) == 0 && ok ? 0 : -1;
+}
+
+/* N texts -> N PCM spans (or, with flac, N .flac files; with a G.711 law, N spans of codes) of one pinned buffer through
+ * ctts_b200_synth_texts(_flac, _g711) (the front end's planner threads feed the device piece by piece): r->out (release
+ * with ctts_gpu_host_free), r->off[u], r->bytes[u] (FLAC: file sizes) and r->cnt[u] (malloc'ed, n entries each); stats
+ * may be NULL (2n: found, missing).  on_chunk (may be NULL) is called as soon as a range of utterances is in host
+ * memory; it finds the arrays through r, which is filled before the device starts. */
 typedef struct {
-    void* out;   /* int16_t PCM, or the FLAC files */
+    void* out;   /* int16_t PCM, the FLAC files, or the G.711 codes */
     uint64_t* off;
     uint32_t* bytes;
     uint32_t* cnt;
@@ -155,21 +181,22 @@ static void result_free(batch_result* r) {
 }
 
 static int ctts_b200_synthesize_batch(engine* e, const char* const* texts, const float* speeds, uint32_t n, int flac,
-                                      batch_result* r, uint32_t* stats, ctts_gpu_chunk_fn on_chunk, void* user) {
+                                      int law, batch_result* r, uint32_t* stats, ctts_gpu_chunk_fn on_chunk, void* user) {
     int rc = 0;
-    /* replaces the SampleBuffer growth policy */
+    /* replaces the SampleBuffer growth policy; G.711: the sample capacity, read as bytes */
     const uint64_t cap = flac ? ctts_b200_capacity_hint_flac(e->front, texts, speeds, n, e->rate)
                               : ctts_b200_capacity_hint_rate(e->front, texts, speeds, n, e->rate);
     r->off = malloc(sizeof *r->off * ((size_t)n + 1));
     r->bytes = calloc(n ? n : 1, sizeof *r->bytes);
     r->cnt = calloc(n ? n : 1, sizeof *r->cnt);
-    r->out = ctts_gpu_host_alloc((flac ? 1 : sizeof(int16_t)) * (cap ? cap : 16));
+    r->out = ctts_gpu_host_alloc((flac || law ? 1 : sizeof(int16_t)) * (cap ? cap : 16));
     if (!r->off || !r->bytes || !r->cnt || !r->out) rc = CTTS_GPU_ERR_OUT_OF_MEMORY;
     ctts_b200_options opt;
     memset(&opt, 0, sizeof opt);
     opt.on_piece = on_chunk;
     opt.user = user;
     if (!rc && flac) rc = ctts_b200_synth_texts_flac(e->front, e->gpu, texts, speeds, n, r->out, cap, r->off, r->bytes, r->cnt, stats, NULL, &opt, NULL);
+    else if (!rc && law) rc = ctts_b200_synth_texts_g711(e->front, e->gpu, law, texts, speeds, n, r->out, cap, r->off, r->cnt, stats, NULL, &opt, NULL);
     else if (!rc) rc = ctts_b200_synth_texts(e->front, e->gpu, texts, speeds, n, r->out, cap, r->off, r->cnt, stats, NULL, &opt, NULL);
     if (rc) {
         fprintf(stderr, "synthesis failed: %d %s\n", rc, ctts_gpu_last_error(e->gpu));
@@ -201,8 +228,10 @@ static uint32_t parse_rate(const char* a) {
 
 static int cmd_synth(int argc, char** argv) {
     loudness_arg ld;
-    if (take_lufs(&argc, argv, &ld) || argc < 5 || argc > 7) {
-        fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav> [speed] [rate] [lufs=<target> [dbtp=<ceiling>]]\n", argv[0]);
+    int law;
+    if (take_options(&argc, argv, &ld, &law) || argc < 5 || argc > 7 || (law && ends_with(argv[4], ".flac"))) {
+        fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav|output.flac> [speed] [rate] [lufs=<target> [dbtp=<ceiling>]] [g711=ulaw|alaw]\n"
+                        "       (g711= writes a G.711 .wav file, not FLAC)\n", argv[0]);
         return 1;
     }
     float speed = 1.0f;
@@ -219,11 +248,12 @@ static int cmd_synth(int argc, char** argv) {
     const int flac = ends_with(argv[4], ".flac");
     batch_result r;
     uint32_t stats[2] = {0, 0};
-    if (ctts_b200_synthesize_batch(&e, texts, &speed, 1, flac, &r, stats, NULL, NULL)) { engine_close(&e); return 1; }
+    if (ctts_b200_synthesize_batch(&e, texts, &speed, 1, flac, law, &r, stats, NULL, NULL)) { engine_close(&e); return 1; }
     printf("Synthesized %u samples (%.2f seconds)\n", r.cnt[0], (float)r.cnt[0] / (float)e.rate);
     printf("Units found: %u, missing: %u\n", stats[0], stats[1]);
-    int rc = flac ? write_flac(argv[4], (const uint8_t*)r.out + r.off[0], r.bytes[0])
-                  : write_wav(argv[4], (const int16_t*)r.out + r.off[0], r.cnt[0], e.rate);
+    int rc = flac  ? write_flac(argv[4], (const uint8_t*)r.out + r.off[0], r.bytes[0])
+             : law ? write_g711_wav(argv[4], (const uint8_t*)r.out + r.off[0], r.cnt[0], e.rate, law)
+                   : write_wav(argv[4], (const int16_t*)r.out + r.off[0], r.cnt[0], e.rate);
     if (rc) fprintf(stderr, "Failed to write %s: %s\n", flac ? "FLAC" : "WAV", argv[4]);
     else printf("Written to %s\n", argv[4]);
     result_free(&r);
@@ -237,7 +267,7 @@ typedef struct {
     const char* dir;
     uint32_t rate;
     uint32_t base;   /* first utterance of the group being synthesised */
-    int flac;
+    int flac, law;
     const batch_result* r;
     double seconds;
     int rc;
@@ -248,16 +278,20 @@ static void write_chunk(void* user, uint32_t u0, uint32_t u1) {
     for (uint32_t u = u0; u < u1 && !w->rc; u++) {
         char path[4096];
         snprintf(path, sizeof path, "%s/%06u.%s", w->dir, w->base + u, w->flac ? "flac" : "wav");
-        w->rc = w->flac ? write_flac(path, (const uint8_t*)w->r->out + w->r->off[u], w->r->bytes[u])
-                        : write_wav(path, (const int16_t*)w->r->out + w->r->off[u], w->r->cnt[u], w->rate);
+        w->rc = w->flac  ? write_flac(path, (const uint8_t*)w->r->out + w->r->off[u], w->r->bytes[u])
+                : w->law ? write_g711_wav(path, (const uint8_t*)w->r->out + w->r->off[u], w->r->cnt[u], w->rate, w->law)
+                         : write_wav(path, (const int16_t*)w->r->out + w->r->off[u], w->r->cnt[u], w->rate);
         w->seconds += (double)w->r->cnt[u] / w->rate;
     }
 }
 
 static int cmd_synth_batch(int argc, char** argv) {
     loudness_arg ld;
-    if (take_lufs(&argc, argv, &ld) || argc < 5 || argc > 7 || (argc == 7 && strcmp(argv[6], "flac") != 0)) {
-        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target> [dbtp=<ceiling>]]\n", argv[0]);
+    int law;
+    if (take_options(&argc, argv, &ld, &law) || argc < 5 || argc > 7 || (argc == 7 && strcmp(argv[6], "flac") != 0) ||
+        (law && argc == 7)) {
+        fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target> [dbtp=<ceiling>]] [g711=ulaw|alaw]\n"
+                        "       (g711= writes G.711 .wav files, not FLAC)\n", argv[0]);
         return 1;
     }
     const uint32_t rate = argc > 5 ? parse_rate(argv[5]) : SAMPLE_RATE;
@@ -295,13 +329,13 @@ static int cmd_synth_batch(int argc, char** argv) {
     }
     if (mkdir(argv[4], 0777) != 0 && errno != EEXIST) { fprintf(stderr, "cannot create %s\n", argv[4]); engine_close(&e); return 1; }
     batch_result r;
-    wav_sink sink = {argv[4], e.rate, 0, flac, &r, 0.0, 0};
+    wav_sink sink = {argv[4], e.rate, 0, flac, law, &r, 0.0, 0};
     /* groups of 1024 utterances: the pinned buffer is sized from the texts alone (ctts_b200_capacity_hint) */
     int rc = 0;
     for (uint32_t g0 = 0; g0 < n && !rc; g0 += 1024) {
         const uint32_t gn = n - g0 < 1024 ? n - g0 : 1024;
         sink.base = g0;
-        rc = ctts_b200_synthesize_batch(&e, (const char* const*)texts + g0, speeds + g0, gn, flac, &r, NULL, write_chunk, &sink);
+        rc = ctts_b200_synthesize_batch(&e, (const char* const*)texts + g0, speeds + g0, gn, flac, law, &r, NULL, write_chunk, &sink);
         if (!rc) {
             rc = sink.rc;
             result_free(&r);
@@ -319,7 +353,8 @@ static int cmd_synth_batch(int argc, char** argv) {
 int main(int argc, char** argv) {
     if (argc >= 2 && strcmp(argv[1], "synth") == 0) return cmd_synth(argc, argv);
     if (argc >= 2 && strcmp(argv[1], "synth-batch") == 0) return cmd_synth_batch(argc, argv);
-    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav|output.flac> [speed] [rate] [lufs=<target> [dbtp=<ceiling>]]\n       %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target> [dbtp=<ceiling>]]\n",
+    fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav|output.flac> [speed] [rate] [lufs=<target> [dbtp=<ceiling>]] [g711=ulaw|alaw]\n"
+                    "       %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target> [dbtp=<ceiling>]] [g711=ulaw|alaw]\n",
             argv[0], argv[0]);
     return 1;
 }

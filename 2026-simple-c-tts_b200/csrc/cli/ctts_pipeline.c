@@ -331,11 +331,16 @@ uint64_t ctts_b200_capacity_hint_flac(ctts_front* front, const char* const* text
     return capacity_hint(front, texts, speeds, n, hz, 1);
 }
 
-/* ctts_b200_synth_texts and ctts_b200_synth_texts_flac: the same pipeline over a PCM or a FLAC session */
+/* what synth_texts delivers: PCM, a FLAC file per utterance, or G.711 bytes of one law */
+enum out_kind { OUT_PCM, OUT_FLAC, OUT_ULAW, OUT_ALAW };
+
+/* ctts_b200_synth_texts, ctts_b200_synth_texts_flac and ctts_b200_synth_texts_g711: the same pipeline over a PCM, a
+ * FLAC or a G.711 session; byte_out is the output of the last two */
 static int synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* const* texts, const float* speeds, uint32_t n,
-                       int flac, int16_t* pcm_out, uint8_t* flac_out, uint64_t capacity, uint64_t* out_offsets, uint32_t* out_bytes,
-                       uint32_t* out_counts, uint32_t* stats, uint64_t* used, const ctts_b200_options* opt,
-                       ctts_b200_timing* timing) {
+                       enum out_kind kind, int16_t* pcm_out, uint8_t* byte_out, uint64_t capacity, uint64_t* out_offsets,
+                       uint32_t* out_bytes, uint32_t* out_counts, uint32_t* stats, uint64_t* used,
+                       const ctts_b200_options* opt, ctts_b200_timing* timing) {
+    const int flac = kind == OUT_FLAC;
     if (!front || !gpu || (n && (!texts || !out_offsets || !out_counts || (flac && !out_bytes)))) return CTTS_GPU_ERR_INVALID_ARG;
     pipeline P;
     memset(&P, 0, sizeof P);
@@ -362,8 +367,12 @@ static int synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* const* 
     ctts_assembly_params prm;
     ctts_front_params(front, &prm);
     ctts_gpu_session* ses = NULL;
-    int rc = flac ? ctts_gpu_session_begin_flac(gpu, &prm, flac_out, capacity, opt ? opt->on_piece : NULL, opt ? opt->user : NULL, &ses)
-                      : ctts_gpu_session_begin(gpu, &prm, pcm_out, capacity, opt ? opt->on_piece : NULL, opt ? opt->user : NULL, &ses);
+    ctts_gpu_chunk_fn on_piece = opt ? opt->on_piece : NULL;
+    void* user = opt ? opt->user : NULL;
+    int rc = kind == OUT_PCM ? ctts_gpu_session_begin(gpu, &prm, pcm_out, capacity, on_piece, user, &ses)
+             : flac          ? ctts_gpu_session_begin_flac(gpu, &prm, byte_out, capacity, on_piece, user, &ses)
+                             : ctts_gpu_session_begin_g711(gpu, &prm, kind == OUT_ULAW ? CTTS_GPU_G711_ULAW : CTTS_GPU_G711_ALAW,
+                                                           byte_out, capacity, on_piece, user, &ses);
     if (rc) {
         free(P.piece_begin);
         return rc;
@@ -450,8 +459,9 @@ static int synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* const* 
             joined.ops = j_ops;
             piece = &joined;
         }
-        rc = flac ? ctts_gpu_session_submit_flac(ses, piece, out_offsets + u0, out_bytes + u0, out_counts + u0)
-                      : ctts_gpu_session_submit(ses, piece, out_offsets + u0, out_counts + u0);
+        rc = kind == OUT_PCM ? ctts_gpu_session_submit(ses, piece, out_offsets + u0, out_counts + u0)
+             : flac          ? ctts_gpu_session_submit_flac(ses, piece, out_offsets + u0, out_bytes + u0, out_counts + u0)
+                             : ctts_gpu_session_submit_g711(ses, piece, out_offsets + u0, out_counts + u0);
         for (uint32_t k = i; k < j; k++) {
             ctts_front_plan_free(&P.slots[k].plan);   /* the session keeps nothing of the plan */
             P.slots[k].state = 2;
@@ -497,7 +507,7 @@ int ctts_b200_synth_texts(ctts_front* front, ctts_gpu_ctx* gpu, const char* cons
                           uint32_t n, int16_t* pcm_out, uint64_t capacity, uint64_t* out_offsets,
                           uint32_t* out_counts, uint32_t* stats, uint64_t* samples_used,
                           const ctts_b200_options* opt, ctts_b200_timing* timing) {
-    return synth_texts(front, gpu, texts, speeds, n, 0, pcm_out, NULL, capacity, out_offsets, NULL, out_counts, stats,
+    return synth_texts(front, gpu, texts, speeds, n, OUT_PCM, pcm_out, NULL, capacity, out_offsets, NULL, out_counts, stats,
                        samples_used, opt, timing);
 }
 
@@ -505,6 +515,15 @@ int ctts_b200_synth_texts_flac(ctts_front* front, ctts_gpu_ctx* gpu, const char*
                                uint32_t n, uint8_t* out, uint64_t capacity_bytes, uint64_t* out_offsets,
                                uint32_t* out_bytes, uint32_t* out_counts, uint32_t* stats, uint64_t* bytes_used,
                                const ctts_b200_options* opt, ctts_b200_timing* timing) {
-    return synth_texts(front, gpu, texts, speeds, n, 1, NULL, out, capacity_bytes, out_offsets, out_bytes,
+    return synth_texts(front, gpu, texts, speeds, n, OUT_FLAC, NULL, out, capacity_bytes, out_offsets, out_bytes,
                        out_counts, stats, bytes_used, opt, timing);
+}
+
+int ctts_b200_synth_texts_g711(ctts_front* front, ctts_gpu_ctx* gpu, int law, const char* const* texts,
+                               const float* speeds, uint32_t n, uint8_t* out, uint64_t capacity_bytes,
+                               uint64_t* out_offsets, uint32_t* out_counts, uint32_t* stats, uint64_t* bytes_used,
+                               const ctts_b200_options* opt, ctts_b200_timing* timing) {
+    if (law != CTTS_GPU_G711_ULAW && law != CTTS_GPU_G711_ALAW) return CTTS_GPU_ERR_INVALID_ARG;
+    return synth_texts(front, gpu, texts, speeds, n, law == CTTS_GPU_G711_ULAW ? OUT_ULAW : OUT_ALAW, NULL, out,
+                       capacity_bytes, out_offsets, NULL, out_counts, stats, bytes_used, opt, timing);
 }

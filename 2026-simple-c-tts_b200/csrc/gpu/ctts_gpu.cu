@@ -23,6 +23,7 @@
 #include "wsola.cuh"
 #include "resample.cuh"
 #include "flac.cuh"
+#include "g711.cuh"
 #include "loudness.cuh"
 
 extern "C" void ctts_host_tables(float* fade_out, float* fade_in, float* sine, float* hann256,
@@ -2048,12 +2049,16 @@ int ctts_gpu_plan_read_pre(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t u, int1
 
 }  // extern "C"
 
+// What a session delivers: PCM samples, or bytes (one FLAC file per utterance, or one G.711 code per sample)
+enum SessionOutput { OUT_PCM = 0, OUT_ULAW = CTTS_GPU_G711_ULAW, OUT_ALAW = CTTS_GPU_G711_ALAW, OUT_FLAC };
+static_assert(OUT_ULAW == ctts::G711_ULAW && OUT_ALAW == ctts::G711_ALAW, "G.711 law constants");
+
 struct ctts_gpu_session {
     ctts_gpu_ctx* ctx = nullptr;
     ctts_assembly_params prm{};
     int16_t* pcm_out = nullptr;
-    uint8_t* flac_out = nullptr;  // FLAC session: the files go here, and capacity and cursor count bytes
-    bool flac = false;
+    uint8_t* byte_out = nullptr;  // FLAC and G.711 sessions: the output goes here, and capacity and cursor count bytes
+    SessionOutput kind = OUT_PCM;
     uint64_t capacity = 0;        // samples
     uint64_t cursor = 0;          // next free sample (library-chosen layout)
     uint32_t submitted = 0, harvested = 0;   // pieces
@@ -2062,7 +2067,7 @@ struct ctts_gpu_session {
     ctts_gpu_chunk_fn on_piece = nullptr;
     void* user = nullptr;
     int error = 0;
-    uint64_t d2h_samples = 0;     // samples (FLAC: bytes) copied to the host
+    uint64_t d2h_samples = 0;     // samples (FLAC, G.711: bytes) copied to the host
     std::chrono::steady_clock::time_point t0;
 };
 
@@ -2128,7 +2133,8 @@ int harvest_one(ctts_gpu_session* s) {
 // One piece: compile, launch, copy.  Utterance i of the piece is delivered to pcm_out[slot_off[i] ..),
 // slot_cap[i] samples of room (>= its bound); slot_off == nullptr: the library appends packed slots at the
 // session's cursor and reports them through offsets_out.  Asynchronous: returns once everything is enqueued.
-// A FLAC session (packed only) encodes every utterance into a file instead and reports the sizes through out_bytes.
+// A FLAC session (packed only) encodes every utterance into a file instead and reports the sizes through out_bytes;
+// a G.711 session (packed only) encodes every sample into one byte of the same packed layout.
 int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64_t* slot_off, const uint64_t* slot_cap,
                  uint64_t* offsets_out, uint32_t* out_counts, uint32_t* out_bytes = nullptr) {
     ctts_gpu_ctx* ctx = s->ctx;
@@ -2168,7 +2174,7 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
     };
     if ((rc = grow(&l.d_out, &l.d_out_cap, p->n_offsets[n])) != 0) return bail(rc);
     if (p->rs && (rc = grow(&l.d_rs, &l.d_rs_cap, total)) != 0) return bail(rc);
-    const bool flac = s->flac;
+    const bool flac = s->kind == OUT_FLAC;
     if (packed && !flac && (rc = grow(&l.d_pack, &l.d_pack_cap, total)) != 0) return bail(rc);
     // FLAC: the files and the frame descriptors are sized by the slots (>= the bounds): ctts_gpu_flac_bound each
     uint64_t flac_bytes = 0, n_frames = 0, max_frames = 1;
@@ -2275,7 +2281,13 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
                 for (uint32_t u = 0; u < n; u++) max_slot = std::max<uint64_t>(max_slot, p->offsets[u + 1] - p->offsets[u]);
                 for (uint32_t u0 = 0; u0 < n && e == cudaSuccess; u0 += 65535u) {   // grid.y limit
                     const dim3 grid((unsigned)((max_slot + ctts::PACK_TILE - 1) / ctts::PACK_TILE), std::min<uint32_t>(n - u0, 65535u));
-                    ctts::pack_copy_kernel<<<grid, ctts::PACK_THREADS, 0, ctx->stream>>>(d_final, d_slot + u0, p->d_final_counts + u0, l.d_pack_off + u0, l.d_pack);
+                    uint8_t* const d_bytes = reinterpret_cast<uint8_t*>(l.d_pack);   // G.711: one byte per sample
+                    if (s->kind == OUT_ULAW)
+                        ctts::g711_pack_kernel<ctts::G711_ULAW><<<grid, ctts::PACK_THREADS, 0, ctx->stream>>>(d_final, d_slot + u0, p->d_final_counts + u0, l.d_pack_off + u0, d_bytes);
+                    else if (s->kind == OUT_ALAW)
+                        ctts::g711_pack_kernel<ctts::G711_ALAW><<<grid, ctts::PACK_THREADS, 0, ctx->stream>>>(d_final, d_slot + u0, p->d_final_counts + u0, l.d_pack_off + u0, d_bytes);
+                    else
+                        ctts::pack_copy_kernel<<<grid, ctts::PACK_THREADS, 0, ctx->stream>>>(d_final, d_slot + u0, p->d_final_counts + u0, l.d_pack_off + u0, l.d_pack);
                     e = cudaGetLastError();
                 }
             }
@@ -2335,19 +2347,21 @@ int enqueue_packed_copy(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l) {
     }
     const uint32_t* h_cnt = l.h_res;
     const uint32_t* h_bytes = l.h_res + 2 * (size_t)l.n;   // FLAC: file sizes
+    const bool flac = s->kind == OUT_FLAC;
     uint64_t o = s->cursor;
     for (uint32_t u = 0; u < l.n; u++) {
         if (l.user_offsets) l.user_offsets[u] = o;
-        o += s->flac ? (h_bytes[u] + 15ull) & ~15ull : up8(h_cnt[u]);
+        o += flac ? (h_bytes[u] + 15ull) & ~15ull : up8(h_cnt[u]);
     }
     const uint64_t len = o - s->cursor;
     if (o > s->capacity) {
         if (!s->error)
             s->error = fail(ctx, CTTS_GPU_ERR_BOUNDS, "output buffer too small: %llu %s needed up to utterance %u", (unsigned long long)o,
-                            s->flac ? "bytes" : "samples", l.utt_base + l.n);
+                            s->kind != OUT_PCM ? "bytes" : "samples", l.utt_base + l.n);
         return s->error;
     }
-    if (len && s->flac) e = cudaMemcpyAsync(s->flac_out + s->cursor, l.d_flac, len, cudaMemcpyDeviceToHost, ctx->copy_stream);
+    if (len && flac) e = cudaMemcpyAsync(s->byte_out + s->cursor, l.d_flac, len, cudaMemcpyDeviceToHost, ctx->copy_stream);
+    else if (len && s->kind != OUT_PCM) e = cudaMemcpyAsync(s->byte_out + s->cursor, l.d_pack, len, cudaMemcpyDeviceToHost, ctx->copy_stream);
     else if (len) e = cudaMemcpyAsync(s->pcm_out + s->cursor, l.d_pack, len * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
     if (e == cudaSuccess) e = cudaEventRecord(l.copied, ctx->copy_stream);
     if (e != cudaSuccess) {
@@ -2408,7 +2422,8 @@ int ctts_gpu_session_begin(ctts_gpu_ctx* ctx, const ctts_assembly_params* params
 
 int ctts_gpu_session_submit(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets, uint32_t* out_counts) {
     if (!s || !piece || !out_counts || (piece->n_utts && !out_offsets)) return CTTS_GPU_ERR_INVALID_ARG;
-    if (s->flac) return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, "a FLAC session takes ctts_gpu_session_submit_flac");
+    if (s->kind == OUT_FLAC) return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, "a FLAC session takes ctts_gpu_session_submit_flac");
+    if (s->kind != OUT_PCM) return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, "a G.711 session takes ctts_gpu_session_submit_g711");
     if (s->error) return s->error;
     ctts_gpu_ctx* ctx = s->ctx;
     CU(ctx, cudaSetDevice(ctx->device));
@@ -2424,8 +2439,8 @@ int ctts_gpu_session_begin_flac(ctts_gpu_ctx* ctx, const ctts_assembly_params* p
     if (capacity_bytes && !out) return CTTS_GPU_ERR_INVALID_ARG;
     const int rc = ctts_gpu_session_begin(ctx, params, nullptr, 0, on_piece, user, s);
     if (rc) return rc;
-    (*s)->flac = true;
-    (*s)->flac_out = out;
+    (*s)->kind = OUT_FLAC;
+    (*s)->byte_out = out;
     (*s)->capacity = capacity_bytes;
     return CTTS_GPU_OK;
 }
@@ -2433,11 +2448,39 @@ int ctts_gpu_session_begin_flac(ctts_gpu_ctx* ctx, const ctts_assembly_params* p
 int ctts_gpu_session_submit_flac(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets, uint32_t* out_bytes,
                                  uint32_t* out_counts) {
     if (!s || !piece || (piece->n_utts && (!out_offsets || !out_bytes || !out_counts))) return CTTS_GPU_ERR_INVALID_ARG;
-    if (!s->flac) return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, "a PCM session takes ctts_gpu_session_submit");
+    if (s->kind != OUT_FLAC)
+        return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, s->kind == OUT_PCM ? "a PCM session takes ctts_gpu_session_submit"
+                                                                          : "a G.711 session takes ctts_gpu_session_submit_g711");
     if (s->error) return s->error;
     ctts_gpu_ctx* ctx = s->ctx;
     CU(ctx, cudaSetDevice(ctx->device));
     return submit_piece(s, piece, nullptr, nullptr, out_offsets, out_counts, out_bytes);
+}
+
+int ctts_gpu_session_begin_g711(ctts_gpu_ctx* ctx, const ctts_assembly_params* params, int law, uint8_t* out,
+                                uint64_t capacity_bytes, ctts_gpu_chunk_fn on_piece, void* user, ctts_gpu_session** s) {
+    if (!ctx || !s || (capacity_bytes && !out)) return CTTS_GPU_ERR_INVALID_ARG;
+    if (law != CTTS_GPU_G711_ULAW && law != CTTS_GPU_G711_ALAW) {
+        *s = nullptr;
+        return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "G.711 law %d: CTTS_GPU_G711_ULAW or CTTS_GPU_G711_ALAW", law);
+    }
+    const int rc = ctts_gpu_session_begin(ctx, params, nullptr, 0, on_piece, user, s);
+    if (rc) return rc;
+    (*s)->kind = law == CTTS_GPU_G711_ULAW ? OUT_ULAW : OUT_ALAW;
+    (*s)->byte_out = out;
+    (*s)->capacity = capacity_bytes;
+    return CTTS_GPU_OK;
+}
+
+int ctts_gpu_session_submit_g711(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets, uint32_t* out_counts) {
+    if (!s || !piece || !out_counts || (piece->n_utts && !out_offsets)) return CTTS_GPU_ERR_INVALID_ARG;
+    if (s->kind != OUT_ULAW && s->kind != OUT_ALAW)
+        return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, s->kind == OUT_PCM ? "a PCM session takes ctts_gpu_session_submit"
+                                                                          : "a FLAC session takes ctts_gpu_session_submit_flac");
+    if (s->error) return s->error;
+    ctts_gpu_ctx* ctx = s->ctx;
+    CU(ctx, cudaSetDevice(ctx->device));
+    return submit_piece(s, piece, nullptr, nullptr, out_offsets, out_counts);
 }
 
 int ctts_gpu_session_end(ctts_gpu_session* s, uint64_t* samples_used) {
@@ -2448,7 +2491,7 @@ int ctts_gpu_session_end(ctts_gpu_session* s, uint64_t* samples_used) {
     if (samples_used) *samples_used = s->cursor;
     if (ctx->knobs.trace)
         fprintf(stderr, "ctts_gpu session: %u utterances in %u pieces, %.1f MB to the host, %.1f ms\n", s->utts, s->submitted,
-                (s->flac ? 1e-6 : 2e-6) * (double)s->d2h_samples, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - s->t0).count());
+                (s->kind != OUT_PCM ? 1e-6 : 2e-6) * (double)s->d2h_samples, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - s->t0).count());
     const int rc = s->error;
     ctx->session = nullptr;
     delete s;

@@ -15,6 +15,7 @@ from . import _build
 from .front import AssemblyParams, BatchPlan, CBatchPlan
 
 ERR_CUDA, ERR_BOUNDS, ERR_DEVICE = -100, -101, -102
+G711_ULAW, G711_ALAW = 1, 2   # CTTS_GPU_G711_ULAW, CTTS_GPU_G711_ALAW
 
 
 class WsolaStats(C.Structure):
@@ -80,6 +81,8 @@ def lib(build: bool = True) -> C.CDLL:
         L.ctts_gpu_session_submit_flac.argtypes = [vp, C.POINTER(CBatchPlan), vp, vp, vp]
         L.ctts_gpu_flac_bound.argtypes = [C.c_uint64]
         L.ctts_gpu_flac_bound.restype = C.c_uint64
+        L.ctts_gpu_session_begin_g711.argtypes = [vp, C.POINTER(AssemblyParams), C.c_int, vp, C.c_uint64, vp, vp, C.POINTER(vp)]
+        L.ctts_gpu_session_submit_g711.argtypes = [vp, C.POINTER(CBatchPlan), vp, vp]
         L.ctts_gpu_synth_batch_packed.argtypes = [vp, C.POINTER(CBatchPlan), C.POINTER(AssemblyParams), vp, C.c_uint64, vp, vp, u64p]
         L.ctts_gpu_multi_synth_batch.argtypes = [C.POINTER(vp), C.c_uint32, C.POINTER(CBatchPlan), C.POINTER(AssemblyParams),
                                                  vp, vp, vp, vp]
@@ -333,6 +336,29 @@ class GpuSynth:
         rc_end = L.ctts_gpu_session_end(h, C.byref(used))
         self._check(rc or rc_end)
         return off[:n], nbytes[:n], cnt[:n], int(used.value)
+
+    def synth_pieces_g711(self, pieces: list[BatchPlan], params: AssemblyParams, law: int, out: np.ndarray):
+        """A G.711 session of `law` (G711_ULAW or G711_ALAW) fed with the given plans, one piece each
+        (ctts_gpu_session_begin_g711 / _submit_g711): one byte per sample in the uint8 buffer `out`, in the packed
+        layout.  Returns (byte offsets, sample counts, bytes used) over all utterances of all pieces, in order."""
+        assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
+        L = lib()
+        h = C.c_void_p()
+        self._check(L.ctts_gpu_session_begin_g711(self._h, C.byref(params), law, out.ctypes.data, out.size, None, None, C.byref(h)))
+        n = sum(p.n_utts for p in pieces)
+        off = np.zeros(max(n, 1), dtype=np.uint64)
+        cnt = np.zeros(max(n, 1), dtype=np.uint32)
+        at, rc = 0, 0
+        for p in pieces:
+            cp = p.as_c()
+            rc = L.ctts_gpu_session_submit_g711(h, C.byref(cp), off[at:].ctypes.data, cnt[at:].ctypes.data)
+            if rc:
+                break
+            at += p.n_utts
+        used = C.c_uint64()
+        rc_end = L.ctts_gpu_session_end(h, C.byref(used))
+        self._check(rc or rc_end)
+        return off[:n], cnt[:n], int(used.value)
 
     def flac_bound(self, plan: BatchPlan) -> int:
         """Bytes that are always enough for a FLAC session over the plan: ctts_gpu_flac_bound of every bound, rounded up to 16."""

@@ -45,6 +45,8 @@ def lib() -> C.CDLL:
                                                  C.POINTER(C.c_uint64), C.POINTER(Options), C.POINTER(Timing)]
         L.ctts_b200_capacity_hint_flac.argtypes = [vp, vp, vp, C.c_uint32, C.c_uint32]
         L.ctts_b200_capacity_hint_flac.restype = C.c_uint64
+        L.ctts_b200_synth_texts_g711.argtypes = [vp, vp, C.c_int, vp, vp, C.c_uint32, vp, C.c_uint64, vp, vp, vp,
+                                                 C.POINTER(C.c_uint64), C.POINTER(Options), C.POINTER(Timing)]
         L.ctts_b200_plan_cache_create.argtypes = [C.c_size_t]
         L.ctts_b200_plan_cache_create.restype = vp
         L.ctts_b200_plan_cache_destroy.argtypes = [vp]
@@ -147,3 +149,23 @@ def synth_texts_flac(front, gpu, batch: TextBatch, out: np.ndarray, piece_utts: 
         msg = _gpu.lib().ctts_gpu_last_error(gpu._h)
         raise _gpu.GpuError(f"ctts_b200_synth_texts_flac: {rc}: {msg.decode(errors='replace') if msg else ''}")
     return off[:n], nbytes[:n], cnt[:n], int(used.value), tm
+
+
+def synth_texts_g711(front, gpu, batch: TextBatch, law: int, out: np.ndarray, piece_utts: int = 0, threads: int = 0,
+                     cache: PlanCache | None = None):
+    """ctts_b200_synth_texts_g711: one G.711 byte of `law` (gpu.G711_ULAW or gpu.G711_ALAW) per sample in the uint8
+    buffer `out`, in the packed layout; capacity_hint(front, batch, rate) bytes are always enough.
+    Returns (byte offsets[n], sample counts[n], bytes_used, Timing)."""
+    assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
+    n = batch.n
+    off = np.zeros(max(n, 1), dtype=np.uint64)
+    cnt = np.zeros(max(n, 1), dtype=np.uint32)
+    used = C.c_uint64()
+    opt = Options(piece_utts, threads, None, None, cache._h if cache is not None else None)
+    tm = Timing()
+    rc = lib().ctts_b200_synth_texts_g711(front._h, gpu._h, law, batch.ptrs, batch.speeds_ptr, n, out.ctypes.data, out.size,
+                                          off.ctypes.data, cnt.ctypes.data, None, C.byref(used), C.byref(opt), C.byref(tm))
+    if rc != 0:
+        msg = _gpu.lib().ctts_gpu_last_error(gpu._h)
+        raise _gpu.GpuError(f"ctts_b200_synth_texts_g711: {rc}: {msg.decode(errors='replace') if msg else ''}")
+    return off[:n], cnt[:n], int(used.value), tm

@@ -71,5 +71,6 @@ uint64_t ctts_b200_capacity_hint(ctts_front* front, const char* const* texts, co
 
 #include "ctts_b200_rate.h"
 #include "ctts_b200_flac.h"
+#include "ctts_b200_g711.h"
 
 #endif /* CTTS_B200_H */

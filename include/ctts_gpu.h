@@ -77,8 +77,8 @@ int ctts_gpu_set_output_rate(ctts_gpu_ctx* ctx, uint32_t hz);
  * is then unchanged.
  *
  * It applies to every path: resident plans (a plan keeps the setting it was created under), all ctts_gpu_synth_batch*
- * calls, PCM and FLAC sessions, ctts_b200_synth_texts(_flac) and ctts_gpu_multi_synth_batch, which rejects contexts
- * whose settings differ. */
+ * calls, PCM, FLAC and G.711 sessions, ctts_b200_synth_texts(_flac, _g711) and ctts_gpu_multi_synth_batch, which
+ * rejects contexts whose settings differ. */
 int ctts_gpu_set_loudness(ctts_gpu_ctx* ctx, float target_lufs, float ceiling_dbfs);
 /* The same loudness normalization with a TRUE-PEAK ceiling of C dBTP (ITU-R BS.1770-4 Annex 2, DESIGN.md 3.6), for
  * delivery specifications such as EBU R128 (-1 dBTP).  The peak is that of the signal interpolated 4x with the 49-tap
@@ -180,6 +180,36 @@ int ctts_gpu_session_submit_flac(ctts_gpu_session* s, const ctts_batch_plan* pie
 /* Largest .flac file of an utterance of `samples` samples: 42 + ceil(samples / 4096) * (16 + 1 + 8192 + 2) bytes
  * (a VERBATIM subframe caps every frame). */
 uint64_t ctts_gpu_flac_bound(uint64_t samples);
+
+/* ---- G.711 sessions: the same session, every sample delivered as one μ-law or A-law byte (DESIGN.md 3.7) --------
+ * For telephony: 8-bit G.711 at the context's output rate (8000 Hz for the classic telephone channel), as IVR and
+ * contact-center systems play it.  The encoder is the ITU-T G.711 reference (the G.191 tools, Sun's g711.c, CPython's
+ * audioop.lin2ulaw / lin2alaw on 16-bit input), applied to the int16 samples a PCM session delivers for the same piece
+ * on the same context settings (after assembly, time stretching, rate conversion and loudness):
+ *   μ-law  v = x >> 2 (arithmetic); m = min(|v|, 8159) + 33; segment s = the first of 0..7 with m <= (64 << s) - 1
+ *          (none: code 0x7F), else code = (s << 4) | ((m >> (s + 1)) & 0xF); the byte is code ^ 0x7F for v < 0,
+ *          code ^ 0xFF otherwise.
+ *   A-law  v = x >> 3; m = -v - 1 for v < 0, else v; s = the first of 0..7 with m <= (32 << s) - 1;
+ *          code = (s << 4) | ((m >> max(s, 1)) & 0xF); the byte is code ^ 0x55 for v < 0, code ^ 0xD5 otherwise.
+ * No zero-code suppression.  E.g. x = 0, -1, 100, -100, 32767, -32768 -> μ-law ff 7e f2 72 80 00, A-law d5 55 d3 53 aa 2a.
+ * Layout: the PCM session's packed layout with bytes in place of samples.  Utterance u is out[out_offsets[u] ..
+ * out_offsets[u] + out_counts[u]), one byte per sample; every offset is a multiple of 8 and the next utterance starts
+ * at out_offsets[u] + up8(out_counts[u]); the padding bytes hold the law's code for silence (0xFF μ-law, 0xD5 A-law),
+ * not zero (a zero byte decodes to a near full-scale sample).
+ * begin_g711   as ctts_gpu_session_begin with law CTTS_GPU_G711_ULAW or CTTS_GPU_G711_ALAW; out (page-locked for full
+ *              copy speed) holds capacity_bytes bytes.  The sum of up8(bound) over the ctts_gpu_plan_bounds, read as
+ *              bytes, is always enough.
+ * submit_g711  as ctts_gpu_session_submit, offsets in bytes.  A buffer that turns out too small ends the session with
+ *              CTTS_GPU_ERR_BOUNDS.
+ * ctts_gpu_session_end closes it; *samples_used is then the number of BYTES taken in out.  Any other law, a second
+ * session on the context, and a submit call of another kind on a G.711 session (or submit_g711 on a PCM or FLAC
+ * session) is CTTS_GPU_ERR_INVALID_ARG. */
+#define CTTS_GPU_G711_ULAW 1
+#define CTTS_GPU_G711_ALAW 2
+int ctts_gpu_session_begin_g711(ctts_gpu_ctx* ctx, const ctts_assembly_params* params, int law, uint8_t* out,
+                                uint64_t capacity_bytes, ctts_gpu_chunk_fn on_piece, void* user, ctts_gpu_session** s);
+int ctts_gpu_session_submit_g711(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets,
+                                 uint32_t* out_counts);
 
 /* ---- one batch on several GPUs of one box ---------------------------------------------------------
  * ctxs[d] is a context on device d (each holds its own replica of the voice: ctts_gpu_init per device).
