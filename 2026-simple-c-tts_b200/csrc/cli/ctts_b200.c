@@ -34,6 +34,9 @@
 
 #define SAMPLE_RATE CTTS_PLAN_SAMPLE_RATE
 
+/* what the files hold: 16-bit PCM WAV, G.711 WAV of either law, or FLAC */
+typedef enum { OUT_WAV = 0, OUT_ULAW = CTTS_GPU_G711_ULAW, OUT_ALAW = CTTS_GPU_G711_ALAW, OUT_FLAC } out_kind;
+
 /* the loudness options: lufs = 0 without lufs=; true_peak when dbtp= was given */
 typedef struct {
     float lufs, dbtp;
@@ -99,19 +102,19 @@ static int engine_open(engine* e, const char* db_path, uint32_t rate, const loud
 }
 
 /* Optional last arguments lufs=<target>, dbtp=<ceiling> and g711=ulaw|alaw, in any order (after the output argument):
- * taken off the argument list.  ld->lufs = 0 without lufs=; *law = 0 without g711=, else CTTS_GPU_G711_ULAW or
- * CTTS_GPU_G711_ALAW.  -1 when a value is not a number or not a law, an option repeats or dbtp= comes without lufs=
+ * taken off the argument list.  ld->lufs = 0 without lufs=; *kind = OUT_WAV without g711=, else OUT_ULAW or OUT_ALAW.
+ * -1 when a value is not a number or not a law, an option repeats or dbtp= comes without lufs=
  * (any other value is checked by ctts_gpu_set_loudness(_true_peak)). */
-static int take_options(int* argc, char** argv, loudness_arg* ld, int* law) {
+static int take_options(int* argc, char** argv, loudness_arg* ld, out_kind* kind) {
     memset(ld, 0, sizeof *ld);
-    *law = 0;
+    *kind = OUT_WAV;
     int have_lufs = 0;
     while (*argc >= 6) {   /* behind the required arguments only */
         const char* a = argv[*argc - 1];
         if (strncmp(a, "g711=", 5) == 0) {
-            if (*law) return -1;
-            *law = strcmp(a + 5, "ulaw") == 0 ? CTTS_GPU_G711_ULAW : strcmp(a + 5, "alaw") == 0 ? CTTS_GPU_G711_ALAW : -1;
-            if (*law < 0) return -1;
+            if (*kind) return -1;
+            *kind = strcmp(a + 5, "ulaw") == 0 ? OUT_ULAW : strcmp(a + 5, "alaw") == 0 ? OUT_ALAW : OUT_WAV;
+            if (!*kind) return -1;
             (*argc)--;
             continue;
         }
@@ -133,34 +136,7 @@ static int take_options(int* argc, char** argv, loudness_arg* ld, int* law) {
     return ld->true_peak && !have_lufs ? -1 : 0;
 }
 
-/* ctts_write_wav, ctts.c:809: 44-byte RIFF/WAVE header (PCM, mono, 16 bit) + samples */
-static int write_wav(const char* path, const int16_t* samples, size_t count, uint32_t rate) {
-    FILE* f = fopen(path, "wb");
-    if (!f) return -1;
-    const uint32_t data = (uint32_t)(count * sizeof(int16_t)), riff = 36 + data, fmt = 16, sr = rate, br = rate * 2;
-    const uint16_t pcm = 1, ch = 1, align = 2, bits = 16;
-    fwrite("RIFF", 1, 4, f); fwrite(&riff, 4, 1, f); fwrite("WAVE", 1, 4, f);
-    fwrite("fmt ", 1, 4, f); fwrite(&fmt, 4, 1, f);
-    fwrite(&pcm, 2, 1, f); fwrite(&ch, 2, 1, f); fwrite(&sr, 4, 1, f); fwrite(&br, 4, 1, f);
-    fwrite(&align, 2, 1, f); fwrite(&bits, 2, 1, f);
-    fwrite("data", 1, 4, f); fwrite(&data, 4, 1, f);
-    fwrite(samples, sizeof(int16_t), count, f);
-    return fclose(f) == 0 ? 0 : -1;
-}
-
-/* G.711 .wav (g711_wav.h): the header, the count code bytes and a pad byte when the count is odd */
-static int write_g711_wav(const char* path, const uint8_t* codes, size_t count, uint32_t rate, int law) {
-    FILE* f = fopen(path, "wb");
-    if (!f) return -1;
-    uint8_t h[G711_WAV_HEADER_BYTES];
-    g711_wav_header(h, law, rate, (uint32_t)count);
-    const uint8_t pad = 0;
-    int ok = fwrite(h, 1, sizeof h, f) == sizeof h && fwrite(codes, 1, count, f) == count;
-    if (count & 1) ok = ok && fwrite(&pad, 1, 1, f) == 1;
-    return fclose(f) == 0 && ok ? 0 : -1;
-}
-
-/* N texts -> N PCM spans (or, with flac, N .flac files; with a G.711 law, N spans of codes) of one pinned buffer through
+/* N texts -> N PCM spans (or N .flac files, or N spans of G.711 codes) of one pinned buffer through
  * ctts_b200_synth_texts(_flac, _g711) (the front end's planner threads feed the device piece by piece): r->out (release
  * with ctts_gpu_host_free), r->off[u], r->bytes[u] (FLAC: file sizes) and r->cnt[u] (malloc'ed, n entries each); stats
  * may be NULL (2n: found, missing).  on_chunk (may be NULL) is called as soon as a range of utterances is in host
@@ -180,24 +156,23 @@ static void result_free(batch_result* r) {
     memset(r, 0, sizeof *r);
 }
 
-static int ctts_b200_synthesize_batch(engine* e, const char* const* texts, const float* speeds, uint32_t n, int flac,
-                                      int law, batch_result* r, uint32_t* stats, ctts_gpu_chunk_fn on_chunk, void* user) {
-    int rc = 0;
+static int ctts_b200_synthesize_batch(engine* e, const char* const* texts, const float* speeds, uint32_t n, out_kind kind,
+                                      batch_result* r, uint32_t* stats, ctts_gpu_chunk_fn on_chunk, void* user) {
     /* replaces the SampleBuffer growth policy; G.711: the sample capacity, read as bytes */
-    const uint64_t cap = flac ? ctts_b200_capacity_hint_flac(e->front, texts, speeds, n, e->rate)
-                              : ctts_b200_capacity_hint_rate(e->front, texts, speeds, n, e->rate);
+    const uint64_t cap = kind == OUT_FLAC ? ctts_b200_capacity_hint_flac(e->front, texts, speeds, n, e->rate)
+                                          : ctts_b200_capacity_hint_rate(e->front, texts, speeds, n, e->rate);
     r->off = malloc(sizeof *r->off * ((size_t)n + 1));
     r->bytes = calloc(n ? n : 1, sizeof *r->bytes);
     r->cnt = calloc(n ? n : 1, sizeof *r->cnt);
-    r->out = ctts_gpu_host_alloc((flac || law ? 1 : sizeof(int16_t)) * (cap ? cap : 16));
-    if (!r->off || !r->bytes || !r->cnt || !r->out) rc = CTTS_GPU_ERR_OUT_OF_MEMORY;
+    r->out = ctts_gpu_host_alloc((kind == OUT_WAV ? sizeof(int16_t) : 1) * (cap ? cap : 16));
     ctts_b200_options opt;
     memset(&opt, 0, sizeof opt);
     opt.on_piece = on_chunk;
     opt.user = user;
-    if (!rc && flac) rc = ctts_b200_synth_texts_flac(e->front, e->gpu, texts, speeds, n, r->out, cap, r->off, r->bytes, r->cnt, stats, NULL, &opt, NULL);
-    else if (!rc && law) rc = ctts_b200_synth_texts_g711(e->front, e->gpu, law, texts, speeds, n, r->out, cap, r->off, r->cnt, stats, NULL, &opt, NULL);
-    else if (!rc) rc = ctts_b200_synth_texts(e->front, e->gpu, texts, speeds, n, r->out, cap, r->off, r->cnt, stats, NULL, &opt, NULL);
+    int rc = !r->off || !r->bytes || !r->cnt || !r->out ? CTTS_GPU_ERR_OUT_OF_MEMORY
+           : kind == OUT_FLAC ? ctts_b200_synth_texts_flac(e->front, e->gpu, texts, speeds, n, r->out, cap, r->off, r->bytes, r->cnt, stats, NULL, &opt, NULL)
+           : kind != OUT_WAV  ? ctts_b200_synth_texts_g711(e->front, e->gpu, kind, texts, speeds, n, r->out, cap, r->off, r->cnt, stats, NULL, &opt, NULL)
+                              : ctts_b200_synth_texts(e->front, e->gpu, texts, speeds, n, r->out, cap, r->off, r->cnt, stats, NULL, &opt, NULL);
     if (rc) {
         fprintf(stderr, "synthesis failed: %d %s\n", rc, ctts_gpu_last_error(e->gpu));
         result_free(r);
@@ -205,10 +180,38 @@ static int ctts_b200_synthesize_batch(engine* e, const char* const* texts, const
     return rc;
 }
 
-static int write_flac(const char* path, const uint8_t* data, size_t bytes) {
+/* utterance u of r as the file `path`: a WAV file as ctts_write_wav (ctts.c:809) writes it (44-byte RIFF/WAVE header,
+ * PCM, mono, 16 bit), a G.711 .wav file (g711_wav.h: the header, the codes and a pad byte when the count is odd) or the
+ * .flac file */
+static int write_utterance(const char* path, out_kind kind, const batch_result* r, uint32_t u, uint32_t rate) {
     FILE* f = fopen(path, "wb");
     if (!f) return -1;
-    const int ok = fwrite(data, 1, bytes, f) == bytes;
+    const uint8_t* bytes = (const uint8_t*)r->out + r->off[u];
+    const uint32_t count = r->cnt[u];
+    int ok = 1;
+    switch (kind) {
+    case OUT_WAV: {
+        const uint32_t data = count * (uint32_t)sizeof(int16_t), riff = 36 + data, fmt = 16, sr = rate, br = rate * 2;
+        const uint16_t pcm = 1, ch = 1, align = 2, bits = 16;
+        fwrite("RIFF", 1, 4, f); fwrite(&riff, 4, 1, f); fwrite("WAVE", 1, 4, f);
+        fwrite("fmt ", 1, 4, f); fwrite(&fmt, 4, 1, f);
+        fwrite(&pcm, 2, 1, f); fwrite(&ch, 2, 1, f); fwrite(&sr, 4, 1, f); fwrite(&br, 4, 1, f);
+        fwrite(&align, 2, 1, f); fwrite(&bits, 2, 1, f);
+        fwrite("data", 1, 4, f); fwrite(&data, 4, 1, f);
+        fwrite((const int16_t*)r->out + r->off[u], sizeof(int16_t), count, f);
+        break;
+    }
+    case OUT_ULAW:
+    case OUT_ALAW: {
+        uint8_t h[G711_WAV_HEADER_BYTES];
+        const uint8_t pad = 0;
+        g711_wav_header(h, kind, rate, count);
+        ok = fwrite(h, 1, sizeof h, f) == sizeof h && fwrite(bytes, 1, count, f) == count;
+        if (count & 1) ok = ok && fwrite(&pad, 1, 1, f) == 1;
+        break;
+    }
+    case OUT_FLAC: ok = fwrite(bytes, 1, r->bytes[u], f) == r->bytes[u]; break;
+    }
     return fclose(f) == 0 && ok ? 0 : -1;
 }
 
@@ -228,8 +231,8 @@ static uint32_t parse_rate(const char* a) {
 
 static int cmd_synth(int argc, char** argv) {
     loudness_arg ld;
-    int law;
-    if (take_options(&argc, argv, &ld, &law) || argc < 5 || argc > 7 || (law && ends_with(argv[4], ".flac"))) {
+    out_kind kind;
+    if (take_options(&argc, argv, &ld, &kind) || argc < 5 || argc > 7 || (kind && ends_with(argv[4], ".flac"))) {
         fprintf(stderr, "Usage: %s synth <database.db> \"text\" <output.wav|output.flac> [speed] [rate] [lufs=<target> [dbtp=<ceiling>]] [g711=ulaw|alaw]\n"
                         "       (g711= writes a G.711 .wav file, not FLAC)\n", argv[0]);
         return 1;
@@ -245,16 +248,14 @@ static int cmd_synth(int argc, char** argv) {
     if (argc <= 5 && e.cfg.default_speed != 1.0f) speed = e.cfg.default_speed;
     printf("Loaded database with %u units\n", ctts_front_unit_count(e.front));
     const char* texts[1] = {argv[3]};
-    const int flac = ends_with(argv[4], ".flac");
+    if (ends_with(argv[4], ".flac")) kind = OUT_FLAC;
     batch_result r;
     uint32_t stats[2] = {0, 0};
-    if (ctts_b200_synthesize_batch(&e, texts, &speed, 1, flac, law, &r, stats, NULL, NULL)) { engine_close(&e); return 1; }
+    if (ctts_b200_synthesize_batch(&e, texts, &speed, 1, kind, &r, stats, NULL, NULL)) { engine_close(&e); return 1; }
     printf("Synthesized %u samples (%.2f seconds)\n", r.cnt[0], (float)r.cnt[0] / (float)e.rate);
     printf("Units found: %u, missing: %u\n", stats[0], stats[1]);
-    int rc = flac  ? write_flac(argv[4], (const uint8_t*)r.out + r.off[0], r.bytes[0])
-             : law ? write_g711_wav(argv[4], (const uint8_t*)r.out + r.off[0], r.cnt[0], e.rate, law)
-                   : write_wav(argv[4], (const int16_t*)r.out + r.off[0], r.cnt[0], e.rate);
-    if (rc) fprintf(stderr, "Failed to write %s: %s\n", flac ? "FLAC" : "WAV", argv[4]);
+    int rc = write_utterance(argv[4], kind, &r, 0, e.rate);
+    if (rc) fprintf(stderr, "Failed to write %s: %s\n", kind == OUT_FLAC ? "FLAC" : "WAV", argv[4]);
     else printf("Written to %s\n", argv[4]);
     result_free(&r);
     engine_close(&e);
@@ -267,7 +268,7 @@ typedef struct {
     const char* dir;
     uint32_t rate;
     uint32_t base;   /* first utterance of the group being synthesised */
-    int flac, law;
+    out_kind kind;
     const batch_result* r;
     double seconds;
     int rc;
@@ -277,25 +278,23 @@ static void write_chunk(void* user, uint32_t u0, uint32_t u1) {
     wav_sink* w = user;
     for (uint32_t u = u0; u < u1 && !w->rc; u++) {
         char path[4096];
-        snprintf(path, sizeof path, "%s/%06u.%s", w->dir, w->base + u, w->flac ? "flac" : "wav");
-        w->rc = w->flac  ? write_flac(path, (const uint8_t*)w->r->out + w->r->off[u], w->r->bytes[u])
-                : w->law ? write_g711_wav(path, (const uint8_t*)w->r->out + w->r->off[u], w->r->cnt[u], w->rate, w->law)
-                         : write_wav(path, (const int16_t*)w->r->out + w->r->off[u], w->r->cnt[u], w->rate);
+        snprintf(path, sizeof path, "%s/%06u.%s", w->dir, w->base + u, w->kind == OUT_FLAC ? "flac" : "wav");
+        w->rc = write_utterance(path, w->kind, w->r, u, w->rate);
         w->seconds += (double)w->r->cnt[u] / w->rate;
     }
 }
 
 static int cmd_synth_batch(int argc, char** argv) {
     loudness_arg ld;
-    int law;
-    if (take_options(&argc, argv, &ld, &law) || argc < 5 || argc > 7 || (argc == 7 && strcmp(argv[6], "flac") != 0) ||
-        (law && argc == 7)) {
+    out_kind kind;
+    if (take_options(&argc, argv, &ld, &kind) || argc < 5 || argc > 7 || (argc == 7 && strcmp(argv[6], "flac") != 0) ||
+        (kind && argc == 7)) {
         fprintf(stderr, "Usage: %s synth-batch <database.db> <texts.tsv> <out_dir> [rate] [flac] [lufs=<target> [dbtp=<ceiling>]] [g711=ulaw|alaw]\n"
                         "       (g711= writes G.711 .wav files, not FLAC)\n", argv[0]);
         return 1;
     }
     const uint32_t rate = argc > 5 ? parse_rate(argv[5]) : SAMPLE_RATE;
-    const int flac = argc == 7;
+    if (argc == 7) kind = OUT_FLAC;
     FILE* f = fopen(argv[3], "rb");
     if (!f) { fprintf(stderr, "cannot read %s\n", argv[3]); return 1; }
     char** texts = NULL;
@@ -329,19 +328,19 @@ static int cmd_synth_batch(int argc, char** argv) {
     }
     if (mkdir(argv[4], 0777) != 0 && errno != EEXIST) { fprintf(stderr, "cannot create %s\n", argv[4]); engine_close(&e); return 1; }
     batch_result r;
-    wav_sink sink = {argv[4], e.rate, 0, flac, law, &r, 0.0, 0};
+    wav_sink sink = {argv[4], e.rate, 0, kind, &r, 0.0, 0};
     /* groups of 1024 utterances: the pinned buffer is sized from the texts alone (ctts_b200_capacity_hint) */
     int rc = 0;
     for (uint32_t g0 = 0; g0 < n && !rc; g0 += 1024) {
         const uint32_t gn = n - g0 < 1024 ? n - g0 : 1024;
         sink.base = g0;
-        rc = ctts_b200_synthesize_batch(&e, (const char* const*)texts + g0, speeds + g0, gn, flac, law, &r, NULL, write_chunk, &sink);
+        rc = ctts_b200_synthesize_batch(&e, (const char* const*)texts + g0, speeds + g0, gn, kind, &r, NULL, write_chunk, &sink);
         if (!rc) {
             rc = sink.rc;
             result_free(&r);
         }
     }
-    if (rc) fprintf(stderr, "Failed to write %s files into %s\n", flac ? "FLAC" : "WAV", argv[4]);
+    if (rc) fprintf(stderr, "Failed to write %s files into %s\n", kind == OUT_FLAC ? "FLAC" : "WAV", argv[4]);
     else printf("Synthesized %u utterances (%.1f seconds of audio) into %s\n", n, sink.seconds, argv[4]);
     for (uint32_t u = 0; u < n; u++) free(texts[u]);
     free(texts);

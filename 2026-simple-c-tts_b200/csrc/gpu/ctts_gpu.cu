@@ -170,7 +170,7 @@ struct ctts_gpu_ctx {
     int smem_optin = 0;
     // A batch is worked on in PIECES (contiguous utterance ranges); up to kLanes (4) pieces are in flight: the
     // host compiles piece c+1 while the device assembles piece c and piece c-1 is copied to the caller.
-    // Every lane owns grow-only workspaces (no cudaMalloc / cudaFree per call).
+    // Every lane owns grow-only workspaces (no cudaMalloc / cudaFree per call); device capacities count bytes.
     static constexpr int kLanes = 4;
     struct Lane {
         Arena arena;                       // device workspace + pinned staging of the plan upload
@@ -178,18 +178,15 @@ struct ctts_gpu_ctx {
         uint64_t d_out_cap = 0;
         int16_t* d_rs = nullptr;           // output-rate slots (only when the context converts the rate)
         uint64_t d_rs_cap = 0;
-        int16_t* d_pack = nullptr;         // packed mode: the utterances' samples back to back
+        uint8_t* d_pack = nullptr;         // packed mode: the utterances back to back (PCM samples, G.711 codes or FLAC files)
         uint64_t d_pack_cap = 0;
-        unsigned long long* d_pack_off = nullptr;   // n + 1 (+ the n + 1 slot offsets behind them)
-        size_t d_pack_off_cap = 0;
-        uint8_t* d_flac = nullptr;         // FLAC sessions: the utterances' files back to back (DESIGN.md 3.5)
-        uint64_t d_flac_cap = 0;           // bytes
+        unsigned long long* d_pack_off = nullptr;   // packed mode: ResLayout
+        uint64_t d_pack_off_cap = 0;
         ctts::FlacFrame* d_frames = nullptr;   // FLAC sessions: one descriptor per frame a slot can hold
-        uint64_t d_frames_cap = 0;         // bytes
+        uint64_t d_frames_cap = 0;
         uint32_t* d_flac_info = nullptr;   // FLAC sessions: per utterance file bytes, min and max frame bytes
-        uint64_t d_flac_info_cap = 0;      // bytes
-        uint32_t* h_res = nullptr;         // pinned: counts [n], then device error flags [n], (FLAC: file bytes [n],) then
-                                           // (8-byte aligned) slot offsets [n + 1] (FLAC: and frame bases [n + 1])
+        uint64_t d_flac_info_cap = 0;
+        uint32_t* h_res = nullptr;         // pinned: ResLayout
         size_t h_res_cap = 0;              // in 4-byte words
         cudaEvent_t kernels_done = nullptr, counts_ready = nullptr, copied = nullptr;
         ctts_gpu_plan* plan = nullptr;     // piece in flight
@@ -579,7 +576,6 @@ void ctts_gpu_free(ctts_gpu_ctx* ctx) {
         cudaFree(l.d_rs);
         cudaFree(l.d_pack);
         cudaFree(l.d_pack_off);
-        cudaFree(l.d_flac);
         cudaFree(l.d_frames);
         cudaFree(l.d_flac_info);
         if (l.h_res) cudaFreeHost(l.h_res);
@@ -1913,6 +1909,15 @@ int launch_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_final, cudaS
     return sliced(ctts::ld_apply_kernel, p->ld_apply_tiles, ctts::LD_APPLY_THREADS);
 }
 
+// Enqueue the plan's stage chain: assembly and WSOLA into the native-rate slots d_nat, output-rate conversion into
+// d_final (the same slots at the native rate), loudness normalization in place there.
+int launch_chain(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_nat, int16_t* d_final, cudaStream_t st) {
+    int rc = launch_assemble(ctx, p, d_nat, st);
+    if (!rc) rc = launch_stretch(ctx, p, d_nat, st);
+    if (!rc) rc = launch_resample(ctx, p, d_nat, d_final, st);
+    return rc ? rc : launch_loudness(ctx, p, d_final, st);
+}
+
 }  // namespace
 
 extern "C" {
@@ -1961,12 +1966,8 @@ int ctts_gpu_plan_run(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out) {
             CU(ctx, cudaMalloc(reinterpret_cast<void**>(&p->d_nat_owned), std::max<uint64_t>(p->n_offsets[p->n_utts], 8) * sizeof(int16_t)));
         d_nat = p->d_nat_owned;
     }
-    int rc = begin_run(ctx, p);
-    if (!rc) rc = launch_assemble(ctx, p, d_nat, ctx->stream);
-    if (!rc) rc = launch_stretch(ctx, p, d_nat, ctx->stream);
-    if (!rc) rc = launch_resample(ctx, p, d_nat, d_pcm_out, ctx->stream);
-    if (!rc) rc = launch_loudness(ctx, p, d_pcm_out, ctx->stream);
-    return rc;
+    const int rc = begin_run(ctx, p);
+    return rc ? rc : launch_chain(ctx, p, d_nat, d_pcm_out, ctx->stream);
 }
 
 int ctts_gpu_plan_read_counts(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t* out_counts) {
@@ -2053,22 +2054,48 @@ int ctts_gpu_plan_read_pre(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t u, int1
 enum SessionOutput { OUT_PCM = 0, OUT_ULAW = CTTS_GPU_G711_ULAW, OUT_ALAW = CTTS_GPU_G711_ALAW, OUT_FLAC };
 static_assert(OUT_ULAW == ctts::G711_ULAW && OUT_ALAW == ctts::G711_ALAW, "G.711 law constants");
 
+// What the delivery path needs to know of each output kind, indexed by SessionOutput
+struct OutputKind {
+    uint32_t unit_bytes;   // host bytes of one unit: capacity, cursor and offsets count units
+    uint32_t align;        // a packed utterance takes its size rounded up to this many units
+    const char *unit, *name, *submit;   // for error messages: the units, the kind, the submit call it takes
+};
+constexpr OutputKind kOutput[] = {{2, 8, "samples", "PCM", "ctts_gpu_session_submit"},
+                                  {1, 8, "bytes", "G.711", "ctts_gpu_session_submit_g711"},
+                                  {1, 8, "bytes", "G.711", "ctts_gpu_session_submit_g711"},
+                                  {1, 16, "bytes", "FLAC", "ctts_gpu_session_submit_flac"}};
+
+// Where a piece of n utterances keeps its results.  h_res (pinned, 4-byte words): counts [n], device error flags [n],
+// (FLAC: file bytes [n],) then, 8-byte aligned, the slot offsets [n + 1] (FLAC: and the first frame descriptor of
+// every utterance [n + 1]).  Packed mode uploads those slot words to d_pack_off behind the n + 1 packed offsets.
+struct ResLayout {
+    size_t flags, bytes, size, slots;          // word offsets in h_res; size: what sizes a packed utterance
+    size_t slot_words, res_words, off_words;   // 8-byte words at slots; the words h_res and d_pack_off need
+    ResLayout(uint32_t n, SessionOutput k) : flags(n), bytes(2 * (size_t)n) {
+        const size_t heads = k == OUT_FLAC ? 3 : 2;
+        size = k == OUT_FLAC ? bytes : 0;   // the file bytes, else the count
+        slots = (heads * n + 1) & ~(size_t)1;
+        slot_words = (heads - 1) * ((size_t)n + 1);
+        res_words = slots + 2 + 2 * slot_words;
+        off_words = (size_t)n + 1 + slot_words;
+    }
+};
+
 struct ctts_gpu_session {
-    ctts_gpu_ctx* ctx = nullptr;
-    ctts_assembly_params prm{};
-    int16_t* pcm_out = nullptr;
-    uint8_t* byte_out = nullptr;  // FLAC and G.711 sessions: the output goes here, and capacity and cursor count bytes
-    SessionOutput kind = OUT_PCM;
-    uint64_t capacity = 0;        // samples
-    uint64_t cursor = 0;          // next free sample (library-chosen layout)
-    uint32_t submitted = 0, harvested = 0;   // pieces
-    uint32_t copy_next = 0;       // packed mode: first piece whose PCM copy is not enqueued yet
-    uint32_t utts = 0;            // utterances submitted so far
-    ctts_gpu_chunk_fn on_piece = nullptr;
-    void* user = nullptr;
-    int error = 0;
-    uint64_t d2h_samples = 0;     // samples (FLAC, G.711: bytes) copied to the host
+    ctts_gpu_ctx* ctx;
+    ctts_assembly_params prm;
+    SessionOutput kind;
+    uint8_t* out;                 // the caller's buffer
+    uint64_t capacity;            // units of kOutput[kind]
+    ctts_gpu_chunk_fn on_piece;
+    void* user;
     std::chrono::steady_clock::time_point t0;
+    uint64_t cursor = 0;          // next free unit (library-chosen layout)
+    uint32_t submitted = 0, harvested = 0;   // pieces
+    uint32_t copy_next = 0;       // packed mode: first piece whose copy is not enqueued yet
+    uint32_t utts = 0;            // utterances submitted so far
+    int error = 0;
+    uint64_t d2h_bytes = 0;       // copied to the host
 };
 
 namespace {
@@ -2079,10 +2106,39 @@ void drain(ctts_gpu_ctx* ctx) {
 }
 
 // Packed mode: the counts of the lane's piece are (or will shortly be) on the host; lay its utterances out
-// back to back at the session's cursor and enqueue ONE copy of exactly the samples that exist.
-int enqueue_packed_copy(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l);
+// back to back at the session's cursor and enqueue ONE copy of exactly the units that exist.
+int enqueue_packed_copy(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l) {
+    ctts_gpu_ctx* ctx = s->ctx;
+    const OutputKind& k = kOutput[s->kind];
+    l.copy_pending = false;
+    cudaError_t e = cudaEventSynchronize(l.counts_ready);
+    if (e != cudaSuccess) {
+        if (!s->error) s->error = fail(ctx, CTTS_GPU_ERR_CUDA, "piece of utterances %u..%u: %s", l.utt_base, l.utt_base + l.n, cudaGetErrorString(e));
+        return s->error;
+    }
+    const uint32_t* h_size = l.h_res + ResLayout(l.n, s->kind).size;
+    uint64_t o = s->cursor;
+    for (uint32_t u = 0; u < l.n; u++) {
+        if (l.user_offsets) l.user_offsets[u] = o;
+        o += (h_size[u] + (k.align - 1ull)) & ~(k.align - 1ull);
+    }
+    const uint64_t len = o - s->cursor;
+    if (o > s->capacity) {
+        if (!s->error) s->error = fail(ctx, CTTS_GPU_ERR_BOUNDS, "output buffer too small: %llu %s needed up to utterance %u", (unsigned long long)o, k.unit, l.utt_base + l.n);
+        return s->error;
+    }
+    if (len) e = cudaMemcpyAsync(s->out + s->cursor * k.unit_bytes, l.d_pack, len * k.unit_bytes, cudaMemcpyDeviceToHost, ctx->copy_stream);
+    if (e == cudaSuccess) e = cudaEventRecord(l.copied, ctx->copy_stream);
+    if (e != cudaSuccess) {
+        if (!s->error) s->error = fail(ctx, CTTS_GPU_ERR_CUDA, "D2H: %s", cudaGetErrorString(e));
+        return s->error;
+    }
+    s->d2h_bytes += len * k.unit_bytes;
+    s->cursor = o;
+    return CTTS_GPU_OK;
+}
 
-// Packed mode: enqueue, in order, the PCM copies of the pieces whose counts have arrived; pieces up to and
+// Packed mode: enqueue, in order, the copies of the pieces whose counts have arrived; pieces up to and
 // including `must` (a piece index, or none: 0xffffffff... never) are waited for.  Keeps the copy stream fed
 // while the host is about to block on an older piece.
 void pump_copies(ctts_gpu_session* s, uint32_t must_upto) {
@@ -2108,10 +2164,10 @@ int harvest_one(ctts_gpu_session* s) {
     cudaError_t e = cudaEventSynchronize(l.copied);
     if (e != cudaSuccess && !rc) rc = fail(ctx, CTTS_GPU_ERR_CUDA, "piece of utterances %u..%u: %s", l.utt_base, l.utt_base + l.n, cudaGetErrorString(e));
     if (!rc) {
-        const uint32_t* h_cnt = l.h_res;
-        const uint32_t* h_err = l.h_res + l.n;
-        if (l.user_counts) memcpy(l.user_counts, h_cnt, (size_t)l.n * 4);
-        if (l.user_bytes) memcpy(l.user_bytes, l.h_res + 2 * (size_t)l.n, (size_t)l.n * 4);
+        const ResLayout r(l.n, s->kind);
+        const uint32_t* h_err = l.h_res + r.flags;
+        if (l.user_counts) memcpy(l.user_counts, l.h_res, (size_t)l.n * 4);
+        if (l.user_bytes) memcpy(l.user_bytes, l.h_res + r.bytes, (size_t)l.n * 4);
         for (uint32_t u = 0; u < l.n && !rc; u++)
             if (h_err[u]) rc = fail(ctx, CTTS_GPU_ERR_DEVICE, "utterance %u: device error %u", l.utt_base + u, h_err[u]);
     }
@@ -2130,11 +2186,143 @@ int harvest_one(ctts_gpu_session* s) {
     return rc;
 }
 
-// One piece: compile, launch, copy.  Utterance i of the piece is delivered to pcm_out[slot_off[i] ..),
-// slot_cap[i] samples of room (>= its bound); slot_off == nullptr: the library appends packed slots at the
-// session's cursor and reports them through offsets_out.  Asynchronous: returns once everything is enqueued.
-// A FLAC session (packed only) encodes every utterance into a file instead and reports the sizes through out_bytes;
-// a G.711 session (packed only) encodes every sample into one byte of the same packed layout.
+// Grow-only device buffer: at least `bytes` afterwards, *cap in bytes.  zero: a new allocation is zero-filled on the
+// context's stream, so that bytes no kernel writes do not carry an earlier allocation's to the host.
+template <class T>
+int grow(ctts_gpu_ctx* ctx, T** buf, uint64_t* cap, uint64_t bytes, bool zero, const char* what) {
+    if (bytes <= *cap) return CTTS_GPU_OK;
+    cudaFree(*buf);
+    *buf = nullptr;
+    *cap = 0;
+    const uint64_t c = bytes + bytes / 8 + 32768;
+    if (cudaMalloc(reinterpret_cast<void**>(buf), c) != cudaSuccess)
+        return fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "%s of %llu bytes", what, (unsigned long long)c);
+    if (zero && cudaMemsetAsync(*buf, 0, c, ctx->stream) != cudaSuccess) return fail(ctx, CTTS_GPU_ERR_CUDA, "memset");
+    *cap = c;
+    return CTTS_GPU_OK;
+}
+
+// FLAC frames of the slot of utterance u
+uint64_t slot_frames(const ctts_gpu_plan* p, uint32_t u) { return (p->offsets[u + 1] - p->offsets[u] + ctts::FLAC_BLOCK - 1) / ctts::FLAC_BLOCK; }
+
+// Grow the lane's workspace for the piece p: slots, packed output and offsets, pinned results.
+int grow_lane(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l, const ctts_gpu_plan* p, bool packed) {
+    ctts_gpu_ctx* ctx = s->ctx;
+    const uint32_t n = p->n_utts;
+    const uint64_t total = p->offsets[n];
+    const ResLayout r(n, s->kind);
+    int rc = grow(ctx, &l.d_out, &l.d_out_cap, p->n_offsets[n] * sizeof(int16_t), true, "output slots");
+    if (!rc && p->rs) rc = grow(ctx, &l.d_rs, &l.d_rs_cap, total * sizeof(int16_t), true, "output-rate slots");
+    uint64_t pack_bytes = total * kOutput[s->kind].unit_bytes;
+    if (s->kind == OUT_FLAC) {   // files and frame descriptors are sized by the slots (>= the bounds): ctts_gpu_flac_bound each
+        uint64_t frames = 0;
+        pack_bytes = 0;
+        for (uint32_t u = 0; u < n; u++) {
+            frames += slot_frames(p, u);
+            pack_bytes += (ctts_gpu_flac_bound(p->offsets[u + 1] - p->offsets[u]) + 15) & ~15ull;
+        }
+        if (!rc) rc = grow(ctx, &l.d_frames, &l.d_frames_cap, frames * sizeof(ctts::FlacFrame), false, "FLAC frames");
+        if (!rc) rc = grow(ctx, &l.d_flac_info, &l.d_flac_info_cap, 3 * (uint64_t)n * 4, false, "FLAC sizes");
+    }
+    if (!rc && packed) rc = grow(ctx, &l.d_pack, &l.d_pack_cap, pack_bytes, true, "packed output");
+    if (!rc && packed) rc = grow(ctx, &l.d_pack_off, &l.d_pack_off_cap, r.off_words * 8, false, "pack offsets");
+    if (rc) return rc;
+    if (r.res_words > l.h_res_cap) {
+        if (l.h_res) cudaFreeHost(l.h_res);
+        l.h_res = nullptr;
+        l.h_res_cap = 0;
+        const size_t cap = r.res_words + 4096;
+        if (cudaHostAlloc(reinterpret_cast<void**>(&l.h_res), cap * 4, cudaHostAllocDefault) != cudaSuccess)
+            return fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "pinned counts");
+        l.h_res_cap = cap;
+    }
+    return CTTS_GPU_OK;
+}
+
+// Packed mode: encode the piece's output-rate slots d_final into d_pack, its utterances back to back.  The scan kernel
+// stores the counts and flags (FLAC: and file sizes) straight into h_res; counts_ready is recorded behind it, and the
+// copy to the caller is enqueued once they are on the host.
+cudaError_t encode_packed(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l, const ctts_gpu_plan* p, const int16_t* d_final) {
+    const cudaStream_t st = s->ctx->stream;
+    const uint32_t n = p->n_utts;
+    const ResLayout r(n, s->kind);
+    const uint32_t* const cnt = p->d_final_counts;
+    unsigned long long* const h_slot = reinterpret_cast<unsigned long long*>(l.h_res + r.slots);
+    unsigned long long* const d_slot = l.d_pack_off + (n + 1);
+    uint64_t max_slot = 0;
+    for (uint32_t u = 0; u < n; u++) max_slot = std::max<uint64_t>(max_slot, p->offsets[u + 1] - p->offsets[u]);
+    for (uint32_t u = 0; u <= n; u++) h_slot[u] = p->offsets[u];
+    cudaError_t e = cudaSuccess;
+    auto sliced = [&](uint64_t tiles, auto launch) {   // grid.y limit
+        for (uint32_t u0 = 0; u0 < n && e == cudaSuccess; u0 += 65535u) {
+            launch(dim3((unsigned)tiles, std::min<uint32_t>(n - u0, 65535u)), u0);
+            e = cudaGetLastError();
+        }
+    };
+    // PCM and G.711: device prefix sum of the counts -> packed positions -> `kernel` copies or encodes every
+    // utterance there, padding included
+    auto pack = [&](auto kernel, auto* dst) {
+        e = cudaMemcpyAsync(d_slot, h_slot, r.slot_words * 8, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) {
+            ctts::pack_scan_kernel<<<1, 1024, 0, st>>>(cnt, p->d_err, n, l.d_pack_off, l.h_res);
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) e = cudaEventRecord(l.counts_ready, st);   // counts and flags are on the host
+        sliced((max_slot + ctts::PACK_TILE - 1) / ctts::PACK_TILE, [&](dim3 grid, uint32_t u0) {
+            kernel<<<grid, ctts::PACK_THREADS, 0, st>>>(d_final, d_slot + u0, cnt + u0, l.d_pack_off + u0, dst);
+        });
+        return e;
+    };
+    switch (s->kind) {
+    case OUT_PCM: return pack(ctts::pack_copy_kernel, reinterpret_cast<int16_t*>(l.d_pack));
+    case OUT_ULAW: return pack(ctts::g711_pack_kernel<ctts::G711_ULAW>, l.d_pack);
+    case OUT_ALAW: return pack(ctts::g711_pack_kernel<ctts::G711_ALAW>, l.d_pack);
+    case OUT_FLAC: break;
+    }
+    // FLAC: the first frame descriptor of every utterance goes behind the slot offsets; analyse every frame -> sizes
+    // and packed byte offsets (counts, flags and sizes into h_res) -> emit each frame at its offset
+    h_slot[n + 1] = 0;
+    for (uint32_t u = 0; u < n; u++) h_slot[n + 2 + u] = h_slot[n + 1 + u] + slot_frames(p, u);
+    e = cudaMemcpyAsync(d_slot, h_slot, r.slot_words * 8, cudaMemcpyHostToDevice, st);
+    const ctts::FlacArgs fa{d_final, d_slot, cnt, d_slot + (n + 1), l.d_frames, l.d_pack_off, l.d_flac_info, l.d_pack,
+                            p->rs ? p->rs->hz : (uint32_t)CTTS_PLAN_SAMPLE_RATE};
+    const uint64_t frames = std::max<uint64_t>((max_slot + ctts::FLAC_BLOCK - 1) / ctts::FLAC_BLOCK, 1);
+    sliced(frames, [&](dim3 grid, uint32_t u0) { ctts::flac_analyze_kernel<<<grid, ctts::FLAC_THREADS, 0, st>>>(fa, u0); });
+    if (e == cudaSuccess) {
+        ctts::flac_scan_kernel<<<1, 1024, 0, st>>>(fa, p->d_err, n, l.h_res);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaEventRecord(l.counts_ready, st);   // counts, flags and sizes are on the host
+    sliced(frames, [&](dim3 grid, uint32_t u0) { ctts::flac_emit_kernel<<<grid, ctts::FLAC_THREADS, 0, st>>>(fa, u0); });
+    return e;
+}
+
+// Slot mode: copy the piece from the device slots (packed by their bounds, up8(bound) + 8 each) to the caller's
+// (runs of utterances whose host slots are laid out the same way go in one copy), then its counts and flags to h_res.
+cudaError_t copy_slots(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l, const ctts_gpu_plan* p, const int16_t* d_final,
+                       const uint64_t* slot_off, const uint64_t* slot_cap) {
+    const cudaStream_t cs = s->ctx->copy_stream;
+    const uint32_t n = p->n_utts;
+    const std::vector<uint64_t>& o = p->offsets;
+    cudaError_t e = cudaSuccess;
+    for (uint32_t u = 0; u < n && e == cudaSuccess;) {
+        uint32_t v = u;
+        while (v + 1 < n && slot_off[v + 1] == slot_off[v] + (o[v + 1] - o[v]) && slot_cap[v] >= o[v + 1] - o[v]) v++;
+        const uint64_t len = (o[v] - o[u]) + std::min<uint64_t>(o[v + 1] - o[v], slot_cap[v]);
+        if (len) e = cudaMemcpyAsync(s->out + slot_off[u] * sizeof(int16_t), d_final + o[u], len * sizeof(int16_t), cudaMemcpyDeviceToHost, cs);
+        s->d2h_bytes += len * sizeof(int16_t);
+        u = v + 1;
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(l.h_res, p->d_final_counts, (size_t)n * 4, cudaMemcpyDeviceToHost, cs);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(l.h_res + ResLayout(n, s->kind).flags, p->d_err, (size_t)n * 4, cudaMemcpyDeviceToHost, cs);
+    if (e == cudaSuccess) e = cudaEventRecord(l.copied, cs);
+    return e;
+}
+
+// One piece: compile, launch, copy.  Utterance i of the piece is delivered to the caller's buffer at slot_off[i],
+// slot_cap[i] samples of room (>= its bound); slot_off == nullptr (FLAC and G.711 always): the library appends packed
+// slots at the session's cursor and reports them through offsets_out (FLAC: and the file sizes through out_bytes).
+// Asynchronous: returns once everything is enqueued.
 int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64_t* slot_off, const uint64_t* slot_cap,
                  uint64_t* offsets_out, uint32_t* out_counts, uint32_t* out_bytes = nullptr) {
     ctts_gpu_ctx* ctx = s->ctx;
@@ -2158,165 +2346,30 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
         if ((slot_off[u] & 7) || slot_cap[u] < p->bounds[u] || slot_off[u] + slot_cap[u] > s->capacity)
             return bail(fail(ctx, CTTS_GPU_ERR_BOUNDS, "output slot of utterance %u is misaligned, outside the buffer or smaller than its bound %llu",
                              s->utts + u, (unsigned long long)p->bounds[u]));
-    const uint64_t total = p->offsets[n];
-    auto grow = [&](int16_t** buf, uint64_t* cap_now, uint64_t total) -> int {
-        if (total <= *cap_now) return 0;
-        cudaFree(*buf);
-        *buf = nullptr;
-        *cap_now = 0;
-        const uint64_t cap = std::max<uint64_t>(total + total / 8, 8);
-        if (cudaMalloc(reinterpret_cast<void**>(buf), cap * sizeof(int16_t)) != cudaSuccess)
-            return fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "output buffer of %llu samples", (unsigned long long)cap);
-        // never-written slot tails must not carry an earlier allocation's bytes to the host
-        if (cudaMemsetAsync(*buf, 0, cap * sizeof(int16_t), ctx->stream) != cudaSuccess) return fail(ctx, CTTS_GPU_ERR_CUDA, "memset");
-        *cap_now = cap;
-        return 0;
-    };
-    if ((rc = grow(&l.d_out, &l.d_out_cap, p->n_offsets[n])) != 0) return bail(rc);
-    if (p->rs && (rc = grow(&l.d_rs, &l.d_rs_cap, total)) != 0) return bail(rc);
-    const bool flac = s->kind == OUT_FLAC;
-    if (packed && !flac && (rc = grow(&l.d_pack, &l.d_pack_cap, total)) != 0) return bail(rc);
-    // FLAC: the files and the frame descriptors are sized by the slots (>= the bounds): ctts_gpu_flac_bound each
-    uint64_t flac_bytes = 0, n_frames = 0, max_frames = 1;
-    for (uint32_t u = 0; u < n && flac; u++) {
-        const uint64_t frames = (p->offsets[u + 1] - p->offsets[u] + ctts::FLAC_BLOCK - 1) / ctts::FLAC_BLOCK;
-        flac_bytes += (ctts_gpu_flac_bound(p->offsets[u + 1] - p->offsets[u]) + 15) & ~15ull;
-        n_frames += frames;
-        max_frames = std::max(max_frames, frames);
-    }
-    auto grow_raw = [&](void** buf, uint64_t* cap_now, uint64_t bytes, const char* what) -> int {
-        if (bytes <= *cap_now) return 0;
-        cudaFree(*buf);
-        *buf = nullptr;
-        *cap_now = 0;
-        const uint64_t cap = std::max<uint64_t>(bytes + bytes / 8, 64);
-        if (cudaMalloc(buf, cap) != cudaSuccess) return fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "%s of %llu bytes", what, (unsigned long long)cap);
-        *cap_now = cap;
-        return 0;
-    };
-    if (flac) {
-        if ((rc = grow_raw(reinterpret_cast<void**>(&l.d_flac), &l.d_flac_cap, flac_bytes, "FLAC output")) != 0) return bail(rc);
-        if ((rc = grow_raw(reinterpret_cast<void**>(&l.d_frames), &l.d_frames_cap, n_frames * sizeof(ctts::FlacFrame), "FLAC frames")) != 0) return bail(rc);
-        if ((rc = grow_raw(reinterpret_cast<void**>(&l.d_flac_info), &l.d_flac_info_cap, 3 * (uint64_t)n * 4, "FLAC sizes")) != 0) return bail(rc);
-    }
+    if ((rc = grow_lane(s, l, p, packed)) != 0) return bail(rc);
     int16_t* const d_final = p->rs ? l.d_rs : l.d_out;   // the slots callers see
-    // h_res: counts, flags (, FLAC: file bytes), then 8-byte aligned: slot offsets (, FLAC: frame bases)
-    const size_t res_head = ((flac ? 3 : 2) * (size_t)n + 1) & ~(size_t)1;
-    const size_t res_words = res_head + 2 + (flac ? 4 : 2) * ((size_t)n + 1);
-    if (res_words > l.h_res_cap) {
-        if (l.h_res) cudaFreeHost(l.h_res);
-        l.h_res = nullptr;
-        l.h_res_cap = 0;
-        const size_t cap = res_words + 4096;
-        if (cudaHostAlloc(reinterpret_cast<void**>(&l.h_res), cap * 4, cudaHostAllocDefault) != cudaSuccess)
-            return bail(fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "pinned counts"));
-        l.h_res_cap = cap;
-    }
-    const size_t off_words = (flac ? 3 : 2) * ((size_t)n + 1);   // packed offsets, slot offsets (, FLAC: frame bases)
-    if (packed && off_words > l.d_pack_off_cap) {
-        cudaFree(l.d_pack_off);
-        l.d_pack_off = nullptr;
-        l.d_pack_off_cap = 0;
-        const size_t cap = off_words + 4096;
-        if (cudaMalloc(reinterpret_cast<void**>(&l.d_pack_off), cap * 8) != cudaSuccess)
-            return bail(fail(ctx, CTTS_GPU_ERR_OUT_OF_MEMORY, "pack offsets"));
-        l.d_pack_off_cap = cap;
-    }
-    if (!l.kernels_done) {
-        cudaError_t e = cudaEventCreateWithFlags(&l.kernels_done, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&l.copied, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&l.counts_ready, cudaEventDisableTiming);
-        if (e != cudaSuccess) return bail(fail(ctx, CTTS_GPU_ERR_CUDA, "event: %s", cudaGetErrorString(e)));
-    }
     p->d_out_last = d_final;
-    l.copy_pending = false;
+    cudaError_t e = cudaSuccess;
     if (n) {
         rc = begin_run(ctx, p);
         if (!rc) rc = build_tasks(ctx, p, piece, ctx->stream);
         const auto tp2 = std::chrono::steady_clock::now();
-        if (!rc) rc = launch_assemble(ctx, p, l.d_out, ctx->stream);
-        if (!rc) rc = launch_stretch(ctx, p, l.d_out, ctx->stream);
-        if (!rc) rc = launch_resample(ctx, p, l.d_out, d_final, ctx->stream);
-        if (!rc) rc = launch_loudness(ctx, p, d_final, ctx->stream);
+        if (!rc) rc = launch_chain(ctx, p, l.d_out, d_final, ctx->stream);
         if (rc) return bail(rc);
         if (ctx->knobs.trace) {
             auto msf = [](auto a, auto b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
             fprintf(stderr, "  submit %u utterances at %.1f ms: waited %.2f, prepare %.2f, build %.2f, launch %.2f ms\n", n, msf(s->t0, tp0),
                     msf(tsub0, tp0), msf(tp0, tp1), msf(tp1, tp2), msf(tp2, std::chrono::steady_clock::now()));
         }
-        cudaError_t e = cudaSuccess;
-        if (packed) {
-            // device prefix sum of the counts -> packed positions -> gather; the scan kernel also stores counts
-            // and flags into page-locked host memory, and the PCM copy is enqueued once they are here
-            unsigned long long* h_slot = reinterpret_cast<unsigned long long*>(l.h_res + res_head);
-            for (uint32_t u = 0; u <= n; u++) h_slot[u] = p->offsets[u];
-            for (uint32_t u = 0, fb = 0; u <= n && flac; u++) {   // first frame descriptor of every utterance
-                h_slot[n + 1 + u] = fb;
-                if (u < n) fb += (uint32_t)((p->offsets[u + 1] - p->offsets[u] + ctts::FLAC_BLOCK - 1) / ctts::FLAC_BLOCK);
-            }
-            unsigned long long* d_slot = l.d_pack_off + (n + 1);
-            e = cudaMemcpyAsync(d_slot, h_slot, (flac ? 2 : 1) * ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, ctx->stream);
-            if (e == cudaSuccess && flac) {
-                // analyse every frame -> sizes and packed byte offsets (counts, flags and sizes into h_res) -> emit
-                const ctts::FlacArgs fa{d_final, d_slot, p->d_final_counts, d_slot + (n + 1), l.d_frames, l.d_pack_off,
-                                        l.d_flac_info, l.d_flac, p->rs ? p->rs->hz : (uint32_t)CTTS_PLAN_SAMPLE_RATE};
-                for (uint32_t u0 = 0; u0 < n && e == cudaSuccess; u0 += 65535u) {   // grid.y limit
-                    ctts::flac_analyze_kernel<<<dim3((unsigned)max_frames, std::min<uint32_t>(n - u0, 65535u)), ctts::FLAC_THREADS, 0, ctx->stream>>>(fa, u0);
-                    e = cudaGetLastError();
-                }
-                if (e == cudaSuccess) {
-                    ctts::flac_scan_kernel<<<1, 1024, 0, ctx->stream>>>(fa, p->d_err, n, l.h_res);
-                    e = cudaGetLastError();
-                }
-                if (e == cudaSuccess) e = cudaEventRecord(l.counts_ready, ctx->stream);   // counts, flags and sizes are on the host
-                for (uint32_t u0 = 0; u0 < n && e == cudaSuccess; u0 += 65535u) {
-                    ctts::flac_emit_kernel<<<dim3((unsigned)max_frames, std::min<uint32_t>(n - u0, 65535u)), ctts::FLAC_THREADS, 0, ctx->stream>>>(fa, u0);
-                    e = cudaGetLastError();
-                }
-            } else if (e == cudaSuccess) {
-                ctts::pack_scan_kernel<<<1, 1024, 0, ctx->stream>>>(p->d_final_counts, p->d_err, n, l.d_pack_off, l.h_res);
-                e = cudaGetLastError();
-                if (e == cudaSuccess) e = cudaEventRecord(l.counts_ready, ctx->stream);   // counts and flags are on the host
-                uint64_t max_slot = 0;
-                for (uint32_t u = 0; u < n; u++) max_slot = std::max<uint64_t>(max_slot, p->offsets[u + 1] - p->offsets[u]);
-                for (uint32_t u0 = 0; u0 < n && e == cudaSuccess; u0 += 65535u) {   // grid.y limit
-                    const dim3 grid((unsigned)((max_slot + ctts::PACK_TILE - 1) / ctts::PACK_TILE), std::min<uint32_t>(n - u0, 65535u));
-                    uint8_t* const d_bytes = reinterpret_cast<uint8_t*>(l.d_pack);   // G.711: one byte per sample
-                    if (s->kind == OUT_ULAW)
-                        ctts::g711_pack_kernel<ctts::G711_ULAW><<<grid, ctts::PACK_THREADS, 0, ctx->stream>>>(d_final, d_slot + u0, p->d_final_counts + u0, l.d_pack_off + u0, d_bytes);
-                    else if (s->kind == OUT_ALAW)
-                        ctts::g711_pack_kernel<ctts::G711_ALAW><<<grid, ctts::PACK_THREADS, 0, ctx->stream>>>(d_final, d_slot + u0, p->d_final_counts + u0, l.d_pack_off + u0, d_bytes);
-                    else
-                        ctts::pack_copy_kernel<<<grid, ctts::PACK_THREADS, 0, ctx->stream>>>(d_final, d_slot + u0, p->d_final_counts + u0, l.d_pack_off + u0, l.d_pack);
-                    e = cudaGetLastError();
-                }
-            }
-        }
+        if (packed) e = encode_packed(s, l, p, d_final);
         if (e == cudaSuccess) e = cudaEventRecord(l.kernels_done, ctx->stream);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, l.kernels_done, 0);
-        // slots mode: device slots are packed by their bounds (up8(bound) + 8 each); runs of utterances whose
-        // host slots are laid out the same way go in one copy
-        for (uint32_t u = 0; u < n && e == cudaSuccess && !packed;) {
-            uint32_t v = u;
-            while (v + 1 < n && slot_off[v + 1] == slot_off[v] + (p->offsets[v + 1] - p->offsets[v]) &&
-                   slot_cap[v] >= p->offsets[v + 1] - p->offsets[v])
-                v++;
-            const uint64_t len = (p->offsets[v] - p->offsets[u]) + std::min<uint64_t>(p->offsets[v + 1] - p->offsets[v], slot_cap[v]);
-            if (len) e = cudaMemcpyAsync(s->pcm_out + slot_off[u], d_final + p->offsets[u], len * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
-            s->d2h_samples += len;
-            u = v + 1;
-        }
-        if (e == cudaSuccess && !packed) {
-            e = cudaMemcpyAsync(l.h_res, p->d_final_counts, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->copy_stream);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(l.h_res + n, p->d_err, (size_t)n * 4, cudaMemcpyDeviceToHost, ctx->copy_stream);
-            if (e == cudaSuccess) e = cudaEventRecord(l.copied, ctx->copy_stream);
-        }
-        if (e != cudaSuccess) return bail(fail(ctx, CTTS_GPU_ERR_CUDA, "enqueue: %s", cudaGetErrorString(e)));
-        l.copy_pending = packed;
+        if (e == cudaSuccess && !packed) e = copy_slots(s, l, p, d_final, slot_off, slot_cap);
     } else {
-        cudaError_t e = cudaEventRecord(l.copied, ctx->copy_stream);
-        if (e != cudaSuccess) return bail(fail(ctx, CTTS_GPU_ERR_CUDA, "enqueue: %s", cudaGetErrorString(e)));
+        e = cudaEventRecord(l.copied, ctx->copy_stream);
     }
+    if (e != cudaSuccess) return bail(fail(ctx, CTTS_GPU_ERR_CUDA, "enqueue: %s", cudaGetErrorString(e)));
+    l.copy_pending = packed && n;   // packed mode: the copy is enqueued once the counts are on the host
     l.plan = p;
     l.user_counts = out_counts;
     l.user_offsets = offsets_out;
@@ -2326,7 +2379,7 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
     l.busy = true;
     s->submitted++;
     s->utts += n;
-    // packed mode: enqueue the PCM copies of the pieces whose counts have arrived (in order; never blocks)
+    // packed mode: enqueue the copies of the pieces whose counts have arrived (in order; never blocks)
     pump_copies(s, 0);
     // hand over whatever has arrived in the meantime (never blocks)
     while (s->harvested < s->submitted) {
@@ -2337,40 +2390,9 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
     return s->error;
 }
 
-int enqueue_packed_copy(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l) {
-    ctts_gpu_ctx* ctx = s->ctx;
-    l.copy_pending = false;
-    cudaError_t e = cudaEventSynchronize(l.counts_ready);
-    if (e != cudaSuccess) {
-        if (!s->error) s->error = fail(ctx, CTTS_GPU_ERR_CUDA, "piece of utterances %u..%u: %s", l.utt_base, l.utt_base + l.n, cudaGetErrorString(e));
-        return s->error;
-    }
-    const uint32_t* h_cnt = l.h_res;
-    const uint32_t* h_bytes = l.h_res + 2 * (size_t)l.n;   // FLAC: file sizes
-    const bool flac = s->kind == OUT_FLAC;
-    uint64_t o = s->cursor;
-    for (uint32_t u = 0; u < l.n; u++) {
-        if (l.user_offsets) l.user_offsets[u] = o;
-        o += flac ? (h_bytes[u] + 15ull) & ~15ull : up8(h_cnt[u]);
-    }
-    const uint64_t len = o - s->cursor;
-    if (o > s->capacity) {
-        if (!s->error)
-            s->error = fail(ctx, CTTS_GPU_ERR_BOUNDS, "output buffer too small: %llu %s needed up to utterance %u", (unsigned long long)o,
-                            s->kind != OUT_PCM ? "bytes" : "samples", l.utt_base + l.n);
-        return s->error;
-    }
-    if (len && flac) e = cudaMemcpyAsync(s->byte_out + s->cursor, l.d_flac, len, cudaMemcpyDeviceToHost, ctx->copy_stream);
-    else if (len && s->kind != OUT_PCM) e = cudaMemcpyAsync(s->byte_out + s->cursor, l.d_pack, len, cudaMemcpyDeviceToHost, ctx->copy_stream);
-    else if (len) e = cudaMemcpyAsync(s->pcm_out + s->cursor, l.d_pack, len * sizeof(int16_t), cudaMemcpyDeviceToHost, ctx->copy_stream);
-    if (e == cudaSuccess) e = cudaEventRecord(l.copied, ctx->copy_stream);
-    if (e != cudaSuccess) {
-        if (!s->error) s->error = fail(ctx, CTTS_GPU_ERR_CUDA, "D2H: %s", cudaGetErrorString(e));
-        return s->error;
-    }
-    s->d2h_samples += len;
-    s->cursor = o;
-    return CTTS_GPU_OK;
+// Utterances u0 .. u1 - 1 of the plan as a plan of their own (the ops stay where they are)
+ctts_batch_plan sub_plan(const ctts_batch_plan* plan, uint32_t u0, uint32_t u1) {
+    return {u1 - u0, plan->n_ops, plan->utt_op_begin + u0, plan->speed + u0, plan->ops};
 }
 
 // Caller-defined slots: utterance u goes to pcm_out[off[u] ..), cap[u] samples of room.  The batch is cut into
@@ -2384,10 +2406,7 @@ int submit_slot_pieces(ctts_gpu_session* s, const ctts_batch_plan* plan, const u
     for (uint32_t u0 = 0, u = 0; u < n && !rc; u++) {
         acc += cap[u];
         if (acc >= s->ctx->knobs.piece_samples || u + 1 == n) {
-            ctts_batch_plan piece = *plan;
-            piece.n_utts = u + 1 - u0;
-            piece.utt_op_begin = plan->utt_op_begin + u0;
-            piece.speed = plan->speed + u0;
+            const ctts_batch_plan piece = sub_plan(plan, u0, u + 1);
             rc = submit_piece(s, &piece, off + u0, cap + u0, nullptr, out_counts + u0);
             u0 = u + 1;
             acc = 0;
@@ -2396,38 +2415,43 @@ int submit_slot_pieces(ctts_gpu_session* s, const ctts_batch_plan* plan, const u
     return rc;
 }
 
+int session_open(ctts_gpu_ctx* ctx, const ctts_assembly_params* params, SessionOutput kind, void* out, uint64_t capacity,
+                 ctts_gpu_chunk_fn on_piece, void* user, ctts_gpu_session** s_out) {
+    if (!ctx || !params || !s_out || (capacity && !out)) return CTTS_GPU_ERR_INVALID_ARG;
+    *s_out = nullptr;
+    if (ctx->session) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "a session is already open on this context");
+    CU(ctx, cudaSetDevice(ctx->device));
+    if (!ctx->copy_stream) CU(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+    for (ctts_gpu_ctx::Lane& l : ctx->lane)
+        for (cudaEvent_t* ev : {&l.kernels_done, &l.counts_ready, &l.copied})
+            if (!*ev) CU(ctx, cudaEventCreateWithFlags(ev, cudaEventDisableTiming));
+    ctx->session = new ctts_gpu_session{ctx, *params, kind, static_cast<uint8_t*>(out), capacity, on_piece, user, std::chrono::steady_clock::now()};
+    *s_out = ctx->session;
+    return CTTS_GPU_OK;
+}
+
+// kind: the submit call's (either law for G.711)
+int session_submit(ctts_gpu_session* s, SessionOutput kind, const ctts_batch_plan* piece, uint64_t* out_offsets,
+                   uint32_t* out_bytes, uint32_t* out_counts) {
+    const OutputKind& k = kOutput[s->kind];
+    if (strcmp(k.submit, kOutput[kind].submit) != 0) return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, "a %s session takes %s", k.name, k.submit);
+    if (s->error) return s->error;
+    CU(s->ctx, cudaSetDevice(s->ctx->device));
+    return submit_piece(s, piece, nullptr, nullptr, out_offsets, out_counts, out_bytes);
+}
+
 }  // namespace
 
 extern "C" {
 
 int ctts_gpu_session_begin(ctts_gpu_ctx* ctx, const ctts_assembly_params* params, int16_t* pcm_out, uint64_t capacity,
                            ctts_gpu_chunk_fn on_piece, void* user, ctts_gpu_session** out) {
-    if (!ctx || !params || !out || (capacity && !pcm_out)) return CTTS_GPU_ERR_INVALID_ARG;
-    *out = nullptr;
-    if (ctx->session) return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "a session is already open on this context");
-    CU(ctx, cudaSetDevice(ctx->device));
-    if (!ctx->copy_stream) CU(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-    ctts_gpu_session* s = new ctts_gpu_session();
-    s->ctx = ctx;
-    s->prm = *params;
-    s->pcm_out = pcm_out;
-    s->capacity = capacity;
-    s->on_piece = on_piece;
-    s->user = user;
-    s->t0 = std::chrono::steady_clock::now();
-    ctx->session = s;
-    *out = s;
-    return CTTS_GPU_OK;
+    return session_open(ctx, params, OUT_PCM, pcm_out, capacity, on_piece, user, out);
 }
 
 int ctts_gpu_session_submit(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets, uint32_t* out_counts) {
     if (!s || !piece || !out_counts || (piece->n_utts && !out_offsets)) return CTTS_GPU_ERR_INVALID_ARG;
-    if (s->kind == OUT_FLAC) return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, "a FLAC session takes ctts_gpu_session_submit_flac");
-    if (s->kind != OUT_PCM) return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, "a G.711 session takes ctts_gpu_session_submit_g711");
-    if (s->error) return s->error;
-    ctts_gpu_ctx* ctx = s->ctx;
-    CU(ctx, cudaSetDevice(ctx->device));
-    return submit_piece(s, piece, nullptr, nullptr, out_offsets, out_counts);
+    return session_submit(s, OUT_PCM, piece, out_offsets, nullptr, out_counts);
 }
 
 uint64_t ctts_gpu_flac_bound(uint64_t samples) {
@@ -2436,25 +2460,13 @@ uint64_t ctts_gpu_flac_bound(uint64_t samples) {
 
 int ctts_gpu_session_begin_flac(ctts_gpu_ctx* ctx, const ctts_assembly_params* params, uint8_t* out, uint64_t capacity_bytes,
                                 ctts_gpu_chunk_fn on_piece, void* user, ctts_gpu_session** s) {
-    if (capacity_bytes && !out) return CTTS_GPU_ERR_INVALID_ARG;
-    const int rc = ctts_gpu_session_begin(ctx, params, nullptr, 0, on_piece, user, s);
-    if (rc) return rc;
-    (*s)->kind = OUT_FLAC;
-    (*s)->byte_out = out;
-    (*s)->capacity = capacity_bytes;
-    return CTTS_GPU_OK;
+    return session_open(ctx, params, OUT_FLAC, out, capacity_bytes, on_piece, user, s);
 }
 
 int ctts_gpu_session_submit_flac(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets, uint32_t* out_bytes,
                                  uint32_t* out_counts) {
     if (!s || !piece || (piece->n_utts && (!out_offsets || !out_bytes || !out_counts))) return CTTS_GPU_ERR_INVALID_ARG;
-    if (s->kind != OUT_FLAC)
-        return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, s->kind == OUT_PCM ? "a PCM session takes ctts_gpu_session_submit"
-                                                                          : "a G.711 session takes ctts_gpu_session_submit_g711");
-    if (s->error) return s->error;
-    ctts_gpu_ctx* ctx = s->ctx;
-    CU(ctx, cudaSetDevice(ctx->device));
-    return submit_piece(s, piece, nullptr, nullptr, out_offsets, out_counts, out_bytes);
+    return session_submit(s, OUT_FLAC, piece, out_offsets, out_bytes, out_counts);
 }
 
 int ctts_gpu_session_begin_g711(ctts_gpu_ctx* ctx, const ctts_assembly_params* params, int law, uint8_t* out,
@@ -2464,23 +2476,12 @@ int ctts_gpu_session_begin_g711(ctts_gpu_ctx* ctx, const ctts_assembly_params* p
         *s = nullptr;
         return fail(ctx, CTTS_GPU_ERR_INVALID_ARG, "G.711 law %d: CTTS_GPU_G711_ULAW or CTTS_GPU_G711_ALAW", law);
     }
-    const int rc = ctts_gpu_session_begin(ctx, params, nullptr, 0, on_piece, user, s);
-    if (rc) return rc;
-    (*s)->kind = law == CTTS_GPU_G711_ULAW ? OUT_ULAW : OUT_ALAW;
-    (*s)->byte_out = out;
-    (*s)->capacity = capacity_bytes;
-    return CTTS_GPU_OK;
+    return session_open(ctx, params, static_cast<SessionOutput>(law), out, capacity_bytes, on_piece, user, s);
 }
 
 int ctts_gpu_session_submit_g711(ctts_gpu_session* s, const ctts_batch_plan* piece, uint64_t* out_offsets, uint32_t* out_counts) {
     if (!s || !piece || !out_counts || (piece->n_utts && !out_offsets)) return CTTS_GPU_ERR_INVALID_ARG;
-    if (s->kind != OUT_ULAW && s->kind != OUT_ALAW)
-        return fail(s->ctx, CTTS_GPU_ERR_INVALID_ARG, s->kind == OUT_PCM ? "a PCM session takes ctts_gpu_session_submit"
-                                                                          : "a FLAC session takes ctts_gpu_session_submit_flac");
-    if (s->error) return s->error;
-    ctts_gpu_ctx* ctx = s->ctx;
-    CU(ctx, cudaSetDevice(ctx->device));
-    return submit_piece(s, piece, nullptr, nullptr, out_offsets, out_counts);
+    return session_submit(s, OUT_ULAW, piece, out_offsets, nullptr, out_counts);
 }
 
 int ctts_gpu_session_end(ctts_gpu_session* s, uint64_t* samples_used) {
@@ -2491,7 +2492,7 @@ int ctts_gpu_session_end(ctts_gpu_session* s, uint64_t* samples_used) {
     if (samples_used) *samples_used = s->cursor;
     if (ctx->knobs.trace)
         fprintf(stderr, "ctts_gpu session: %u utterances in %u pieces, %.1f MB to the host, %.1f ms\n", s->utts, s->submitted,
-                (s->kind != OUT_PCM ? 1e-6 : 2e-6) * (double)s->d2h_samples, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - s->t0).count());
+                1e-6 * (double)s->d2h_bytes, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - s->t0).count());
     const int rc = s->error;
     ctx->session = nullptr;
     delete s;
@@ -2543,10 +2544,7 @@ int ctts_gpu_synth_batch_packed(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, 
     const uint64_t ops_per_piece = std::max<uint64_t>(ctx->knobs.piece_samples / 2800, 64);
     for (uint32_t u0 = 0, u = 0; u < n && !rc; u++) {
         if (plan->utt_op_begin[u + 1] - plan->utt_op_begin[u0] >= ops_per_piece || u + 1 == n) {
-            ctts_batch_plan piece = *plan;
-            piece.n_utts = u + 1 - u0;
-            piece.utt_op_begin = plan->utt_op_begin + u0;
-            piece.speed = plan->speed + u0;
+            const ctts_batch_plan piece = sub_plan(plan, u0, u + 1);
             rc = submit_piece(s, &piece, nullptr, nullptr, out_offsets + u0, out_counts + u0);
             u0 = u + 1;
         }

@@ -292,35 +292,13 @@ class GpuSynth:
                                                   out_offsets.ctypes.data, counts.ctypes.data, cb, None))
         return pcm_out, out_offsets, counts[:plan.n_utts]
 
-    def synth_pieces(self, pieces: list[BatchPlan], params: AssemblyParams, pcm_out: np.ndarray):
-        """A session fed with the given plans, one piece each (ctts_gpu_session_*).
-        Returns (offsets, counts) over all utterances of all pieces, in order."""
+    def _session(self, begin, submit, pieces: list[BatchPlan]):
+        """A session opened by begin(handle) and fed with the given plans, one piece each, through
+        submit(handle, plan, offsets, file bytes, counts).  Returns (offsets, file bytes, counts, units used) over all
+        utterances of all pieces, in order."""
         L = lib()
         h = C.c_void_p()
-        self._check(L.ctts_gpu_session_begin(self._h, C.byref(params), pcm_out.ctypes.data, pcm_out.size, None, None, C.byref(h)))
-        n = sum(p.n_utts for p in pieces)
-        off = np.zeros(max(n, 1), dtype=np.uint64)
-        cnt = np.zeros(max(n, 1), dtype=np.uint32)
-        at, rc = 0, 0
-        for p in pieces:
-            cp = p.as_c()
-            rc = L.ctts_gpu_session_submit(h, C.byref(cp), off[at:].ctypes.data, cnt[at:].ctypes.data)
-            if rc:
-                break
-            at += p.n_utts
-        used = C.c_uint64()
-        rc_end = L.ctts_gpu_session_end(h, C.byref(used))
-        self._check(rc or rc_end)
-        return off[:n], cnt[:n]
-
-    def synth_pieces_flac(self, pieces: list[BatchPlan], params: AssemblyParams, out: np.ndarray):
-        """A FLAC session fed with the given plans, one piece each (ctts_gpu_session_begin_flac / _submit_flac): every
-        utterance becomes one .flac file in the uint8 buffer `out`.  Returns (byte offsets, file bytes, sample counts,
-        bytes used) over all utterances of all pieces, in order."""
-        assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
-        L = lib()
-        h = C.c_void_p()
-        self._check(L.ctts_gpu_session_begin_flac(self._h, C.byref(params), out.ctypes.data, out.size, None, None, C.byref(h)))
+        self._check(begin(C.byref(h)))
         n = sum(p.n_utts for p in pieces)
         off = np.zeros(max(n, 1), dtype=np.uint64)
         nbytes = np.zeros(max(n, 1), dtype=np.uint32)
@@ -328,7 +306,7 @@ class GpuSynth:
         at, rc = 0, 0
         for p in pieces:
             cp = p.as_c()
-            rc = L.ctts_gpu_session_submit_flac(h, C.byref(cp), off[at:].ctypes.data, nbytes[at:].ctypes.data, cnt[at:].ctypes.data)
+            rc = submit(h, C.byref(cp), off[at:].ctypes.data, nbytes[at:].ctypes.data, cnt[at:].ctypes.data)
             if rc:
                 break
             at += p.n_utts
@@ -337,28 +315,35 @@ class GpuSynth:
         self._check(rc or rc_end)
         return off[:n], nbytes[:n], cnt[:n], int(used.value)
 
+    def synth_pieces(self, pieces: list[BatchPlan], params: AssemblyParams, pcm_out: np.ndarray):
+        """A session fed with the given plans, one piece each (ctts_gpu_session_*).
+        Returns (offsets, counts) over all utterances of all pieces, in order."""
+        L = lib()
+        off, _, cnt, _ = self._session(
+            lambda h: L.ctts_gpu_session_begin(self._h, C.byref(params), pcm_out.ctypes.data, pcm_out.size, None, None, h),
+            lambda h, cp, o, b, c: L.ctts_gpu_session_submit(h, cp, o, c), pieces)
+        return off, cnt
+
+    def synth_pieces_flac(self, pieces: list[BatchPlan], params: AssemblyParams, out: np.ndarray):
+        """A FLAC session fed with the given plans, one piece each (ctts_gpu_session_begin_flac / _submit_flac): every
+        utterance becomes one .flac file in the uint8 buffer `out`.  Returns (byte offsets, file bytes, sample counts,
+        bytes used) over all utterances of all pieces, in order."""
+        assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
+        L = lib()
+        return self._session(
+            lambda h: L.ctts_gpu_session_begin_flac(self._h, C.byref(params), out.ctypes.data, out.size, None, None, h),
+            L.ctts_gpu_session_submit_flac, pieces)
+
     def synth_pieces_g711(self, pieces: list[BatchPlan], params: AssemblyParams, law: int, out: np.ndarray):
         """A G.711 session of `law` (G711_ULAW or G711_ALAW) fed with the given plans, one piece each
         (ctts_gpu_session_begin_g711 / _submit_g711): one byte per sample in the uint8 buffer `out`, in the packed
         layout.  Returns (byte offsets, sample counts, bytes used) over all utterances of all pieces, in order."""
         assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
         L = lib()
-        h = C.c_void_p()
-        self._check(L.ctts_gpu_session_begin_g711(self._h, C.byref(params), law, out.ctypes.data, out.size, None, None, C.byref(h)))
-        n = sum(p.n_utts for p in pieces)
-        off = np.zeros(max(n, 1), dtype=np.uint64)
-        cnt = np.zeros(max(n, 1), dtype=np.uint32)
-        at, rc = 0, 0
-        for p in pieces:
-            cp = p.as_c()
-            rc = L.ctts_gpu_session_submit_g711(h, C.byref(cp), off[at:].ctypes.data, cnt[at:].ctypes.data)
-            if rc:
-                break
-            at += p.n_utts
-        used = C.c_uint64()
-        rc_end = L.ctts_gpu_session_end(h, C.byref(used))
-        self._check(rc or rc_end)
-        return off[:n], cnt[:n], int(used.value)
+        off, _, cnt, used = self._session(
+            lambda h: L.ctts_gpu_session_begin_g711(self._h, C.byref(params), law, out.ctypes.data, out.size, None, None, h),
+            lambda h, cp, o, b, c: L.ctts_gpu_session_submit_g711(h, cp, o, c), pieces)
+        return off, cnt, used
 
     def flac_bound(self, plan: BatchPlan) -> int:
         """Bytes that are always enough for a FLAC session over the plan: ctts_gpu_flac_bound of every bound, rounded up to 16."""

@@ -104,24 +104,32 @@ def capacity_hint(front, batch: TextBatch, rate: int = 22050) -> int:
     return int(lib().ctts_b200_capacity_hint_rate(front._h, batch.ptrs, batch.speeds_ptr, batch.n, rate))
 
 
+def _synth(entry: str, front, gpu, batch: TextBatch, out: np.ndarray, arrays, piece_utts: int, threads: int,
+           cache: PlanCache | None, law=()):
+    """Calls entry(front, gpu, [law,] texts, speeds, n, out, capacity, *arrays, &used, options, timing) of
+    libctts_b200.so, an array None for NULL.  Returns (units used, Timing); raises GpuError when it fails."""
+    assert out.flags["C_CONTIGUOUS"]
+    used = C.c_uint64()
+    opt = Options(piece_utts, threads, None, None, cache._h if cache is not None else None)
+    tm = Timing()
+    rc = getattr(lib(), entry)(front._h, gpu._h, *law, batch.ptrs, batch.speeds_ptr, batch.n, out.ctypes.data, out.size,
+                               *(None if a is None else a.ctypes.data for a in arrays), C.byref(used), C.byref(opt), C.byref(tm))
+    if rc != 0:
+        msg = _gpu.lib().ctts_gpu_last_error(gpu._h)
+        raise _gpu.GpuError(f"{entry}: {rc}: {msg.decode(errors='replace') if msg else ''}")
+    return int(used.value), tm
+
+
 def synth_texts(front, gpu, batch: TextBatch, pcm_out: np.ndarray, piece_utts: int = 0, threads: int = 0,
                 want_stats: bool = False, cache: PlanCache | None = None):
     """ctts_b200_synth_texts.  Returns (offsets[n], counts[n], samples_used, Timing[, stats])."""
-    assert pcm_out.dtype == np.int16 and pcm_out.flags["C_CONTIGUOUS"]
+    assert pcm_out.dtype == np.int16
     n = batch.n
     off = np.zeros(max(n, 1), dtype=np.uint64)
     cnt = np.zeros(max(n, 1), dtype=np.uint32)
     stats = np.zeros(2 * max(n, 1), dtype=np.uint32) if want_stats else None
-    used = C.c_uint64()
-    opt = Options(piece_utts, threads, None, None, cache._h if cache is not None else None)
-    tm = Timing()
-    rc = lib().ctts_b200_synth_texts(front._h, gpu._h, batch.ptrs, batch.speeds_ptr, n, pcm_out.ctypes.data,
-                                     pcm_out.size, off.ctypes.data, cnt.ctypes.data,
-                                     stats.ctypes.data if want_stats else None, C.byref(used), C.byref(opt), C.byref(tm))
-    if rc != 0:
-        msg = _gpu.lib().ctts_gpu_last_error(gpu._h)
-        raise _gpu.GpuError(f"ctts_b200_synth_texts: {rc}: {msg.decode(errors='replace') if msg else ''}")
-    res = (off[:n], cnt[:n], int(used.value), tm)
+    res = (off[:n], cnt[:n]) + _synth("ctts_b200_synth_texts", front, gpu, batch, pcm_out, (off, cnt, stats), piece_utts,
+                                      threads, cache)
     return res + (stats[:2 * n].reshape(n, 2),) if want_stats else res
 
 
@@ -134,21 +142,13 @@ def synth_texts_flac(front, gpu, batch: TextBatch, out: np.ndarray, piece_utts: 
                      cache: PlanCache | None = None):
     """ctts_b200_synth_texts_flac: one .flac file per utterance in the uint8 buffer `out`.
     Returns (byte offsets[n], file bytes[n], sample counts[n], bytes_used, Timing)."""
-    assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
+    assert out.dtype == np.uint8
     n = batch.n
     off = np.zeros(max(n, 1), dtype=np.uint64)
     nbytes = np.zeros(max(n, 1), dtype=np.uint32)
     cnt = np.zeros(max(n, 1), dtype=np.uint32)
-    used = C.c_uint64()
-    opt = Options(piece_utts, threads, None, None, cache._h if cache is not None else None)
-    tm = Timing()
-    rc = lib().ctts_b200_synth_texts_flac(front._h, gpu._h, batch.ptrs, batch.speeds_ptr, n, out.ctypes.data, out.size,
-                                          off.ctypes.data, nbytes.ctypes.data, cnt.ctypes.data, None, C.byref(used),
-                                          C.byref(opt), C.byref(tm))
-    if rc != 0:
-        msg = _gpu.lib().ctts_gpu_last_error(gpu._h)
-        raise _gpu.GpuError(f"ctts_b200_synth_texts_flac: {rc}: {msg.decode(errors='replace') if msg else ''}")
-    return off[:n], nbytes[:n], cnt[:n], int(used.value), tm
+    return (off[:n], nbytes[:n], cnt[:n]) + _synth("ctts_b200_synth_texts_flac", front, gpu, batch, out,
+                                                   (off, nbytes, cnt, None), piece_utts, threads, cache)
 
 
 def synth_texts_g711(front, gpu, batch: TextBatch, law: int, out: np.ndarray, piece_utts: int = 0, threads: int = 0,
@@ -156,16 +156,9 @@ def synth_texts_g711(front, gpu, batch: TextBatch, law: int, out: np.ndarray, pi
     """ctts_b200_synth_texts_g711: one G.711 byte of `law` (gpu.G711_ULAW or gpu.G711_ALAW) per sample in the uint8
     buffer `out`, in the packed layout; capacity_hint(front, batch, rate) bytes are always enough.
     Returns (byte offsets[n], sample counts[n], bytes_used, Timing)."""
-    assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
+    assert out.dtype == np.uint8
     n = batch.n
     off = np.zeros(max(n, 1), dtype=np.uint64)
     cnt = np.zeros(max(n, 1), dtype=np.uint32)
-    used = C.c_uint64()
-    opt = Options(piece_utts, threads, None, None, cache._h if cache is not None else None)
-    tm = Timing()
-    rc = lib().ctts_b200_synth_texts_g711(front._h, gpu._h, law, batch.ptrs, batch.speeds_ptr, n, out.ctypes.data, out.size,
-                                          off.ctypes.data, cnt.ctypes.data, None, C.byref(used), C.byref(opt), C.byref(tm))
-    if rc != 0:
-        msg = _gpu.lib().ctts_gpu_last_error(gpu._h)
-        raise _gpu.GpuError(f"ctts_b200_synth_texts_g711: {rc}: {msg.decode(errors='replace') if msg else ''}")
-    return off[:n], cnt[:n], int(used.value), tm
+    return (off[:n], cnt[:n]) + _synth("ctts_b200_synth_texts_g711", front, gpu, batch, out, (off, cnt, None), piece_utts,
+                                       threads, cache, law=(law,))
