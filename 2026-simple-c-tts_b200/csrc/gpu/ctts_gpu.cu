@@ -211,13 +211,15 @@ struct ctts_gpu_plan {
     std::vector<uint64_t> bounds;   // output-rate bounds
     ctts_gpu_ctx::RsTable* rs = nullptr;   // rate conversion the plan was created under (nullptr: native rate)
     std::vector<uint64_t> n_offsets;       // native-rate slots, where the assembly and WSOLA kernels write (== offsets without rs)
-    unsigned long long* d_rs_off = nullptr;   // rs: native slot offsets [n + 1], then output-rate ones [n + 1]
+    // the plan's offset table: (rs: native slot offsets [n + 1],) output-rate slot offsets [n + 1], (ld: the first
+    // chunk of every utterance [n + 1], ld->true_peak: its first ld_true_peak_kernel tile [n + 1]); slot_off() is
+    // the output-rate section
+    unsigned long long* d_off = nullptr;
     uint32_t* d_rs_counts = nullptr;       // rs: output-rate counts
     uint32_t* d_final_counts = nullptr;    // the counts callers see: d_rs_counts with rs, else d_counts
     uint32_t rs_tiles = 0;                 // rs: grid.x of resample_kernel
     int16_t* d_nat_owned = nullptr;        // resident plan with rs: its native slots
     const ctts_gpu_ctx::LdTable* ld = nullptr;   // loudness setting the plan was created under (nullptr: off)
-    unsigned long long* d_ld_off = nullptr;      // ld: output-rate slot offsets [n + 1], then first chunks [n + 1] (+ first tiles [n + 1] for a true peak)
     double* d_ld_state = nullptr;                // ld: 4 per chunk
     double* d_ld_energy = nullptr;               // ld: per chunk
     uint32_t* d_ld_peak = nullptr;               // ld: per chunk
@@ -312,6 +314,9 @@ uint64_t stretch_bound(uint64_t pre, uint32_t hop) {
 
 // samples at the output rate of n native samples: ceil(n * L / M)
 uint64_t rate_bound(const ctts_gpu_ctx::RsTable* rs, uint64_t n) { return rs ? (n * rs->L + rs->M - 1) / rs->M : n; }
+
+// the output-rate slot offsets in the plan's offset table
+unsigned long long* slot_off(const ctts_gpu_plan* p) { return p->d_off + (p->rs ? (size_t)p->n_utts + 1 : 0); }
 
 // Upper bound of the samples a UNIT op appends, given a lower bound L of the samples already in
 // the current region.  The crossfade consumes a = min(xf, count, n) samples of the tail
@@ -1142,8 +1147,8 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
     const size_t tasks_cap = (size_t)sc.n_regions + (size_t)sc.n_regions / 2 + 2;
     ctts::StretchTask* h_st = nullptr;
     uint32_t *h_ot = nullptr, *h_of = nullptr;
-    unsigned long long* h_ro = nullptr;
-    unsigned long long* h_lo = nullptr;
+    unsigned long long* h_off = nullptr;
+    const size_t off_words = ((rs ? 2 : 1) + (ld ? 1 : 0) + (tp ? 1 : 0)) * ((size_t)n + 1);   // of d_off
     auto layout = [&](PlanAlloc& al) {
         p->d_ops = al.dev<ctts_plan_op>(n_ops_local);
         p->d_tasks = al.dev<ctts::RegionTask>(tasks_cap);
@@ -1153,15 +1158,14 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         p->d_counts = al.dev<uint32_t>(n);
         p->d_pre_counts = al.dev<uint32_t>(n);
         p->d_err = al.dev<uint32_t>(n);
+        p->d_off = al.dev<unsigned long long>(off_words);
         p->d_final_counts = p->d_counts;
         if (rs) {
             p->d_rs_counts = al.dev<uint32_t>(n);
-            p->d_rs_off = al.dev<unsigned long long>(2 * ((size_t)n + 1));
             p->d_final_counts = p->d_rs_counts;
         }
         if (ld) {
             const uint64_t chunks = ld_chunk0[n];
-            p->d_ld_off = al.dev<unsigned long long>((tp ? 3 : 2) * ((size_t)n + 1));
             p->d_ld_state = al.dev<double>(4 * chunks);
             p->d_ld_energy = al.dev<double>(chunks);
             p->d_ld_peak = al.dev<uint32_t>(chunks);
@@ -1187,8 +1191,7 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
             h_ot = al.host<uint32_t>(ola_task.size());
             h_of = al.host<uint32_t>(ola_first.size());
         }
-        if (rs) h_ro = al.host<unsigned long long>(2 * ((size_t)n + 1));
-        if (ld) h_lo = al.host<unsigned long long>((tp ? 3 : 2) * ((size_t)n + 1));
+        h_off = al.host<unsigned long long>(off_words);
     };
     PlanAlloc al{p, true};
     layout(al);
@@ -1235,33 +1238,17 @@ int prepare_plan(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const ctts_asse
         CUP(cudaMemcpyAsync(p->d_ola_task, h_ot, ola_task.size() * 4, cudaMemcpyHostToDevice, st));
         CUP(cudaMemcpyAsync(p->d_ola_first, h_of, ola_first.size() * 4, cudaMemcpyHostToDevice, st));
     }
-    if (rs) {
-        for (uint32_t u = 0; u <= n; u++) {
-            h_ro[u] = p->n_offsets[u];
-            h_ro[n + 1 + u] = p->offsets[u];
-        }
-        CUP(cudaMemcpyAsync(p->d_rs_off, h_ro, 2 * ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, st));
-    }
-    if (ld) {
-        for (uint32_t u = 0; u <= n; u++) {
-            h_lo[u] = p->offsets[u];
-            h_lo[n + 1 + u] = ld_chunk0[u];
-            if (tp) h_lo[2 * ((size_t)n + 1) + u] = ld_tile0[u];
-        }
-        CUP(cudaMemcpyAsync(p->d_ld_off, h_lo, (tp ? 3 : 2) * ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, st));
-    }
+    unsigned long long* o = h_off;
+    if (rs) o = std::copy(p->n_offsets.begin(), p->n_offsets.end(), o);
+    o = std::copy(p->offsets.begin(), p->offsets.end(), o);
+    if (ld) o = std::copy(ld_chunk0.begin(), ld_chunk0.end(), o);
+    if (tp) std::copy(ld_tile0.begin(), ld_tile0.end(), o);
+    CUP(cudaMemcpyAsync(p->d_off, h_off, off_words * 8, cudaMemcpyHostToDevice, st));
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ctts::assemble_kernel, ctts::ASM_THREADS, p->smem_bytes) != cudaSuccess || occ < 1)
         occ = 1;
     p->occ = (uint32_t)occ;
 
-    p->info.kernel_launches = 1;   // assemble_kernel, counted also when a plan without tasks skips it
-    if (p->n_stretch)   // scan, verify, repair (chain walk), overlap-add
-        p->info.kernel_launches += 2 + (p->verify_tiles && ctx->knobs.wsola_speculate ? (p->n_stretch + 65534) / 65535 : 0) +
-                                   (p->n_ola_blocks ? 1 : 0);
-    if (rs) p->info.kernel_launches += (uint32_t)(((uint64_t)n + 65534) / 65535);   // resample_kernel
-    if (ld && n)   // the two chunk passes and ld_apply_kernel per grid.y slice, ld_scan_kernel, ld_gain_kernel
-        p->info.kernel_launches += (tp ? 4 : 3) * (uint32_t)(((uint64_t)n + 65534) / 65535) + 2;   // + ld_true_peak_kernel
     p->info.n_stretch = p->n_stretch;
     p->info.bound_samples = std::accumulate(bound.begin(), bound.end(), (uint64_t)0);
     p->info.smem_bytes = p->smem_bytes;
@@ -1738,9 +1725,41 @@ int build_tasks(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const ctts_batch_plan* plan
 }
 #undef CUP
 
-// Enqueue the plan's assembly kernel.
-int launch_assemble(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out, cudaStream_t st) {
-    if (p->n_tasks == 0) return CTTS_GPU_OK;
+// Enqueues kernels on one stream, checks each launch and counts it.  A counting Launch enqueues nothing: run over a
+// plan's launch code, it gives the plan's kernel_launches.
+struct Launch {
+    ctts_gpu_ctx* ctx;
+    cudaStream_t st;
+    bool count_only = false;
+    uint32_t count = 0;
+
+    template <class... P, class... A>
+    int operator()(void (*kernel)(P...), dim3 grid, uint32_t threads, size_t smem, A... args) {
+        count++;
+        if (count_only) return CTTS_GPU_OK;
+        kernel<<<grid, threads, smem, st>>>(args...);
+        CU(ctx, cudaGetLastError());
+        return CTTS_GPU_OK;
+    }
+};
+
+// Rows 0 .. n - 1 of a launch cut into grid.y slices: slice(first row, rows) for each, up to the first error.
+template <class F>
+int grid_y_slices(uint32_t n, F slice) {
+    constexpr uint32_t kMaxGridY = 65535;
+    for (uint32_t r0 = 0; r0 < n; r0 += kMaxGridY)
+        if (const int rc = slice(r0, std::min(n - r0, kMaxGridY))) return rc;
+    return CTTS_GPU_OK;
+}
+
+// Enqueue the plan's assembly kernel.  A plan without tasks skips the launch but counts it all the same: the assembly
+// kernel is part of every plan's kernel_launches, an empty plan's 1 included.
+int launch_assemble(Launch& launch, ctts_gpu_plan* p, int16_t* d_pcm_out) {
+    if (p->n_tasks == 0) {
+        launch.count++;
+        return CTTS_GPU_OK;
+    }
+    const ctts_gpu_ctx* ctx = launch.ctx;
     ctts::AsmArgs a{};
     a.pool = p->np->d_pool;
     a.unit_meta = p->np->d_meta;
@@ -1773,9 +1792,7 @@ int launch_assemble(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out, cud
     a.prm = p->prm;
     a.wcap = p->wcap;
     a.hcap = p->hcap;
-    ctts::assemble_kernel<<<p->grid, ctts::ASM_THREADS, p->smem_bytes, st>>>(a);
-    CU(ctx, cudaGetLastError());
-    return CTTS_GPU_OK;
+    return launch(ctts::assemble_kernel, p->grid, ctts::ASM_THREADS, p->smem_bytes, a);
 }
 
 int begin_run(ctts_gpu_ctx* ctx, ctts_gpu_plan* p) {
@@ -1790,9 +1807,10 @@ int begin_run(ctts_gpu_ctx* ctx, ctts_gpu_plan* p) {
 }
 
 // Enqueue the WSOLA kernels of the plan's stretched utterances (after its assembly kernel).
-int launch_stretch(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out, cudaStream_t st) {
+int launch_stretch(Launch& launch, ctts_gpu_plan* p, int16_t* d_pcm_out) {
     const uint32_t ns = p->n_stretch;
     if (!ns) return CTTS_GPU_OK;
+    const ctts_gpu_ctx* ctx = launch.ctx;
     ctts::WsolaArgs w{};
     w.tasks = p->d_stasks;
     w.n_tasks = ns;
@@ -1812,39 +1830,31 @@ int launch_stretch(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out, cuda
     w.ola_block_task = p->d_ola_task;
     w.ola_block_first = p->d_ola_first;
     // speculate (scan) -> verify every frame in parallel -> walk the chain only where that failed -> overlap-add
-    ctts::wsola_scan_kernel<<<(ns + 7) / 8, 256, 0, st>>>(w);
-    CU(ctx, cudaGetLastError());
-    if (w.speculate && p->verify_tiles) {
-        for (uint32_t t0 = 0; t0 < ns; t0 += 65535u) {   // grid.y limit
+    int rc = launch(ctts::wsola_scan_kernel, (ns + 7) / 8, 256, 0, w);
+    if (!rc && w.speculate && p->verify_tiles)
+        rc = grid_y_slices(ns, [&](uint32_t t0, uint32_t rows) {
             ctts::WsolaArgs wv = w;
             wv.task_first = t0;
-            const dim3 grid(p->verify_tiles, std::min<uint32_t>(ns - t0, 65535u));
-            ctts::wsola_verify_kernel<<<grid, ctts::WV_THREADS, sizeof(ctts::WvSmem), st>>>(wv);
-            CU(ctx, cudaGetLastError());
-        }
-    }
-    ctts::wsola_search_kernel<<<ns, ctts::WS_THREADS, 0, st>>>(w);
-    CU(ctx, cudaGetLastError());
-    if (p->n_ola_blocks) {
-        ctts::wsola_ola_kernel<<<p->n_ola_blocks, ctts::OLA_THREADS, 0, st>>>(w);
-        CU(ctx, cudaGetLastError());
-    }
-    return CTTS_GPU_OK;
+            return launch(ctts::wsola_verify_kernel, dim3(p->verify_tiles, rows), ctts::WV_THREADS, sizeof(ctts::WvSmem), wv);
+        });
+    if (!rc) rc = launch(ctts::wsola_search_kernel, ns, ctts::WS_THREADS, 0, w);
+    if (!rc && p->n_ola_blocks) rc = launch(ctts::wsola_ola_kernel, p->n_ola_blocks, ctts::OLA_THREADS, 0, w);
+    return rc;
 }
 
 // Enqueue the output-rate conversion of the plan (after its WSOLA kernels): native slots d_nat and
 // counts -> output-rate slots d_final and d_rs_counts.  Nothing at the native rate.
-int launch_resample(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const int16_t* d_nat, int16_t* d_final, cudaStream_t st) {
+int launch_resample(Launch& launch, ctts_gpu_plan* p, const int16_t* d_nat, int16_t* d_final) {
     const ctts_gpu_ctx::RsTable* rs = p->rs;
     if (!rs || !p->n_utts) return CTTS_GPU_OK;
     const uint32_t n = p->n_utts;
-    for (uint32_t u0 = 0; u0 < n; u0 += 65535u) {   // grid.y limit
+    return grid_y_slices(n, [&](uint32_t u0, uint32_t rows) {
         ctts::ResampleArgs r{};
         r.in = d_nat;
-        r.in_off = p->d_rs_off + u0;
+        r.in_off = p->d_off + u0;
         r.in_counts = p->d_counts + u0;
         r.out = d_final;
-        r.out_off = p->d_rs_off + (n + 1) + u0;
+        r.out_off = slot_off(p) + u0;
         r.out_counts = p->d_rs_counts + u0;
         r.taps = reinterpret_cast<const float4*>(rs->d_taps);
         r.L = rs->L;
@@ -1852,29 +1862,26 @@ int launch_resample(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, const int16_t* d_nat, i
         r.kp = rs->kp;
         r.c = rs->c;
         r.smem_floats = rs->smem_floats;
-        const dim3 grid(p->rs_tiles, std::min<uint32_t>(n - u0, 65535u));
-        ctts::resample_kernel<<<grid, ctts::RS_THREADS, rs->smem_floats * sizeof(float), st>>>(r);
-        CU(ctx, cudaGetLastError());
-    }
-    return CTTS_GPU_OK;
+        return launch(ctts::resample_kernel, dim3(p->rs_tiles, rows), ctts::RS_THREADS, rs->smem_floats * sizeof(float), r);
+    });
 }
 
 // Enqueue the loudness normalization of the plan (after its output-rate conversion), in place on the output-rate
 // slots d_final.  Nothing when the stage is off.
-int launch_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_final, cudaStream_t st) {
+int launch_loudness(Launch& launch, ctts_gpu_plan* p, int16_t* d_final) {
     const ctts_gpu_ctx::LdTable* ld = p->ld;
     if (!ld || !p->n_utts) return CTTS_GPU_OK;
     const uint32_t n = p->n_utts;
     ctts::LdArgs a{};
     a.pcm = d_final;
-    a.off = p->d_ld_off;
+    a.off = slot_off(p);
     a.counts = p->d_final_counts;
     a.state = p->d_ld_state;
     a.energy = p->d_ld_energy;
     a.peak = p->d_ld_peak;
     a.lufs = p->d_ld_lufs;
     a.gain = p->d_ld_gain;
-    a.table = ctx->d_ld_gains;
+    a.table = launch.ctx->d_ld_gains;
     a.gate_abs = pow(10.0, (-70.0 + 0.691) / 10.0);
     a.n = n;
     a.ceiling = ld->ceiling_q;
@@ -1885,37 +1892,29 @@ int launch_loudness(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_final, cudaS
         a.tp_peak = p->d_ld_tp;
         memcpy(a.tp_h, ld->tp_h, sizeof a.tp_h);
     }
-    auto sliced = [&](auto kernel, uint32_t tiles, int threads) -> int {
-        for (uint32_t u0 = 0; u0 < n; u0 += 65535u) {   // grid.y limit
+    auto sliced = [&](auto kernel, uint32_t tiles, uint32_t threads) {
+        const int rc = grid_y_slices(n, [&](uint32_t u0, uint32_t rows) {
             a.u0 = u0;
-            kernel<<<dim3(tiles, std::min<uint32_t>(n - u0, 65535u)), threads, 0, st>>>(a);
-            CU(ctx, cudaGetLastError());
-        }
+            return launch(kernel, dim3(tiles, rows), threads, 0, a);
+        });
         a.u0 = 0;
-        return CTTS_GPU_OK;
+        return rc;
     };
     int rc = sliced(ctts::ld_chunk_kernel<false>, p->ld_tiles, ctts::LD_THREADS);
-    if (rc) return rc;
-    ctts::ld_scan_kernel<<<(n + ctts::LD_SCAN_THREADS - 1) / ctts::LD_SCAN_THREADS, ctts::LD_SCAN_THREADS, 0, st>>>(a);
-    CU(ctx, cudaGetLastError());
-    if ((rc = sliced(ctts::ld_chunk_kernel<true>, p->ld_tiles, ctts::LD_THREADS)) != 0) return rc;
-    if (ld->true_peak) {
-        if ((rc = sliced(ctts::ld_true_peak_kernel, p->ld_tp_tiles, ctts::LD_TP_THREADS)) != 0) return rc;
-        ctts::ld_gain_kernel<true><<<n, ctts::LD_GAIN_THREADS, 0, st>>>(a);
-    } else {
-        ctts::ld_gain_kernel<false><<<n, ctts::LD_GAIN_THREADS, 0, st>>>(a);
-    }
-    CU(ctx, cudaGetLastError());
-    return sliced(ctts::ld_apply_kernel, p->ld_apply_tiles, ctts::LD_APPLY_THREADS);
+    if (!rc) rc = launch(ctts::ld_scan_kernel, (n + ctts::LD_SCAN_THREADS - 1) / ctts::LD_SCAN_THREADS, ctts::LD_SCAN_THREADS, 0, a);
+    if (!rc) rc = sliced(ctts::ld_chunk_kernel<true>, p->ld_tiles, ctts::LD_THREADS);
+    if (!rc && ld->true_peak) rc = sliced(ctts::ld_true_peak_kernel, p->ld_tp_tiles, ctts::LD_TP_THREADS);
+    if (!rc) rc = launch(ld->true_peak ? ctts::ld_gain_kernel<true> : ctts::ld_gain_kernel<false>, n, ctts::LD_GAIN_THREADS, 0, a);
+    return rc ? rc : sliced(ctts::ld_apply_kernel, p->ld_apply_tiles, ctts::LD_APPLY_THREADS);
 }
 
 // Enqueue the plan's stage chain: assembly and WSOLA into the native-rate slots d_nat, output-rate conversion into
 // d_final (the same slots at the native rate), loudness normalization in place there.
-int launch_chain(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_nat, int16_t* d_final, cudaStream_t st) {
-    int rc = launch_assemble(ctx, p, d_nat, st);
-    if (!rc) rc = launch_stretch(ctx, p, d_nat, st);
-    if (!rc) rc = launch_resample(ctx, p, d_nat, d_final, st);
-    return rc ? rc : launch_loudness(ctx, p, d_final, st);
+int launch_chain(Launch& launch, ctts_gpu_plan* p, int16_t* d_nat, int16_t* d_final) {
+    int rc = launch_assemble(launch, p, d_nat);
+    if (!rc) rc = launch_stretch(launch, p, d_nat);
+    if (!rc) rc = launch_resample(launch, p, d_nat, d_final);
+    return rc ? rc : launch_loudness(launch, p, d_final);
 }
 
 }  // namespace
@@ -1931,6 +1930,9 @@ int ctts_gpu_plan_create(ctts_gpu_ctx* ctx, const ctts_batch_plan* plan, const c
         ctts_gpu_plan_destroy(p);
         return rc;
     }
+    Launch count{ctx, ctx->stream, true};
+    launch_chain(count, p, nullptr, nullptr);   // (launches nothing: cannot fail)
+    p->info.kernel_launches = count.count;
     *out = p;
     return CTTS_GPU_OK;
 }
@@ -1966,8 +1968,9 @@ int ctts_gpu_plan_run(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, int16_t* d_pcm_out) {
             CU(ctx, cudaMalloc(reinterpret_cast<void**>(&p->d_nat_owned), std::max<uint64_t>(p->n_offsets[p->n_utts], 8) * sizeof(int16_t)));
         d_nat = p->d_nat_owned;
     }
+    Launch launch{ctx, ctx->stream};
     const int rc = begin_run(ctx, p);
-    return rc ? rc : launch_chain(ctx, p, d_nat, d_pcm_out, ctx->stream);
+    return rc ? rc : launch_chain(launch, p, d_nat, d_pcm_out);
 }
 
 int ctts_gpu_plan_read_counts(ctts_gpu_ctx* ctx, ctts_gpu_plan* p, uint32_t* out_counts) {
@@ -2066,18 +2069,18 @@ constexpr OutputKind kOutput[] = {{2, 8, "samples", "PCM", "ctts_gpu_session_sub
                                   {1, 16, "bytes", "FLAC", "ctts_gpu_session_submit_flac"}};
 
 // Where a piece of n utterances keeps its results.  h_res (pinned, 4-byte words): counts [n], device error flags [n],
-// (FLAC: file bytes [n],) then, 8-byte aligned, the slot offsets [n + 1] (FLAC: and the first frame descriptor of
-// every utterance [n + 1]).  Packed mode uploads those slot words to d_pack_off behind the n + 1 packed offsets.
+// (FLAC: file bytes [n], then, 8-byte aligned, the first frame descriptor of every utterance [n + 1]).  FLAC uploads
+// those frame bases to d_pack_off behind the n + 1 packed offsets.
 struct ResLayout {
-    size_t flags, bytes, size, slots;          // word offsets in h_res; size: what sizes a packed utterance
-    size_t slot_words, res_words, off_words;   // 8-byte words at slots; the words h_res and d_pack_off need
+    size_t flags, bytes, size, bases;          // word offsets in h_res; size: what sizes a packed utterance
+    size_t base_words, res_words, off_words;   // 8-byte words at bases; the words h_res and d_pack_off need
     ResLayout(uint32_t n, SessionOutput k) : flags(n), bytes(2 * (size_t)n) {
         const size_t heads = k == OUT_FLAC ? 3 : 2;
         size = k == OUT_FLAC ? bytes : 0;   // the file bytes, else the count
-        slots = (heads * n + 1) & ~(size_t)1;
-        slot_words = (heads - 1) * ((size_t)n + 1);
-        res_words = slots + 2 + 2 * slot_words;
-        off_words = (size_t)n + 1 + slot_words;
+        bases = (heads * n + 1) & ~(size_t)1;
+        base_words = k == OUT_FLAC ? (size_t)n + 1 : 0;
+        res_words = bases + 2 + 2 * base_words;
+        off_words = (size_t)n + 1 + base_words;
     }
 };
 
@@ -2242,36 +2245,24 @@ int grow_lane(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l, const ctts_gpu_plan* p
 // Packed mode: encode the piece's output-rate slots d_final into d_pack, its utterances back to back.  The scan kernel
 // stores the counts and flags (FLAC: and file sizes) straight into h_res; counts_ready is recorded behind it, and the
 // copy to the caller is enqueued once they are on the host.
-cudaError_t encode_packed(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l, const ctts_gpu_plan* p, const int16_t* d_final) {
-    const cudaStream_t st = s->ctx->stream;
+int encode_packed(Launch& launch, ctts_gpu_session* s, ctts_gpu_ctx::Lane& l, const ctts_gpu_plan* p, const int16_t* d_final) {
+    ctts_gpu_ctx* ctx = s->ctx;
+    const cudaStream_t st = launch.st;
     const uint32_t n = p->n_utts;
-    const ResLayout r(n, s->kind);
     const uint32_t* const cnt = p->d_final_counts;
-    unsigned long long* const h_slot = reinterpret_cast<unsigned long long*>(l.h_res + r.slots);
-    unsigned long long* const d_slot = l.d_pack_off + (n + 1);
+    const unsigned long long* const d_slot = slot_off(p);
     uint64_t max_slot = 0;
     for (uint32_t u = 0; u < n; u++) max_slot = std::max<uint64_t>(max_slot, p->offsets[u + 1] - p->offsets[u]);
-    for (uint32_t u = 0; u <= n; u++) h_slot[u] = p->offsets[u];
-    cudaError_t e = cudaSuccess;
-    auto sliced = [&](uint64_t tiles, auto launch) {   // grid.y limit
-        for (uint32_t u0 = 0; u0 < n && e == cudaSuccess; u0 += 65535u) {
-            launch(dim3((unsigned)tiles, std::min<uint32_t>(n - u0, 65535u)), u0);
-            e = cudaGetLastError();
-        }
-    };
     // PCM and G.711: device prefix sum of the counts -> packed positions -> `kernel` copies or encodes every
     // utterance there, padding included
     auto pack = [&](auto kernel, auto* dst) {
-        e = cudaMemcpyAsync(d_slot, h_slot, r.slot_words * 8, cudaMemcpyHostToDevice, st);
-        if (e == cudaSuccess) {
-            ctts::pack_scan_kernel<<<1, 1024, 0, st>>>(cnt, p->d_err, n, l.d_pack_off, l.h_res);
-            e = cudaGetLastError();
-        }
-        if (e == cudaSuccess) e = cudaEventRecord(l.counts_ready, st);   // counts and flags are on the host
-        sliced((max_slot + ctts::PACK_TILE - 1) / ctts::PACK_TILE, [&](dim3 grid, uint32_t u0) {
-            kernel<<<grid, ctts::PACK_THREADS, 0, st>>>(d_final, d_slot + u0, cnt + u0, l.d_pack_off + u0, dst);
+        int rc = launch(ctts::pack_scan_kernel, 1, 1024, 0, cnt, p->d_err, n, l.d_pack_off, l.h_res);
+        if (rc) return rc;
+        CU(ctx, cudaEventRecord(l.counts_ready, st));   // counts and flags are on the host
+        const uint32_t tiles = (uint32_t)((max_slot + ctts::PACK_TILE - 1) / ctts::PACK_TILE);
+        return grid_y_slices(n, [&](uint32_t u0, uint32_t rows) {
+            return launch(kernel, dim3(tiles, rows), ctts::PACK_THREADS, 0, d_final, d_slot + u0, cnt + u0, l.d_pack_off + u0, dst);
         });
-        return e;
     };
     switch (s->kind) {
     case OUT_PCM: return pack(ctts::pack_copy_kernel, reinterpret_cast<int16_t*>(l.d_pack));
@@ -2279,22 +2270,24 @@ cudaError_t encode_packed(ctts_gpu_session* s, ctts_gpu_ctx::Lane& l, const ctts
     case OUT_ALAW: return pack(ctts::g711_pack_kernel<ctts::G711_ALAW>, l.d_pack);
     case OUT_FLAC: break;
     }
-    // FLAC: the first frame descriptor of every utterance goes behind the slot offsets; analyse every frame -> sizes
+    // FLAC: the first frame descriptor of every utterance goes behind the packed offsets; analyse every frame -> sizes
     // and packed byte offsets (counts, flags and sizes into h_res) -> emit each frame at its offset
-    h_slot[n + 1] = 0;
-    for (uint32_t u = 0; u < n; u++) h_slot[n + 2 + u] = h_slot[n + 1 + u] + slot_frames(p, u);
-    e = cudaMemcpyAsync(d_slot, h_slot, r.slot_words * 8, cudaMemcpyHostToDevice, st);
-    const ctts::FlacArgs fa{d_final, d_slot, cnt, d_slot + (n + 1), l.d_frames, l.d_pack_off, l.d_flac_info, l.d_pack,
+    unsigned long long* const h_base = reinterpret_cast<unsigned long long*>(l.h_res + ResLayout(n, s->kind).bases);
+    unsigned long long* const d_base = l.d_pack_off + (n + 1);
+    h_base[0] = 0;
+    for (uint32_t u = 0; u < n; u++) h_base[u + 1] = h_base[u] + slot_frames(p, u);
+    CU(ctx, cudaMemcpyAsync(d_base, h_base, ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, st));
+    const ctts::FlacArgs fa{d_final, d_slot, cnt, d_base, l.d_frames, l.d_pack_off, l.d_flac_info, l.d_pack,
                             p->rs ? p->rs->hz : (uint32_t)CTTS_PLAN_SAMPLE_RATE};
-    const uint64_t frames = std::max<uint64_t>((max_slot + ctts::FLAC_BLOCK - 1) / ctts::FLAC_BLOCK, 1);
-    sliced(frames, [&](dim3 grid, uint32_t u0) { ctts::flac_analyze_kernel<<<grid, ctts::FLAC_THREADS, 0, st>>>(fa, u0); });
-    if (e == cudaSuccess) {
-        ctts::flac_scan_kernel<<<1, 1024, 0, st>>>(fa, p->d_err, n, l.h_res);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaEventRecord(l.counts_ready, st);   // counts, flags and sizes are on the host
-    sliced(frames, [&](dim3 grid, uint32_t u0) { ctts::flac_emit_kernel<<<grid, ctts::FLAC_THREADS, 0, st>>>(fa, u0); });
-    return e;
+    const uint32_t frames = (uint32_t)std::max<uint64_t>((max_slot + ctts::FLAC_BLOCK - 1) / ctts::FLAC_BLOCK, 1);
+    auto frame_grid = [&](auto kernel) {
+        return grid_y_slices(n, [&](uint32_t u0, uint32_t rows) { return launch(kernel, dim3(frames, rows), ctts::FLAC_THREADS, 0, fa, u0); });
+    };
+    int rc = frame_grid(ctts::flac_analyze_kernel);
+    if (!rc) rc = launch(ctts::flac_scan_kernel, 1, 1024, 0, fa, p->d_err, n, l.h_res);
+    if (rc) return rc;
+    CU(ctx, cudaEventRecord(l.counts_ready, st));   // counts, flags and sizes are on the host
+    return frame_grid(ctts::flac_emit_kernel);
 }
 
 // Slot mode: copy the piece from the device slots (packed by their bounds, up8(bound) + 8 each) to the caller's
@@ -2351,18 +2344,19 @@ int submit_piece(ctts_gpu_session* s, const ctts_batch_plan* piece, const uint64
     p->d_out_last = d_final;
     cudaError_t e = cudaSuccess;
     if (n) {
+        Launch launch{ctx, ctx->stream};
         rc = begin_run(ctx, p);
         if (!rc) rc = build_tasks(ctx, p, piece, ctx->stream);
         const auto tp2 = std::chrono::steady_clock::now();
-        if (!rc) rc = launch_chain(ctx, p, l.d_out, d_final, ctx->stream);
+        if (!rc) rc = launch_chain(launch, p, l.d_out, d_final);
         if (rc) return bail(rc);
         if (ctx->knobs.trace) {
             auto msf = [](auto a, auto b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
             fprintf(stderr, "  submit %u utterances at %.1f ms: waited %.2f, prepare %.2f, build %.2f, launch %.2f ms\n", n, msf(s->t0, tp0),
                     msf(tsub0, tp0), msf(tp0, tp1), msf(tp1, tp2), msf(tp2, std::chrono::steady_clock::now()));
         }
-        if (packed) e = encode_packed(s, l, p, d_final);
-        if (e == cudaSuccess) e = cudaEventRecord(l.kernels_done, ctx->stream);
+        if (packed && (rc = encode_packed(launch, s, l, p, d_final)) != 0) return bail(rc);
+        e = cudaEventRecord(l.kernels_done, ctx->stream);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->copy_stream, l.kernels_done, 0);
         if (e == cudaSuccess && !packed) e = copy_slots(s, l, p, d_final, slot_off, slot_cap);
     } else {
